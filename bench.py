@@ -24,7 +24,8 @@ Further legs in the same JSON line:
   general_text FORMAT=GT:GQ:DP text (the shape of the reference's own fixture): tokenizer + general decode.
   dataset      kernel 5 at BASELINE.json configs[4] shapes.
 
-Contract: python bench.py --gpus N --steps K --warmup W [--impl reference]; rank 0 prints ONE JSON line.
+Contract: python bench.py --gpus N --steps K --warmup W [--impl reference] [--dump-outputs DIR]; rank 0 prints ONE JSON
+line.  --dump-outputs writes a fixed sample of what rank 0's last timed step computed as DIR/<name>.npy (see dump_outputs).
 """
 from __future__ import annotations
 
@@ -192,6 +193,51 @@ def workload_config(args):
             "variants": args.variants, "samples": args.samples,
             "l2": "inputs (GBs of text) are far larger than the 126 MB L2; no flush needed",
             "per_rank": "each rank parses its own shard of this shape (seed + rank)"}
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, p, frames, seed):
+    """--dump-outputs: what the timed step hands its caller, as float32 / float64 .npy files, so that two builds can be
+    compared output for output.  The genotype matrix, the site columns and the stored chunks are GBs at the bench shape,
+    so a fixed sample drawn with `seed` is written (under 64 MB in all):
+      index_donors [D], index_records [R]   the sampled donors (rows of the matrix) and records (columns)
+      gt0, gt1 [D, R]                       allele calls of those donors at those records (-9 = missing)
+      start, stop [R]; ref, alt [R]         site columns at those records (REF / ALT as byte values)
+      chunk_sizes [D, n_chunks]             size in bytes of every stored chunk (Blosc frame) of the sampled donors
+      index_chunks [P, 2]                   P of those chunks: (row of index_donors, chunk)
+      chunk_bytes [sum of their sizes]      their stored bytes, back to back in index_chunks order"""
+    import numpy as np
+    rng = np.random.default_rng(seed)
+    info = p.info
+    V, S = int(info.n_records), int(info.n_samples)
+    donors = np.sort(rng.choice(S, min(S, 32), replace=False))
+    records = np.sort(rng.choice(V, min(V, 1 << 16), replace=False))
+    out = {"index_donors": donors.astype(np.float64), "index_records": records.astype(np.float64)}
+    rows = [p.sample(int(s)) for s in donors]
+    out["gt0"] = np.stack([g0[records] for g0, _ in rows]).astype(np.float32)
+    out["gt1"] = np.stack([g1[records] for _, g1 in rows]).astype(np.float32)
+    start, stop, ref, alt = p.sites()
+    out["start"], out["stop"] = start[records].astype(np.float64), stop[records].astype(np.float64)
+    out["ref"], out["alt"] = ref[records].view(np.uint8).astype(np.float32), alt[records].view(np.uint8).astype(np.float32)
+    if frames is not None:
+        fi = frames.info
+        nc, cr = int(fi.n_chunks), int(fi.chunk_records)
+        stored = [frames.sample(int(s)) for s in donors]
+        out["chunk_sizes"] = np.array([[len(f) for f in row] for row in stored], np.float32).reshape(len(donors), nc)
+        # a stored chunk holds at most its cr 35-byte records plus the Blosc header: at most 16 MB of chunk_bytes
+        n_pairs = min(len(donors) * nc, 64, max(1, (4 << 20) // (35 * cr + 1024)))
+        pairs = np.sort(rng.choice(len(donors) * nc, n_pairs, replace=False))
+        out["index_chunks"] = np.stack([pairs // nc, pairs % nc], axis=1).astype(np.float64)
+        blob = b"".join(stored[int(k) // nc][int(k) % nc] for k in pairs)
+        out["chunk_bytes"] = np.frombuffer(blob, np.uint8).astype(np.float32)
+    total = sum(a.nbytes for a in out.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise RuntimeError("--dump-outputs: %d bytes exceed the %d-byte limit" % (total, DUMP_LIMIT_BYTES))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 # =====================================================================================================================
@@ -458,7 +504,13 @@ def main():
     ap.add_argument("--parse-only", action="store_true", help="step = kernels 1-3 only (no frames)")
     ap.add_argument("--site-matcher", choices=["fast", "deep"], default="fast",
                     help="deep: 4-way hash buckets in the site-plane encoder (hb_set_site_matcher): smaller chunks, slower kernel 4a")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write a fixed sample of what rank 0's last step computed as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU path; --impl reference has none")
     args.warmup = max(args.warmup, 3) if args.impl != "reference" else args.warmup
 
     if args.impl == "reference":
@@ -555,6 +607,8 @@ def main():
     value = calls_total / (ms / 1e3 / args.steps)
     fi_head = frames[0].info if frames[0] is not None else None
     c_out_head = float(fi_head.total_bytes) if fi_head is not None else 0.0
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, p, frames[0], args.seed)
 
     # ---- parity of what was just measured (oracle as the checker): whole HDF5 chunks of three donors -- every record
     # of the chunk, site columns and both alleles, through the stored chunk bytes -- plus the genotype matrix rows
