@@ -44,6 +44,26 @@ def _decode(frames, dtype: np.dtype, n: int, chunk: int) -> np.ndarray:
     return raw.reshape(-1).view(dtype)[:n].copy()
 
 
+def _decode_masked(chunks, dtype: np.dtype, n: int, chunk: int) -> np.ndarray:
+    """chunks: [(stored bytes, filter mask)] of a dataset behind the Blosc filter alone.  A chunk with mask bit 0 set was
+    stored unfiltered (hdf5-blosc gives c-blosc an output buffer of the chunk's size, so a chunk Blosc cannot shrink,
+    e.g. one of 1-3 records, fails the optional filter): its bytes are the records.  The others decode on the GPU."""
+    from . import capi
+    nbytes = chunk * dtype.itemsize
+    if not any(m & 1 for _, m in chunks):
+        return _decode([b for b, _ in chunks], dtype, n, chunk)
+    out = np.zeros((len(chunks), nbytes), np.uint8)
+    blosc = [k for k, (_, m) in enumerate(chunks) if not m & 1]
+    if blosc:
+        out[blosc] = capi.decode_frames([chunks[k][0] for k in blosc], nbytes)
+    for k, (b, m) in enumerate(chunks):
+        if m & 1:
+            if len(b) != nbytes:
+                raise OSError(f"unfiltered chunk {k} holds {len(b)} bytes, not {nbytes}")
+            out[k] = np.frombuffer(b, np.uint8)
+    return out.reshape(-1).view(dtype)[:n].copy()
+
+
 class _MiniFile:
     backend = "minih5"
 
@@ -83,21 +103,25 @@ class _MiniFile:
         if info.layout == "contiguous":
             return self._r.read_contiguous(info)
         n = int(info.shape[0])
-        stored = self._r.chunks(info)
+        stored = self._r.chunks_with_masks(info)
         if not info.filters:
-            raw = b"".join(b for _, b in stored)
+            raw = b"".join(b for _, b, _ in stored)
             return np.frombuffer(raw, info.dtype)[:n].copy()
         if [f for f, _ in info.filters] != [FILTER_BLOSC]:
             raise OSError(f"{path}: unsupported filter pipeline {info.filters}")
-        return _decode([b for _, b in stored], info.dtype, n, info.chunk)
+        return _decode_masked([(b, m) for _, b, m in stored], info.dtype, n, info.chunk)
 
     def stored_chunks(self, path: str):
         """The dataset as it is stored: (n_records, chunk_records, dtype, [stored chunk bytes in order]) -- no decoding.
-        None for a dataset that is not a 1-D chunked array behind filter 32001 alone."""
+        None for a dataset that is not a 1-D chunked array behind filter 32001 alone, or that holds a chunk HDF5 stored
+        unfiltered (filter mask bit 0: the optional Blosc filter failed on it); read_dataset reads those."""
         info = self._r.dataset_info(path)
         if info.layout == "contiguous" or [f for f, _ in info.filters] != [FILTER_BLOSC]:
             return None
-        return int(info.shape[0]), int(info.chunk), info.dtype, [b for _, b in self._r.chunks(info)]
+        stored = self._r.chunks_with_masks(info)
+        if any(m & 1 for _, _, m in stored):
+            return None
+        return int(info.shape[0]), int(info.chunk), info.dtype, [b for _, b, _ in stored]
 
     def close(self):
         if self._w is not None:
@@ -146,8 +170,8 @@ class _H5pyFile:
         if d.chunks is None or d.compression is None and not d.id.get_create_plist().get_nfilters():
             return d[()]
         chunk, n = d.chunks[0], d.shape[0]
-        frames = [d.id.read_direct_chunk((off,))[1] for off in range(0, n, chunk)]
-        return _decode(frames, d.dtype, n, chunk)
+        frames = [d.id.read_direct_chunk((off,)) for off in range(0, n, chunk)]       # (filter mask, stored bytes)
+        return _decode_masked([(b, m) for m, b in frames], d.dtype, n, chunk)
 
     def stored_chunks(self, path: str):
         d = self._f[path]
@@ -155,7 +179,10 @@ class _H5pyFile:
         if d.chunks is None or d.ndim != 1 or pl.get_nfilters() != 1 or pl.get_filter(0)[0] != FILTER_BLOSC:
             return None
         chunk, n = d.chunks[0], d.shape[0]
-        return int(n), int(chunk), d.dtype, [d.id.read_direct_chunk((off,))[1] for off in range(0, n, chunk)]
+        frames = [d.id.read_direct_chunk((off,)) for off in range(0, n, chunk)]
+        if any(m & 1 for m, _ in frames):
+            return None
+        return int(n), int(chunk), d.dtype, [b for _, b in frames]
 
     def close(self):
         self._f.close()

@@ -101,8 +101,10 @@ __device__ __forceinline__ int decode_sym(const HuffTab &h, BitReader &br) {
     return decode_slow(h, br);
 }
 
-// lens[0..nsym) in shared memory -> count / sorted / primary table.  Returns false for an over-subscribed code.
-__device__ bool build_table(HuffTab &h, const uint8_t *lens, int nsym, uint16_t *cursor /* [16] scratch */) {
+// lens[0..nsym) in shared memory -> count / sorted / primary table.  Returns false for an over-subscribed code and, as
+// zlib does (inftrees.c), for an incomplete one, except a literal/length or distance code whose longest code is <= 1 bit
+// (a single code, or none); the code-length code (`lengths_code`) must always be complete.
+__device__ bool build_table(HuffTab &h, const uint8_t *lens, int nsym, uint16_t *cursor /* [16] scratch */, bool lengths_code) {
     const int lane = threadIdx.x & 31;
     if (lane < 16) h.count[lane] = 0;
     __syncwarp();
@@ -114,15 +116,17 @@ __device__ bool build_table(HuffTab &h, const uint8_t *lens, int nsym, uint16_t 
         __syncwarp();
     }
     // offsets of each length in `sorted`; Kraft check (every lane, redundantly)
-    int left = 1, off = 0;
+    int left = 1, off = 0, longest = 0;
     bool ok = true;
     for (int len = 1; len <= 15; ++len) {
         left <<= 1;
         left -= h.count[len];
         if (left < 0) ok = false;
+        if (h.count[len]) longest = len;
         if (lane == 0) cursor[len] = (uint16_t)off;
         off += h.count[len];
     }
+    if (left > 0 && (lengths_code || longest > 1)) ok = false;
     __syncwarp();
     for (int base = 0; base < nsym; base += 32) {
         const int s = base + lane;
@@ -216,8 +220,8 @@ __global__ void __launch_bounds__(kInfWarps * 32, 6) inflate_bgzf_kernel(const I
         int nlit, ndist;
         if (type == 1) {                                   // fixed code
             for (int s = lane; s < 288; s += 32) lens[s] = s < 144 ? 8 : s < 256 ? 9 : s < 280 ? 7 : 8;
-            if (lane < 30) lens[288 + lane] = 5;
-            nlit = 288; ndist = 30;
+            lens[288 + lane] = 5;                          // 32 distance codes, so the code is complete; 30 and 31 are rejected below
+            nlit = 288; ndist = 32;
             __syncwarp();
         } else {                                           // dynamic code
             nlit = (int)br.take(5) + 257;
@@ -232,7 +236,7 @@ __global__ void __launch_bounds__(kInfWarps * 32, 6) inflate_bgzf_kernel(const I
                 if (lane == 0) lens[c_clorder[i]] = (uint8_t)v;
             }
             __syncwarp();
-            if (!build_table(cl, lens, 19, cursor)) { err = 5; break; }
+            if (!build_table(cl, lens, 19, cursor, true)) { err = 5; break; }
             // the nlit + ndist code lengths, run-length coded (every lane decodes; lane 0 writes)
             int i = 0, prev = 0;
             while (i < nlit + ndist) {
@@ -253,8 +257,8 @@ __global__ void __launch_bounds__(kInfWarps * 32, 6) inflate_bgzf_kernel(const I
             __syncwarp();
             if (lens[256] == 0) { err = 9; break; }
         }
-        if (!build_table(lit, lens, nlit, cursor)) { err = 10; break; }
-        if (!build_table(dist, lens + 288, ndist, cursor)) { err = 11; break; }
+        if (!build_table(lit, lens, nlit, cursor, false)) { err = 10; break; }
+        if (!build_table(dist, lens + 288, ndist, cursor, false)) { err = 11; break; }
         // ---- symbols
         for (;;) {
             br.refill();

@@ -1750,10 +1750,11 @@ decode_frames_kernel(const uint8_t *__restrict__ frames, const uint64_t *__restr
         for (int i = 0; i < 6; ++i) { if (c[16 + i] == 1) shuffle = true; else if (c[16 + i] != 0) err = 3; }
         if ((c[31] >> 4) & 7) err = 6;                       // special chunks (runs of zeros / NaNs / uninit)
     }
-    if (!err && (flags & 2)) {                               // memcpyed
+    if (!err && (flags & 2)) {                               // memcpyed: the bytes as they were given, never shuffled
         if ((uint64_t)hdr + cn > ccb) err = 7;
         else for (uint32_t i = lane; i < cn; i += 32) t[i] = c[hdr + i];
         shuffle = false;
+        planar = 1;                                          // nothing to undo
     } else if (!err) {
         if ((flags >> 5) != 1 || (!ext && c[1] != 1)) err = 5;       // LZ4 / LZ4HC codec format, its format version
         const bool dont_split = flags & 0x10;
@@ -1880,7 +1881,9 @@ __global__ void __launch_bounds__(128) decode_columns_kernel(const DecodeColsArg
         shuffle = !ext && (flags & 1);
         if (c[0] < 2 || c[0] > 5 || (!ext && (c[0] != 2 || (flags & 0x08)))) err = 2;
         else if (c[3] != 35 || cn != nbytes || ccb > flen || ccb < hdr) err = 4;
-        else if (!(flags & 2) && bs != cn) err = 11;                 // several blocks per chunk: the host-pointer decoder reads those
+        // several blocks per chunk, or a c-blosc2 block split into `typesize` streams (no dont-split flag 0x10): the
+        // host-pointer decoder reads those
+        else if (!(flags & 2) && (bs != cn || (ext && !(flags & 0x10)))) err = 11;
     }
     if (!err && ext) {
         for (int i = 0; i < 6; ++i) { if (c[16 + i] == 1) shuffle = true; else if (c[16 + i] != 0) err = 3; }

@@ -156,12 +156,15 @@ class H5Writer:
         self._link(path, self._object_header(msgs + [(0x0008, layout)]))
 
     def create_dataset_chunked(self, path: str, dtype: np.dtype, n: int, chunk: int, chunks: Sequence[bytes],
-                               filter_id: Optional[int] = None, cd_values: Sequence[int] = (), filter_name: str = ""):
-        """chunks[k] = the bytes to store for chunk k (already filtered when filter_id is given)."""
+                               filter_id: Optional[int] = None, cd_values: Sequence[int] = (), filter_name: str = "",
+                               masks: Optional[Sequence[int]] = None):
+        """chunks[k] = the bytes to store for chunk k (already filtered when filter_id is given).  masks[k] = chunk k's
+        filter mask: bit i set = filter i of the pipeline was skipped, as HDF5 does when an optional filter fails."""
         dtype = np.dtype(dtype)
         entries = []
         for k, payload in enumerate(chunks):
-            entries.append((len(payload), k * chunk, self._write(bytes(payload), align=1)))
+            mask = int(masks[k]) if masks is not None else 0
+            entries.append((len(payload), mask, k * chunk, self._write(bytes(payload), align=1)))
         btree = self._chunk_btree(entries, chunk, len(entries) * chunk) if entries else UNDEF
         layout = struct.pack("<BBBQII", 3, 2, 2, btree, chunk, dtype.itemsize)
         msgs = self._common_messages(dtype, n) + [(0x0008, layout)]
@@ -243,13 +246,13 @@ class H5Writer:
             level += 1
 
     def _chunk_btree(self, entries, chunk: int, end_offset: int) -> int:
-        """v1 B-tree, node type 1.  entries: (stored size, element offset, address), offset-sorted."""
-        def key(size, off):
-            return struct.pack("<IIQQ", size, 0, off, 0)
+        """v1 B-tree, node type 1.  entries: (stored size, filter mask, element offset, address), offset-sorted."""
+        def key(size, mask, off):
+            return struct.pack("<IIQQ", size, mask, off, 0)
         cap = 2 * CHUNK_K
         level = 0
-        nodes = [(key(s, o), a, None) for s, o, a in entries]      # (first key, child address, last key of subtree)
-        last_key = key(0, end_offset)
+        nodes = [(key(s, m, o), a, None) for s, m, o, a in entries]   # (first key, child address, last key of subtree)
+        last_key = key(0, 0, end_offset)
         while True:
             groups = [nodes[i:i + cap] for i in range(0, len(nodes), cap)]
             addrs = []
@@ -486,7 +489,12 @@ class H5Reader:
         return info
 
     def chunks(self, info: DatasetInfo) -> List[Tuple[int, bytes]]:
-        """[(element offset, stored bytes)] in offset order."""
+        """[(element offset, stored bytes)] in offset order (the filter masks dropped: see chunks_with_masks)."""
+        return [(off, b) for off, b, _ in self.chunks_with_masks(info)]
+
+    def chunks_with_masks(self, info: DatasetInfo) -> List[Tuple[int, bytes, int]]:
+        """[(element offset, stored bytes, filter mask)] in offset order.  Bit i of the mask set = filter i of the
+        pipeline was not applied to this chunk (an optional filter that failed on it): those bytes are not filtered."""
         out = []
 
         def walk(node):
@@ -496,12 +504,12 @@ class H5Reader:
             level, used = h[5], struct.unpack_from("<H", h, 6)[0]
             body = self._read(node + 24, used * 32 + 24)
             for i in range(used):
-                size, _, off, _ = struct.unpack_from("<IIQQ", body, 32 * i)
+                size, mask, off, _ = struct.unpack_from("<IIQQ", body, 32 * i)
                 child = struct.unpack_from("<Q", body, 32 * i + 24)[0]
                 if level:
                     walk(child)
                 else:
-                    out.append((off, self._read(child, size)))
+                    out.append((off, self._read(child, size), mask))
 
         if info.btree != UNDEF:
             walk(info.btree)

@@ -122,3 +122,37 @@ def test_bulk_blob_writer_equals_per_chunk_writer(tmp_path, minih5, n_chunks):
     assert [c for _, c in ra.chunks(ia)] == chunks and rb.chunks(ib) == ra.chunks(ia)
     assert ia.filters == ib.filters and ia.chunk == ib.chunk and ia.shape == ib.shape and ia.dtype == ib.dtype
     ra.close(); rb.close()
+
+
+def test_chunk_filter_mask_roundtrip(tmp_path, minih5):
+    """Per-chunk filter masks survive the chunk B-tree (one level and several); a chunk with mask bit 0 (the optional
+    Blosc filter skipped, as HDF5 stores a chunk the filter could not shrink) keeps the dataset out of stored_chunks."""
+    from haplohyped_varawareml_b200 import container
+    rng = np.random.default_rng(3)
+    cd = (2, 2, 35, 350, 5, 1, 2)
+    p = str(tmp_path / "m.h5")
+    small = [rng.integers(0, 256, 350, dtype=np.uint8).tobytes()]
+    many = [rng.integers(0, 256, int(rng.integers(1, 60)), dtype=np.uint8).tobytes() for _ in range(300)]
+    masks = [int(m) for m in rng.choice([0, 1, 2, 0xFFFFFFFF], 300)]
+    with minih5.H5Writer(p) as w:
+        w.create_dataset_chunked("d/chr_1/snp_data", REC, 2, 10, small, filter_id=32001, cd_values=cd,
+                                 filter_name="blosc", masks=[1])
+        w.create_dataset_chunked("d/chr_2/snp_data", REC, 3000, 10, many, filter_id=32001, cd_values=cd,
+                                 filter_name="blosc", masks=masks)
+        w.create_dataset_chunked("d/chr_3/snp_data", REC, 3000, 10, many, filter_id=32001, cd_values=cd,
+                                 filter_name="blosc")
+    r = minih5.H5Reader(p)
+    assert r.chunks_with_masks(r.dataset_info("d/chr_1/snp_data")) == [(0, small[0], 1)]
+    info2 = r.dataset_info("d/chr_2/snp_data")
+    assert r.chunks_with_masks(info2) == [(10 * k, c, m) for k, (c, m) in enumerate(zip(many, masks))]
+    assert r.chunks(info2) == [(10 * k, c) for k, c in enumerate(many)]
+    assert [m for _, _, m in r.chunks_with_masks(r.dataset_info("d/chr_3/snp_data"))] == [0] * 300
+    r.close()
+    f = container.open_h5(p, "r", backend="minih5")
+    assert f.stored_chunks("d/chr_1/snp_data") is None and f.stored_chunks("d/chr_2/snp_data") is None
+    n, cr, dt, chunks = f.stored_chunks("d/chr_3/snp_data")
+    assert (n, cr, dt, chunks) == (3000, 10, REC, many)
+    # every chunk unfiltered: read without any codec, the records as stored (the tail past n dropped)
+    rec = np.frombuffer(small[0], REC)
+    assert f.read_dataset("d/chr_1/snp_data").tobytes() == rec[:2].tobytes()
+    f.close()
