@@ -719,14 +719,13 @@ int hb_parse_host_text(const uint8_t *text, uint64_t nbytes, const hb_parse_opts
 // same options; hb_cache_clear() frees them.
 namespace {
 struct StreamSlot {
-    hb_parse *p = nullptr;
+    hb_parse *p = nullptr;                        // parses the slab text in buf; owns no text
     cudaStream_t compute = nullptr, d2h = nullptr;
     cudaEvent_t fetched = nullptr;
+    uint8_t *buf = nullptr;                       // [carry_cap + 32 | slab text | '\n' + 256]; host text (no carry) sits at buf + 0
     // BGZF streaming only
     hb::InflateScratch sc;
-    uint8_t *buf = nullptr;                       // [carry_cap + 32 | slab text | '\n' + 256]
     unsigned long long *h_pin = nullptr;          // pinned: [last newline | inflate status of every member]
-    std::vector<uint64_t> hc, ho;
     uint64_t x = 0, end = 0, begin = 0;           // slab text at buf + x .. buf + end; the parse starts at buf + begin
 };
 struct StreamSlots {
@@ -742,7 +741,7 @@ struct StreamSlots {
         for (auto &s : slot) {
             if (s.compute) cudaStreamSynchronize(s.compute);
             if (s.d2h) cudaStreamSynchronize(s.d2h);
-            if (s.p) { if (s.buf) s.p->d_text = nullptr; hb_parse_free(s.p); }
+            if (s.p) hb_parse_free(s.p);
             free_dev(s.buf);
             if (s.h_pin) cudaFreeHost(s.h_pin);
             hb::inflate_scratch_free(s.sc);
@@ -791,6 +790,125 @@ void clear_slot_cache(SlotCache &c) {
     std::lock_guard<std::mutex> lk(c.mu);
     if (c.kept && !c.in_use) { c.kept->destroy(); delete c.kept; c.kept = nullptr; }
 }
+
+// the slots of one streaming call from cache c: streams, event and parse are made for a slot that has none, and the buffers of
+// every slot grow together when a capacity is short (the carry offset is part of the layout).  text_cap: text of one slab;
+// carry_cap, comp_cap, n_cap: BGZF only -- host text (all 0) has no inflate scratch and no pinned tables.
+int open_slots(SlotCache &c, const hb_parse_opts &opts, size_t n_slots, uint64_t text_cap, uint64_t carry_cap, uint64_t comp_cap,
+               uint32_t n_cap, StreamSlots **out) {
+    StreamSlots *ss = acquire_slots(c, opts, n_slots);
+    int rc = HB_OK;
+    for (size_t i = ss->n_slots; i < n_slots && rc == HB_OK; ++i) {
+        StreamSlot &s = ss->slot[i];
+        if (cudaStreamCreateWithFlags(&s.compute, cudaStreamNonBlocking) != cudaSuccess ||
+            cudaStreamCreateWithFlags(&s.d2h, cudaStreamNonBlocking) != cudaSuccess ||
+            cudaEventCreateWithFlags(&s.fetched, cudaEventDisableTiming) != cudaSuccess) { rc = fail(HB_ERR_CUDA, "cannot create streams"); break; }
+        hb_parse_opts o = opts;
+        o.stream = s.compute;
+        rc = new_parse(&o, &s.p);
+        if (rc == HB_OK) ss->n_slots = i + 1;
+    }
+    const bool grow = ss->text_cap < text_cap || ss->carry_cap < carry_cap || ss->comp_cap < comp_cap || ss->n_cap < n_cap;
+    if (grow) {
+        ss->text_cap = std::max(ss->text_cap, text_cap + text_cap / 16);
+        ss->carry_cap = std::max(ss->carry_cap, carry_cap);
+        ss->comp_cap = std::max(ss->comp_cap, comp_cap + comp_cap / 8);
+        if (n_cap) ss->n_cap = std::max<uint32_t>(ss->n_cap, n_cap + n_cap / 8 + 16);
+    }
+    for (size_t i = 0; i < ss->n_slots && rc == HB_OK; ++i) {
+        StreamSlot &s = ss->slot[i];
+        s.p->probed = false;                         // this call's text may have another shape than the last one's
+        if (s.buf && !grow) continue;
+        rc = dev_alloc(&s.buf, ss->carry_cap + 32 + ss->text_cap + 1 + 256);
+        if (rc != HB_OK || !ss->n_cap) continue;
+        if (s.h_pin) { cudaFreeHost(s.h_pin); s.h_pin = nullptr; }
+        inflate_scratch_free(s.sc);
+        rc = inflate_scratch_alloc(s.sc, ss->comp_cap, ss->n_cap);
+        // pinned: [last newline 8 | status 4n | coff 8n | ooff 8n | clen 4n | olen 4n] -- copies from / to pageable memory stall here
+        if (rc == HB_OK && cudaMallocHost((void **)&s.h_pin, 8 + 28ull * ss->n_cap + 8) != cudaSuccess) rc = fail(HB_ERR_MEM, "cudaMallocHost failed");
+    }
+    if (rc != HB_OK) { release_slots(c, ss, false); return rc; }
+    *out = ss;
+    return HB_OK;
+}
+
+// the end of a streaming call: the D2H copies of every slot are waited for, a CUDA error becomes the return code, and the slots
+// go back to cache c, kept for the next call when all went well
+int close_slots(SlotCache &c, StreamSlots *ss, int rc, cudaError_t e) {
+    for (size_t i = 0; i < ss->n_slots && rc == HB_OK && e == cudaSuccess; ++i) e = cudaStreamSynchronize(ss->slot[i].d2h);
+    if (e != cudaSuccess && rc == HB_OK) rc = fail(HB_ERR_CUDA, std::string("CUDA: ") + cudaGetErrorString(e));
+    release_slots(c, ss, rc == HB_OK);
+    return rc;
+}
+
+// where the rows of a parsed slab go: host arrays (HostSink) or the growing planes of ONE resident parse (ResidentSink).
+// deliver() enqueues copies on s.d2h (the slot's compute stream is idle by then).  The per-sample error counts of all
+// slabs are summed into ploidy_err / badgt_err, each [n_samples], when set.
+struct SlabSink {
+    hb_parse_opts opts{};
+    uint32_t *ploidy_err = nullptr, *badgt_err = nullptr;
+    std::vector<uint32_t> pl, bg;                 // the counts of one slab
+    virtual ~SlabSink() {}
+    virtual int begin(const hb_parse_opts &o, const std::vector<std::string> &samples, uint64_t total_text) {
+        (void)samples; (void)total_text;
+        opts = o;
+        if (ploidy_err) memset(ploidy_err, 0, 4ull * o.n_samples);
+        if (badgt_err) memset(badgt_err, 0, 4ull * o.n_samples);
+        pl.resize(o.n_samples); bg.resize(o.n_samples);
+        return HB_OK;
+    }
+    virtual int deliver(StreamSlot &s, uint64_t R, uint64_t n, uint64_t slab_text, cudaError_t &e) = 0;
+    void add_errors(const StreamSlot &s, cudaError_t &e) {      // waits for s.d2h
+        if (!(ploidy_err || badgt_err) || !opts.want_gt || !opts.n_samples || e != cudaSuccess) return;
+        e = cudaMemcpyAsync(pl.data(), s.p->d_ploidy, 4ull * opts.n_samples, cudaMemcpyDeviceToHost, s.d2h);
+        if (e == cudaSuccess) e = cudaMemcpyAsync(bg.data(), s.p->d_badgt, 4ull * opts.n_samples, cudaMemcpyDeviceToHost, s.d2h);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(s.d2h);
+        for (uint32_t i = 0; i < opts.n_samples && e == cudaSuccess; ++i) {
+            if (ploidy_err) ploidy_err[i] += pl[i];
+            if (badgt_err) badgt_err[i] += bg[i];
+        }
+    }
+};
+
+// rows into the caller's host arrays: planes [n_samples][out_stride], columns of out_stride records; any of them may be NULL
+struct HostSink : SlabSink {
+    int8_t *gt0, *gt1; uint64_t out_stride; uint32_t *start, *stop; char *ref, *alt;
+    int deliver(StreamSlot &s, uint64_t R, uint64_t n, uint64_t, cudaError_t &e) override {
+        if (R + n > out_stride && (gt0 || gt1 || start || stop || ref || alt)) return fail(HB_ERR_ARG, "more records than the output arrays hold");
+        if (opts.want_gt && opts.n_samples && s.p->d_gt[0]) {
+            if (gt0) e = cudaMemcpy2DAsync(gt0 + R, out_stride, s.p->d_gt[0], s.p->gt_stride, n, opts.n_samples, cudaMemcpyDeviceToHost, s.d2h);
+            if (gt1 && e == cudaSuccess) e = cudaMemcpy2DAsync(gt1 + R, out_stride, s.p->d_gt[1], s.p->gt_stride, n, opts.n_samples, cudaMemcpyDeviceToHost, s.d2h);
+        }
+        if (start && e == cudaSuccess) e = cudaMemcpyAsync(start + R, s.p->d_start, n * 4, cudaMemcpyDeviceToHost, s.d2h);
+        if (stop && e == cudaSuccess) e = cudaMemcpyAsync(stop + R, s.p->d_stop, n * 4, cudaMemcpyDeviceToHost, s.d2h);
+        if (ref && e == cudaSuccess) e = cudaMemcpyAsync(ref + R, s.p->d_ref, n, cudaMemcpyDeviceToHost, s.d2h);
+        if (alt && e == cudaSuccess) e = cudaMemcpyAsync(alt + R, s.p->d_alt, n, cudaMemcpyDeviceToHost, s.d2h);
+        return HB_OK;
+    }
+};
+
+// the nbytes of slab text at s.buf + begin: parsed once the slot's previous rows have left, its rows handed to the sink behind
+// the R rows before them.  Returns with the slot's compute stream idle; a CUDA error is left in e.
+int parse_slab(StreamSlot &s, uint64_t begin, uint64_t nbytes, SlabSink &sink, uint64_t &R, cudaError_t &e) {
+    uint64_t n = 0;
+    if (nbytes) {
+        e = cudaStreamWaitEvent(s.compute, s.fetched, 0);     // (putting the text in place did not need to wait for that)
+        if (e != cudaSuccess) return HB_OK;
+        s.p->d_text = s.buf + begin;
+        s.p->nbytes = nbytes;
+        TRY(run_parse(s.p));
+        n = s.p->h_st.n_records;
+    }
+    if (n) {
+        TRY(sink.deliver(s, R, n, nbytes, e));
+        sink.add_errors(s, e);
+    }
+    if (e == cudaSuccess) e = cudaEventRecord(s.fetched, s.d2h);
+    R += n;
+    return HB_OK;
+}
+
+double now_ms() { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now().time_since_epoch()).count(); }
 }  // namespace
 
 int hb_parse_stream_host(const uint8_t *text, uint64_t nbytes, const hb_parse_opts *opts, uint64_t slab_bytes,
@@ -799,8 +917,10 @@ int hb_parse_stream_host(const uint8_t *text, uint64_t nbytes, const hb_parse_op
     if (!opts || !n_records || (nbytes && !text)) return fail(HB_ERR_ARG, "null argument");
     *n_records = 0;
     if (n_slabs) *n_slabs = 0;
-    if (ploidy_err) memset(ploidy_err, 0, 4ull * opts->n_samples);
-    if (badgt_err) memset(badgt_err, 0, 4ull * opts->n_samples);
+    HostSink sink;
+    sink.gt0 = gt0; sink.gt1 = gt1; sink.out_stride = out_stride; sink.start = start; sink.stop = stop; sink.ref = ref; sink.alt = alt;
+    sink.ploidy_err = ploidy_err; sink.badgt_err = badgt_err;
+    TRY(sink.begin(*opts, {}, nbytes));
     if (nbytes == 0) return HB_OK;
     if (text[nbytes - 1] != '\n') return fail(HB_ERR_ARG, "the text must end with a newline");
     if (slab_bytes == 0) slab_bytes = 1ull << 30;
@@ -821,91 +941,34 @@ int hb_parse_stream_host(const uint8_t *text, uint64_t nbytes, const hb_parse_op
         off = end;
     }
     TRY(ensure_device(opts->device));
-    const bool trace = getenv("HB_TRACE") != nullptr;
-    auto now = []() { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now().time_since_epoch()).count(); };
-    const double t_begin = now();
-    double t_setup = 0, t_loop = 0, t_tail = 0, t_parse = 0, t_maxparse = 0;
-    typedef StreamSlot Slot;
-    int rc = HB_OK;
-    const size_t n_slots = std::min<size_t>(2, slabs.size());
-    StreamSlots *ss = acquire_slots(g_text_slots, *opts, n_slots);
-    Slot *slot = ss->slot;
-    auto cleanup = [&]() { release_slots(g_text_slots, ss, rc == HB_OK); };
-    for (size_t i = ss->n_slots; i < n_slots && rc == HB_OK; ++i) {      // slots the cache did not have
-        Slot &s = slot[i];
-        if (cudaStreamCreateWithFlags(&s.compute, cudaStreamNonBlocking) != cudaSuccess ||
-            cudaStreamCreateWithFlags(&s.d2h, cudaStreamNonBlocking) != cudaSuccess ||
-            cudaEventCreateWithFlags(&s.fetched, cudaEventDisableTiming) != cudaSuccess) { rc = fail(HB_ERR_CUDA, "cannot create streams"); break; }
-        hb_parse_opts o = *opts;
-        o.stream = s.compute;
-        rc = new_parse(&o, &s.p);
-        if (rc == HB_OK) ss->n_slots = i + 1;
-    }
-    for (size_t i = 0; i < ss->n_slots && rc == HB_OK; ++i) {
-        Slot &s = slot[i];
-        s.p->probed = false;                         // this call's text may have another shape than the last one's
-        if (ss->text_cap < cap || !s.p->d_text_owned) {
-            rc = dev_alloc(&s.p->d_text_owned, std::max(cap + cap / 16, ss->text_cap) + 256);
-            if (rc == HB_OK) s.p->d_text = s.p->d_text_owned;
-        }
-    }
-    if (rc == HB_OK && ss->text_cap < cap) ss->text_cap = cap + cap / 16;
-    if (rc != HB_OK) { cleanup(); return rc; }
+    const double t_begin = now_ms();
+    StreamSlots *ss = nullptr;
+    TRY(open_slots(g_text_slots, *opts, std::min<size_t>(2, slabs.size()), cap, 0, 0, 0, &ss));
+    StreamSlot *slot = ss->slot;
     auto h2d = [&](size_t k) -> cudaError_t {
-        Slot &s = slot[k & 1];
-        cudaError_t e = cudaMemcpyAsync(s.p->d_text_owned, text + slabs[k].first, slabs[k].second, cudaMemcpyHostToDevice, s.compute);
-        if (e == cudaSuccess) e = cudaMemsetAsync(s.p->d_text_owned + slabs[k].second, 0, 256, s.compute);
+        StreamSlot &s = slot[k & 1];
+        cudaError_t e = cudaMemcpyAsync(s.buf, text + slabs[k].first, slabs[k].second, cudaMemcpyHostToDevice, s.compute);
+        if (e == cudaSuccess) e = cudaMemsetAsync(s.buf + slabs[k].second, 0, 256, s.compute);
         return e;
     };
-    t_setup = now() - t_begin;
+    const double t_setup = now_ms() - t_begin;
+    double t_parse = 0;
+    int rc = HB_OK;
     cudaError_t e = h2d(0);
     uint64_t R = 0;
-    std::vector<uint32_t> pl(opts->n_samples), bg(opts->n_samples);
     for (size_t k = 0; k < slabs.size() && rc == HB_OK && e == cudaSuccess; ++k) {
         if (k + 1 < slabs.size()) e = h2d(k + 1);
         if (e != cudaSuccess) break;
-        Slot &s = slot[k & 1];
-        s.p->nbytes = slabs[k].second;
-        e = cudaStreamWaitEvent(s.compute, s.fetched, 0);       // the slot's previous results have left (the H2D copy did not need that)
-        if (e != cudaSuccess) break;
-        const double tp = now();
-        rc = run_parse(s.p);                         // returns with the slot's compute stream idle
-        { const double d = now() - tp; t_parse += d; t_maxparse = std::max(t_maxparse, d); }
-        if (rc != HB_OK) break;
-        const uint64_t n = s.p->h_st.n_records;
-        if (R + n > out_stride) { rc = fail(HB_ERR_ARG, "more records than the output arrays hold"); break; }
-        if (n) {
-            if (opts->want_gt && opts->n_samples && s.p->d_gt[0]) {
-                if (gt0) e = cudaMemcpy2DAsync(gt0 + R, out_stride, s.p->d_gt[0], s.p->gt_stride, n, opts->n_samples, cudaMemcpyDeviceToHost, s.d2h);
-                if (gt1 && e == cudaSuccess) e = cudaMemcpy2DAsync(gt1 + R, out_stride, s.p->d_gt[1], s.p->gt_stride, n, opts->n_samples, cudaMemcpyDeviceToHost, s.d2h);
-            }
-            if (start && e == cudaSuccess) e = cudaMemcpyAsync(start + R, s.p->d_start, n * 4, cudaMemcpyDeviceToHost, s.d2h);
-            if (stop && e == cudaSuccess) e = cudaMemcpyAsync(stop + R, s.p->d_stop, n * 4, cudaMemcpyDeviceToHost, s.d2h);
-            if (ref && e == cudaSuccess) e = cudaMemcpyAsync(ref + R, s.p->d_ref, n, cudaMemcpyDeviceToHost, s.d2h);
-            if (alt && e == cudaSuccess) e = cudaMemcpyAsync(alt + R, s.p->d_alt, n, cudaMemcpyDeviceToHost, s.d2h);
-        }
-        if ((ploidy_err || badgt_err) && opts->want_gt && opts->n_samples && e == cudaSuccess) {
-            e = cudaMemcpyAsync(pl.data(), s.p->d_ploidy, 4ull * opts->n_samples, cudaMemcpyDeviceToHost, s.d2h);
-            if (e == cudaSuccess) e = cudaMemcpyAsync(bg.data(), s.p->d_badgt, 4ull * opts->n_samples, cudaMemcpyDeviceToHost, s.d2h);
-            if (e == cudaSuccess) e = cudaStreamSynchronize(s.d2h);
-            for (uint32_t i = 0; i < opts->n_samples && e == cudaSuccess; ++i) {
-                if (ploidy_err) ploidy_err[i] += pl[i];
-                if (badgt_err) badgt_err[i] += bg[i];
-            }
-        }
-        if (e == cudaSuccess) e = cudaEventRecord(s.fetched, s.d2h);
-        R += n;
+        const double t0 = now_ms();
+        rc = parse_slab(slot[k & 1], 0, slabs[k].second, sink, R, e);
+        t_parse += now_ms() - t0;
     }
-    t_loop = now() - t_begin - t_setup;
-    for (size_t i = 0; i < ss->n_slots; ++i) if (slot[i].d2h && e == cudaSuccess) e = cudaStreamSynchronize(slot[i].d2h);
-    t_tail = now() - t_begin - t_setup - t_loop;
-    if (e != cudaSuccess && rc == HB_OK) rc = fail(HB_ERR_CUDA, std::string("CUDA: ") + cudaGetErrorString(e));
-    cleanup();
-    if (trace)
-        fprintf(stderr, "[hb_parse_stream_host] %zu slabs: setup %.1f ms, loop %.1f ms (run_parse %.1f, longest %.1f), D2H tail %.1f ms, cleanup %.1f ms\n",
-                slabs.size(), t_setup, t_loop, t_parse, t_maxparse, t_tail, now() - t_begin - t_setup - t_loop - t_tail);
+    const double t_loop_end = now_ms();
+    rc = close_slots(g_text_slots, ss, rc, e);
+    if (getenv("HB_TRACE"))
+        fprintf(stderr, "[hb_parse_stream_host] %zu slabs: setup %.1f ms, loop %.1f ms (parse + deliver %.1f ms), D2H tail + release %.1f ms\n",
+                slabs.size(), t_setup, t_loop_end - t_begin - t_setup, t_parse, now_ms() - t_loop_end);
     if (rc != HB_OK) return rc;
-    if (e != cudaSuccess) return fail(HB_ERR_CUDA, std::string("CUDA: ") + cudaGetErrorString(e));
     *n_records = R;
     if (n_slabs) *n_slabs = (uint32_t)slabs.size();
     return HB_OK;
@@ -1031,7 +1094,7 @@ int hb_parse_chrom_runs(hb_parse *p, uint64_t *n_runs, uint64_t *row_begin, uint
 }
 
 // =============================================================================================
-// File level: .vcf / .vcf.gz reader (BGZF blocks inflate in parallel) + per-(file, region) cache
+// File level: .vcf / .vcf.gz reader (BGZF members inflate in parallel on the GPU) + per-(file, region) cache
 // =============================================================================================
 namespace hb {
 bool bgzf_index(const uint8_t *raw, uint64_t size, std::vector<uint64_t> &coff, std::vector<uint32_t> &clen,
@@ -1063,74 +1126,10 @@ int read_all(const char *path, std::vector<uint8_t> &raw) {
     return HB_OK;
 }
 
-// BGZF: every gzip member carries a 'BC' extra subfield with the block size (htslib bgzf.c)
-bool bgzf_blocks(const std::vector<uint8_t> &raw, std::vector<std::pair<uint64_t, uint32_t>> &blocks,
-                 std::vector<uint64_t> &out_off, uint64_t &total) {
-    uint64_t p = 0;
-    total = 0;
-    while (p < raw.size()) {
-        if (p + 18 > raw.size()) return false;
-        const uint8_t *h = raw.data() + p;
-        if (h[0] != 0x1f || h[1] != 0x8b || h[2] != 8 || !(h[3] & 4)) return false;
-        uint32_t xlen = h[10] | (h[11] << 8);
-        uint32_t bsize = 0;
-        bool found = false;
-        uint64_t q = p + 12, xe = p + 12 + xlen;
-        if (xe > raw.size()) return false;
-        while (q + 4 <= xe) {
-            uint32_t slen = raw[q + 2] | (raw[q + 3] << 8);
-            if (raw[q] == 'B' && raw[q + 1] == 'C' && slen == 2) { bsize = (raw[q + 4] | (raw[q + 5] << 8)) + 1; found = true; }
-            q += 4 + slen;
-        }
-        if (!found || p + bsize > raw.size() || bsize < 12 + xlen + 8) return false;
-        const uint8_t *tr = raw.data() + p + bsize - 4;
-        uint32_t isize = tr[0] | (tr[1] << 8) | (tr[2] << 16) | ((uint32_t)tr[3] << 24);
-        blocks.emplace_back(p, bsize);
-        out_off.push_back(total);
-        total += isize;
-        p += bsize;
-    }
-    return !blocks.empty();
-}
-
+// what parse_bytes_common does not inflate on the GPU: plain text as it is, and any gzip input that is not bgzip-conformant
+// BGZF (e.g. the reference's own test fixture) through zlib, member after member, each checked against its CRC
 int inflate_all(const std::vector<uint8_t> &raw, std::vector<uint8_t> &out) {
     if (raw.size() < 2 || raw[0] != 0x1f || raw[1] != 0x8b) { out = raw; return HB_OK; }   // plain text
-    std::vector<std::pair<uint64_t, uint32_t>> blocks;
-    std::vector<uint64_t> off;
-    uint64_t total = 0;
-    if (bgzf_blocks(raw, blocks, off, total)) {
-        out.resize(total);
-        unsigned nt = std::max(1u, std::min(std::thread::hardware_concurrency(), 64u));
-        nt = (unsigned)std::min<size_t>(nt, blocks.size());
-        std::atomic<size_t> next{0};
-        std::atomic<int> bad{0};
-        auto work = [&]() {
-            z_stream zs;
-            for (;;) {
-                size_t i = next.fetch_add(1);
-                if (i >= blocks.size()) break;
-                const uint8_t *h = raw.data() + blocks[i].first;
-                uint32_t xlen = h[10] | (h[11] << 8);
-                uint64_t outlen = (i + 1 < blocks.size() ? off[i + 1] : total) - off[i];
-                memset(&zs, 0, sizeof zs);
-                if (inflateInit2(&zs, -15) != Z_OK) { bad = 1; break; }
-                zs.next_in = const_cast<Bytef *>(h + 12 + xlen);
-                zs.avail_in = blocks[i].second - 12 - xlen - 8;
-                zs.next_out = out.data() + off[i];
-                zs.avail_out = (uInt)outlen;
-                int rc = inflate(&zs, Z_FINISH);
-                inflateEnd(&zs);
-                if (rc != Z_STREAM_END || zs.avail_out != 0) { bad = 1; break; }
-            }
-        };
-        std::vector<std::thread> th;
-        for (unsigned t = 1; t < nt; ++t) th.emplace_back(work);
-        work();
-        for (auto &t : th) t.join();
-        if (bad) return fail(HB_ERR_IO, "BGZF inflate failed");
-        return HB_OK;
-    }
-    // plain (possibly multi-member) gzip, e.g. the reference's own test fixture
     z_stream zs;
     memset(&zs, 0, sizeof zs);
     if (inflateInit2(&zs, 15 + 32) != Z_OK) return fail(HB_ERR_IO, "inflateInit2 failed");
@@ -1205,8 +1204,8 @@ int read_vcf(const std::vector<uint8_t> &raw, FileText &ft) {
 
 // One .vcf / .vcf.gz -> device-resident parse.  BGZF files (what bgzip writes, what the reference's tabix path
 // reads) travel over PCIe COMPRESSED and are inflated on the GPU (hb_inflate.cu) straight into the text buffer;
-// only the header members are also inflated on the host, to learn the sample names.  Plain gzip (one DEFLATE
-// stream: nothing to parallelise) and plain text go through zlib / as they are.
+// only the header members are also inflated on the host, to learn the sample names.  Any other gzip input (plain
+// gzip, or BGZF that bgzip would not have written) and plain text go through zlib / as they are.
 int parse_bytes_common(std::vector<uint8_t> &raw_owned, const uint8_t *raw_p, uint64_t raw_n, const char *region, bool want_gt,
                        int device, hb_parse **out, std::vector<std::string> &samples);
 
@@ -1577,31 +1576,20 @@ int hb_bgzf_vcf_info(const uint8_t *bgzf, uint64_t nbytes, uint32_t *n_samples, 
 // BGZF bytes in host memory -> results in host memory, streamed: slabs of whole BGZF members cross PCIe compressed,
 // are inflated on the GPU behind the unfinished last line of the slab before, parsed up to their own last newline and
 // fetched -- H2D + inflate of slab k + 1 and the D2H of slab k - 1 run while slab k is parsed.
-namespace {
-// where the rows of a parsed slab go: host arrays (hb_parse_stream_bgzf_host) or the growing planes of ONE resident parse
-// (hb_parse_stream_bgzf_resident).  deliver() enqueues copies on s.d2h (the slot's compute stream is idle by then).
-struct SlabSink {
-    virtual ~SlabSink() {}
-    virtual int begin(const hb_parse_opts &opts, const std::vector<std::string> &samples, uint64_t total_text) { (void)opts; (void)samples; (void)total_text; return HB_OK; }
-    virtual int deliver(StreamSlot &s, uint64_t R, uint64_t n, uint64_t slab_text, cudaError_t &e) = 0;
-};
-}
-static int stream_bgzf(const uint8_t *bgzf, uint64_t nbytes, const char *region, int want_gt, int device, uint64_t slab_bytes,
-                       SlabSink &sink, uint32_t *ploidy_err, uint32_t *badgt_err, uint64_t *n_records, uint32_t *n_slabs) {
+static int stream_bgzf(const char *entry, const uint8_t *bgzf, uint64_t nbytes, const char *region, int want_gt, int device,
+                       uint64_t slab_bytes, SlabSink &sink, uint64_t *n_records, uint32_t *n_slabs) {
     if (!bgzf || !n_records) return fail(HB_ERR_ARG, "null argument");
     *n_records = 0;
     if (n_slabs) *n_slabs = 0;
-    const bool trace = getenv("HB_TRACE") != nullptr;
-    auto now = []() { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now().time_since_epoch()).count(); };
-    const double t_begin = now();
-    double t_index = 0, t_setup = 0, t_wait = 0, t_parse = 0, t_enq = 0;
+    const double t_begin = now_ms();
+    double t_wait = 0, t_parse = 0, t_enq = 0;
     std::vector<uint64_t> coff, ooff;
     std::vector<uint32_t> clen, olen;
     uint64_t total = 0;
     if (!bgzf_index(bgzf, nbytes, coff, clen, ooff, olen, total)) return fail(HB_ERR_IO, "not a BGZF file");
     FileText ft;
     TRY(bgzf_header(bgzf, coff, clen, olen, ft));
-    t_index = now() - t_begin;
+    const double t_index = now_ms() - t_begin;
     hb_parse_opts opts;
     memset(&opts, 0, sizeof opts);
     opts.region = region;
@@ -1609,8 +1597,6 @@ static int stream_bgzf(const uint8_t *bgzf, uint64_t nbytes, const char *region,
     opts.device = device;
     opts.n_samples = (uint32_t)ft.samples.size();
     opts.end_is_int = ft.end_is_int;
-    if (ploidy_err) memset(ploidy_err, 0, 4ull * opts.n_samples);
-    if (badgt_err) memset(badgt_err, 0, 4ull * opts.n_samples);
     TRY(ensure_device(device));
     TRY(sink.begin(opts, ft.samples, total));
     if (total <= ft.body) return HB_OK;
@@ -1631,50 +1617,15 @@ static int stream_bgzf(const uint8_t *bgzf, uint64_t nbytes, const char *region,
     if (slabs.empty()) return HB_OK;
     if (ft.body >= slabs[0].text) return fail(HB_ERR_ARG, "the VCF header is longer than a slab: raise slab_bytes");
     const uint64_t carry_cap = std::min<uint64_t>((text_cap + 15) & ~15ull, 256ull << 20);   // longest unfinished line carried over
-    TRY(ensure_device(device));
-    typedef StreamSlot Slot;
-    int rc = HB_OK;
-    const size_t n_slots = std::min<size_t>(2, slabs.size());
-    StreamSlots *ss = acquire_slots(g_bgzf_slots, opts, n_slots);
-    Slot *slot = ss->slot;
-    auto cleanup = [&]() { release_slots(g_bgzf_slots, ss, rc == HB_OK); };
-    // buffers grow together when any capacity is short (the carry offset is part of the layout)
-    const bool grow = ss->text_cap < text_cap || ss->comp_cap < comp_cap || ss->n_cap < n_cap || ss->carry_cap < carry_cap;
-    if (grow) {
-        ss->text_cap = std::max(ss->text_cap, text_cap + text_cap / 16);
-        ss->comp_cap = std::max(ss->comp_cap, comp_cap + comp_cap / 8);
-        ss->n_cap = std::max<uint32_t>(ss->n_cap, (uint32_t)(n_cap + n_cap / 8 + 16));
-        ss->carry_cap = std::max(ss->carry_cap, carry_cap);
-    }
-    for (size_t i = 0; i < n_slots && rc == HB_OK; ++i) {
-        Slot &s = slot[i];
-        if (!s.p) {
-            if (cudaStreamCreateWithFlags(&s.compute, cudaStreamNonBlocking) != cudaSuccess ||
-                cudaStreamCreateWithFlags(&s.d2h, cudaStreamNonBlocking) != cudaSuccess ||
-                cudaEventCreateWithFlags(&s.fetched, cudaEventDisableTiming) != cudaSuccess) { rc = fail(HB_ERR_CUDA, "cannot create streams"); break; }
-            hb_parse_opts o = opts;
-            o.stream = s.compute;
-            rc = new_parse(&o, &s.p);
-            if (rc == HB_OK) ss->n_slots = std::max(ss->n_slots, i + 1);
-        }
-        if (rc != HB_OK) break;
-        s.p->probed = false;
-        if (grow || !s.buf) {
-            if (s.h_pin) { cudaFreeHost(s.h_pin); s.h_pin = nullptr; }
-            inflate_scratch_free(s.sc);
-            rc = dev_alloc(&s.buf, ss->carry_cap + 32 + ss->text_cap + 1 + 256);
-            if (rc == HB_OK) rc = inflate_scratch_alloc(s.sc, ss->comp_cap, ss->n_cap);
-            s.hc.resize(ss->n_cap); s.ho.resize(ss->n_cap);
-            // pinned: [last newline 8 | status 4n | coff 8n | ooff 8n | clen 4n | olen 4n] -- copies from / to pageable memory stall here
-            if (rc == HB_OK && cudaMallocHost((void **)&s.h_pin, 8 + 28ull * ss->n_cap + 8) != cudaSuccess) rc = fail(HB_ERR_MEM, "cudaMallocHost failed");
-        }
-    }
-    if (rc != HB_OK) { cleanup(); return rc; }
+    StreamSlots *ss = nullptr;
+    TRY(open_slots(g_bgzf_slots, opts, std::min<size_t>(2, slabs.size()), text_cap, carry_cap, comp_cap, (uint32_t)n_cap, &ss));
+    StreamSlot *slot = ss->slot;
     const uint64_t carry_base = ss->carry_cap;                 // offset of a slab's text when nothing is carried
+    int rc = HB_OK;
     cudaError_t e = cudaSuccess;
     // H2D + inflate of slab k behind a carry of carry_len bytes, then the search for its last newline
     auto enqueue = [&](size_t k, uint64_t carry_len) -> int {
-        Slot &s = slot[k & 1];
+        StreamSlot &s = slot[k & 1];
         const Slab &sl = slabs[k];
         const uint64_t skip = k == 0 ? ft.body : 0;            // slab 0 starts with the header
         s.x = carry_base + (k == 0 ? (16 - ft.body % 16) % 16 : carry_len % 16);   // the parse starts on a 16-byte boundary
@@ -1700,15 +1651,14 @@ static int stream_bgzf(const uint8_t *bgzf, uint64_t nbytes, const char *region,
         if (ee != cudaSuccess) return fail(HB_ERR_CUDA, std::string("CUDA: ") + cudaGetErrorString(ee));
         return HB_OK;
     };
-    t_setup = now() - t_begin - t_index;
+    const double t_setup = now_ms() - t_begin - t_index;
     rc = enqueue(0, 0);
     uint64_t R = 0;
-    std::vector<uint32_t> pl(opts.n_samples), bg(opts.n_samples);
     for (size_t k = 0; k < slabs.size() && rc == HB_OK && e == cudaSuccess; ++k) {
-        Slot &s = slot[k & 1];
-        { const double t0 = now();
+        StreamSlot &s = slot[k & 1];
+        { const double t0 = now_ms();
         e = cudaStreamSynchronize(s.compute);                  // slab k is inflated, its last newline is known
-        t_wait += now() - t0; }
+        t_wait += now_ms() - t0; }
         if (e != cudaSuccess) break;
         const unsigned long long last_nl = s.h_pin[0];
         const int *status = reinterpret_cast<const int *>(s.h_pin + 1);
@@ -1725,7 +1675,7 @@ static int stream_bgzf(const uint8_t *bgzf, uint64_t nbytes, const char *region,
         const uint64_t carry_len = last ? 0 : s.end - parse_end;
         if (carry_len > carry_base) { rc = fail(HB_ERR_ARG, "a line is longer than the carry buffer: raise slab_bytes"); break; }
         if (!last) {
-            Slot &nx = slot[(k + 1) & 1];
+            StreamSlot &nx = slot[(k + 1) & 1];
             // the unfinished line goes in front of the next slab's text (that buffer's last parse has returned)
             const uint64_t nx_x = carry_base + carry_len % 16;
             if (carry_len) e = cudaMemcpyAsync(nx.buf + nx_x - carry_len, s.buf + parse_end, carry_len, cudaMemcpyDeviceToDevice, s.compute);
@@ -1733,78 +1683,36 @@ static int stream_bgzf(const uint8_t *bgzf, uint64_t nbytes, const char *region,
         }
         e = cudaMemsetAsync(s.buf + parse_end, 0, 256, s.compute);
         if (e != cudaSuccess) break;
-        if (!last) { const double t0 = now(); rc = enqueue(k + 1, carry_len); t_enq += now() - t0; if (rc != HB_OK) break; }
-        uint64_t n = 0;
-        if (parse_end > s.begin) {
-            e = cudaStreamWaitEvent(s.compute, s.fetched, 0);   // the slot's previous results have left (the inflate did not need that)
-            if (e != cudaSuccess) break;
-            s.p->d_text = s.buf + s.begin;
-            s.p->nbytes = parse_end - s.begin;
-            const double t0 = now();
-            rc = run_parse(s.p);                                // returns with the slot's compute stream idle
-            t_parse += now() - t0;
-            if (rc != HB_OK) break;
-            n = s.p->h_st.n_records;
-        }
-        if (n) {
-            rc = sink.deliver(s, R, n, s.p->nbytes, e);
-            if (rc != HB_OK) break;
-            if ((ploidy_err || badgt_err) && opts.want_gt && opts.n_samples && e == cudaSuccess) {
-                e = cudaMemcpyAsync(pl.data(), s.p->d_ploidy, 4ull * opts.n_samples, cudaMemcpyDeviceToHost, s.d2h);
-                if (e == cudaSuccess) e = cudaMemcpyAsync(bg.data(), s.p->d_badgt, 4ull * opts.n_samples, cudaMemcpyDeviceToHost, s.d2h);
-                if (e == cudaSuccess) e = cudaStreamSynchronize(s.d2h);
-                for (uint32_t i = 0; i < opts.n_samples && e == cudaSuccess; ++i) {
-                    if (ploidy_err) ploidy_err[i] += pl[i];
-                    if (badgt_err) badgt_err[i] += bg[i];
-                }
-            }
-        }
-        if (e == cudaSuccess) e = cudaEventRecord(s.fetched, s.d2h);
-        R += n;
+        if (!last) { const double t0 = now_ms(); rc = enqueue(k + 1, carry_len); t_enq += now_ms() - t0; if (rc != HB_OK) break; }
+        const double t0 = now_ms();
+        rc = parse_slab(s, s.begin, parse_end > s.begin ? parse_end - s.begin : 0, sink, R, e);
+        t_parse += now_ms() - t0;
     }
-    for (size_t i = 0; i < ss->n_slots; ++i) if (slot[i].d2h && e == cudaSuccess && rc == HB_OK) e = cudaStreamSynchronize(slot[i].d2h);
-    if (e != cudaSuccess && rc == HB_OK) rc = fail(HB_ERR_CUDA, std::string("CUDA: ") + cudaGetErrorString(e));
-    const double t_loop_end = now();
-    cleanup();
-    if (trace)
-        fprintf(stderr, "[hb_parse_stream_bgzf_host] %zu slabs: index+header %.1f ms, setup %.1f ms, waits for inflate %.1f ms, enqueue %.1f ms, "
-                        "run_parse %.1f ms, loop+tail %.1f ms, release %.1f ms\n", slabs.size(), t_index, t_setup, t_wait, t_enq, t_parse,
-                t_loop_end - t_begin - t_index - t_setup, now() - t_loop_end);
+    const double t_loop_end = now_ms();
+    rc = close_slots(g_bgzf_slots, ss, rc, e);
+    if (getenv("HB_TRACE"))
+        fprintf(stderr, "[%s] %zu slabs: index+header %.1f ms, setup %.1f ms, waits for inflate %.1f ms, enqueue %.1f ms, "
+                        "parse + deliver %.1f ms, loop %.1f ms, D2H tail + release %.1f ms\n", entry, slabs.size(), t_index, t_setup,
+                t_wait, t_enq, t_parse, t_loop_end - t_begin - t_index - t_setup, now_ms() - t_loop_end);
     if (rc != HB_OK) return rc;
-    if (e != cudaSuccess) return fail(HB_ERR_CUDA, std::string("CUDA: ") + cudaGetErrorString(e));
     *n_records = R;
     if (n_slabs) *n_slabs = (uint32_t)slabs.size();
     return HB_OK;
 }
 
 namespace {
-struct HostSink : SlabSink {
-    int8_t *gt0, *gt1; uint64_t out_stride; uint32_t *start, *stop; char *ref, *alt;
-    hb_parse_opts opts{};
-    int begin(const hb_parse_opts &o, const std::vector<std::string> &, uint64_t) override { opts = o; return HB_OK; }
-    int deliver(StreamSlot &s, uint64_t R, uint64_t n, uint64_t, cudaError_t &e) override {
-        if (R + n > out_stride && (gt0 || gt1 || start || stop || ref || alt)) return fail(HB_ERR_ARG, "more records than the output arrays hold");
-        if (opts.want_gt && opts.n_samples && s.p->d_gt[0]) {
-            if (gt0) e = cudaMemcpy2DAsync(gt0 + R, out_stride, s.p->d_gt[0], s.p->gt_stride, n, opts.n_samples, cudaMemcpyDeviceToHost, s.d2h);
-            if (gt1 && e == cudaSuccess) e = cudaMemcpy2DAsync(gt1 + R, out_stride, s.p->d_gt[1], s.p->gt_stride, n, opts.n_samples, cudaMemcpyDeviceToHost, s.d2h);
-        }
-        if (start && e == cudaSuccess) e = cudaMemcpyAsync(start + R, s.p->d_start, n * 4, cudaMemcpyDeviceToHost, s.d2h);
-        if (stop && e == cudaSuccess) e = cudaMemcpyAsync(stop + R, s.p->d_stop, n * 4, cudaMemcpyDeviceToHost, s.d2h);
-        if (ref && e == cudaSuccess) e = cudaMemcpyAsync(ref + R, s.p->d_ref, n, cudaMemcpyDeviceToHost, s.d2h);
-        if (alt && e == cudaSuccess) e = cudaMemcpyAsync(alt + R, s.p->d_alt, n, cudaMemcpyDeviceToHost, s.d2h);
-        return HB_OK;
-    }
-};
-
 // The rows of every slab appended to ONE resident parse: genotype planes and site columns grow in HBM (2.5 bytes per call),
 // the text never holds more than two slabs.  The result is the handle a whole-file parse would have given (without its
 // text): same rows, so hb_compress_records cuts it into the same HDF5 chunks -- chunk boundaries do not see slab boundaries.
 struct ResidentSink : SlabSink {
     hb_parse *big = nullptr;
     uint64_t total_text = 0, text_seen = 0, cap = 0;
-    std::vector<uint32_t> ploidy, badgt;
+    std::vector<uint32_t> ploidy, badgt;       // per-sample error counts, summed on the host and put on the device at the end
     ~ResidentSink() override { if (big) hb_parse_free(big); }
     int begin(const hb_parse_opts &o, const std::vector<std::string> &samples, uint64_t total) override {
+        ploidy.assign(std::max<uint32_t>(o.n_samples, 1), 0); badgt.assign(std::max<uint32_t>(o.n_samples, 1), 0);
+        ploidy_err = ploidy.data(); badgt_err = badgt.data();
+        TRY(SlabSink::begin(o, samples, total));
         total_text = total;
         hb_parse_opts oo = o;
         oo.stream = nullptr;
@@ -1896,7 +1804,8 @@ int hb_parse_stream_bgzf_host(const uint8_t *bgzf, uint64_t nbytes, const char *
                               uint64_t *n_records, uint32_t *n_slabs) {
     HostSink sink;
     sink.gt0 = gt0; sink.gt1 = gt1; sink.out_stride = out_stride; sink.start = start; sink.stop = stop; sink.ref = ref; sink.alt = alt;
-    return stream_bgzf(bgzf, nbytes, region, want_gt, device, slab_bytes, sink, ploidy_err, badgt_err, n_records, n_slabs);
+    sink.ploidy_err = ploidy_err; sink.badgt_err = badgt_err;
+    return stream_bgzf("hb_parse_stream_bgzf_host", bgzf, nbytes, region, want_gt, device, slab_bytes, sink, n_records, n_slabs);
 }
 
 int hb_parse_stream_bgzf_resident(const uint8_t *bgzf, uint64_t nbytes, const char *region, int want_gt, int device,
@@ -1905,15 +1814,10 @@ int hb_parse_stream_bgzf_resident(const uint8_t *bgzf, uint64_t nbytes, const ch
     *out = nullptr;
     ResidentSink sink;
     uint64_t n = 0;
-    uint32_t S = 0;
-    {   // per-sample error counts are summed on the host and put on the device at the end
-        uint64_t tb = 0, bo = 0;
-        TRY(hb_bgzf_vcf_info(bgzf, nbytes, &S, &tb, &bo));
-    }
-    sink.ploidy.assign(S ? S : 1, 0); sink.badgt.assign(S ? S : 1, 0);
-    TRY(stream_bgzf(bgzf, nbytes, region, want_gt, device, slab_bytes, sink, sink.ploidy.data(), sink.badgt.data(), &n, n_slabs));
+    TRY(stream_bgzf("hb_parse_stream_bgzf_resident", bgzf, nbytes, region, want_gt, device, slab_bytes, sink, &n, n_slabs));
     hb_parse *p = sink.big;
     if (!p) return fail(HB_ERR_IO, "empty input");
+    const uint32_t S = p->n_samples;
     cudaError_t e = cudaSuccess;
     if (want_gt && S) {
         int rc = dev_alloc(&p->d_ploidy, S);

@@ -3,6 +3,7 @@ produced by Python's zlib (an independent, third-party DEFLATE encoder) in BGZF 
 and compared byte for byte with the input.  Dynamic, fixed and stored DEFLATE blocks, all levels."""
 import gzip
 import os
+import struct
 import zlib
 
 import numpy as np
@@ -94,6 +95,31 @@ def test_bgzf_file_through_the_reference_api(capi, tmp_path, built):
     assert np.array_equal(g0, ora["gt0"]) and np.array_equal(g1, ora["gt1"])
 
 
+def test_gzip_members_with_a_file_name_are_read(capi):
+    """Members that carry FNAME next to the BGZF 'BC' subfield (FLG = FEXTRA | FNAME) are valid gzip but not what bgzip
+    writes: the GPU inflater refuses them and the host's zlib reads them, member by member, with their CRCs checked."""
+    text, _ = _vcf_text(2000, 23, seed=4)
+    name = b"chr22.vcf\0"
+    members = []
+    for i in range(0, len(text), 40_000):
+        chunk = text[i:i + 40_000]
+        c = zlib.compressobj(6, zlib.DEFLATED, -15)
+        payload = c.compress(chunk) + c.flush()
+        bsize = 12 + 6 + len(name) + len(payload) + 8
+        head = struct.pack("<BBBBIBBH", 0x1f, 0x8b, 8, 4 | 8, 0, 0, 0xff, 6) + b"BC" + struct.pack("<HH", 2, bsize - 1)
+        members.append(head + name + payload + struct.pack("<II", zlib.crc32(chunk), len(chunk)))
+    data = b"".join(members)
+    assert len(members) > 1 and gzip.decompress(data) == text
+    ora = oracle.parse_text(text, "*", "chr22")
+    p = capi.Parse.from_vcf_bytes(data, region="chr22")
+    assert p.info.n_records == ora["n"]
+    g0, g1 = p.matrix()
+    assert np.array_equal(g0, ora["gt0"]) and np.array_equal(g1, ora["gt1"])
+    start, stop, ref, alt = p.sites()
+    assert np.array_equal(start, ora["start"]) and np.array_equal(stop, ora["stop"])
+    assert np.array_equal(ref, ora["ref"]) and np.array_equal(alt, ora["alt"])
+
+
 @pytest.mark.parametrize("fmt,kinds,slab,block", [("GT", "phased", 5000, 0xff00), ("GT", "mixed", 30000, 4000),
                                                   ("GT:GQ:DP", "mixed", 9000, 1500), ("GT", "mixed", 1 << 30, 0xff00)])
 def test_stream_bgzf_host_equals_oracle(capi, fmt, kinds, slab, block):
@@ -134,6 +160,20 @@ def test_stream_bgzf_host_edges(capi):
     r = capi.parse_stream_bgzf_host(synth.bgzf_compress(text), capacity=4000, region="chr22", slab_bytes=len(text) // 7)
     assert r["n"] == ora["n"] and r["n_slabs"] >= 7
     assert np.array_equal(r["gt0"], ora["gt0"]) and np.array_equal(r["gt1"], ora["gt1"]) and np.array_equal(r["start"], ora["start"])
+
+
+def test_stream_bgzf_host_grows_every_cached_slot(capi):
+    """A one-slab call grows the buffers of both cached slots, so a later two-slab call of that size finds room in each."""
+    text, _ = synth.random_vcf(1500, 41, seed=79, fmt="GT", kinds="mixed")
+    ora = oracle.parse_text(text, "*", "chr22")
+    gz = synth.bgzf_compress(text, block=4000)
+    capi.lib().hb_cache_clear()
+    for slab in (8000, 1 << 30, len(text) // 2 + 4000):
+        r = capi.parse_stream_bgzf_host(gz, capacity=1500, region="chr22", slab_bytes=slab)
+        assert r["n"] == ora["n"] and np.array_equal(r["gt0"], ora["gt0"]) and np.array_equal(r["gt1"], ora["gt1"])
+        assert np.array_equal(r["start"], ora["start"]) and np.array_equal(r["alt"], ora["alt"])
+    assert r["n_slabs"] == 2
+    capi.lib().hb_cache_clear()
 
 
 def test_streamed_resident_parse_gives_the_whole_file_chunks(capi):

@@ -305,6 +305,14 @@ def test_stream_host_uniform_text_and_errors(capi):
     lines[333] = "chr22\t433\t.\tA\tC\t.\t.\t.\tGT\t0|1\t1\t0|0\n"
     r = capi.parse_stream_host("".join(lines).encode(), 3, capacity=400, region="", slab_bytes=2000)
     assert r["n"] == 400 and list(r["ploidy_err"]) == [0, 1, 0] and r["n_slabs"] > 3
+    # the same lines behind a header, in BGZF: streamed into host arrays, and into one resident parse
+    gz = synth.bgzf_compress((synth.header(S) + "".join(lines)).encode(), block=1000)
+    r = capi.parse_stream_bgzf_host(gz, capacity=400, region="", slab_bytes=2000)
+    assert r["n"] == 400 and list(r["ploidy_err"]) == [0, 1, 0] and r["n_slabs"] > 3
+    p, n_slabs = capi.Parse.from_vcf_bytes_streamed(gz, region="", slab_bytes=2000)
+    assert p.info.n_records == 400 and n_slabs > 3
+    pl, bg = p.sample_errors()
+    assert list(pl) == [0, 1, 0] and list(bg) == [0, 0, 0]
 
 
 def test_biobank_width_200k_samples(capi):
