@@ -77,7 +77,7 @@ EXPORTS = [
     "hb_bgzf_inflate", "hb_bgzf_compress_host",
     "hb_compress_records", "hb_compress_sample_range", "hb_frames_set_window", "hb_parse_release_text", "hb_parse_attach_frames", "hb_frames_rerun", "hb_frames_get_info", "hb_frames_layout", "hb_frames_fetch_all", "hb_frames_fetch_packed", "hb_set_fetch_mode", "hb_set_host_threads", "hb_frames_last_d2h_bytes",
     "hb_frames_fetch_sample", "hb_frames_free",
-    "hb_guess_chunk_records", "hb_set_site_matcher", "hb_decode_frames", "hb_decode_columns_device",
+    "hb_guess_chunk_records", "hb_set_site_matcher", "hb_decode_frames", "hb_decode_columns_device", "hb_decode_columns_device_large",
     "hb_encode_haplotypes",
     "hb_synth_body_bytes", "hb_synth_header", "hb_synth_device", "hb_synth_host",
 ]
@@ -156,6 +156,7 @@ def lib():
             L.hb_set_site_matcher.restype = None
             L.hb_decode_frames.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64, C.c_void_p, C.c_int, C.c_int]
             L.hb_decode_columns_device.argtypes = [C.c_void_p] * 4 + [C.c_uint64, C.c_uint32] + [C.c_void_p] * 8
+            L.hb_decode_columns_device_large.argtypes = [C.c_void_p] * 4 + [C.c_uint64, C.c_uint32] + [C.c_void_p] * 8
         L.hb_encode_haplotypes.argtypes = [C.POINTER(HapBatch)]
         L.hb_synth_body_bytes.argtypes = [C.POINTER(SynthSpec)]
         L.hb_synth_body_bytes.restype = C.c_uint64

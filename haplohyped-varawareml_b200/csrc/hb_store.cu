@@ -168,6 +168,9 @@ __device__ int warp_lz4_segment(const uint8_t *src, int n, int hist, uint8_t *ds
 //                          the block (bit-parallel matcher, below) into shared memory; the frame then leaves as two
 //                          TMA bulk stores (template body from the shared copy, own tail) + two 16-byte header
 //                          vectors with the size fields filled in.  C_out is written exactly once.
+//   site_template_large_kernel / donor_frames_large_kernel   the same frames for chunks of 2,731 - 7,489 records (still ONE
+//                          Blosc block): site planes in a global scratch, allele tails in passes, template read from
+//                          global memory.  The host picks the pair from cr; below 2,731 nothing changes.
 // Output: ONE buffer of slots in [sample][chunk] order.  The slot of (sample s, chunk c) starts at
 // s * row_stride + slot_off[c]; slot_off is the running sum of round16(template_len[c] + worst-case
 // allele tail), so every frame's address is known before it is encoded (no scan, no look-back) and the
@@ -352,6 +355,113 @@ __global__ void __launch_bounds__(kSiteSegs * 32) site_template_kernel(const Sit
     for (uint32_t i = threadIdx.x; i < TMPL_HDR; i += blockDim.x) g[i] = s_head[i];
     for (uint32_t i = tl + threadIdx.x; i < ((tl + 15) & ~15u); i += blockDim.x) g[i] = 0;
     if (threadIdx.x == 0) a.tmpl_len[c] = tl;
+}
+
+// ------------------------------------------------------------------------------------------
+// Kernel 4a-L: the site templates of chunks of kSmallChunkMax < cr <= kMaxChunkRecords records.  Up to 7,489 records
+// such a chunk is still ONE Blosc block with ONE LZ4 stream (c-blosc 1.x cuts blocks of 262,115 bytes for typesize 35
+// at clevel 5 with LZ4HC), so the template has exactly the layout of site_template_kernel's: the same segments, the
+// same matcher, the same stitch, the same closing offset-1 match over planes 24-32.  What changes is where the bytes
+// live: 33 * cr bytes of planes no longer fit shared memory, so the head [0, 24 * cr + 1) that is encoded and the
+// per-segment outputs sit in a per-CTA global scratch (L2-resident: ~2 * 24 * cr bytes per CTA), and only the hash
+// tables stay in shared memory.  The 16-bit table entries still hold: positions are relative to a segment, and the
+// longest segment (the five CHROM planes) is 5 * 7,489 < 65,535 bytes; far = 4 * cr and 2 * cr are legal LZ4 offsets.
+// The grid is smaller than the chunk count (the scratch is per CTA): CTA b encodes chunks b, b + gridDim.x, ...
+// ------------------------------------------------------------------------------------------
+constexpr uint32_t kSmallChunkMax = 2730;        // largest chunk of site_template_kernel / donor_frames_kernel
+constexpr uint32_t kMaxChunkRecords = 7489;      // largest chunk that is ONE c-blosc 1.x block at typesize 35
+constexpr uint32_t kSitePad = 48;                // zero bytes behind the head: look-ahead reads of the last segment
+__host__ __device__ inline uint32_t site_large_head_bytes(uint32_t cr) { return (16 + 24 * cr + 1 + kSitePad + 15) & ~15u; }
+__host__ __device__ inline uint32_t site_large_scratch(uint32_t cr) {
+    return site_large_head_bytes(cr) + ((site_seg_cap(24 * cr + 1) + kSiteSegs * 48 + 15) & ~15u);
+}
+
+__global__ void __launch_bounds__(kSiteSegs * 32) site_template_large_kernel(const SiteArgs4 a, uint8_t *scratch) {
+    extern __shared__ __align__(16) uint8_t smem[];
+    __shared__ int s_len[kSiteSegs], s_pend[kSiteSegs], s_flit[kSiteSegs], s_fhdr[kSiteSegs];
+    __shared__ int s_dst[kSiteSegs], s_carry[kSiteSegs], s_final[2];
+    __shared__ uint8_t s_head[TMPL_HDR + 7];
+    const uint32_t cr = a.cr;
+    const uint32_t n = 33u * cr;
+    const int n1 = 24 * (int)cr + 1;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    uint8_t *planes = scratch + (size_t)blockIdx.x * site_large_scratch(cr) + 16;   // 16 zero bytes of history in front
+    uint8_t *outs = planes - 16 + site_large_head_bytes(cr);
+    uint16_t *table = reinterpret_cast<uint16_t *>(smem) + ((size_t)warp << kSiteHashLog);
+    const int sb = (int)site_seg_begin(warp, cr), se = (int)site_seg_begin(warp + 1, cr);
+    uint32_t out_off = 0;
+    for (int w = 0; w < warp; ++w) out_off += site_seg_cap(site_seg_begin(w + 1, cr) - site_seg_begin(w, cr));
+    uint8_t *my_out = outs + out_off;
+    const uint64_t n_chunks = (a.n_records + cr - 1) / cr;
+    if (threadIdx.x < 16) planes[(int)threadIdx.x - 16] = 0;
+    for (uint32_t i = 24 * cr + threadIdx.x; i < (uint32_t)n1 + kSitePad; i += blockDim.x) planes[i] = 0;   // planes 24.. are zero
+    if (threadIdx.x == 0) write_frame_head(s_head, 35u * cr);
+    for (uint64_t c = blockIdx.x; c < n_chunks; c += gridDim.x) {
+        const uint64_t r0 = c * cr;
+        for (uint32_t i = threadIdx.x; i < cr; i += blockDim.x) {
+            const uint64_t r = r0 + i;
+            uint64_t ch = 0;
+            uint32_t st = 0, sp = 0;
+            uint8_t rf = 0, al = 0;
+            if (r < a.n_records) { ch = a.chrom5[r]; st = a.start[r]; sp = a.stop[r]; rf = a.ref[r]; al = a.alt[r]; }
+#pragma unroll
+            for (int k = 0; k < 5; ++k) planes[k * cr + i] = (uint8_t)(ch >> (8 * k));
+#pragma unroll
+            for (int k = 0; k < 4; ++k) {
+                planes[(5 + k) * cr + i] = (uint8_t)(st >> (8 * k));
+                planes[(9 + k) * cr + i] = (uint8_t)(sp >> (8 * k));
+            }
+            planes[13 * cr + i] = rf;
+            planes[23 * cr + i] = al;
+#pragma unroll
+            for (int k = 0; k < 9; ++k) planes[(14 + k) * cr + i] = 0;
+        }
+        __syncthreads();
+        {
+            int flit, fhdr, pend;
+            const int len = warp_lz4_segment(planes + sb, se - sb, sb, my_out, table, kSiteHashLog, 4 * (int)cr, a.deep != 0, &flit, &fhdr, &pend);
+            if (lane == 0) { s_len[warp] = len; s_pend[warp] = pend; s_flit[warp] = flit; s_fhdr[warp] = fhdr; }
+        }
+        __syncthreads();
+        if (threadIdx.x == 0) {                   // stitch, as in site_template_kernel
+            int carry = 0, off = 0;
+            for (int w = 0; w < kSiteSegs; ++w) {
+                s_dst[w] = off; s_carry[w] = carry;
+                if (s_len[w] == 0) { carry += s_pend[w]; continue; }
+                const int lit = s_flit[w] + carry;
+                off += 1 + (lit >= 15 ? 1 + (lit - 15) / 255 : 0) + carry + (s_len[w] - s_fhdr[w]);
+                carry = s_pend[w];
+            }
+            s_final[0] = off; s_final[1] = carry;
+        }
+        __syncthreads();
+        uint8_t *g = a.tmpl + c * a.tmpl_cap;
+        uint8_t *lz = g + TMPL_HDR;
+        if (s_len[warp] > 0) {
+            const int carry = s_carry[warp], lit = s_flit[warp] + carry;
+            int o = s_dst[warp];
+            if (lane == 0) lz[o] = (uint8_t)((min(lit, 15) << 4) | (my_out[0] & 15));
+            ++o;
+            if (lit >= 15) {
+                int rem = lit - 15;
+                while (rem >= 255) { if (lane == 0) lz[o] = 255; ++o; rem -= 255; }
+                if (lane == 0) lz[o] = (uint8_t)rem;
+                ++o;
+            }
+            for (int i = lane; i < carry; i += 32) lz[o + i] = planes[sb - carry + i];
+            o += carry;
+            const int rest = s_len[warp] - s_fhdr[warp];
+            for (int i = lane; i < rest; i += 32) lz[o + i] = my_out[s_fhdr[warp] + i];
+        }
+        int o = s_final[0];
+        if (warp == 0) o = warp_emit_seq(lz, o, planes + n1 - s_final[1], s_final[1], 1, (int)n - n1);
+        else o = o + 1 + (s_final[1] >= 15 ? 1 + (s_final[1] - 15) / 255 : 0) + s_final[1] + 2 + ((int)n - n1 >= 19 ? 1 + ((int)n - n1 - 19) / 255 : 0);
+        const uint32_t tl = TMPL_HDR + (uint32_t)o;
+        for (uint32_t i = threadIdx.x; i < TMPL_HDR; i += blockDim.x) g[i] = s_head[i];
+        for (uint32_t i = tl + threadIdx.x; i < ((tl + 15) & ~15u); i += blockDim.x) g[i] = 0;
+        if (threadIdx.x == 0) a.tmpl_len[c] = tl;
+        __syncthreads();                          // the scratch and the stitch table are re-used by the next chunk
+    }
 }
 
 // ------------------------------------------------------------------------------------------
@@ -825,6 +935,354 @@ __global__ void __launch_bounds__(kWpc * 32) donor_frames_kernel(const FusedArgs
     if (lane == 0) tma_store_wait_read();    // shared memory must outlive the bulk stores that read it
 }
 
+// ------------------------------------------------------------------------------------------
+// Kernel 4b-L: the allele tails of chunks of kSmallChunkMax < cr <= kMaxChunkRecords records.  The parse, the scans and
+// the emission are donor_frames_kernel's, run in PASSES: a pass covers 32 lanes x 32 * NW block positions, and the
+// literals a pass leaves at its end are carried into the first sequence of the next pass exactly as a lane carries
+// them into the next lane's.  Z and C match sources (offsets 2 * cr and cr) and the closing literals are unchanged,
+// so the slot bound (template + 2 cr + 2 cr / 255 + 24) still holds.  The template is NOT staged in shared memory
+// (a chunk with high-entropy sites makes a template of up to ~24 * cr bytes): the warp copies its body from global
+// memory (L2-resident: every warp of the chunk reads the same bytes).  Shared memory per warp = bit-plane staging +
+// the two bit strings + the whole tail buffer, zeroed up front because the tail's length is known after the last pass.
+// ------------------------------------------------------------------------------------------
+constexpr int kLargeNW = 4;                   // mask words per lane and pass: 4,096 block positions per pass
+constexpr int kWpcL = 4;                      // warps per CTA: 2-6 CTAs per SM from cr 7,489 down to 2,731
+
+// __maxnreg__(96) instead of __launch_bounds__: with the bounds alone ptxas settles on 64 registers and spills
+template <int NW>
+__global__ void __maxnreg__(96) donor_frames_large_kernel(const FusedArgs A) {
+    extern __shared__ __align__(128) uint8_t smem[];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const uint32_t c = blockIdx.x / A.groups, grp = blockIdx.x - c * A.groups;
+    const int cr = (int)A.cr, n = 2 * cr;
+    uint8_t *wbase = smem + (size_t)warp * A.warp_smem;
+    uint64_t *wbar = reinterpret_cast<uint64_t *>(wbase);
+    uint32_t *stage = reinterpret_cast<uint32_t *>(wbase + 16);
+    uint32_t *strB = reinterpret_cast<uint32_t *>(wbase + 16 + A.stg_bytes) + 4;      // 4 zero words in front of each string
+    uint32_t *strN = strB + A.strw + 4;
+    uint8_t *outb = reinterpret_cast<uint8_t *>(strN + A.strw);
+    const uint8_t *tmpl = A.tmpl + (size_t)c * A.tmpl_cap;
+
+    const uint32_t tl = A.tmpl_len[c];
+    const uint32_t tl16 = tl & ~15u, sh16 = tl & 15u;                  // tl >= TMPL_HDR: tl16 >= 16
+    const uint32_t s_end = min(A.n_samples, (grp + 1) * A.gs);
+    uint32_t s = grp * A.gs + warp;
+    if (s >= s_end) return;
+    if (lane == 0) mbar_init(wbar, 1);
+    if (lane < 4) { strB[lane - 4] = 0; strN[lane - 4] = 0; }
+    mbar_fence_init();
+    __syncwarp();
+
+    const uint64_t r0 = (uint64_t)c * (uint64_t)cr;
+    const int valid = (int)min((uint64_t)cr, A.n_records - r0);
+    const int alpha = (int)(r0 & 127);
+    const uint32_t g0 = (uint32_t)(r0 >> 7);
+    const uint32_t ngrp = (uint32_t)((r0 + (uint64_t)valid - 1) >> 7) - g0 + 1;
+    const uint32_t stg = ngrp * (kBitGroupWords * 4);
+    const int nwst = 4 * (int)ngrp;
+    if (lane == 0) {
+        mbar_expect_tx(wbar, stg);
+        tma_load_1d(stage, A.bits + (uint64_t)(A.s0 + s) * A.bits_stride + (uint64_t)g0 * kBitGroupWords, stg, wbar);
+    }
+    uint32_t phase = 0;
+    const unsigned long long row_stride = A.slot_off[A.n_chunks], slot = A.slot_off[c];
+    const int strw = (int)A.strw;
+    const int sh = cr & 31, wsh = cr >> 5;
+    constexpr int seg = 32 * NW;                 // block positions per lane and pass
+    const int npass = (n + 32 * seg - 1) / (32 * seg);
+
+    for (; s < s_end; s += kWpcL) {
+        const uint64_t grow = (uint64_t)(A.s0 + s) * A.gt_stride + r0;
+        // ---- 1. bit strings, as in donor_frames_kernel
+        mbar_wait(wbar, phase);
+        phase ^= 1;
+        uint32_t nacc = 0;
+        for (int w = lane; w < nwst; w += 32) {
+            const uint32_t mk = low_mask(alpha + valid - 32 * w) & ~low_mask(alpha - 32 * w);
+            uint32_t *gq = stage + (w >> 2) * kBitGroupWords + (w & 3);
+            if (mk != 0xFFFFFFFFu) { gq[0] &= mk; gq[4] &= mk; gq[8] &= mk; gq[12] &= mk; }
+            nacc |= gq[8] | gq[12];
+        }
+        const bool any_n = __any_sync(0xffffffffu, nacc != 0);
+        __syncwarp();
+        for (int k = lane; k < strw; k += 32) {
+            const int j = k - wsh;
+            uint32_t b = 0, b1lo = 0, b1hi = 0;
+            if (k < nwst) b = stage[(k >> 2) * kBitGroupWords + (k & 3)];
+            if (j >= 1 && j <= nwst) b1lo = stage[((j - 1) >> 2) * kBitGroupWords + 4 + ((j - 1) & 3)];
+            if (j >= 0 && j < nwst) b1hi = stage[(j >> 2) * kBitGroupWords + 4 + (j & 3)];
+            strB[k] = b | __funnelshift_l(b1lo, b1hi, sh);
+            if (any_n) {
+                uint32_t x = 0, x1lo = 0, x1hi = 0;
+                if (k < nwst) x = stage[(k >> 2) * kBitGroupWords + 8 + (k & 3)];
+                if (j >= 1 && j <= nwst) x1lo = stage[((j - 1) >> 2) * kBitGroupWords + 12 + ((j - 1) & 3)];
+                if (j >= 0 && j < nwst) x1hi = stage[(j >> 2) * kBitGroupWords + 12 + (j & 3)];
+                strN[k] = x | __funnelshift_l(x1lo, x1hi, sh);
+            }
+        }
+        fence_proxy_async();
+        __syncwarp();
+        if (lane == 0 && s + kWpcL < s_end) {
+            mbar_expect_tx(wbar, stg);
+            tma_load_1d(stage, A.bits + (uint64_t)(A.s0 + s + kWpcL) * A.bits_stride + (uint64_t)g0 * kBitGroupWords, stg, wbar);
+        }
+        // ---- 2. the tail buffer: zeroed whole, the template's last partial 16 bytes in front
+        if (lane == 0) tma_store_wait_read();           // the previous frame's bulk store has read the buffer
+        __syncwarp();
+        for (uint32_t i = lane; i < A.outcap / 16u; i += 32) reinterpret_cast<uint4 *>(outb)[i] = make_uint4(0, 0, 0, 0);
+        __syncwarp();
+        if ((uint32_t)lane < sh16) outb[lane] = tmpl[tl16 + lane];
+        __syncwarp();
+        uint8_t *seq = outb + sh16;
+
+        int carry_in = 0, pass_base = 0, final_lit = 0;
+        for (int q = 0; q < npass; ++q) {
+            // ---- 3. per-lane parse of one segment of this pass (donor_frames_kernel, step 2)
+            const int x0 = q * 32 * seg + lane * seg;
+            uint32_t Rp[NW], K[NW];
+            int m = 0;
+            const int seglen = max(0, min(seg, n - x0));
+            const int mlim = min(seglen, n - 11 - x0);
+            const int bi = alpha + x0, j0 = bi >> 5, shb = bi & 31;
+            const int ci = bi - cr, jc = ci >> 5, shc = ci & 31;
+            uint32_t Z[NW], C[NW], ZR[NW], S[NW], E[NW];
+#pragma unroll
+            for (int k = 0; k < NW; ++k) {
+                const uint32_t bw = __funnelshift_r(strB[j0 + k], strB[j0 + k + 1], shb);
+                const uint32_t nw = any_n ? __funnelshift_r(strN[j0 + k], strN[j0 + k + 1], shb) : 0u;
+                const uint32_t vm = low_mask(mlim - 32 * k);
+                Z[k] = ~(bw | nw) & vm;
+                C[k] = 0;
+                const uint32_t cm = vm & ~low_mask(cr - x0 - 32 * k);
+                if (cm) {
+                    const uint32_t b0w = __funnelshift_r(strB[jc + k], strB[jc + k + 1], shc);
+                    const uint32_t n0w = any_n ? __funnelshift_r(strN[jc + k], strN[jc + k + 1], shc) : 0u;
+                    C[k] = ~((bw ^ b0w) | nw | n0w) & cm;
+                }
+            }
+            runs_cover<NW, kMinZ>(Z, ZR);
+#pragma unroll
+            for (int k = 0; k < NW; ++k) C[k] &= ~ZR[k];
+            runs_cover<NW, kMinC>(C, K);
+            int matched = 0;
+#pragma unroll
+            for (int k = 0; k < NW; ++k) {
+                const uint32_t zp = k > 0 ? ZR[k - 1] : 0u, zn = k + 1 < NW ? ZR[k + 1] : 0u;
+                const uint32_t cp = k > 0 ? K[k - 1] : 0u, cn = k + 1 < NW ? K[k + 1] : 0u;
+                S[k] = (ZR[k] & ~__funnelshift_l(zp, ZR[k], 1)) | (K[k] & ~__funnelshift_l(cp, K[k], 1));
+                E[k] = (ZR[k] & ~__funnelshift_r(ZR[k], zn, 1)) | (K[k] & ~__funnelshift_r(K[k], cn, 1));
+                m += __popc(S[k]);
+                matched += __popc(ZR[k] | K[k]);
+            }
+            int prev_end = 0, first_lit = 0, n_ext = 0;
+            if (m > 0) {
+                bool f = false;
+#pragma unroll
+                for (int k = NW - 1; k >= 0; --k)
+                    if (!f && E[k]) { prev_end = 32 * k + 32 - __clz(E[k]); f = true; }
+                f = false;
+#pragma unroll
+                for (int k = 0; k < NW; ++k)
+                    if (!f && S[k]) { first_lit = 32 * k + ctz32(S[k]); f = true; }
+                uint32_t e1[NW], w[NW];
+                or_shr<NW>(E, 1, e1);
+                or_shr<NW>(e1, 2, w);
+                or_shr<NW>(w, 4, w);
+                or_shr<NW>(w, 8, w);
+#pragma unroll
+                for (int k = 0; k < NW; ++k) n_ext += __popc(S[k] & ~(w[k] | shr_word<NW>(e1, k, 16)));
+                uint32_t s1[NW], s2[NW], s3[NW];
+                or_shr<NW>(S, 1, s1);
+                or_shr<NW>(s1, 2, s2);
+                or_shr<NW>(s2, 4, s3);
+#pragma unroll
+                for (int k = 0; k < NW; ++k) {
+                    uint32_t ek = E[k];
+                    if (32 * k <= prev_end - 1 && prev_end - 1 < 32 * k + 32) ek &= ~(1u << ((prev_end - 1) & 31));
+                    const uint32_t near = shr_word<NW>(s3, k, 1) | shr_word<NW>(s2, k, 9) | shr_word<NW>(s1, k, 13) | shr_word<NW>(S, k, 15);
+                    n_ext += __popc(ek & ~near);
+                }
+            }
+            const int trail = seglen - prev_end;
+#pragma unroll
+            for (int k = 0; k < NW; ++k) Rp[k] = (ZR[k] | K[k]) & ~E[k];
+
+            // ---- 4. carry trailing literals forward (lane 0 takes what the previous pass left); scan: output offsets
+            int val = trail + (lane == 0 && m == 0 ? carry_in : 0), flag = m > 0;
+#pragma unroll
+            for (int d = 1; d < 32; d <<= 1) {
+                const int v2 = __shfl_up_sync(0xffffffffu, val, d), f2 = __shfl_up_sync(0xffffffffu, flag, d);
+                if (lane >= d && !flag) { val += v2; flag = f2; }
+            }
+            int carry = __shfl_up_sync(0xffffffffu, val, 1);
+            if (lane == 0) carry = carry_in;
+            carry_in = __shfl_sync(0xffffffffu, val, 31);
+            const bool last = q == npass - 1;
+            if (last) final_lit = carry_in;
+            const int mysize = m > 0 ? 3 * m + (prev_end - matched) + carry + lit_ext(first_lit + carry) + n_ext : 0;
+            int inc = mysize;
+#pragma unroll
+            for (int d = 1; d < 32; d <<= 1) {
+                const int t1 = __shfl_up_sync(0xffffffffu, inc, d);
+                if (lane >= d) inc += t1;
+            }
+            const int total = __shfl_sync(0xffffffffu, inc, 31);
+            const int out_base = pass_base + inc - mysize;
+            pass_base += total;
+
+            // ---- 5. emission (donor_frames_kernel, step 5); lane 31 of the last pass opens the closing literals
+            uint32_t waddr = smem_u32(seq) + (uint32_t)out_base;
+            uint32_t fill = waddr & 7u;
+            waddr &= ~7u;
+            const uint32_t faddr = waddr;
+            uint64_t acc = 0, fw = 0;
+            uint32_t first = 1;
+            auto put = [&](uint64_t v, uint32_t nb) {
+                const uint32_t sh = 8u * fill;
+                acc |= v << sh;
+                const uint64_t spill = (v >> 1) >> (63u - sh);
+                fill += nb;
+                const bool full = fill >= 8u;
+                if (full && !first) sts64(waddr, acc);
+                fw = (full && first) ? acc : fw;
+                first = full ? 0u : first;
+                waddr += full ? 8u : 0u;
+                acc = full ? spill : acc;
+                fill -= full ? 8u : 0u;
+            };
+            auto lit8 = [&](int x, int nb) -> uint64_t {
+                const int G = alpha + x;
+                const uint32_t keep = (1u << nb) - 1u;
+                const uint32_t bits = __funnelshift_r(strB[G >> 5], strB[(G >> 5) + 1], G) & keep;
+                uint64_t v = (uint64_t)spread4(bits) | ((uint64_t)spread4(bits >> 4) << 32);
+                if (any_n) {
+                    uint32_t nb8 = __funnelshift_r(strN[G >> 5], strN[(G >> 5) + 1], G) & keep;
+#pragma unroll 1
+                    while (nb8) {
+                        const int i = ctz32(nb8);
+                        nb8 &= nb8 - 1;
+                        const int xx = x + i;
+                        const uint64_t byte = (uint8_t)(xx < cr ? A.gt0 : A.gt1)[grow + (xx < cr ? xx : xx - cr)];
+                        v = (v & ~(0xFFull << (8 * i))) | (byte << (8 * i));
+                    }
+                }
+                return v;
+            };
+            int pos = x0 - carry;
+            int base = x0;
+            int left = m;
+            uint32_t fin = lane == 31 && last ? 1u : 0u;
+            int litrem = 0, cur_ml = 0;
+            uint32_t cur_off = 0, pend = 0;
+            while ((left | litrem | (int)pend | (int)fin) != 0) {
+                uint64_t v = 0;
+                uint32_t nb = 0;
+                if ((litrem | (int)pend) == 0) {
+                    int lit;
+                    uint32_t tok;
+                    if (left > 0) {
+#pragma unroll
+                        for (int r = 0; r + 1 < NW; ++r) {
+                            const bool z = Rp[0] == 0u;
+#pragma unroll
+                            for (int k = 0; k + 1 < NW; ++k) { Rp[k] = z ? Rp[k + 1] : Rp[k]; K[k] = z ? K[k + 1] : K[k]; }
+                            Rp[NW - 1] = z ? 0u : Rp[NW - 1];
+                            base += z ? 32 : 0;
+                        }
+                        const uint32_t low = Rp[0] & (0u - Rp[0]);
+                        const int ts = __popc(low - 1u);
+                        const bool is_k = (K[0] & low) != 0u;
+                        uint64_t cy = low;
+                        int ml = 1;
+#pragma unroll
+                        for (int k = 0; k < NW; ++k) {
+                            cy += Rp[k];
+                            const uint32_t t = (uint32_t)cy;
+                            cy >>= 32;
+                            ml += __popc(Rp[k] & ~t);
+                            Rp[k] &= t;
+                        }
+                        lit = base + ts - pos;
+                        cur_ml = ml;
+                        cur_off = is_k ? (uint32_t)cr : 2u * (uint32_t)cr;
+                        pend = 1;
+                        --left;
+                        tok = (uint32_t)((min(lit, 15) << 4) | min(ml - 4, 15));
+                    } else {
+                        lit = final_lit;
+                        fin = 0;
+                        tok = (uint32_t)(min(lit, 15) << 4);
+                    }
+                    v = tok; nb = 1;
+                    if (lit >= 15) {
+                        int rem = lit - 15;
+#pragma unroll 1
+                        while (rem >= 255) { put(v, nb); v = 255u; nb = 1; rem -= 255; }
+                        v |= (uint64_t)(uint32_t)rem << (8u * nb);
+                        ++nb;
+                    }
+                    litrem = pend ? lit : 0;
+                }
+                const int take = min(litrem, 8 - (int)nb);
+                if (take > 0) {
+                    v |= lit8(pos, take) << (8u * nb);
+                    nb += (uint32_t)take; pos += take; litrem -= take;
+                }
+                if (pend != 0 && litrem == 0) {
+                    const uint32_t ob = cur_ml >= 19 ? 3u : 2u;
+                    if (nb + ob <= 8u) {
+                        v |= (uint64_t)(cur_off | (cur_ml >= 19 ? (uint32_t)(cur_ml - 19) << 16 : 0u)) << (8u * nb);
+                        nb += ob; pend = 0; pos += cur_ml;
+                    }
+                }
+                put(v, nb);
+            }
+            {
+                const uint64_t fv = first ? acc : fw;
+                if ((uint32_t)fv) sts_or32(faddr, (uint32_t)fv);
+                if ((uint32_t)(fv >> 32)) sts_or32(faddr + 4u, (uint32_t)(fv >> 32));
+                if (!first) {
+                    if ((uint32_t)acc) sts_or32(waddr, (uint32_t)acc);
+                    if ((uint32_t)(acc >> 32)) sts_or32(waddr + 4u, (uint32_t)(acc >> 32));
+                }
+            }
+        }
+        const int dlen = pass_base + 1 + lit_ext(final_lit) + final_lit;
+        __syncwarp();
+        {   // the block's closing literals: one byte per lane and step
+            uint8_t *fdst = seq + (dlen - final_lit);
+            const int fx = n - final_lit;
+            for (int i = lane; i < final_lit; i += 32) {
+                const int x = fx + i, G = alpha + x;
+                uint32_t byte = (strB[G >> 5] >> (G & 31)) & 1u;
+                if (any_n && ((strN[G >> 5] >> (G & 31)) & 1u))
+                    byte = (uint8_t)(x < cr ? A.gt0 : A.gt1)[grow + (x < cr ? x : x - cr)];
+                fdst[i] = (uint8_t)byte;
+            }
+        }
+        // ---- 6. the frame leaves: header + template body from global memory (size fields filled in), own tail by a
+        //         TMA bulk store.  A size field that lies behind tl16 sits in the tail buffer's first bytes.
+        const uint32_t flen = tl + (uint32_t)dlen;
+        const uint32_t lz = flen - TMPL_HDR;
+        if (lane == 0 && tl16 < 24) for (int i = 0; i < 4; ++i) outb[20 - tl16 + i] = (uint8_t)(lz >> (8 * i));
+        fence_proxy_async();
+        __syncwarp();
+        uint8_t *dst = A.frames + (unsigned long long)(s) * row_stride + slot;
+        for (uint32_t k = lane; k < tl16 / 16u; k += 32) {
+            uint4 v = __ldg(reinterpret_cast<const uint4 *>(tmpl) + k);
+            if (k == 0) v.w = flen;
+            if (k == 1) v.y = lz;
+            stg_stream(reinterpret_cast<uint4 *>(dst) + k, v);
+        }
+        if (lane == 0) {
+            tma_store_1d(dst + tl16, outb, (sh16 + (uint32_t)dlen + 15u) & ~15u);
+            tma_store_commit();
+            A.size[(uint64_t)s * A.n_chunks + c] = flen;
+        }
+    }
+    if (lane == 0) tma_store_wait_read();    // shared memory must outlive the bulk stores that read it
+}
+
 __global__ void __launch_bounds__(256) sum_sizes_kernel(const uint32_t *__restrict__ size, uint64_t n, unsigned long long *__restrict__ total) {
     unsigned long long acc = 0;
     for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (uint64_t)gridDim.x * blockDim.x) acc += size[i];
@@ -905,6 +1363,9 @@ struct hb_frames {
     size_t smem_site = 0;
     FusedArgs fa;                            // geometry of the fused kernel
     int nw = 1;
+    bool large = false;                      // cr > kSmallChunkMax: kernels 4a-L / 4b-L
+    uint8_t *d_site_scratch = nullptr;       // 4a-L: site_large_scratch(cr) bytes per CTA
+    uint32_t site_ctas = 0;                  // 4a-L: CTAs the scratch was made for
     uint8_t *d_tmpl = nullptr, *d_frames = nullptr;
     uint32_t *d_tmpl_len = nullptr, *d_size = nullptr;
     uint64_t *d_slot_off = nullptr;
@@ -987,8 +1448,12 @@ static int frames_site_pass(hb_frames *f, hb_parse *p, bool early) {
         CUF(cudaStreamWaitEvent(f->side, f->ev_sites, 0));
     }
     CUF(cudaEventRecord(early ? f->ev_side0 : f->ev[0], st));
-    raise_smem_limit(reinterpret_cast<const void *>(site_template_kernel));
-    site_template_kernel<<<(unsigned)f->n_chunks, kSiteSegs * 32, f->smem_site, st>>>(sa);
+    if (f->large) {
+        site_template_large_kernel<<<(unsigned)std::min<uint64_t>(f->n_chunks, f->site_ctas), kSiteSegs * 32, f->smem_site, st>>>(sa, f->d_site_scratch);
+    } else {
+        raise_smem_limit(reinterpret_cast<const void *>(site_template_kernel));
+        site_template_kernel<<<(unsigned)f->n_chunks, kSiteSegs * 32, f->smem_site, st>>>(sa);
+    }
     count_launch();
     CUF(cudaEventRecord(early ? f->ev_tmpl : f->ev[1], st));
     f->early_site = early;
@@ -1073,14 +1538,17 @@ static int frames_prepare(hb_frames *f, hb_parse *p, bool early) {
     {
         uint32_t mx = 0;
         for (uint64_t c = 0; c < f->n_chunks; ++c) mx = std::max(mx, f->h_tmpl_len[c]);
-        fa.tmpl_smem = (mx + 15u) & ~15u;
-        fa.gs = kWpc * kFramesPerWarp;
+        fa.tmpl_smem = f->large ? 0u : (mx + 15u) & ~15u;            // 4b-L reads the template from global memory
+        fa.gs = (f->large ? kWpcL : kWpc) * kFramesPerWarp;
         fa.groups = (f->n_samples + fa.gs - 1) / fa.gs;
-        if (16 + (size_t)fa.tmpl_smem + (size_t)kWpc * fa.warp_smem > 227 * 1024)
+        if (!f->large && 16 + (size_t)fa.tmpl_smem + (size_t)kWpc * fa.warp_smem > 227 * 1024)
             return api_fail(HB_ERR_ARG, "chunk too large for the allele encoder (template + tail buffers exceed shared memory)");
     }
     const uint64_t n_ctas = f->n_chunks * fa.groups;
-    switch (f->nw) {
+    if (f->large) {
+        raise_smem_limit(reinterpret_cast<const void *>(donor_frames_large_kernel<kLargeNW>));
+        donor_frames_large_kernel<kLargeNW><<<(unsigned)n_ctas, kWpcL * 32, (size_t)kWpcL * fa.warp_smem, f->stream>>>(fa);
+    } else switch (f->nw) {
         case 1: launch_donor_frames<1>(fa, n_ctas, f->stream); break;
         case 2: launch_donor_frames<2>(fa, n_ctas, f->stream); break;
         case 3: launch_donor_frames<3>(fa, n_ctas, f->stream); break;
@@ -1155,7 +1623,7 @@ void hb_frames_free(hb_frames *f) {
         if (small->cap < f->frames_cap) { std::swap(small->p, f->d_frames); std::swap(small->cap, f->frames_cap); }
     }
     dev_pool_free(f->d_tmpl); cudaFree(f->d_frames); dev_pool_free(f->d_tmpl_len); dev_pool_free(f->d_size);
-    dev_pool_free(f->d_slot_off); dev_pool_free(f->d_totals);
+    dev_pool_free(f->d_slot_off); dev_pool_free(f->d_totals); dev_pool_free(f->d_site_scratch);
     for (auto &x : f->ev) if (x) cudaEventDestroy(x);
     if (f->ev_sites) cudaEventDestroy(f->ev_sites);
     if (f->ev_tmpl) cudaEventDestroy(f->ev_tmpl);
@@ -1184,20 +1652,32 @@ int hb_compress_sample_range(hb_parse *p, uint64_t chunk_records, uint32_t s0, u
     f->cr_explicit = chunk_records != 0;
     f->n_chunks = n ? (n + f->cr - 1) / f->cr : 0;
     if (!f->n_chunks || !f->n_samples) { f->n_chunks = n ? f->n_chunks : 0; *out = f; return HB_OK; }
-    if (f->cr > 2730) { hb_frames_free(f); return api_fail(HB_ERR_ARG, "chunk_records too large (at most 2730: the site encoder indexes 24*chunk_records+1 positions with 16 bits)"); }
+    if (f->cr > kMaxChunkRecords) {
+        hb_frames_free(f);
+        return api_fail(HB_ERR_ARG, "chunk_records too large (at most 7,489: a stored chunk must be ONE Blosc block, and c-blosc 1.x "
+                                    "cuts blocks of 262,115 bytes = 7,489 records of 35 bytes at clevel 5 with LZ4HC)");
+    }
     const uint32_t cr = (uint32_t)f->cr;
     const uint32_t n_site = 33u * cr, n_gt = 2u * cr;
     auto bound = [](uint32_t x) { return x + x / 255 + 64; };
     f->tmpl_cap = (TMPL_HDR + bound(n_site) + 15) & ~15u;
-    f->smem_site = 16 + ((n_site + 19) & ~15u) + ((site_seg_cap(24 * cr + 1) + kSiteSegs * 48 + 15) & ~15u) +
-                   ((size_t)kSiteSegs << kSiteHashLog) * 2;
-    if (f->smem_site > 220 * 1024) { hb_frames_free(f); return api_fail(HB_ERR_ARG, "chunk too large for the site encoder (33*chunk_records must fit shared memory)"); }
-    uint32_t seg = (n_gt + 31) / 32;
-    f->nw = (int)((seg + 31) / 32);
-    if (f->nw > 1 && 1024u * (uint32_t)(f->nw - 1) + kSlack >= n_gt) { f->nw -= 1; seg = 32u * (uint32_t)f->nw; }
+    f->large = cr > kSmallChunkMax;
     FusedArgs &fa = f->fa;
-    fa.seg = seg;
-    fa.strw = (((127 + 2 * cr) >> 5) + (uint32_t)f->nw + 3 + 3) & ~3u;   // both planes from bit alpha <= 127 on, + look-ahead words
+    if (f->large) {                          // kernels 4a-L / 4b-L: hash tables in shared memory, 4b-L in passes
+        f->smem_site = ((size_t)kSiteSegs << kSiteHashLog) * 2;
+        f->nw = kLargeNW;
+        fa.seg = 32u * kLargeNW;
+        const uint32_t span = 32u * fa.seg, npass = (n_gt + span - 1) / span;
+        fa.strw = (((127 + npass * span) >> 5) + (uint32_t)f->nw + 3 + 3) & ~3u;   // every pass's words + look-ahead
+    } else {
+        f->smem_site = 16 + ((n_site + 19) & ~15u) + ((site_seg_cap(24 * cr + 1) + kSiteSegs * 48 + 15) & ~15u) +
+                       ((size_t)kSiteSegs << kSiteHashLog) * 2;
+        uint32_t seg = (n_gt + 31) / 32;
+        f->nw = (int)((seg + 31) / 32);
+        if (f->nw > 1 && 1024u * (uint32_t)(f->nw - 1) + kSlack >= n_gt) { f->nw -= 1; seg = 32u * (uint32_t)f->nw; }
+        fa.seg = seg;
+        fa.strw = (((127 + 2 * cr) >> 5) + (uint32_t)f->nw + 3 + 3) & ~3u;   // both planes from bit alpha <= 127 on, + look-ahead words
+    }
     fa.stg_bytes = (((127 + cr - 1) >> 7) + 1) * (kBitGroupWords * 4);   // 128-row groups a chunk's rows can touch
     fa.outcap = (16 + n_gt + n_gt / 255 + 24 + 15) & ~15u;
     fa.warp_smem = 16 + fa.stg_bytes + 2 * (16 + 4 * fa.strw) + fa.outcap;
@@ -1212,6 +1692,12 @@ int hb_compress_sample_range(hb_parse *p, uint64_t chunk_records, uint32_t s0, u
     ck(dev_pool_alloc((void **)&f->d_size, n_frames * 4));
     ck(dev_pool_alloc((void **)&f->d_slot_off, (f->chunk_cap + 1) * 8));
     ck(dev_pool_alloc((void **)&f->d_totals, 8));
+    if (f->large) {                          // 4a-L scratch: two CTAs per SM at most, each loops over its chunks
+        int sms = 0;
+        ck(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, f->device));
+        f->site_ctas = (uint32_t)std::min<uint64_t>(f->chunk_cap, 2ull * (uint64_t)std::max(1, sms));
+        ck(dev_pool_alloc((void **)&f->d_site_scratch, (uint64_t)f->site_ctas * site_large_scratch(cr)));
+    }
     for (auto &x : f->ev) ck(cudaEventCreate(&x));
     {   // highest priority: its few long CTAs must get SM slots while the decoder's many short ones stream through
         int lo = 0, hi = 0;
@@ -1926,11 +2412,163 @@ __global__ void __launch_bounds__(128) decode_columns_kernel(const DecodeColsArg
     if (lane == 0) a.status[wid] = err;
 }
 
+// ---------------------------------------------------------------------------------------------
+// Kernel 6-L: decode_columns_kernel for single-block chunks whose 35 * cr bytes do not fit a warp's shared memory (up to
+// kMaxChunkRecords).  One warp (= one CTA) per chunk.  An LZ4 offset is at most 65,535, so the decoded block streams
+// through a 64 KiB history ring in shared memory and every byte of the planes the columns need (5-13, 23, 33, 34) goes
+// straight to its column.  The stream is first walked once without copying -- the checks of warp_lz4_decode_smem are
+// all structural -- so a chunk that fails writes no row, as in kernel 6.  Stored-raw, memcpyed and zero-run chunks are
+// read in place.  The header checks and status codes are kernel 6's.
+// ---------------------------------------------------------------------------------------------
+constexpr uint32_t kHistRing = 1u << 16;
+
+// The checks of warp_lz4_decode_smem without the copies: true iff the block decodes to exactly cap bytes.
+__device__ bool lz4_block_valid(const uint8_t *__restrict__ src, uint32_t n, uint32_t cap) {
+    uint32_t ip = 0, op = 0;
+    if (n == 0) return false;
+    for (;;) {
+        if (ip >= n) return false;
+        const uint32_t tok = src[ip++];
+        uint32_t ll = tok >> 4;
+        if (ll == 15) { uint32_t b; do { if (ip >= n) return false; b = src[ip++]; ll += b; } while (b == 255 && ll <= cap); }
+        if (ll > n - ip || ll > cap - op) return false;
+        ip += ll; op += ll;
+        if (ip == n) break;
+        if (ip + 2 > n) return false;
+        const uint32_t off = src[ip] | ((uint32_t)src[ip + 1] << 8);
+        ip += 2;
+        if (off == 0 || off > op) return false;
+        uint32_t ml = tok & 15;
+        if (ml == 15) { uint32_t b; do { if (ip >= n) return false; b = src[ip++]; ml += b; } while (b == 255 && ml <= cap); }
+        ml += 4;
+        if (ml > cap - op) return false;
+        op += ml;
+    }
+    return op == cap;
+}
+
+// byte f of record r -> its column (f outside the six columns: nothing)
+__device__ __forceinline__ void put_column_byte(const DecodeColsArgs &a, uint64_t row, uint32_t f, uint8_t v) {
+    if (f >= 5 && f < 9) { if (a.start) reinterpret_cast<uint8_t *>(a.start + row)[f - 5] = v; }
+    else if (f >= 9 && f < 13) { if (a.stop) reinterpret_cast<uint8_t *>(a.stop + row)[f - 9] = v; }
+    else if (f == 13) { if (a.ref) a.ref[row] = v; }
+    else if (f == 23) { if (a.alt) a.alt[row] = v; }
+    else if (f == 33) { if (a.p1) a.p1[row] = (int8_t)v; }
+    else if (f == 34) { if (a.p2) a.p2[row] = (int8_t)v; }
+}
+
+__global__ void __launch_bounds__(32) decode_columns_large_kernel(const DecodeColsArgs a) {
+    extern __shared__ __align__(16) uint8_t ring[];
+    const int lane = threadIdx.x;
+    const uint64_t wid = blockIdx.x;
+    const uint8_t *c = a.frames + a.off[wid];
+    const uint32_t flen = a.len[wid];
+    const uint32_t cr = a.cr, nbytes = 35u * cr;
+    int err = 0;
+    uint32_t flags = 0, bs = 0, ccb = 0, hdr = 16;
+    bool ext = false, shuffle = false;
+    if (flen < 16) err = 1;
+    if (!err) {
+        flags = c[2];
+        const uint32_t cn = ld_le32(c + 4);
+        bs = ld_le32(c + 8); ccb = ld_le32(c + 12);
+        ext = (flags & 1) && (flags & 4);
+        hdr = ext ? 32 : 16;
+        shuffle = !ext && (flags & 1);
+        if (c[0] < 2 || c[0] > 5 || (!ext && (c[0] != 2 || (flags & 0x08)))) err = 2;
+        else if (c[3] != 35 || cn != nbytes || ccb > flen || ccb < hdr) err = 4;
+        else if (!(flags & 2) && (bs != cn || (ext && !(flags & 0x10)))) err = 11;
+    }
+    if (!err && ext) {
+        for (int i = 0; i < 6; ++i) { if (c[16 + i] == 1) shuffle = true; else if (c[16 + i] != 0) err = 3; }
+        if ((c[31] >> 4) & 7) err = 6;
+    }
+    const uint8_t *src = nullptr;                     // the block's bytes in place (memcpyed / stored raw); null + lz: LZ4
+    bool zero = false, lz = false;
+    uint32_t cs = 0;
+    if (!err && (flags & 2)) {                        // memcpyed: record-major
+        if ((uint64_t)hdr + nbytes > ccb) err = 7;
+        else src = c + hdr;
+        shuffle = false;
+    } else if (!err) {
+        if ((flags >> 5) != 1 || (!ext && c[1] != 1)) err = 5;
+        const uint64_t data0 = (uint64_t)hdr + 4;
+        uint64_t ip = 0;
+        if (!err && data0 + 4 > ccb) err = 7;
+        if (!err) { ip = ld_le32(c + hdr); if (ip < data0 || ip + 4 > ccb) err = 7; }
+        if (!err) {
+            const int32_t s32 = (int32_t)ld_le32(c + ip);
+            ip += 4;
+            cs = (uint32_t)s32;
+            if (s32 == 0 && ext) zero = true;
+            else if (s32 <= 0 || ip + cs > ccb) err = 8;
+            else if (cs == nbytes) src = c + ip;
+            else if (!lz4_block_valid(c + ip, cs, nbytes)) err = 9;
+            else { src = c + ip; lz = true; }
+        }
+    }
+    if (lane == 0) a.status[wid] = err;
+    if (err) return;
+    const uint64_t row0 = a.row[wid];
+    if (!lz) {                                        // in place, one record per lane and step (kernel 6's loop)
+        for (uint32_t r = lane; r < cr; r += 32) {
+            auto B = [&](uint32_t f) -> uint32_t { return zero ? 0u : shuffle ? src[f * cr + r] : src[r * 35u + f]; };
+            if (a.start) a.start[row0 + r] = B(5) | (B(6) << 8) | (B(7) << 16) | (B(8) << 24);
+            if (a.stop) a.stop[row0 + r] = B(9) | (B(10) << 8) | (B(11) << 16) | (B(12) << 24);
+            if (a.ref) a.ref[row0 + r] = (uint8_t)B(13);
+            if (a.alt) a.alt[row0 + r] = (uint8_t)B(23);
+            if (a.p1) a.p1[row0 + r] = (int8_t)B(33);
+            if (a.p2) a.p2[row0 + r] = (int8_t)B(34);
+        }
+        return;
+    }
+    // block position q -> (plane, record) when shuffled, (record, field) otherwise: q / d by a multiply-high, exact for
+    // q < 2^18 and d < 2^13
+    const uint32_t d = shuffle ? cr : 35u, magic = 0xFFFFFFFFu / d + 1u;
+    auto put = [&](uint32_t q, uint8_t v) {
+        const uint32_t hi = __umulhi(q, magic), lo = q - hi * d;
+        if (shuffle) put_column_byte(a, row0 + lo, hi, v);
+        else put_column_byte(a, row0 + hi, lo, v);
+    };
+    uint32_t ip = 0, op = 0;
+    for (;;) {                                        // the stream is valid: no bounds checks
+        const uint32_t tok = src[ip++];
+        uint32_t ll = tok >> 4;
+        if (ll == 15) { uint32_t b; do { b = src[ip++]; ll += b; } while (b == 255); }
+        for (uint32_t i = lane; i < ll; i += 32) {
+            const uint8_t v = src[ip + i];
+            ring[(op + i) & (kHistRing - 1)] = v;
+            put(op + i, v);
+        }
+        ip += ll; op += ll;
+        if (ip == cs) break;
+        const uint32_t off = src[ip] | ((uint32_t)src[ip + 1] << 8);
+        ip += 2;
+        uint32_t ml = tok & 15;
+        if (ml == 15) { uint32_t b; do { b = src[ip++]; ml += b; } while (b == 255); }
+        ml += 4;
+        __syncwarp();
+        // step b copies positions [op + b, op + b + 32): position op + i repeats position op + i - k * off, k >= 1 the
+        // smallest with a source written before this step (k = 1 unless off < 32).  Such a source is at most 65,535
+        // bytes back, so its ring slot still holds it; reads and writes of a step are split by a barrier.
+        for (uint32_t b = 0; b < ml; b += 32) {
+            const uint32_t i = b + lane;
+            uint8_t v = 0;
+            if (i < ml) v = ring[(op + i - off * ((i - b + off) / off)) & (kHistRing - 1)];
+            __syncwarp();
+            if (i < ml) { ring[(op + i) & (kHistRing - 1)] = v; put(op + i, v); }
+            __syncwarp();
+        }
+        op += ml;
+    }
+}
+
 }  // namespace hb
 
-extern "C" int hb_decode_columns_device(const uint8_t *d_frames, const uint64_t *d_off, const uint32_t *d_len, const uint64_t *d_row,
-                                        uint64_t n_chunks, uint32_t chunk_records, uint32_t *d_start, uint32_t *d_stop, uint8_t *d_ref,
-                                        uint8_t *d_alt, int8_t *d_p1, int8_t *d_p2, int *d_status, void *stream) {
+// kernel 6 where a chunk fits a warp's shared memory; above that kernel 6-L when `large` allows it
+static int decode_columns(const uint8_t *d_frames, const uint64_t *d_off, const uint32_t *d_len, const uint64_t *d_row,
+                          uint64_t n_chunks, uint32_t chunk_records, uint32_t *d_start, uint32_t *d_stop, uint8_t *d_ref,
+                          uint8_t *d_alt, int8_t *d_p1, int8_t *d_p2, int *d_status, void *stream, bool large) {
     if (!n_chunks) return HB_OK;
     if (!d_off || !d_len || !d_row || !d_status || !chunk_records) return api_fail(HB_ERR_ARG, "bad argument");
     const uint64_t nbytes = 35ull * chunk_records;
@@ -1939,7 +2577,20 @@ extern "C" int hb_decode_columns_device(const uint8_t *d_frames, const uint64_t 
     if (cudaGetDevice(&dev) != cudaSuccess) return api_fail(HB_ERR_CUDA, "no CUDA device: libhaplo_b200 has no CPU fallback");
     cudaDeviceGetAttribute(&smem_max, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
     smem_max -= 1024;
-    if (nbytes > (uint64_t)smem_max) return api_fail(HB_ERR_ARG, "chunk too large for the device-side decoder (use hb_decode_frames)");
+    if (nbytes > (uint64_t)smem_max) {
+        if (!large)
+            return api_fail(HB_ERR_ARG, "chunk too large for the device-side decoder (hb_decode_columns_device_large reads up to "
+                                        "7,489 records, hb_decode_frames any chunk)");
+        if (chunk_records > kMaxChunkRecords)
+            return api_fail(HB_ERR_ARG, "chunk too large for the device-side decoder (at most 7,489 records: ONE Blosc block of "
+                                        "c-blosc 1.x at typesize 35; use hb_decode_frames)");
+        DecodeColsArgs a{d_frames, d_off, d_len, d_row, n_chunks, chunk_records, d_start, d_stop, d_ref, d_alt, d_p1, d_p2, d_status, 0};
+        cudaFuncSetAttribute(decode_columns_large_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kHistRing);
+        decode_columns_large_kernel<<<(unsigned)n_chunks, 32, kHistRing, (cudaStream_t)stream>>>(a);
+        count_launch();
+        if (cudaGetLastError() != cudaSuccess) return api_fail(HB_ERR_CUDA, "decode_columns_large_kernel launch failed");
+        return HB_OK;
+    }
     const int warps = (int)std::max<uint64_t>(1, std::min<uint64_t>(4, (uint64_t)smem_max / warp_smem));
     DecodeColsArgs a{d_frames, d_off, d_len, d_row, n_chunks, chunk_records, d_start, d_stop, d_ref, d_alt, d_p1, d_p2, d_status, warp_smem};
     cudaFuncSetAttribute(decode_columns_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max);
@@ -1947,6 +2598,21 @@ extern "C" int hb_decode_columns_device(const uint8_t *d_frames, const uint64_t 
     count_launch();
     if (cudaGetLastError() != cudaSuccess) return api_fail(HB_ERR_CUDA, "decode_columns_kernel launch failed");
     return HB_OK;
+}
+
+extern "C" int hb_decode_columns_device(const uint8_t *d_frames, const uint64_t *d_off, const uint32_t *d_len, const uint64_t *d_row,
+                                        uint64_t n_chunks, uint32_t chunk_records, uint32_t *d_start, uint32_t *d_stop, uint8_t *d_ref,
+                                        uint8_t *d_alt, int8_t *d_p1, int8_t *d_p2, int *d_status, void *stream) {
+    return decode_columns(d_frames, d_off, d_len, d_row, n_chunks, chunk_records, d_start, d_stop, d_ref, d_alt, d_p1, d_p2, d_status,
+                          stream, false);
+}
+
+extern "C" int hb_decode_columns_device_large(const uint8_t *d_frames, const uint64_t *d_off, const uint32_t *d_len,
+                                              const uint64_t *d_row, uint64_t n_chunks, uint32_t chunk_records, uint32_t *d_start,
+                                              uint32_t *d_stop, uint8_t *d_ref, uint8_t *d_alt, int8_t *d_p1, int8_t *d_p2, int *d_status,
+                                              void *stream) {
+    return decode_columns(d_frames, d_off, d_len, d_row, n_chunks, chunk_records, d_start, d_stop, d_ref, d_alt, d_p1, d_p2, d_status,
+                          stream, true);
 }
 
 extern "C" int hb_decode_frames(const uint8_t *frames, const uint64_t *offsets, uint64_t n_frames,

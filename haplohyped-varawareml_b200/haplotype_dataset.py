@@ -163,7 +163,9 @@ class GenotypeStore:
         got = self._reader.stored_chunks(donor, chrom) if (self._reader is not None and hasattr(self._reader, "stored_chunks")) else None
         if got is not None:
             n, cr, dtype, chunks = got
-            if dtype.itemsize == 35 and n > 0 and 35 * cr <= 200 * 1024:
+            # up to 7,489 records a chunk of the reference's writer is ONE Blosc block, which the device decoder reads;
+            # chunks with several blocks make the first decode fail and the dataset is then read whole (_chunk_first)
+            if dtype.itemsize == 35 and n > 0 and cr <= 7489:
                 sizes = np.array([len(c) for c in chunks], np.uint32)
                 offs = np.zeros(len(chunks), np.uint64)
                 offs[1:] = np.cumsum((sizes[:-1].astype(np.uint64) + 15) // 16 * 16)
@@ -190,7 +192,8 @@ class GenotypeStore:
         return self._first[key]
 
     def _decode(self, st, chunk_ids, rows, start=None, ref=None, alt=None, p1=None, p2=None, frames=None, offs=None, lens=None):
-        """hb_decode_columns_device on chunks `chunk_ids` of one stored dataset (or on pre-built device lists)."""
+        """hb_decode_columns_device_large (every single-block chunk size) on chunks `chunk_ids` of one stored dataset (or on
+        pre-built device lists)."""
         dev = self.device
         n = len(chunk_ids)
         if offs is None:
@@ -201,7 +204,7 @@ class GenotypeStore:
         rows_t = torch.from_numpy(np.asarray(rows, np.uint64).view(np.int64)).to(dev)
         status = torch.empty(n, dtype=torch.int32, device=dev)
         ptr = lambda t: t.data_ptr() if t is not None else None
-        capi.check(capi.lib().hb_decode_columns_device(frames, offs.data_ptr(), lens.data_ptr(), rows_t.data_ptr(), n, st.cr,
+        capi.check(capi.lib().hb_decode_columns_device_large(frames, offs.data_ptr(), lens.data_ptr(), rows_t.data_ptr(), n, st.cr,
                                                        ptr(start), None, ptr(ref), ptr(alt), ptr(p1), ptr(p2), status.data_ptr(),
                                                        torch.cuda.current_stream(dev).cuda_stream))
         return status

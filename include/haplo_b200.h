@@ -206,7 +206,10 @@ typedef struct hb_frames_info {
     uint64_t site_lz4_bytes;        /* LZ4 bytes of the site planes, summed over chunks (shared by every sample) */
 } hb_frames_info;
 
-/* chunk_records = 0 -> h5py's auto-chunk heuristic for a 1-D dataset of 35-byte items (at most 2730).
+/* chunk_records = 0 -> h5py's auto-chunk heuristic for a 1-D dataset of 35-byte items (hb_guess_chunk_records; it is not
+ * clamped, and stays <= 7,489 for every dataset below ~122.7 M records).  chunk_records may be at most 7,489: up to there
+ * a stored chunk is ONE Blosc block with ONE LZ4 stream, as c-blosc 1.x cuts blocks of 262,115 bytes at typesize 35,
+ * clevel 5, LZ4HC; larger values fail with HB_ERR_ARG.  Chunks above 2,730 records take kernels 4a-L / 4b-L.
  * All frames of all samples are produced in one pass and stay in HBM as ONE buffer, laid out
  * [sample][chunk] with every frame starting on a 16-byte boundary: a sample's dataset is one contiguous
  * byte range, and the whole buffer can be written to the HDF5 file with one write. */
@@ -268,11 +271,20 @@ int hb_decode_frames(const uint8_t *frames, const uint64_t *offsets, uint64_t n_
  * d_off[i] is the chunk's device address itself, so one call serves chunks of many datasets -- are decoded into
  * record COLUMNS: the chunk_records records of chunk i go to rows [d_row[i], d_row[i] + chunk_records) of d_start /
  * d_stop (uint32), d_ref / d_alt (first byte of the S10 field), d_p1 / d_p2 (int8); any column may be NULL.
+ * 35 * chunk_records must fit a warp's shared memory (kernel 6: 6,612 records on a B200); larger values fail with
+ * HB_ERR_ARG.
  * d_status[i] = 0 or a non-zero code (corrupt or unsupported chunk; 11 = several Blosc blocks per chunk, which
  * hb_decode_frames reads).  Asynchronous on `stream` (the current device's); all pointers are device pointers. */
 int hb_decode_columns_device(const uint8_t *d_frames, const uint64_t *d_off, const uint32_t *d_len, const uint64_t *d_row,
                              uint64_t n_chunks, uint32_t chunk_records, uint32_t *d_start, uint32_t *d_stop, uint8_t *d_ref,
                              uint8_t *d_alt, int8_t *d_p1, int8_t *d_p2, int *d_status, void *stream);
+/* The same call for every single-block chunk size, chunk_records <= 7,489 (one c-blosc 1.x block at typesize 35): kernel 6
+ * where a chunk fits a warp's shared memory, above that kernel 6-L (one warp per chunk, the block streamed through a
+ * 64 KiB history ring, a bad chunk writes no row).  Same arguments, statuses and untouched rows; larger values fail
+ * with HB_ERR_ARG. */
+int hb_decode_columns_device_large(const uint8_t *d_frames, const uint64_t *d_off, const uint32_t *d_len, const uint64_t *d_row,
+                                   uint64_t n_chunks, uint32_t chunk_records, uint32_t *d_start, uint32_t *d_stop, uint8_t *d_ref,
+                                   uint8_t *d_alt, int8_t *d_p1, int8_t *d_p2, int *d_status, void *stream);
 
 /* ------------------------------------------------------------------------------------------
  * D. Dataset: batched on-the-fly haplotype construction, replacing
