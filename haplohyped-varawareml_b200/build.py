@@ -18,7 +18,7 @@ LIB = os.path.join(HERE, "libhaplo_b200.so")
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 CU_SOURCES = ["hb_tokenize.cu", "hb_sites.cu", "hb_walk.cu", "hb_gt.cu", "hb_inflate.cu", "hb_hap.cu", "hb_synth.cu", "hb_api.cu",
-              "hb_store.cu"]
+              "hb_store.cu", "hb_bcf.cu"]
 
 
 def _newer(target: str, deps) -> bool:

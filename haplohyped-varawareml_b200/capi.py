@@ -71,7 +71,7 @@ class SynthSpec(C.Structure):
 EXPORTS = [
     "hb_last_error", "hb_version", "hb_kernel_launches",
     "hb_load_vcf", "hb_load_vcf_without_sample", "hb_records_free", "hb_cache_clear", "hb_cache_set_limit",
-    "hb_parse_host_text", "hb_parse_stream_host", "hb_parse_stream_bgzf_host", "hb_parse_stream_bgzf_resident", "hb_parse_set_text_limit", "hb_set_walker_lines", "hb_bgzf_vcf_info", "hb_parse_device_text", "hb_parse_file", "hb_parse_vcf_bytes", "hb_parse_samples", "hb_parse_rerun", "hb_parse_rerun_bytes", "hb_parse_get_info",
+    "hb_parse_host_text", "hb_parse_stream_host", "hb_parse_stream_bgzf_host", "hb_parse_stream_bgzf_resident", "hb_parse_set_text_limit", "hb_set_walker_lines", "hb_set_bcf_segment_bytes", "hb_bgzf_vcf_info", "hb_parse_device_text", "hb_parse_file", "hb_parse_vcf_bytes", "hb_parse_samples", "hb_parse_rerun", "hb_parse_rerun_bytes", "hb_parse_get_info",
     "hb_parse_fetch_sites", "hb_parse_fetch_sample", "hb_parse_fetch_matrix", "hb_parse_fetch_sample_errors",
     "hb_parse_chrom_runs", "hb_parse_free",
     "hb_bgzf_inflate", "hb_bgzf_compress_host",
@@ -101,6 +101,8 @@ def lib():
         L.hb_cache_set_limit.restype = None
         L.hb_set_walker_lines.argtypes = [C.c_uint32]
         L.hb_set_walker_lines.restype = None
+        L.hb_set_bcf_segment_bytes.argtypes = [C.c_uint64]
+        L.hb_set_bcf_segment_bytes.restype = None
         L.hb_set_fetch_mode.argtypes = [C.c_int]
         L.hb_set_fetch_mode.restype = None
         L.hb_set_host_threads.argtypes = [C.c_int]
@@ -229,7 +231,7 @@ class Parse:
 
     @classmethod
     def from_vcf_bytes(cls, data, region="", want_gt=True, device=0, nbytes=None):
-        """The bytes of a .vcf / .vcf.gz in host memory (bytes, uint8 array, or address + nbytes)."""
+        """The bytes of a .vcf / .vcf.gz / .bcf in host memory (bytes, uint8 array, or address + nbytes)."""
         if isinstance(data, (bytes, bytearray)):
             keep = np.frombuffer(data, np.uint8); addr, n = keep.ctypes.data, keep.size
         elif isinstance(data, np.ndarray):

@@ -33,6 +33,9 @@ static thread_local std::string g_err;
 static std::atomic<uint64_t> g_launches{0};
 static std::atomic<uint64_t> g_text_limit{0};
 static std::atomic<uint32_t> g_walker_lines{16};   // hb_set_walker_lines      // hb_parse_set_text_limit: 0 = from free device memory
+static std::atomic<uint64_t> g_bcf_segment{0};     // hb_set_bcf_segment_bytes: 0 = max(64 KiB, 8 x the first record)
+static const char *const kBcfNoStream =
+    "BCF streaming is not supported: read a .bcf with hb_parse_file, hb_parse_vcf_bytes or hb_load_vcf";
 void count_launch(uint64_t n) { g_launches += n; }
 
 static int fail(int code, const std::string &msg) {
@@ -305,6 +308,12 @@ void hb_parse_free(hb_parse *p) {
     free_dev(p->d_wstart); free_dev(p->d_wrow); free_dev(p->d_verify); free_dev(p->d_wcount);
     free_dev(p->walk_pad.start); free_dev(p->walk_pad.stop); free_dev(p->walk_pad.ref); free_dev(p->walk_pad.alt);
     free_dev(p->walk_pad.chrom_abs); free_dev(p->walk_pad.chrom_len); free_dev(p->walk_pad.chrom5); free_dev(p->walk_pad.rowinfo);
+    if (hb_parse::Bcf *b = p->bcf) {
+        free_dev(b->d_contigs); free_dev(b->d_names); free_dev(b->d_rec_off); free_dev(b->d_blk_count); free_dev(b->d_blk_base);
+        free_dev(b->seg.start); free_dev(b->seg.exit); free_dev(b->seg.bad); free_dev(b->seg.base); free_dev(b->seg.count);
+        free_dev(b->seg.flag);
+        delete b;
+    }
     for (auto &e : p->ev) if (e) cudaEventDestroy(e);
     if (p->side) { cudaStreamSynchronize(p->side); cudaStreamDestroy(p->side); }
     if (p->ev_runs) cudaEventDestroy(p->ev_runs);
@@ -528,19 +537,116 @@ static int index_by_walker(hb_parse *p, const Launch &L) {
     return HB_OK;
 }
 
+static int bcf_malformed(uint64_t bad, uint32_t n_samples, uint32_t n_contigs) {
+    const std::string at = "BCF record at byte " + std::to_string(bad & ((1ull << 56) - 1)) + " of the body";
+    switch ((uint32_t)(bad >> 56)) {
+        case kBcfTruncated: return fail(HB_ERR_FORMAT, at + " is truncated: its length runs past the end of the data");
+        case kBcfNSample: return fail(HB_ERR_FORMAT, at + ": n_sample differs from the header's " + std::to_string(n_samples) + " samples");
+        case kBcfContig: return fail(HB_ERR_FORMAT, at + ": CHROM is not an index of the header's " + std::to_string(n_contigs) + " contigs");
+        default: return fail(HB_ERR_FORMAT, at + " has a malformed record header");
+    }
+}
+
+// ---- BCF records located by chaining their lengths, proven exact segment by segment: hb_bcf.cu
+static int index_bcf(hb_parse *p, const Launch &L) {
+    hb_parse::Bcf &b = *p->bcf;
+    const uint32_t nc = (uint32_t)b.contigs.size();
+    if (!b.first_len) {
+        uint32_t h[2] = {0, 0};
+        if (p->nbytes >= 8) {
+            CU(cudaMemcpyAsync(h, p->d_text, 8, cudaMemcpyDeviceToHost, p->stream));
+            CU(cudaStreamSynchronize(p->stream));
+        }
+        b.first_len = 8ull + h[0] + h[1];
+    }
+    // segments of several records each: the warp that finds a segment's first record scans at most about one record
+    BcfSegs &sg = b.seg;
+    const uint64_t knob = g_bcf_segment.load();
+    sg.bytes = knob ? knob : std::max<uint64_t>(64ull << 10, std::min<uint64_t>(8 * b.first_len, 1ull << 40));
+    sg.n = (p->nbytes + sg.bytes - 1) / sg.bytes;
+    if (sg.cap < sg.n || !sg.start) {
+        TRY(dev_alloc(&sg.start, sg.n)); TRY(dev_alloc(&sg.exit, sg.n)); TRY(dev_alloc(&sg.bad, sg.n));
+        TRY(dev_alloc(&sg.base, sg.n)); TRY(dev_alloc(&sg.count, sg.n)); TRY(dev_alloc(&sg.flag, sg.n));
+        sg.cap = sg.n;
+    }
+    CU(cudaEventRecord(p->ev[0], p->stream));
+    launch_bcf_chain(p->d_text, p->nbytes, p->n_samples, nc, sg, true, L);
+    for (;;) {                                   // until every segment's start is the exit of the segment before it
+        CU(cudaMemsetAsync(&p->d_st->bcf_fail, 0xff, 8, p->stream));
+        CU(cudaMemsetAsync(&p->d_st->bcf_records, 0, 8, p->stream));
+        launch_bcf_verify(sg, p->d_st, L);
+        TRY(fetch_status(p));
+        CU(cudaGetLastError());
+        const uint64_t f = p->h_st.bcf_fail;
+        if (f == ~0ull) break;
+        if (f & 1) {                             // a proven chain met a record that fails the header test
+            uint64_t bad = 0;
+            CU(cudaMemcpy(&bad, sg.bad + (f >> 1), 8, cudaMemcpyDeviceToHost));
+            return bcf_malformed(bad, p->n_samples, nc);
+        }
+        launch_bcf_chain(p->d_text, p->nbytes, p->n_samples, nc, sg, false, L);
+    }
+    const uint64_t n_all = p->h_st.bcf_records;
+    p->n_lines = n_all;
+    if (b.rec_cap < n_all || !b.d_rec_off) { TRY(dev_alloc(&b.d_rec_off, n_all)); b.rec_cap = n_all; }
+    launch_bcf_emit(p->d_text, p->nbytes, sg, b.d_rec_off, L);
+    CU(cudaEventRecord(p->ev[1], p->stream));
+    if (p->row_cap < n_all || !p->d_start) {
+        uint64_t cap = p->d_start ? std::max(n_all + n_all / 8 + 1024, p->row_cap) : n_all;
+        TRY(dev_alloc(&p->d_start, cap)); TRY(dev_alloc(&p->d_stop, cap));
+        TRY(dev_alloc(&p->d_ref, cap)); TRY(dev_alloc(&p->d_alt, cap));
+        TRY(dev_alloc(&p->d_chrom_abs, cap)); TRY(dev_alloc(&p->d_chrom_len, cap)); TRY(dev_alloc(&p->d_chrom5, cap));
+        TRY(dev_alloc(&p->d_rowinfo, cap));
+        p->row_cap = cap;
+    }
+    const uint64_t blocks = (n_all + 255) / 256;
+    if (b.blk_cap < blocks || !b.d_blk_count) {
+        TRY(dev_alloc(&b.d_blk_count, blocks)); TRY(dev_alloc(&b.d_blk_base, blocks));
+        b.blk_cap = blocks;
+    }
+    BcfSiteArgs a;
+    a.text = p->d_text; a.rec_off = b.d_rec_off; a.n_rec = n_all; a.n_samples = p->n_samples; a.n_contigs = nc;
+    a.contigs = b.d_contigs; a.gt_key = b.gt_key;
+    a.rid = -1;
+    if (p->rg.has_region) {
+        const std::string want(p->rg.chrom, p->rg.chrom_len);
+        a.rid = -2;
+        for (uint32_t i = 0; i < nc; ++i) if (b.contigs[i] == want) { a.rid = (int)i; break; }
+    }
+    a.beg0 = p->rg.beg0; a.end0 = p->rg.end0; a.want_gt = p->want_gt;
+    a.start = p->d_start; a.stop = p->d_stop; a.ref = p->d_ref; a.alt = p->d_alt; a.chrom_len = p->d_chrom_len;
+    a.chrom_abs = p->d_chrom_abs; a.chrom5 = p->d_chrom5; a.rowinfo = p->d_rowinfo;
+    a.blk_count = b.d_blk_count; a.blk_base = b.d_blk_base; a.st = p->d_st;
+    launch_bcf_sites(a, L);
+    CU(cudaEventRecord(p->ev[2], p->stream));
+    TRY(fetch_status(p));
+    CU(cudaGetLastError());
+    if (p->h_st.bcf_bad_fmt)
+        return fail(HB_ERR_FORMAT, "BCF record whose alleles or FORMAT fields run past its length (" +
+                                       std::to_string(p->h_st.bcf_bad_fmt) + " records)");
+    p->index_used = 4;
+    return HB_OK;
+}
+
 // the CHROM runs of the last run_parse, on the host (needs the text: hb_parse_release_text calls it first)
 static int ensure_runs(hb_parse *p) {
     if (p->runs_valid) return HB_OK;
     CU(cudaSetDevice(p->device));
     p->run_rows.clear(); p->run_names.clear();
     const uint64_t n_runs = std::min<uint64_t>(p->h_st.n_chrom_runs, hb_parse::kMaxRuns);
-    if (n_runs && p->d_run_rows && p->d_text) {
+    if (n_runs && p->d_run_rows && (p->d_text || p->bcf)) {
         p->run_rows.resize(n_runs);
         CU(cudaMemcpy(p->run_rows.data(), p->d_run_rows, n_runs * 8, cudaMemcpyDeviceToHost));
         std::sort(p->run_rows.begin(), p->run_rows.end());
         for (uint64_t r : p->run_rows) {
             uint64_t abs; uint8_t len; char name[256];
             CU(cudaMemcpy(&abs, p->d_chrom_abs + r, 8, cudaMemcpyDeviceToHost));
+            if (p->bcf) {                        // BCF rows point into the contig names: the name from the dictionary
+                const auto &off = p->bcf->name_off;
+                const size_t i = (size_t)(std::lower_bound(off.begin(), off.end(), abs) - off.begin());
+                p->run_names.push_back(i < off.size() ? p->bcf->contigs[i] : std::string());
+                continue;
+            }
             CU(cudaMemcpy(&len, p->d_chrom_len + r, 1, cudaMemcpyDeviceToHost));
             CU(cudaMemcpy(name, p->d_text + abs, len, cudaMemcpyDeviceToHost));
             p->run_names.emplace_back(name, name + len);
@@ -561,7 +667,7 @@ static int run_parse(hb_parse *p) {
     if (p->nbytes == 0) return HB_OK;
 
     // ---- how to locate the records, from the first one
-    if (!p->probed) {
+    if (!p->probed && !p->bcf) {
         // the whole first record: 4 bytes per sample when it is GT-only (800 KB at 200,000 samples) + its head
         std::vector<uint8_t> head((size_t)std::min<uint64_t>(4ull * p->n_samples + 65536, p->nbytes));
         const size_t hn = head.size();
@@ -583,7 +689,8 @@ static int run_parse(hb_parse *p) {
     }
     CU(cudaMemsetAsync(p->d_ploidy, 0, std::max<uint64_t>(1, p->n_samples) * 4, p->stream));
     CU(cudaMemsetAsync(p->d_badgt, 0, std::max<uint64_t>(1, p->n_samples) * 4, p->stream));
-    if (p->use_walker) TRY(index_by_walker(p, L));
+    if (p->bcf) TRY(index_bcf(p, L));
+    else if (p->use_walker) TRY(index_by_walker(p, L));
     else TRY(index_by_tokenizer(p, L));
     const uint64_t n_rec = p->h_st.n_records;
     if (p->attached_frames && n_rec) frames_early_site_pass(p->attached_frames, p);
@@ -594,7 +701,7 @@ static int run_parse(hb_parse *p) {
         CU(cudaStreamWaitEvent(p->side, p->ev_runs, 0));
         Launch Ls = L;
         Ls.stream = p->side;
-        launch_chrom_runs(p->d_text, p->d_chrom_abs, p->d_chrom_len, n_rec, p->d_run_rows, hb_parse::kMaxRuns, p->d_st, Ls);
+        launch_chrom_runs(p->bcf ? p->bcf->d_names : p->d_text, p->d_chrom_abs, p->d_chrom_len, n_rec, p->d_run_rows, hb_parse::kMaxRuns, p->d_st, Ls);
         CU(cudaEventRecord(p->ev_runs, p->side));
     }
 
@@ -626,8 +733,12 @@ static int run_parse(hb_parse *p) {
             CU(cudaMemsetAsync(p->d_cp, 0xff, p->cp_rows * p->ncp * sizeof(uint64_t), p->stream));
             launch_index_columns(p->d_text, p->d_rowinfo, p->d_nu_rows, n_nu, p->d_cp, p->ncp, L);
         }
-        launch_decode_gt(p->d_text, p->d_rowinfo, n_rec, p->n_samples, p->d_cp, p->ncp, p->d_gt[0], p->d_gt[1],
-                         p->gt_stride, p->d_bits, p->bits_stride, p->d_ploidy, p->d_badgt, p->d_st, L);
+        if (p->bcf)
+            launch_bcf_decode(p->d_text, p->d_rowinfo, n_rec, p->n_samples, p->d_gt[0], p->d_gt[1], p->gt_stride, p->d_bits,
+                              p->bits_stride, p->d_ploidy, p->d_badgt, p->d_st, L);
+        else
+            launch_decode_gt(p->d_text, p->d_rowinfo, n_rec, p->n_samples, p->d_cp, p->ncp, p->d_gt[0], p->d_gt[1],
+                             p->gt_stride, p->d_bits, p->bits_stride, p->d_ploidy, p->d_badgt, p->d_st, L);
     }
     CU(cudaEventRecord(p->ev[3], p->stream));
     // frames attached to this parse: their kernel is queued right behind the decoder now (the host waits for the templates
@@ -915,6 +1026,7 @@ int hb_parse_stream_host(const uint8_t *text, uint64_t nbytes, const hb_parse_op
                          int8_t *gt0, int8_t *gt1, uint64_t out_stride, uint32_t *start, uint32_t *stop, char *ref,
                          char *alt, uint32_t *ploidy_err, uint32_t *badgt_err, uint64_t *n_records, uint32_t *n_slabs) {
     if (!opts || !n_records || (nbytes && !text)) return fail(HB_ERR_ARG, "null argument");
+    if (nbytes >= 4 && memcmp(text, "BCF\2", 4) == 0) return fail(HB_ERR_ARG, kBcfNoStream);
     *n_records = 0;
     if (n_slabs) *n_slabs = 0;
     HostSink sink;
@@ -1111,6 +1223,9 @@ struct FileText {
     uint64_t body = 0;           // offset of the first record
     std::vector<std::string> samples;
     int end_is_int = 0;
+    bool bcf = false;            // BCF 2.2: body = the records after the header text
+    std::vector<std::string> contigs;   // BCF contig dictionary
+    int gt_key = -1;             // BCF string-dictionary index of GT (-1: not declared)
 };
 
 int read_all(const char *path, std::vector<uint8_t> &raw) {
@@ -1195,8 +1310,92 @@ bool parse_header(const uint8_t *d, uint64_t n, bool whole, FileText &ft) {
     return false;                                          // text without a #CHROM line
 }
 
+// attribute `key` of a structured header line "##X=<ID=...,key=value,...>" (values may be quoted)
+bool hrec_attr(const std::string &line, const std::string &key, std::string &val) {
+    size_t p = line.find('<');
+    if (p == std::string::npos) return false;
+    ++p;
+    while (p < line.size()) {
+        const size_t eq = line.find('=', p);
+        if (eq == std::string::npos) return false;
+        const std::string k = line.substr(p, eq - p);
+        size_t q = eq + 1;
+        std::string v;
+        if (q < line.size() && line[q] == '"') {
+            for (++q; q < line.size() && line[q] != '"'; ++q) {
+                if (line[q] == '\\' && q + 1 < line.size()) ++q;
+                v.push_back(line[q]);
+            }
+            ++q;
+        } else {
+            while (q < line.size() && line[q] != ',' && line[q] != '>') v.push_back(line[q++]);
+        }
+        if (k == key) { val = v; return true; }
+        if (q >= line.size() || line[q] != ',') return false;
+        p = q + 1;
+    }
+    return false;
+}
+
+// The header of a BCF 2.2 file (VCF v4.3 specification, section 6.3): magic "BCF\2\2", uint32 l_text, then l_text bytes of
+// NUL-terminated VCF header text.  complete = false while [d, d + n) does not hold all of it.  Sample names come from the
+// #CHROM line as for text.  Dictionaries, as htslib builds them: IDX= attributes (which htslib writes into BCF headers)
+// win; without them the string dictionary is PASS = 0, then the FILTER / INFO / FORMAT IDs in order of first appearance
+// (an ID shared by several lines gets one index), and the contig dictionary is the ##contig lines in order.
+int bcf_header(const uint8_t *d, uint64_t n, FileText &ft, bool &complete) {
+    complete = false;
+    if (n < 5) return HB_OK;
+    if (d[3] != 2 || d[4] != 2)
+        return fail(HB_ERR_FORMAT, "BCF version " + std::to_string(d[3]) + "." + std::to_string(d[4]) +
+                                       " is not supported: only BCF 2.2 is read");
+    if (n < 9) return HB_OK;
+    const uint32_t l_text = d[5] | d[6] << 8 | d[7] << 16 | (uint32_t)d[8] << 24;
+    if (n < 9ull + l_text) return HB_OK;
+    uint64_t len = l_text;
+    while (len && d[9 + len - 1] == 0) --len;
+    if (!parse_header(d + 9, len, true, ft)) return fail(HB_ERR_HEADER, "no #CHROM header line");
+    std::map<std::string, int> strs{{"PASS", 0}};
+    int next = 1, cnext = 0;
+    std::vector<std::pair<int, std::string>> ctg;
+    for (uint64_t p = 0; p < len;) {
+        const uint8_t *e = (const uint8_t *)memchr(d + 9 + p, '\n', len - p);
+        const uint64_t le = e ? (uint64_t)(e - d - 9) : len;
+        const std::string line((const char *)d + 9 + p, (const char *)d + 9 + le);
+        p = le + 1;
+        const bool dict = line.rfind("##FILTER=<", 0) == 0 || line.rfind("##INFO=<", 0) == 0 || line.rfind("##FORMAT=<", 0) == 0;
+        const bool contig = line.rfind("##contig=<", 0) == 0;
+        std::string id, idx;
+        if ((!dict && !contig) || !hrec_attr(line, "ID", id)) continue;
+        const bool has_idx = hrec_attr(line, "IDX", idx) && !idx.empty() && idx.find_first_not_of("0123456789") == std::string::npos;
+        const int i = has_idx ? std::atoi(idx.c_str()) : -1;
+        if (contig) {
+            const int c = i >= 0 ? i : cnext;
+            cnext = std::max(cnext, c + 1);
+            ctg.emplace_back(c, id);
+        } else if (i >= 0) {
+            strs[id] = i;
+            next = std::max(next, i + 1);
+        } else if (!strs.count(id)) strs[id] = next++;
+    }
+    ft.contigs.assign((size_t)cnext, std::string());
+    for (auto &c : ctg) ft.contigs[(size_t)c.first] = c.second;
+    const auto gt = strs.find("GT");
+    ft.gt_key = gt == strs.end() ? -1 : gt->second;
+    ft.bcf = true;
+    ft.body = 9ull + l_text;
+    complete = true;
+    return HB_OK;
+}
+
+bool is_bcf(const uint8_t *d, uint64_t n) { return n >= 3 && memcmp(d, "BCF", 3) == 0; }
+
 int read_vcf(const std::vector<uint8_t> &raw, FileText &ft) {
     TRY(inflate_all(raw, ft.data));
+    if (is_bcf(ft.data.data(), ft.data.size())) {
+        bool complete = false;
+        TRY(bcf_header(ft.data.data(), ft.data.size(), ft, complete));
+        return complete ? HB_OK : fail(HB_ERR_FORMAT, "BCF header is truncated");
+    }
     if (!ft.data.empty() && ft.data.back() != '\n') ft.data.push_back('\n');
     if (!parse_header(ft.data.data(), ft.data.size(), true, ft)) return fail(HB_ERR_HEADER, "no #CHROM header line");
     return HB_OK;
@@ -1234,13 +1433,79 @@ static int bgzf_header(const uint8_t *raw, const std::vector<uint64_t> &coff, co
         const int zr = inflate(&zs, Z_FINISH);
         inflateEnd(&zs);
         if (zr != Z_STREAM_END || zs.avail_out != 0) return fail(HB_ERR_IO, "BGZF inflate failed (header)");
-        have = parse_header(head.data(), head.size(), i + 1 == coff.size(), ft);
+        if (is_bcf(head.data(), head.size())) TRY(bcf_header(head.data(), head.size(), ft, have));
+        else have = parse_header(head.data(), head.size(), i + 1 == coff.size(), ft);
     }
+    if (!have && is_bcf(head.data(), head.size())) return fail(HB_ERR_FORMAT, "BCF header is truncated");
     if (!have) return fail(HB_ERR_HEADER, "no #CHROM header line");
     return HB_OK;
 }
 
-// raw_p[0..raw_n): the bytes of a .vcf / .vcf.gz; raw_owned: the vector that holds them when the caller read a file
+// text bytes a whole-file parse may hold in HBM (hb_parse_set_text_limit, else from free device memory); slab: the slab
+// size of the streamed route
+uint64_t text_limit(uint64_t &slab) {
+    uint64_t limit = g_text_limit.load();
+    slab = limit ? std::max<uint64_t>(limit / 2, 1 << 16) : 0;      // two slabs of text are resident at a time
+    if (!limit) {
+        size_t fr = 0, tot = 0;
+        if (cudaMemGetInfo(&fr, &tot) != cudaSuccess) { cudaGetLastError(); fr = 0; }
+        // GT-only text is ~4 bytes per call, the planes + bit planes it leaves 2.125: text + 0.55 x text must fit
+        limit = (uint64_t)(0.9 * (double)(fr + hb::dev_pool_idle_bytes()) / 1.55);
+    }
+    return limit;
+}
+
+// a BCF's contig table and names on the device, and the dictionaries on the handle
+int bcf_attach(hb_parse *p, const FileText &ft) {
+    hb_parse::Bcf *b = p->bcf = new hb_parse::Bcf();
+    b->contigs = ft.contigs;
+    b->gt_key = ft.gt_key;
+    std::string names;
+    std::vector<BcfContig> tab;
+    for (const std::string &c : ft.contigs) {
+        BcfContig x{0, names.size(), (uint32_t)std::min<size_t>(c.size(), 255), 0};
+        for (size_t k = 0; k < 5 && k < c.size(); ++k) x.name5 |= (uint64_t)(uint8_t)c[k] << (8 * k);
+        b->name_off.push_back(names.size());
+        tab.push_back(x);
+        names += c;
+        names.push_back('\0');
+    }
+    TRY(dev_alloc(&b->d_contigs, tab.size()));
+    TRY(dev_alloc(&b->d_names, names.size() + 1));
+    if (!tab.empty()) CU(cudaMemcpy(b->d_contigs, tab.data(), tab.size() * sizeof(BcfContig), cudaMemcpyHostToDevice));
+    if (!names.empty()) CU(cudaMemcpy(b->d_names, names.data(), names.size(), cudaMemcpyHostToDevice));
+    return HB_OK;
+}
+
+int bcf_too_big(uint64_t body) {
+    return fail(HB_ERR_ARG, "BCF body of " + std::to_string(body) + " bytes exceeds the text limit and BCF streaming is not supported");
+}
+
+// the body of an uncompressed or plain-gzip BCF, inflated on the host
+int parse_bcf_host(const FileText &ft, const hb_parse_opts &o, hb_parse **out) {
+    const uint64_t n = ft.data.size() - ft.body;
+    uint64_t slab;
+    TRY(ensure_device(o.device));
+    if (n > text_limit(slab)) return bcf_too_big(n);
+    hb_parse *p = nullptr;
+    TRY(new_parse(&o, &p));
+    int rc = dev_alloc(&p->d_text_owned, n + 256);
+    cudaError_t e = cudaSuccess;
+    if (rc == HB_OK) e = cudaMemcpyAsync(p->d_text_owned, ft.data.data() + ft.body, n, cudaMemcpyHostToDevice, p->stream);
+    if (rc == HB_OK && e == cudaSuccess) e = cudaMemsetAsync(p->d_text_owned + n, 0, 256, p->stream);
+    if (rc == HB_OK && e != cudaSuccess) rc = fail(HB_ERR_CUDA, std::string("CUDA: ") + cudaGetErrorString(e));
+    if (rc == HB_OK) {
+        p->d_text = p->d_text_owned;
+        p->nbytes = n;
+        rc = bcf_attach(p, ft);
+    }
+    if (rc == HB_OK) rc = run_parse(p);
+    if (rc != HB_OK) { hb_parse_free(p); return rc; }
+    *out = p;
+    return HB_OK;
+}
+
+// raw_p[0..raw_n): the bytes of a .vcf / .vcf.gz / .bcf; raw_owned: the vector that holds them when the caller read a file
 // (released early on the zlib path), empty when they belong to the caller
 int parse_bytes_common(std::vector<uint8_t> &raw_owned, const uint8_t *raw_p, uint64_t raw_n, const char *region, bool want_gt,
                        int device, hb_parse **out, std::vector<std::string> &samples) {
@@ -1264,6 +1529,7 @@ int parse_bytes_common(std::vector<uint8_t> &raw_owned, const uint8_t *raw_p, ui
         samples = ft.samples;
         o.n_samples = (uint32_t)ft.samples.size();
         o.end_is_int = ft.end_is_int;
+        if (ft.bcf) return parse_bcf_host(ft, o, out);
         return hb_parse_host_text(ft.data.data() + ft.body, ft.data.size() - ft.body, &o, out);
     }
     // ---- header: inflate leading members on the host until the #CHROM line is complete
@@ -1273,14 +1539,9 @@ int parse_bytes_common(std::vector<uint8_t> &raw_owned, const uint8_t *raw_p, ui
     {   // a file whose text does not fit HBM next to its genotype planes passes through in slabs instead: same rows, same
         // handle minus the text (hb_parse_stream_bgzf_resident)
         TRY(ensure_device(device));
-        uint64_t limit = g_text_limit.load();
-        const uint64_t slab = limit ? std::max<uint64_t>(limit / 2, 1 << 16) : 0;      // two slabs of text are resident at a time
-        if (!limit) {
-            size_t fr = 0, tot = 0;
-            if (cudaMemGetInfo(&fr, &tot) != cudaSuccess) { cudaGetLastError(); fr = 0; }
-            // GT-only text is ~4 bytes per call, the planes + bit planes it leaves 2.125: text + 0.55 x text must fit
-            limit = (uint64_t)(0.9 * (double)(fr + hb::dev_pool_idle_bytes()) / 1.55);
-        }
+        uint64_t slab;
+        const uint64_t limit = text_limit(slab);
+        if (total > limit && ft.bcf) return bcf_too_big(total - ft.body);
         if (total > limit) return hb_parse_stream_bgzf_resident(raw_p, raw_n, region, want_gt ? 1 : 0, device, slab, out, nullptr);
     }
     o.n_samples = (uint32_t)ft.samples.size();
@@ -1298,7 +1559,7 @@ int parse_bytes_common(std::vector<uint8_t> &raw_owned, const uint8_t *raw_p, ui
     cudaError_t e = cudaSuccess;
     if (rc == HB_OK) e = cudaMemcpy(&last, p->d_text_owned + pad + total - 1, 1, cudaMemcpyDeviceToHost);
     uint64_t end = pad + total;
-    if (rc == HB_OK && e == cudaSuccess && last != '\n') { e = cudaMemset(p->d_text_owned + end, '\n', 1); ++end; }
+    if (rc == HB_OK && e == cudaSuccess && last != '\n' && !ft.bcf) { e = cudaMemset(p->d_text_owned + end, '\n', 1); ++end; }
     if (rc == HB_OK && e == cudaSuccess) e = cudaMemset(p->d_text_owned + end, 0, 256);
     if (rc == HB_OK && e != cudaSuccess) rc = fail(HB_ERR_CUDA, std::string("CUDA: ") + cudaGetErrorString(e));
     if (rc == HB_OK) {
@@ -1306,7 +1567,8 @@ int parse_bytes_common(std::vector<uint8_t> &raw_owned, const uint8_t *raw_p, ui
         p->nbytes = end - pad - ft.body;
         p->compressed_bytes = raw.size();
         const double t2 = now();
-        rc = run_parse(p);
+        if (ft.bcf) rc = bcf_attach(p, ft);
+        if (rc == HB_OK) rc = run_parse(p);
         if (trace) fprintf(stderr, "[parse_bytes_common] text buffer %.1f ms, H2D + inflate %.1f ms, parse %.1f ms\n", t1 - t0, t2 - t1, now() - t2);
     }
     if (rc != HB_OK) { hb_parse_free(p); return rc; }
@@ -1531,6 +1793,7 @@ void hb_cache_set_limit(uint64_t hbm_bytes) {
 
 void hb_parse_set_text_limit(uint64_t text_bytes) { g_text_limit.store(text_bytes); }
 void hb_set_walker_lines(uint32_t lines) { g_walker_lines.store(lines == 0 ? 16u : std::min(lines, 20u)); }
+void hb_set_bcf_segment_bytes(uint64_t bytes) { g_bcf_segment.store(bytes == 0 ? 0 : std::max<uint64_t>(bytes, 64)); }
 
 void hb_cache_clear(void) {
     {
@@ -1567,6 +1830,7 @@ int hb_bgzf_vcf_info(const uint8_t *bgzf, uint64_t nbytes, uint32_t *n_samples, 
     if (!bgzf_index(bgzf, nbytes, coff, clen, ooff, olen, total)) return fail(HB_ERR_IO, "not a BGZF file");
     FileText ft;
     TRY(bgzf_header(bgzf, coff, clen, olen, ft));
+    if (ft.bcf) return fail(HB_ERR_ARG, kBcfNoStream);
     if (n_samples) *n_samples = (uint32_t)ft.samples.size();
     if (text_bytes) *text_bytes = total;
     if (body_offset) *body_offset = ft.body;
@@ -1589,6 +1853,7 @@ static int stream_bgzf(const char *entry, const uint8_t *bgzf, uint64_t nbytes, 
     if (!bgzf_index(bgzf, nbytes, coff, clen, ooff, olen, total)) return fail(HB_ERR_IO, "not a BGZF file");
     FileText ft;
     TRY(bgzf_header(bgzf, coff, clen, olen, ft));
+    if (ft.bcf) return fail(HB_ERR_ARG, kBcfNoStream);
     const double t_index = now_ms() - t_begin;
     hb_parse_opts opts;
     memset(&opts, 0, sizeof opts);

@@ -42,6 +42,10 @@ struct DevStatus {
     unsigned int ticket;               // tile tickets of the site kernel
     unsigned int walk_broken;          // walker: a chain did not land on the next walker's start
     unsigned int index_invalid;        // a newline was found inside a span taken for one record's samples
+    unsigned long long bcf_fail;       // BCF locator: least of 2k (segment k's start is not segment k - 1's exit) and
+                                       // 2k + 1 (segment k's chain met a record that fails the header test); ~0 = none
+    unsigned long long bcf_records;    // BCF locator: records that start in the segments
+    unsigned long long bcf_bad_fmt;    // BCF sites: kept records whose FORMAT fields run past the record
 };
 
 // Per tokenizer CTA (one contiguous byte range each).
@@ -109,6 +113,55 @@ void launch_decode_gt(const uint8_t *d_text, const RowInfo *d_rowinfo, uint64_t 
 
 void launch_bits_from_planes(const int8_t *d_gt0, const int8_t *d_gt1, uint64_t gt_stride, uint64_t n_rows, uint32_t n_samples,
                              uint32_t *d_bits, uint64_t bits_stride, const Launch &L);
+
+// ---- BCF 2.2 input (hb_bcf.cu): kernel 1b locates records by chaining their lengths, kernel 3b decodes typed GT values.
+// BCF rows use RowInfo as: samp_abs = offset of the GT values of sample 0, samp_len = values per sample, misc [7:0] = value
+// type (1 int8, 2 int16, 3 int32; 255 = no GT) | kRowHasSamples.
+struct BcfContig {                 // one entry of the header's contig dictionary
+    uint64_t name5;                // first 5 name bytes, NUL padded (the S5 field)
+    uint64_t name_off;             // offset of the name in the parse's name buffer: what d_chrom_abs holds for BCF rows
+    uint32_t name_len;             // min(length, 255)
+    uint32_t pad;
+};
+constexpr uint64_t kBcfNone = ~0ull;
+struct BcfSegs {                   // the locator's segments, [k * bytes, (k + 1) * bytes) of the body
+    uint64_t n = 0, bytes = 0, cap = 0;
+    uint64_t *start = nullptr;     // first record start at or past the segment's begin (kBcfNone: none found)
+    uint64_t *exit = nullptr;      // first record start at or past its end, from chaining `start`
+    uint64_t *bad = nullptr;       // 0, or reason << 56 | offset of the record that failed the header test
+    uint64_t *base = nullptr;      // exclusive prefix sums of count
+    uint32_t *count = nullptr;     // records that start in the segment
+    uint32_t *flag = nullptr;      // chain the segment (again)
+};
+// header-test failures (BcfSegs::bad >> 56)
+constexpr uint32_t kBcfTruncated = 1, kBcfNSample = 2, kBcfContig = 3, kBcfHead = 4;
+struct BcfSiteArgs {
+    const uint8_t *text;
+    const uint64_t *rec_off;       // [n_rec] record starts
+    uint64_t n_rec;
+    uint32_t n_samples, n_contigs;
+    const BcfContig *contigs;
+    int gt_key;                    // string-dictionary index of GT, -1 = not declared
+    int rid;                       // region: -1 none, -2 contig not in the dictionary, else its index
+    long long beg0, end0;
+    int want_gt;
+    uint32_t *start, *stop;
+    uint8_t *ref, *alt, *chrom_len;
+    uint64_t *chrom_abs, *chrom5;
+    RowInfo *rowinfo;
+    uint32_t *blk_count;           // [ceil(n_rec / 256)] kept records per block of 256
+    uint64_t *blk_base;
+    DevStatus *st;
+};
+// find (round 0: every segment's first start) and chain the flagged segments
+void launch_bcf_chain(const uint8_t *d_text, uint64_t nbytes, uint32_t n_samples, uint32_t n_contigs, const BcfSegs &sg, bool find,
+                      const Launch &L);
+void launch_bcf_verify(const BcfSegs &sg, DevStatus *d_st, const Launch &L);
+void launch_bcf_emit(const uint8_t *d_text, uint64_t nbytes, const BcfSegs &sg, uint64_t *d_rec_off, const Launch &L);
+void launch_bcf_sites(const BcfSiteArgs &a, const Launch &L);
+void launch_bcf_decode(const uint8_t *d_text, const RowInfo *d_rowinfo, uint64_t n_rows, uint32_t n_samples, int8_t *d_gt0,
+                       int8_t *d_gt1, uint64_t gt_stride, uint32_t *d_bits, uint64_t bits_stride, uint32_t *d_ploidy_err,
+                       uint32_t *d_badgt_err, DevStatus *d_st, const Launch &L);
 
 void count_launch(uint64_t n = 1);
 

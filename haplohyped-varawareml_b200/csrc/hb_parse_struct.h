@@ -29,7 +29,20 @@ struct hb_parse {
     uint64_t verify_cap = 0;
     hb::WalkPad walk_pad;                // padded site rows of the walk (compacted into d_start ... d_rowinfo)
     int walker_fallbacks = 0;
-    int index_used = 0;                 // 1 newline tokenizer, 2 newline+tab tokenizer, 3 walker
+    int index_used = 0;                 // 1 newline tokenizer, 2 newline+tab tokenizer, 3 walker, 4 BCF records
+    struct Bcf {                        // BCF input: the header's dictionaries and the locator's buffers (hb_bcf.cu)
+        std::vector<std::string> contigs;
+        std::vector<uint64_t> name_off;  // of each contig name in d_names (ascending)
+        int gt_key = -1;                 // string-dictionary index of GT, -1 = not declared
+        hb::BcfContig *d_contigs = nullptr;
+        uint8_t *d_names = nullptr;      // the contig names, NUL-separated: the "text" of the CHROM runs
+        uint64_t first_len = 0;          // bytes of the first record
+        hb::BcfSegs seg;
+        uint64_t *d_rec_off = nullptr, rec_cap = 0;
+        uint32_t *d_blk_count = nullptr;
+        uint64_t *d_blk_base = nullptr, blk_cap = 0;
+    };
+    Bcf *bcf = nullptr;
     uint32_t ncp = 0;
 
     uint64_t *d_nl_after = nullptr; uint64_t nl_after_cap = 0;

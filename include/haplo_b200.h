@@ -59,6 +59,7 @@ typedef struct hb_records {
     void *owner_;               /* private */
 } hb_records;
 
+/* in_vcf: a .vcf, .vcf.gz or .bcf, as the reference's hts_open reads all three (vcfpp.h:1381) */
 int hb_load_vcf(const char *in_vcf, const char *sample, const char *chrom, hb_records *out);
 int hb_load_vcf_without_sample(const char *in_vcf, const char *chrom, hb_records *out);
 void hb_records_free(hb_records *r);
@@ -98,7 +99,8 @@ typedef struct hb_parse_info {
     uint64_t n_nonuniform;          /* records that took the general (tab-scan) decode path */
     uint64_t n_bad_gt, n_bad_cols;  /* malformed alleles / column-count mismatches */
     uint64_t n_nogt;                /* kept records without a GT key or without sample columns */
-    int tokenizer_used;             /* 1 newline-only, 2 newline + tab checkpoints, 3 head walker */
+    int tokenizer_used;             /* 1 newline-only, 2 newline + tab checkpoints, 3 head walker, 4 BCF records (ms_tokenize
+                                       = locate, ms_sites = site columns, ms_decode = GT decode) */
     float ms_tokenize, ms_sites, ms_decode;   /* CUDA-event kernel times of the last parse */
     int walker_fallbacks;           /* times the head walker could not prove itself exact and the tokenizer re-ran */
     float ms_inflate;               /* GPU BGZF inflate kernel time (file-level parses of BGZF input), else 0 */
@@ -120,10 +122,12 @@ int hb_parse_device_text(const uint8_t *d_text, uint64_t nbytes, const hb_parse_
 int hb_parse_stream_host(const uint8_t *text, uint64_t nbytes, const hb_parse_opts *opts, uint64_t slab_bytes,
                          int8_t *gt0, int8_t *gt1, uint64_t out_stride, uint32_t *start, uint32_t *stop, char *ref,
                          char *alt, uint32_t *ploidy_err, uint32_t *badgt_err, uint64_t *n_records, uint32_t *n_slabs);
-/* a whole .vcf / .vcf.gz (BGZF or plain gzip): header + body, all samples, no per-sample cache.
+/* a whole .vcf / .vcf.gz / .bcf (BGZF, plain gzip or uncompressed; BCF 2.2 is recognised by its magic): header + body,
+ * all samples, no per-sample cache.  A BCF gives the rows the VCF text of the same records gives (tokenizer_used 4).
+ * BCF is not streamed: a BCF body above the text limit (hb_parse_set_text_limit) fails with HB_ERR_ARG.
  * What the vcf_to_h5 converter drives (src/haplohyped/vcf_to_h5.py:98-101 without the per-donor re-scan). */
 int hb_parse_file(const char *in_vcf, const char *region, int want_gt, int device, hb_parse **out);
-/* the same for the bytes of a .vcf / .vcf.gz already in host memory (BGZF bytes cross PCIe compressed and are
+/* the same for the bytes of a .vcf / .vcf.gz / .bcf already in host memory (BGZF bytes cross PCIe compressed and are
  * inflated on the GPU; pinned memory makes that copy asynchronous) */
 int hb_parse_vcf_bytes(const uint8_t *data, uint64_t nbytes, const char *region, int want_gt, int device, hb_parse **out);
 /* BGZF bytes of a .vcf.gz in (pinned) host memory -> the same results as hb_parse_stream_host, streamed: slabs of whole
@@ -132,6 +136,8 @@ int hb_parse_vcf_bytes(const uint8_t *data, uint64_t nbytes, const char *region,
  * overlap the parse of slab k.  This is the reference's whole read path (tbx_itr_next + vcf_parse1 + getGenotypes,
  * vcfpp.h:1468-1472, :546-588) for all samples at once.  hb_bgzf_vcf_info gives what is needed to size the outputs. */
 int hb_bgzf_vcf_info(const uint8_t *bgzf, uint64_t nbytes, uint32_t *n_samples, uint64_t *text_bytes, uint64_t *body_offset);
+/* The streaming entry points (hb_parse_stream_host, hb_bgzf_vcf_info, hb_parse_stream_bgzf_host / _resident) read VCF text
+ * only: BCF input fails with HB_ERR_ARG. */
 int hb_parse_stream_bgzf_host(const uint8_t *bgzf, uint64_t nbytes, const char *region, int want_gt, int device,
                               uint64_t slab_bytes, int8_t *gt0, int8_t *gt1, uint64_t out_stride, uint32_t *start,
                               uint32_t *stop, char *ref, char *alt, uint32_t *ploidy_err, uint32_t *badgt_err,
@@ -150,6 +156,10 @@ void hb_parse_set_text_limit(uint64_t text_bytes);
 /* Lines per walker of the head walker (kernel 1a): 0 = the default (16), at most 20 (a walker has 24 row slots).  Tests
  * use 1-3 to put a walker boundary at every line. */
 void hb_set_walker_lines(uint32_t lines);
+/* Bytes per segment of the BCF record locator (kernel 1b): 0 = the default, max(64 KiB, 8 x the first record's length);
+ * other values are raised to at least 64.  Tests use small segments to put segment boundaries at every offset of a
+ * record and to make records longer than a segment. */
+void hb_set_bcf_segment_bytes(uint64_t bytes);
 /* sample names of a file-level parse, NUL-separated */
 int hb_parse_samples(hb_parse *p, uint32_t *n, char *names, uint64_t cap, uint64_t *len);
 /* re-run the kernels of an existing handle on (new contents of) the same device buffer: no allocation */
