@@ -5,6 +5,7 @@ CPU fallback -- if the library is missing or no sm_100 device is present, calls 
 """
 from __future__ import annotations
 
+import contextlib
 import ctypes as C
 import os
 
@@ -75,7 +76,7 @@ EXPORTS = [
     "hb_parse_fetch_sites", "hb_parse_fetch_sample", "hb_parse_fetch_matrix", "hb_parse_fetch_sample_errors",
     "hb_parse_chrom_runs", "hb_parse_free",
     "hb_bgzf_inflate", "hb_bgzf_compress_host",
-    "hb_compress_records", "hb_compress_sample_range", "hb_frames_set_window", "hb_parse_release_text", "hb_parse_attach_frames", "hb_frames_rerun", "hb_frames_get_info", "hb_frames_layout", "hb_frames_fetch_all", "hb_frames_fetch_packed", "hb_set_fetch_mode", "hb_set_host_threads", "hb_frames_last_d2h_bytes",
+    "hb_compress_records", "hb_compress_sample_range", "hb_frames_set_window", "hb_parse_release_text", "hb_parse_attach_frames", "hb_frames_rerun", "hb_frames_get_info", "hb_frames_layout", "hb_frames_fetch_all", "hb_frames_fetch_packed", "hb_set_fetch_mode", "hb_set_bgzf_crc_check", "hb_get_bgzf_crc_check", "hb_set_host_threads", "hb_frames_last_d2h_bytes",
     "hb_frames_fetch_sample", "hb_frames_free",
     "hb_guess_chunk_records", "hb_set_site_matcher", "hb_decode_frames", "hb_decode_columns_device", "hb_decode_columns_device_large",
     "hb_encode_haplotypes",
@@ -105,6 +106,9 @@ def lib():
         L.hb_set_bcf_segment_bytes.restype = None
         L.hb_set_fetch_mode.argtypes = [C.c_int]
         L.hb_set_fetch_mode.restype = None
+        L.hb_set_bgzf_crc_check.argtypes = [C.c_int]
+        L.hb_set_bgzf_crc_check.restype = None
+        L.hb_get_bgzf_crc_check.restype = C.c_int
         L.hb_set_host_threads.argtypes = [C.c_int]
         L.hb_set_host_threads.restype = None
         L.hb_frames_last_d2h_bytes.argtypes = [C.c_void_p]
@@ -507,6 +511,26 @@ def bgzf_compress_host(text, level: int = 6) -> np.ndarray:
     out = np.empty(n.value, np.uint8)
     check(L.hb_bgzf_compress_host(src.ctypes.data, src.size, level, out.ctypes.data, out.size, C.byref(n)))
     return out[:n.value]
+
+
+def set_bgzf_crc_check(on: bool) -> None:
+    """Check every BGZF member's CRC32 against its trailer, as htslib does (hb_set_bgzf_crc_check; process-wide, off by default)."""
+    lib().hb_set_bgzf_crc_check(1 if on else 0)
+
+
+def get_bgzf_crc_check() -> bool:
+    return bool(lib().hb_get_bgzf_crc_check())
+
+
+@contextlib.contextmanager
+def crc_check(on: bool = True):
+    """`with crc_check(): ...` runs the block with the BGZF CRC32 check set to `on` and restores the setting after it."""
+    was = get_bgzf_crc_check()
+    set_bgzf_crc_check(on)
+    try:
+        yield
+    finally:
+        set_bgzf_crc_check(was)
 
 
 def bgzf_inflate(data: bytes, device: int = 0, with_ms: bool = False):

@@ -1415,11 +1415,13 @@ int parse_file_common(const char *path, const char *region, bool want_gt, int de
     return parse_bytes_common(raw, raw.data(), raw.size(), region, want_gt, device, out, samples);
 }
 
-// the VCF header of a BGZF file: leading members are inflated on the host (zlib) until the #CHROM line is complete
+// the VCF header of a BGZF file: leading members are inflated on the host (zlib) until the #CHROM line is complete; with
+// hb_set_bgzf_crc_check on, each is checked against its CRC32 as kernel 0 checks the others
 static int bgzf_header(const uint8_t *raw, const std::vector<uint64_t> &coff, const std::vector<uint32_t> &clen,
                        const std::vector<uint32_t> &olen, FileText &ft) {
     std::vector<uint8_t> head;
     bool have = false;
+    const bool check_crc = bgzf_crc_check();
     for (size_t i = 0; i < coff.size() && !have; ++i) {
         const size_t at = head.size();
         head.resize(at + olen[i]);
@@ -1433,6 +1435,11 @@ static int bgzf_header(const uint8_t *raw, const std::vector<uint64_t> &coff, co
         const int zr = inflate(&zs, Z_FINISH);
         inflateEnd(&zs);
         if (zr != Z_STREAM_END || zs.avail_out != 0) return fail(HB_ERR_IO, "BGZF inflate failed (header)");
+        if (check_crc) {
+            const uint8_t *tr = raw + coff[i] + clen[i];
+            const uint32_t want = tr[0] | tr[1] << 8 | tr[2] << 16 | (uint32_t)tr[3] << 24;
+            if ((uint32_t)crc32(crc32(0L, Z_NULL, 0), head.data() + at, olen[i]) != want) return fail(HB_ERR_IO, bgzf_crc_message(raw, coff[i]));
+        }
         if (is_bcf(head.data(), head.size())) TRY(bcf_header(head.data(), head.size(), ft, have));
         else have = parse_header(head.data(), head.size(), i + 1 == coff.size(), ft);
     }
@@ -1668,7 +1675,9 @@ int build_entry(CacheEntry &ce, const char *path, const char *region, bool want_
 }
 
 std::shared_ptr<CacheEntry> get_entry(const char *path, const char *region, bool want_gt, int &rc) {
-    const std::string base = std::string(path) + "\x01" + file_identity(path) + "\x01" + (region ? region : "");
+    // a parse made without the BGZF CRC check must not answer a call made with it
+    const std::string base = std::string(path) + "\x01" + file_identity(path) + "\x01" + (region ? region : "") +
+                             (bgzf_crc_check() ? "\x01crc" : "");
     const std::string key = base + (want_gt ? "\x01g" : "\x01s");
     std::shared_ptr<CacheEntry> ce;
     bool builder = false;
@@ -1874,7 +1883,7 @@ static int stream_bgzf(const char *entry, const uint8_t *bgzf, uint64_t nbytes, 
     for (size_t m = 0; m < coff.size();) {
         Slab sl{m, m, 0, coff[m], 0};
         while (sl.m1 < coff.size() && (sl.text == 0 || sl.text + olen[sl.m1] <= slab_bytes)) { sl.text += olen[sl.m1]; ++sl.m1; }
-        sl.comp = coff[sl.m1 - 1] + clen[sl.m1 - 1] - sl.comp0;
+        sl.comp = coff[sl.m1 - 1] + clen[sl.m1 - 1] + 8 - sl.comp0;   // through the last member's trailer (CRC32, ISIZE)
         if (sl.text) slabs.push_back(sl);
         text_cap = std::max(text_cap, sl.text); comp_cap = std::max(comp_cap, sl.comp); n_cap = std::max(n_cap, sl.m1 - sl.m0);
         m = sl.m1;
@@ -1927,8 +1936,10 @@ static int stream_bgzf(const char *entry, const uint8_t *bgzf, uint64_t nbytes, 
         if (e != cudaSuccess) break;
         const unsigned long long last_nl = s.h_pin[0];
         const int *status = reinterpret_cast<const int *>(s.h_pin + 1);
-        for (size_t i = 0; i < slabs[k].m1 - slabs[k].m0; ++i)
+        for (size_t i = 0; i < slabs[k].m1 - slabs[k].m0; ++i) {
+            if (status[i] == kInflateCrcMismatch) { rc = fail(HB_ERR_IO, bgzf_crc_message(bgzf, coff[slabs[k].m0 + i])); break; }
             if (status[i]) { rc = fail(HB_ERR_IO, "BGZF inflate failed (member " + std::to_string(slabs[k].m0 + i) + ", code " + std::to_string(status[i]) + ")"); break; }
+        }
         if (rc != HB_OK) break;
         const bool last = k + 1 == slabs.size();
         uint64_t parse_end;                                     // one past the last newline of the slab's text

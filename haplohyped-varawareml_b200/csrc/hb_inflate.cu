@@ -10,7 +10,10 @@
 //   * every lane then runs the same symbol loop on the same bit buffer (no divergence, no communication),
 //   * LZ77 copies are done by all 32 lanes (sources always precede the current output position, so the
 //     32-byte pieces of one match are independent), literals are stored by lane 0.
-// Stored and fixed-Huffman blocks are handled too.  CRC32 is not checked; ISIZE is.
+// Stored and fixed-Huffman blocks are handled too.  ISIZE is always checked.  CRC32 is checked when hb_set_bgzf_crc_check(1)
+// is in force (inflate_bgzf_kernel<true>): after a clean decode each lane takes the CRC of a contiguous slice of the member's
+// text, read back through L2 (slice-by-4 tables in shared memory), and a 5-level warp tree joins the 32 lane CRCs with
+// zlib's crc32_combine operator (multiplication by x^(8 n) mod P); the result is compared with the member's trailer.
 //
 // Round 2 tried to remove the 32-fold redundant decode (profiles/r02g_inflate_experiments.txt): a thread per member with
 // tables in shared memory and an aligned-word byte FIFO (bit-exact, 5 of 32 lanes active on average: copy paths diverge),
@@ -19,6 +22,7 @@
 // here).  Both lose to this kernel at the slab sizes the streaming path uses, so it stays; what was kept from them:
 // one aligned word per refill, length / distance bases computed instead of looked up, runs copied without a per-byte
 // modulo, loads of a match issued before its stores, 48 resident warps per SM.
+#include <atomic>
 #include <cstring>
 #include <mutex>
 #include <string>
@@ -165,15 +169,106 @@ struct InflateArgs {
     const uint32_t *olen;        // [n] ISIZE
     uint8_t *out;
     uint32_t n_blocks;
-    int *status;                 // [n] 0 = ok
+    int *status;                 // [n] 0 = ok; 19 = the text's CRC32 is not the trailer's (inflate_bgzf_kernel<true>)
 };
+
+// ---- CRC32 of a member's text (zlib's: reflected polynomial 0xEDB88320, x^0 = bit 31), for inflate_bgzf_kernel<true>
+constexpr uint32_t kCrcPoly = 0xEDB88320u;
+// a * b mod P (zlib's multmodp), as a fixed 32-step loop
+__host__ __device__ constexpr uint32_t crc_mulmod(uint32_t a, uint32_t b) {
+    uint32_t p = 0;
+    for (int k = 0; k < 32; ++k) {
+        p ^= b & (0u - (a >> 31));
+        a <<= 1;
+        b = (b >> 1) ^ (kCrcPoly & (0u - (b & 1u)));
+    }
+    return p;
+}
+// x^(8 n) mod P = lo[n % 256] * hi[n / 256] for n <= 65,536: one multiplication instead of zlib's one per set bit of n
+struct CrcShift { uint32_t lo[256], hi[257]; };
+constexpr CrcShift crc_shift_tables() {
+    CrcShift t{};
+    t.lo[0] = 0x80000000u;                                  // x^0
+    for (int n = 1; n < 256; ++n) t.lo[n] = crc_mulmod(t.lo[n - 1], 0x00800000u);   // * x^8
+    const uint32_t x2048 = crc_mulmod(t.lo[255], 0x00800000u);
+    t.hi[0] = 0x80000000u;
+    for (int j = 1; j < 257; ++j) t.hi[j] = crc_mulmod(t.hi[j - 1], x2048);
+    return t;
+}
+__device__ const CrcShift g_crc_shift = crc_shift_tables();
+// crc * x^(8 n) mod P: a CRC register followed by n zero bytes, the shift of zlib's crc32_combine
+__device__ __forceinline__ uint32_t crc_shift(uint32_t crc, uint32_t n) {
+    return crc_mulmod(crc_mulmod(__ldg(&g_crc_shift.lo[n & 255]), __ldg(&g_crc_shift.hi[n >> 8])), crc);
+}
+// one 32-bit little-endian word into the register (slice-by-4: t[k][b] = the register after byte b and k zero bytes)
+__device__ __forceinline__ uint32_t crc_word(uint32_t c, uint32_t w, const uint32_t (*t)[256]) {
+    c ^= w;
+    return t[3][c & 255] ^ t[2][(c >> 8) & 255] ^ t[1][(c >> 16) & 255] ^ t[0][c >> 24];
+}
+// CRC32 of out[0, olen), the warp together.  Lane L takes the bytes of [A0 + L S, A0 + (L + 1) S), A0 = out rounded down to 32
+// bytes, S a multiple of 32: aligned 16-byte loads through L2, bytes before `out` read as zeros (which leave a register that
+// starts at 0 unchanged), the last lane's ragged end byte by byte.  Lane registers start at 0 and are joined in a tree,
+// crc(A B) = crc(A) x^(8 |B|) + crc(B); zlib's initial and final inversions are applied to the joined value.
+__device__ uint32_t member_crc32(const uint8_t *out, uint32_t olen, const uint32_t (*t)[256]) {
+    const int lane = threadIdx.x & 31;
+    const uintptr_t a = reinterpret_cast<uintptr_t>(out), e = a + olen, a0 = a & ~uintptr_t(31);
+    const uint32_t S = ((uint32_t)(e - a0) + 1023u) / 1024u * 32u;
+    const uintptr_t lo = a0 + (uintptr_t)lane * S, hi = lo + S < e ? lo + S : e;
+    uint32_t c = 0, n = 0;
+    if (lo < e) {
+        n = (uint32_t)(hi - (lo > a ? lo : a));
+        for (uintptr_t p = lo; p < hi; p += 32) {
+            const uint4 *q = reinterpret_cast<const uint4 *>(p);
+            if (p >= a && p + 32 <= hi) {                  // whole chunk
+                const uint4 v0 = __ldcg(q), v1 = __ldcg(q + 1);
+                c = crc_word(c, v0.x, t); c = crc_word(c, v0.y, t); c = crc_word(c, v0.z, t); c = crc_word(c, v0.w, t);
+                c = crc_word(c, v1.x, t); c = crc_word(c, v1.y, t); c = crc_word(c, v1.z, t); c = crc_word(c, v1.w, t);
+                continue;
+            }
+            uint4 v[2] = {make_uint4(0, 0, 0, 0), make_uint4(0, 0, 0, 0)};
+#pragma unroll
+            for (int h = 0; h < 2; ++h)                    // only 16-byte pieces that hold member bytes are read
+                if (p + 16 * h + 16 > a && p + 16 * h < hi) v[h] = __ldcg(q + h);
+            const uint32_t w[8] = {v[0].x, v[0].y, v[0].z, v[0].w, v[1].x, v[1].y, v[1].z, v[1].w};
+#pragma unroll
+            for (int j = 0; j < 8; ++j) {
+                const uintptr_t wa = p + 4 * j;
+                if (wa >= hi) break;
+                uint32_t x = w[j];
+                if (wa + 4 <= a) x = 0;
+                else if (wa < a) x &= 0xFFFFFFFFu << (8 * (uint32_t)(a - wa));
+                if (wa + 4 <= hi) { c = crc_word(c, x, t); continue; }
+                for (uint32_t b = 0; wa + b < hi; ++b) c = (c >> 8) ^ t[0][(c ^ (x >> (8 * b))) & 255];
+            }
+        }
+    }
+    for (int d = 1; d < 32; d <<= 1) {
+        const uint32_t rc = __shfl_down_sync(0xffffffffu, c, d), rn = __shfl_down_sync(0xffffffffu, n, d);
+        if ((lane & (2 * d - 1)) == 0 && rn) { c = crc_shift(c, rn) ^ rc; n += rn; }
+    }
+    c = __shfl_sync(0xffffffffu, c, 0);
+    return ~(c ^ crc_shift(0xFFFFFFFFu, olen));
+}
 
 constexpr int kInfSmemPerWarp = 2 * (1 << kLitBits) + 2 * (1 << kDistBits) + 2 * 288 + 2 * 32 + 2 * 16 * 3 + 2 * 16 + 320 + 2 * 128 + 2 * 19 + 2 * 16 + 26;
 
+// kCrc: also check each member's CRC32 (4 KiB more shared memory per CTA: still 6 CTAs = 48 warps per SM)
+template <bool kCrc>
 __global__ void __launch_bounds__(kInfWarps * 32, 6) inflate_bgzf_kernel(const InflateArgs a) {
     __shared__ __align__(16) uint8_t smem[kInfWarps][(kInfSmemPerWarp + 15) & ~15];
+    __shared__ uint32_t crc_tab[kCrc ? 4 : 1][256];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const uint32_t blk = blockIdx.x * kInfWarps + warp;
+    if constexpr (kCrc) {                                  // slice-by-4 tables: thread i fills entry i of each
+        uint32_t c = threadIdx.x;
+#pragma unroll
+        for (int k = 0; k < 4; ++k) {
+#pragma unroll
+            for (int b = 0; b < 8; ++b) c = (c >> 1) ^ (kCrcPoly & (0u - (c & 1u)));
+            crc_tab[k][threadIdx.x] = c;
+        }
+        __syncthreads();
+    }
     if (blk >= a.n_blocks) return;
     uint8_t *sm = smem[warp];
     HuffTab lit, dist, cl;
@@ -315,7 +410,43 @@ __global__ void __launch_bounds__(kInfWarps * 32, 6) inflate_bgzf_kernel(const I
         __syncwarp();
     }
     if (!err && op != olen) err = 18;
+    if constexpr (kCrc) {                                  // err is the same in every lane
+        if (!err) {
+            const uint8_t *tr = src + br.n;                // the trailer: CRC32, ISIZE
+            const uint32_t want = (uint32_t)__ldg(tr) | (uint32_t)__ldg(tr + 1) << 8 | (uint32_t)__ldg(tr + 2) << 16 |
+                                  (uint32_t)__ldg(tr + 3) << 24;
+            if (member_crc32(out, olen, crc_tab) != want) err = kInflateCrcMismatch;
+        }
+    }
     if (lane == 0) a.status[blk] = err;
+}
+
+// hb_set_bgzf_crc_check: process-wide, off by default
+std::atomic<int> g_bgzf_crc{0};
+bool bgzf_crc_check() { return g_bgzf_crc.load() != 0; }
+
+// "BGZF CRC32 mismatch (member i, compressed offset X)" for the member whose DEFLATE payload starts at raw[coff]: i counts
+// every member of the file before it (empty ones too) and X is where its gzip header starts.  The headers up to it were
+// validated by bgzf_index.
+std::string bgzf_crc_message(const uint8_t *raw, uint64_t coff) {
+    uint64_t p = 0, i = 0;
+    for (;;) {
+        const uint8_t *h = raw + p;
+        const uint32_t xlen = h[10] | (h[11] << 8);
+        if (p + 12 + xlen >= coff) break;
+        uint32_t bsize = 0;
+        for (uint64_t q = p + 12; q + 4 <= p + 12 + xlen; q += 4 + (raw[q + 2] | (raw[q + 3] << 8)))
+            if (raw[q] == 'B' && raw[q + 1] == 'C') bsize = (raw[q + 4] | (raw[q + 5] << 8)) + 1;
+        p += bsize;
+        ++i;
+    }
+    return "BGZF CRC32 mismatch (member " + std::to_string(i) + ", compressed offset " + std::to_string(p) + ")";
+}
+
+static void launch_inflate(const InflateArgs &a, cudaStream_t stream) {
+    const uint32_t grid = (a.n_blocks + kInfWarps - 1) / kInfWarps;
+    if (bgzf_crc_check()) inflate_bgzf_kernel<true><<<grid, kInfWarps * 32, 0, stream>>>(a);
+    else inflate_bgzf_kernel<false><<<grid, kInfWarps * 32, 0, stream>>>(a);
 }
 
 // BGZF member table of a whole file (host): false when the bytes are not BGZF
@@ -405,7 +536,7 @@ int inflate_bgzf_to_device(const uint8_t *raw, uint64_t size, const std::vector<
         ck(cudaMemcpyAsync(d_olen, staged ? (const void *)h_olen : (const void *)olen.data(), n * 4ull, cudaMemcpyHostToDevice, stream));
         InflateArgs a{d_comp, d_coff, d_clen, d_ooff, d_olen, d_out, n, d_status};
         if (ms) { cudaEventCreate(&ev0); cudaEventCreate(&ev1); cudaEventRecord(ev0, stream); }
-        inflate_bgzf_kernel<<<(n + kInfWarps - 1) / kInfWarps, kInfWarps * 32, 0, stream>>>(a);
+        launch_inflate(a, stream);
         count_launch();
         if (ms) cudaEventRecord(ev1, stream);
         ck(cudaGetLastError());
@@ -418,8 +549,10 @@ int inflate_bgzf_to_device(const uint8_t *raw, uint64_t size, const std::vector<
     if (ev1) cudaEventDestroy(ev1);
     dev_pool_free(d_comp); dev_pool_free(d_coff); dev_pool_free(d_ooff); dev_pool_free(d_clen); dev_pool_free(d_olen); dev_pool_free(d_status);
     if (e != cudaSuccess) return api_fail(HB_ERR_CUDA, std::string("CUDA: ") + cudaGetErrorString(e));
-    for (uint32_t i = 0; i < n; ++i)
+    for (uint32_t i = 0; i < n; ++i) {
+        if (status[i] == kInflateCrcMismatch) return api_fail(HB_ERR_IO, bgzf_crc_message(raw, coff[i]));
         if (status[i]) return api_fail(HB_ERR_IO, "BGZF inflate failed (member " + std::to_string(i) + ", code " + std::to_string(status[i]) + ")");
+    }
     return HB_OK;
 }
 
@@ -455,7 +588,7 @@ int inflate_bgzf_enqueue(InflateScratch &sc, const uint8_t *comp, uint64_t comp_
     ck(cudaMemcpyAsync(sc.d_clen, clen, n * 4ull, cudaMemcpyHostToDevice, stream));
     ck(cudaMemcpyAsync(sc.d_olen, olen, n * 4ull, cudaMemcpyHostToDevice, stream));
     InflateArgs a{sc.d_comp, sc.d_coff, sc.d_clen, sc.d_ooff, sc.d_olen, d_out, n, sc.d_status};
-    inflate_bgzf_kernel<<<(n + kInfWarps - 1) / kInfWarps, kInfWarps * 32, 0, stream>>>(a);
+    launch_inflate(a, stream);
     count_launch();
     ck(cudaGetLastError());
     if (e != cudaSuccess) return api_fail(HB_ERR_CUDA, std::string("CUDA: ") + cudaGetErrorString(e));
@@ -511,3 +644,6 @@ extern "C" int hb_bgzf_inflate(const uint8_t *bgzf, uint64_t nbytes, uint8_t *ou
     cudaFree(d_out);
     return rc;
 }
+
+void hb_set_bgzf_crc_check(int on) { g_bgzf_crc.store(on ? 1 : 0); }
+int hb_get_bgzf_crc_check(void) { return g_bgzf_crc.load(); }

@@ -3,6 +3,8 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include <string>
+
 namespace hb {
 
 // Tile geometry shared by the tokenizer (checkpoints) and the GT decoder (sample tiles).
@@ -190,6 +192,10 @@ int inflate_scratch_alloc(InflateScratch &sc, uint64_t comp_cap, uint32_t n_cap)
 void inflate_scratch_free(InflateScratch &sc);
 int inflate_bgzf_enqueue(InflateScratch &sc, const uint8_t *comp, uint64_t comp_bytes, const uint64_t *coff, const uint32_t *clen,
                          const uint64_t *ooff, const uint32_t *olen, uint32_t n, uint8_t *d_out, cudaStream_t stream);
+// hb_set_bgzf_crc_check: kernel 0 compares each member's CRC32 with its trailer, and so does the host for the header members
+bool bgzf_crc_check();
+constexpr int kInflateCrcMismatch = 19;   // kernel 0 status of a member whose text does not match its CRC32
+std::string bgzf_crc_message(const uint8_t *raw, uint64_t coff);
 void launch_last_newline(const uint8_t *d_buf, uint64_t begin, uint64_t end, unsigned long long *d_res, cudaStream_t stream);
 
 }  // namespace hb

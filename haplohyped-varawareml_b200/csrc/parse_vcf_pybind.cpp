@@ -133,5 +133,7 @@ PYBIND11_MODULE(parse_vcf, m) {
               return VCFLoader().load_vcf_columns(f, s, c); },
           py::arg("in_vcf"), py::arg("sample") = "", py::arg("chrom") = "");
     m.def("cache_clear", &hb_cache_clear, "Drop the device-resident per-(file, region) parse cache");
+    m.def("set_bgzf_crc_check", [](bool on) { hb_set_bgzf_crc_check(on ? 1 : 0); }, py::arg("on"),
+          "Check the CRC32 of every BGZF member against its trailer, as htslib does (process-wide, off by default)");
     m.def("last_error", []() { return std::string(hb_last_error()); });
 }

@@ -17,9 +17,13 @@ Documented deviations (each replaces a crash or a silent loss in the reference, 
 a chromosome file that does not exist is skipped with a warning (the reference dereferences NULL);
 a donor that is not in the VCF header is reported and skipped (the reference's worker exception
 vanishes inside `executor.map`); `tmp_files/` is still created and removed but never used.
+
+`verify_crc=True` (CLI `--verify-crc`) checks the CRC32 of every BGZF member, as htslib's reader does
+(`capi.crc_check`); a file that fails it is skipped, counted and logged like any other unreadable file.
 """
 from __future__ import annotations
 
+import contextlib
 import logging
 import os
 import shutil
@@ -109,7 +113,7 @@ class _ChromParse:
 class VCFtoHDF5Converter:
     def __init__(self, cohort_name: str, vcf_dir: str, out_dir: str, sample_list_path: str, cores: int,
                  cxx_threads: int, device: int = 0, chromosomes=None, backend: Optional[str] = None,
-                 sample_window: Optional[int] = None, devices: Optional[List[int]] = None):
+                 sample_window: Optional[int] = None, devices: Optional[List[int]] = None, verify_crc: bool = False):
         self.cohort_name = cohort_name
         self.vcf_dir = vcf_dir
         self.out_dir = out_dir
@@ -124,6 +128,7 @@ class VCFtoHDF5Converter:
         self._wlock = threading.RLock()
         self.backend = backend
         self.sample_window = sample_window        # None: as many samples per frames pass as free HBM allows
+        self.verify_crc = verify_crc              # BGZF CRC32 check (process-wide while this converter parses)
         self.donor_ids = self.read_sample_list(sample_list_path)
         self.chromosomes = range(1, 23) if chromosomes is None else chromosomes
         self.tmp_dir = os.path.join(out_dir, "tmp_files")
@@ -156,11 +161,15 @@ class VCFtoHDF5Converter:
             for k, v in kw.items():
                 self.stats[k] += v
 
+    def _crc_scope(self):
+        return capi.crc_check(True) if self.verify_crc else contextlib.nullcontext()
+
     def _chrom_parse(self, data_path: str, chromosome: int, device: Optional[int] = None) -> _ChromParse:
         with self._wlock:
             cp = self._chrom.get(chromosome)
         if cp is None:
-            cp = _ChromParse(data_path, chromosome, self.device if device is None else device, self.sample_window)
+            with self._crc_scope():
+                cp = _ChromParse(data_path, chromosome, self.device if device is None else device, self.sample_window)
             with self._wlock:
                 self._chrom[chromosome] = cp
         return cp
@@ -242,23 +251,24 @@ class VCFtoHDF5Converter:
     def run(self):
         start_time = time.time()
         try:
-            # chromosome-major: one device-resident parse is shared by every donor.  `cores` host
-            # threads overlap the BGZF inflate of the next files with the GPU work of the current one.
-            present = [c for c in self.chromosomes
-                       if os.path.exists(os.path.join(self.vcf_dir, f"chr{c}.filtered.vcf.gz"))]
-            self.stats["skipped_files"] += len(list(self.chromosomes)) - len(present)
-            for c in self.chromosomes:
-                if c not in present:
-                    logger.warning(f"chr{c}.filtered.vcf.gz does not exist in {self.vcf_dir}; skipped")
-            if len(self.devices) > 1 and len(present) > 1:
-                self._run_devices(present)
-            else:
-                self._run_files(present, self.devices[0])
-            merge_start_time = time.time()
-            self.merge_h5_files()
-            end_time = time.time()
-            logger.info(f"Time taken to merge HDF5 files: {end_time - merge_start_time:.2f} seconds")
-            logger.info(f"Total time taken: {end_time - start_time:.2f} seconds")
+            with self._crc_scope():
+                # chromosome-major: one device-resident parse is shared by every donor.  `cores` host
+                # threads overlap the BGZF inflate of the next files with the GPU work of the current one.
+                present = [c for c in self.chromosomes
+                           if os.path.exists(os.path.join(self.vcf_dir, f"chr{c}.filtered.vcf.gz"))]
+                self.stats["skipped_files"] += len(list(self.chromosomes)) - len(present)
+                for c in self.chromosomes:
+                    if c not in present:
+                        logger.warning(f"chr{c}.filtered.vcf.gz does not exist in {self.vcf_dir}; skipped")
+                if len(self.devices) > 1 and len(present) > 1:
+                    self._run_devices(present)
+                else:
+                    self._run_files(present, self.devices[0])
+                merge_start_time = time.time()
+                self.merge_h5_files()
+                end_time = time.time()
+                logger.info(f"Time taken to merge HDF5 files: {end_time - merge_start_time:.2f} seconds")
+                logger.info(f"Total time taken: {end_time - start_time:.2f} seconds")
         except Exception as e:
             logger.error(f"An error occurred: {e}")
             raise
@@ -338,7 +348,9 @@ def main(argv=None):
     @click.option("--device", default=0, type=int, help="CUDA device ordinal")
     @click.option("--devices", default=None, type=str,
                   help="CUDA device ordinals, comma-separated (e.g. 0,1,2,3,4,5,6,7) or 'all': chromosome files are spread over them")
-    def _main(cohort_name, vcf, outdir, sample_list, cores, cxx_threads, device, devices):
+    @click.option("--verify-crc", "verify_crc", is_flag=True, default=False,
+                  help="Check the CRC32 of every BGZF member, as htslib does; a file that fails is skipped and logged")
+    def _main(cohort_name, vcf, outdir, sample_list, cores, cxx_threads, device, devices, verify_crc):
         _configure_logging()
         devs = None
         if devices:
@@ -348,7 +360,7 @@ def main(argv=None):
             else:
                 devs = [int(x) for x in devices.split(",") if x.strip() != ""]
         VCFtoHDF5Converter(cohort_name=cohort_name, vcf_dir=vcf, out_dir=outdir, sample_list_path=sample_list,
-                           cores=cores, cxx_threads=cxx_threads, device=device, devices=devs).run()
+                           cores=cores, cxx_threads=cxx_threads, device=device, devices=devs, verify_crc=verify_crc).run()
 
     return _main(args=argv, standalone_mode=argv is None)
 

@@ -258,6 +258,15 @@ int hb_frames_fetch_packed(hb_frames *f, uint8_t *buf, uint64_t cap, uint64_t *o
  * (0 = the CPUs the process may run on, at most 16). */
 void hb_set_fetch_mode(int mode);
 void hb_set_host_threads(int n);
+/* BGZF CRC32 check, process-wide, off by default.  On: every BGZF member (.vcf.gz and BGZF .bcf, on every route:
+ * hb_parse_file, hb_parse_vcf_bytes, hb_load_vcf, the streamed routes, hb_bgzf_inflate) has the CRC32 of its text compared
+ * with its gzip trailer, on the GPU inside the inflate kernel and on the host for the header members.  A mismatch fails
+ * with HB_ERR_IO and "BGZF CRC32 mismatch (member i, compressed offset X)", i and X positions in the whole file.  This is
+ * what htslib's BGZF reader does; off, a member whose DEFLATE stream is valid but whose bytes changed (any byte of a stored
+ * block, many in Huffman-coded data) is accepted as it is.  ISIZE is checked either way; plain gzip input goes through
+ * zlib, which always checks the CRC.  hb_load_vcf keeps parses made with the check on apart from those made with it off. */
+void hb_set_bgzf_crc_check(int on);
+int hb_get_bgzf_crc_check(void);
 /* bytes the last hb_frames_fetch_packed of this handle moved device -> host (frames or tails + headers + templates, + sizes) */
 uint64_t hb_frames_last_d2h_bytes(const hb_frames *f);
 /* sizes[n_chunks] of one sample's frames; then the frames themselves, concatenated without padding */
