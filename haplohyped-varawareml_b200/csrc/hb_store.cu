@@ -37,11 +37,39 @@
 
 namespace hb {
 
+extern __shared__ __align__(128) uint8_t smem[];     // the dynamic shared memory of the encoder kernels
 
 __device__ __forceinline__ uint32_t rd32(const uint8_t *p) {     // unaligned 4-byte read (shared memory)
     const uintptr_t a = reinterpret_cast<uintptr_t>(p);
     const uint32_t *w = reinterpret_cast<const uint32_t *>(a & ~uintptr_t(3));
     return __funnelshift_r(w[0], w[1], (uint32_t)(a & 3) * 8u);
+}
+
+// extension bytes of an LZ4 literal length (or of a match length - 4)
+__device__ __forceinline__ int lit_ext(int lit) { return lit >= 15 ? 1 + (lit - 15) / 255 : 0; }
+
+// one LZ4 sequence, written by the whole warp; returns the new output offset
+__device__ int warp_emit_seq(uint8_t *dst, int o, const uint8_t *lit, int litlen, int off, int ml) {
+    const int lane = threadIdx.x & 31;
+    if (lane == 0) dst[o] = (uint8_t)((min(litlen, 15) << 4) | min(ml - 4, 15));
+    ++o;
+    if (litlen >= 15) {
+        int rem = litlen - 15;
+        while (rem >= 255) { if (lane == 0) dst[o] = 255; ++o; rem -= 255; }
+        if (lane == 0) dst[o] = (uint8_t)rem;
+        ++o;
+    }
+    for (int i = lane; i < litlen; i += 32) dst[o + i] = lit[i];
+    o += litlen;
+    if (lane == 0) { dst[o] = (uint8_t)off; dst[o + 1] = (uint8_t)(off >> 8); }
+    o += 2;
+    if (ml - 4 >= 15) {
+        int rem = ml - 19;
+        while (rem >= 255) { if (lane == 0) dst[o] = 255; ++o; rem -= 255; }
+        if (lane == 0) dst[o] = (uint8_t)rem;
+        ++o;
+    }
+    return o;
 }
 
 // Warp-cooperative LZ4 encoder of one SEGMENT src[0..n) of a block whose earlier bytes (`hist` of them) sit right
@@ -118,28 +146,8 @@ __device__ int warp_lz4_segment(const uint8_t *src, int n, int hist, uint8_t *ds
             break;
         }
         const int litlen = m - anchor;
-        int o = op;
-        if (lane == 0) dst[o] = (uint8_t)((min(litlen, 15) << 4) | min(ml - 4, 15));
-        ++o;
-        if (litlen >= 15) {
-            int rem = litlen - 15;
-            while (rem >= 255) { if (lane == 0) dst[o] = 255; ++o; rem -= 255; }
-            if (lane == 0) dst[o] = (uint8_t)rem;
-            ++o;
-        }
-        if (op == 0) { *first_lit = litlen; *first_hdr = o; }
-        for (int i = lane; i < litlen; i += 32) dst[o + i] = src[anchor + i];
-        o += litlen;
-        const int off = m - c;
-        if (lane == 0) { dst[o] = (uint8_t)off; dst[o + 1] = (uint8_t)(off >> 8); }
-        o += 2;
-        if (ml - 4 >= 15) {
-            int rem = ml - 19;
-            while (rem >= 255) { if (lane == 0) dst[o] = 255; ++o; rem -= 255; }
-            if (lane == 0) dst[o] = (uint8_t)rem;
-            ++o;
-        }
-        op = o;
+        if (op == 0) { *first_lit = litlen; *first_hdr = op + 1 + lit_ext(litlen); }
+        op = warp_emit_seq(dst, op, src + anchor, litlen, m - c, ml);
         anchor = pos = m + ml;
     }
     *pending = n - anchor;
@@ -169,8 +177,10 @@ __device__ int warp_lz4_segment(const uint8_t *src, int n, int hist, uint8_t *ds
 //                          TMA bulk stores (template body from the shared copy, own tail) + two 16-byte header
 //                          vectors with the size fields filled in.  C_out is written exactly once.
 //   site_template_large_kernel / donor_frames_large_kernel   the same frames for chunks of 2,731 - 7,489 records (still ONE
-//                          Blosc block): site planes in a global scratch, allele tails in passes, template read from
-//                          global memory.  The host picks the pair from cr; below 2,731 nothing changes.
+//                          Blosc block), built by the same encoder helpers (site_encode_chunk; build_bit_strings,
+//                          parse_lane, scan_offsets, emit_lane, closing_literals).  What differs: site planes in a global
+//                          scratch, allele tails in passes, template read from global memory.  The host picks the pair
+//                          from cr.
 // Output: ONE buffer of slots in [sample][chunk] order.  The slot of (sample s, chunk c) starts at
 // s * row_stride + slot_off[c]; slot_off is the running sum of round16(template_len[c] + worst-case
 // allele tail), so every frame's address is known before it is encoded (no scan, no look-back) and the
@@ -191,29 +201,9 @@ __device__ void write_frame_head(uint8_t *h, uint32_t nbytes) {
     put_le32(h + 16, BLOSC_HDR + 4);                         // bstarts[0]
 }                                                            // csize @20: patched
 
-// one LZ4 sequence, written by the whole warp; returns the new output offset
-__device__ int warp_emit_seq(uint8_t *dst, int o, const uint8_t *lit, int litlen, int off, int ml) {
-    const int lane = threadIdx.x & 31;
-    if (lane == 0) dst[o] = (uint8_t)((min(litlen, 15) << 4) | min(ml - 4, 15));
-    ++o;
-    if (litlen >= 15) {
-        int rem = litlen - 15;
-        while (rem >= 255) { if (lane == 0) dst[o] = 255; ++o; rem -= 255; }
-        if (lane == 0) dst[o] = (uint8_t)rem;
-        ++o;
-    }
-    for (int i = lane; i < litlen; i += 32) dst[o + i] = lit[i];
-    o += litlen;
-    if (lane == 0) { dst[o] = (uint8_t)off; dst[o + 1] = (uint8_t)(off >> 8); }
-    o += 2;
-    if (ml - 4 >= 15) {
-        int rem = ml - 19;
-        while (rem >= 255) { if (lane == 0) dst[o] = 255; ++o; rem -= 255; }
-        if (lane == 0) dst[o] = (uint8_t)rem;
-        ++o;
-    }
-    return o;
-}
+// byte offsets of the fields of a 35-byte record (plane f of a shuffled chunk holds byte f of every record): CHROM's
+// first 5 bytes at 0, start and stop as LE32, REF and ALT as the first bytes of their 10-byte fields, the two alleles
+constexpr uint32_t kRecStart = 5, kRecStop = 9, kRecRef = 13, kRecAlt = 23, kRecP1 = 33, kRecP2 = 34;
 
 struct SiteArgs4 {
     const uint64_t *chrom5;      // per record: first 5 CHROM bytes, NUL padded, in the low 40 bits
@@ -259,17 +249,12 @@ __host__ __device__ inline uint32_t site_seg_begin(int s, uint32_t cr) {
     }
 }
 
-__global__ void __launch_bounds__(kSiteSegs * 32) site_template_kernel(const SiteArgs4 a) {
-    extern __shared__ __align__(16) uint8_t smem[];
-    __shared__ int s_len[kSiteSegs], s_pend[kSiteSegs], s_flit[kSiteSegs], s_fhdr[kSiteSegs];
-    __shared__ int s_dst[kSiteSegs], s_carry[kSiteSegs], s_final[2];
-    __shared__ uint8_t s_head[TMPL_HDR + 7];
+// ---- The site-template encoder shared by site_template_kernel and site_template_large_kernel.
+
+// site planes 0..23 of chunk c: CHROM, start, stop, REF and its nine zero planes, ALT's first byte.  Planes 24..32 (ALT
+// bytes 1..9) are zero too; the caller clears them.
+__device__ __forceinline__ void site_planes_fill(const SiteArgs4 &a, uint64_t c, uint8_t *planes) {
     const uint32_t cr = a.cr;
-    const uint32_t n = 33u * cr;
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    uint8_t *planes = smem + 16;                            // 16 zero bytes of history in front
-    uint8_t *outs = planes + ((n + 19) & ~15u);             // per-segment output regions
-    const uint64_t c = blockIdx.x;
     const uint64_t r0 = c * cr;
     for (uint32_t i = threadIdx.x; i < cr; i += blockDim.x) {
         const uint64_t r = r0 + i;
@@ -281,60 +266,61 @@ __global__ void __launch_bounds__(kSiteSegs * 32) site_template_kernel(const Sit
         for (int k = 0; k < 5; ++k) planes[k * cr + i] = (uint8_t)(ch >> (8 * k));
 #pragma unroll
         for (int k = 0; k < 4; ++k) {
-            planes[(5 + k) * cr + i] = (uint8_t)(st >> (8 * k));
-            planes[(9 + k) * cr + i] = (uint8_t)(sp >> (8 * k));
+            planes[(kRecStart + k) * cr + i] = (uint8_t)(st >> (8 * k));
+            planes[(kRecStop + k) * cr + i] = (uint8_t)(sp >> (8 * k));
         }
-        planes[13 * cr + i] = rf;
-        planes[23 * cr + i] = al;
+        planes[kRecRef * cr + i] = rf;
+        planes[kRecAlt * cr + i] = al;
 #pragma unroll
-        for (int k = 0; k < 9; ++k) { planes[(14 + k) * cr + i] = 0; planes[(24 + k) * cr + i] = 0; }
+        for (int k = 1; k < 10; ++k) planes[(kRecRef + k) * cr + i] = 0;
     }
-    if (threadIdx.x < 16) smem[threadIdx.x] = 0;
-    if (threadIdx.x == 0) write_frame_head(s_head, 35u * cr);
-    __syncthreads();
-    uint8_t *g = a.tmpl + c * a.tmpl_cap;
-    // Chunks of fewer than 6 records cannot honour LZ4's end-of-block rules (last match >= 12 bytes
-    // before the end) once the 2*cr allele bytes follow: such blocks are stored raw (csize == size).
-    if (cr < 6) {
-        for (uint32_t i = threadIdx.x; i < TMPL_HDR; i += blockDim.x) g[i] = s_head[i];
-        for (uint32_t i = threadIdx.x; i < n; i += blockDim.x) g[TMPL_HDR + i] = planes[i];
-        const uint32_t tl = TMPL_HDR + n;
-        for (uint32_t i = tl + threadIdx.x; i < ((tl + 15) & ~15u); i += blockDim.x) g[i] = 0;
-        if (threadIdx.x == 0) a.tmpl_len[c] = tl;
-        return;
-    }
-    // Planes 24..32 (ALT bytes 1..9) are all zero: the head is encoded up to the first of those zeros, then ONE
-    // offset-1 match covers the other 9*cr-1 -- so the site part always ends on a sequence boundary and every donor
-    // continues the block with nothing pending and zeros behind it.  The head is cut into kSiteSegs segments, one
-    // per warp, encoded independently (own hash table; the fixed-distance candidates reach back across segments).
+}
+
+// per-segment results and the stitch of one chunk (static shared memory of both site kernels)
+struct SiteStitch {
+    int len[kSiteSegs], pend[kSiteSegs], flit[kSiteSegs], fhdr[kSiteSegs];     // warp_lz4_segment's, per segment
+    int dst[kSiteSegs], carry[kSiteSegs];        // where the segment's output goes; literals carried into it
+    int final_off, final_carry;                  // end of the stitched head; literals left behind it
+    uint8_t head[TMPL_HDR];                      // write_frame_head's bytes
+};
+
+// Chunk c's planes (16 zero bytes of history in front of them, planes 24..32 zero) -> its template and tmpl_len[c];
+// `head` is written and the CTA synchronised before the call.  Planes 24..32 (ALT bytes 1..9) are all zero: the head
+// is encoded up to the first of those zeros, then ONE offset-1 match covers the other 9*cr-1 -- so the site part always
+// ends on a sequence boundary and every donor continues the block with nothing pending and zeros behind it.  The head
+// is cut into kSiteSegs segments, one per warp, encoded independently into the warp's region of `outs` (own hash
+// table; the fixed-distance candidates reach back across segments) and then stitched back to back.
+__device__ __forceinline__ void site_encode_chunk(const SiteArgs4 &a, uint64_t c, const uint8_t *planes, uint8_t *outs,
+                                                  uint16_t *table, SiteStitch &S) {
+    const uint32_t cr = a.cr, n = 33u * cr;
     const int n1 = 24 * (int)cr + 1;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int sb = (int)site_seg_begin(warp, cr), se = (int)site_seg_begin(warp + 1, cr);
     uint32_t out_off = 0;
     for (int w = 0; w < warp; ++w) out_off += site_seg_cap(site_seg_begin(w + 1, cr) - site_seg_begin(w, cr));
     uint8_t *my_out = outs + out_off;
-    uint16_t *table = reinterpret_cast<uint16_t *>(outs + ((site_seg_cap((uint32_t)n1) + kSiteSegs * 48 + 15) & ~15u)) + ((size_t)warp << kSiteHashLog);
     {
         int flit, fhdr, pend;
         const int len = warp_lz4_segment(planes + sb, se - sb, sb, my_out, table, kSiteHashLog, 4 * (int)cr, a.deep != 0, &flit, &fhdr, &pend);
-        if (lane == 0) { s_len[warp] = len; s_pend[warp] = pend; s_flit[warp] = flit; s_fhdr[warp] = fhdr; }
+        if (lane == 0) { S.len[warp] = len; S.pend[warp] = pend; S.flit[warp] = flit; S.fhdr[warp] = fhdr; }
     }
     __syncthreads();
     if (threadIdx.x == 0) {                       // stitch: literals left over by a segment open the next one's first sequence
         int carry = 0, off = 0;
         for (int w = 0; w < kSiteSegs; ++w) {
-            s_dst[w] = off; s_carry[w] = carry;
-            if (s_len[w] == 0) { carry += s_pend[w]; continue; }
-            const int lit = s_flit[w] + carry;
-            off += 1 + (lit >= 15 ? 1 + (lit - 15) / 255 : 0) + carry + (s_len[w] - s_fhdr[w]);
-            carry = s_pend[w];
+            S.dst[w] = off; S.carry[w] = carry;
+            if (S.len[w] == 0) { carry += S.pend[w]; continue; }
+            off += 1 + lit_ext(S.flit[w] + carry) + carry + (S.len[w] - S.fhdr[w]);
+            carry = S.pend[w];
         }
-        s_final[0] = off; s_final[1] = carry;
+        S.final_off = off; S.final_carry = carry;
     }
     __syncthreads();
+    uint8_t *g = a.tmpl + c * a.tmpl_cap;
     uint8_t *lz = g + TMPL_HDR;
-    if (s_len[warp] > 0) {
-        const int carry = s_carry[warp], lit = s_flit[warp] + carry;
-        int o = s_dst[warp];
+    if (S.len[warp] > 0) {                        // the segment's first sequence, re-written with the carried literals
+        const int carry = S.carry[warp], lit = S.flit[warp] + carry;
+        int o = S.dst[warp];
         if (lane == 0) lz[o] = (uint8_t)((min(lit, 15) << 4) | (my_out[0] & 15));
         ++o;
         if (lit >= 15) {
@@ -345,28 +331,58 @@ __global__ void __launch_bounds__(kSiteSegs * 32) site_template_kernel(const Sit
         }
         for (int i = lane; i < carry; i += 32) lz[o + i] = planes[sb - carry + i];
         o += carry;
-        const int rest = s_len[warp] - s_fhdr[warp];
-        for (int i = lane; i < rest; i += 32) lz[o + i] = my_out[s_fhdr[warp] + i];
+        const int rest = S.len[warp] - S.fhdr[warp];
+        for (int i = lane; i < rest; i += 32) lz[o + i] = my_out[S.fhdr[warp] + i];
     }
-    int o = s_final[0];
-    if (warp == 0) o = warp_emit_seq(lz, o, planes + n1 - s_final[1], s_final[1], 1, (int)n - n1);
-    else o = o + 1 + (s_final[1] >= 15 ? 1 + (s_final[1] - 15) / 255 : 0) + s_final[1] + 2 + ((int)n - n1 >= 19 ? 1 + ((int)n - n1 - 19) / 255 : 0);
+    const int fl = S.final_carry;
+    int o = S.final_off;
+    if (warp == 0) o = warp_emit_seq(lz, o, planes + n1 - fl, fl, 1, (int)n - n1);
+    else o += 1 + lit_ext(fl) + fl + 2 + lit_ext((int)n - n1 - 4);
     const uint32_t tl = TMPL_HDR + (uint32_t)o;
-    for (uint32_t i = threadIdx.x; i < TMPL_HDR; i += blockDim.x) g[i] = s_head[i];
+    for (uint32_t i = threadIdx.x; i < TMPL_HDR; i += blockDim.x) g[i] = S.head[i];
     for (uint32_t i = tl + threadIdx.x; i < ((tl + 15) & ~15u); i += blockDim.x) g[i] = 0;
     if (threadIdx.x == 0) a.tmpl_len[c] = tl;
+}
+
+__global__ void __launch_bounds__(kSiteSegs * 32) site_template_kernel(const SiteArgs4 a) {
+    __shared__ SiteStitch S;
+    const uint32_t cr = a.cr;
+    const uint32_t n = 33u * cr;
+    const int warp = threadIdx.x >> 5;
+    uint8_t *planes = smem + 16;                            // 16 zero bytes of history in front
+    uint8_t *outs = planes + ((n + 19) & ~15u);             // per-segment output regions, then the hash tables
+    uint16_t *table = reinterpret_cast<uint16_t *>(outs + ((site_seg_cap(24 * cr + 1) + kSiteSegs * 48 + 15) & ~15u)) + ((size_t)warp << kSiteHashLog);
+    const uint64_t c = blockIdx.x;
+    site_planes_fill(a, c, planes);
+    for (uint32_t i = 24 * cr + threadIdx.x; i < n; i += blockDim.x) planes[i] = 0;
+    if (threadIdx.x < 16) smem[threadIdx.x] = 0;
+    if (threadIdx.x == 0) write_frame_head(S.head, 35u * cr);
+    __syncthreads();
+    // Chunks of fewer than 6 records cannot honour LZ4's end-of-block rules (last match >= 12 bytes
+    // before the end) once the 2*cr allele bytes follow: such blocks are stored raw (csize == size).
+    if (cr < 6) {
+        uint8_t *g = a.tmpl + c * a.tmpl_cap;
+        for (uint32_t i = threadIdx.x; i < TMPL_HDR; i += blockDim.x) g[i] = S.head[i];
+        for (uint32_t i = threadIdx.x; i < n; i += blockDim.x) g[TMPL_HDR + i] = planes[i];
+        const uint32_t tl = TMPL_HDR + n;
+        for (uint32_t i = tl + threadIdx.x; i < ((tl + 15) & ~15u); i += blockDim.x) g[i] = 0;
+        if (threadIdx.x == 0) a.tmpl_len[c] = tl;
+        return;
+    }
+    site_encode_chunk(a, c, planes, outs, table, S);
 }
 
 // ------------------------------------------------------------------------------------------
 // Kernel 4a-L: the site templates of chunks of kSmallChunkMax < cr <= kMaxChunkRecords records.  Up to 7,489 records
 // such a chunk is still ONE Blosc block with ONE LZ4 stream (c-blosc 1.x cuts blocks of 262,115 bytes for typesize 35
-// at clevel 5 with LZ4HC), so the template has exactly the layout of site_template_kernel's: the same segments, the
-// same matcher, the same stitch, the same closing offset-1 match over planes 24-32.  What changes is where the bytes
-// live: 33 * cr bytes of planes no longer fit shared memory, so the head [0, 24 * cr + 1) that is encoded and the
-// per-segment outputs sit in a per-CTA global scratch (L2-resident: ~2 * 24 * cr bytes per CTA), and only the hash
-// tables stay in shared memory.  The 16-bit table entries still hold: positions are relative to a segment, and the
-// longest segment (the five CHROM planes) is 5 * 7,489 < 65,535 bytes; far = 4 * cr and 2 * cr are legal LZ4 offsets.
-// The grid is smaller than the chunk count (the scratch is per CTA): CTA b encodes chunks b, b + gridDim.x, ...
+// at clevel 5 with LZ4HC), so the template has exactly the layout of site_template_kernel's, and both kernels encode it
+// with site_planes_fill and site_encode_chunk: the same segments, matcher, stitch and closing offset-1 match over
+// planes 24-32.  What differs is where the bytes live: 33 * cr bytes of planes no longer fit shared memory, so the head
+// [0, 24 * cr + 1) that is encoded and the per-segment outputs sit in a per-CTA global scratch (L2-resident:
+// ~2 * 24 * cr bytes per CTA), and only the hash tables stay in shared memory.  The 16-bit table entries still hold:
+// positions are relative to a segment, and the longest segment (the five CHROM planes) is 5 * 7,489 < 65,535 bytes;
+// far = 4 * cr and 2 * cr are legal LZ4 offsets.  The grid is smaller than the chunk count (the scratch is per CTA):
+// CTA b encodes chunks b, b + gridDim.x, ...
 // ------------------------------------------------------------------------------------------
 constexpr uint32_t kSmallChunkMax = 2730;        // largest chunk of site_template_kernel / donor_frames_kernel
 constexpr uint32_t kMaxChunkRecords = 7489;      // largest chunk that is ONE c-blosc 1.x block at typesize 35
@@ -377,89 +393,20 @@ __host__ __device__ inline uint32_t site_large_scratch(uint32_t cr) {
 }
 
 __global__ void __launch_bounds__(kSiteSegs * 32) site_template_large_kernel(const SiteArgs4 a, uint8_t *scratch) {
-    extern __shared__ __align__(16) uint8_t smem[];
-    __shared__ int s_len[kSiteSegs], s_pend[kSiteSegs], s_flit[kSiteSegs], s_fhdr[kSiteSegs];
-    __shared__ int s_dst[kSiteSegs], s_carry[kSiteSegs], s_final[2];
-    __shared__ uint8_t s_head[TMPL_HDR + 7];
+    __shared__ SiteStitch S;
     const uint32_t cr = a.cr;
-    const uint32_t n = 33u * cr;
-    const int n1 = 24 * (int)cr + 1;
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int warp = threadIdx.x >> 5;
     uint8_t *planes = scratch + (size_t)blockIdx.x * site_large_scratch(cr) + 16;   // 16 zero bytes of history in front
     uint8_t *outs = planes - 16 + site_large_head_bytes(cr);
     uint16_t *table = reinterpret_cast<uint16_t *>(smem) + ((size_t)warp << kSiteHashLog);
-    const int sb = (int)site_seg_begin(warp, cr), se = (int)site_seg_begin(warp + 1, cr);
-    uint32_t out_off = 0;
-    for (int w = 0; w < warp; ++w) out_off += site_seg_cap(site_seg_begin(w + 1, cr) - site_seg_begin(w, cr));
-    uint8_t *my_out = outs + out_off;
     const uint64_t n_chunks = (a.n_records + cr - 1) / cr;
     if (threadIdx.x < 16) planes[(int)threadIdx.x - 16] = 0;
-    for (uint32_t i = 24 * cr + threadIdx.x; i < (uint32_t)n1 + kSitePad; i += blockDim.x) planes[i] = 0;   // planes 24.. are zero
-    if (threadIdx.x == 0) write_frame_head(s_head, 35u * cr);
+    for (uint32_t i = 24 * cr + threadIdx.x; i < 24 * cr + 1 + kSitePad; i += blockDim.x) planes[i] = 0;   // planes 24.. are zero
+    if (threadIdx.x == 0) write_frame_head(S.head, 35u * cr);
     for (uint64_t c = blockIdx.x; c < n_chunks; c += gridDim.x) {
-        const uint64_t r0 = c * cr;
-        for (uint32_t i = threadIdx.x; i < cr; i += blockDim.x) {
-            const uint64_t r = r0 + i;
-            uint64_t ch = 0;
-            uint32_t st = 0, sp = 0;
-            uint8_t rf = 0, al = 0;
-            if (r < a.n_records) { ch = a.chrom5[r]; st = a.start[r]; sp = a.stop[r]; rf = a.ref[r]; al = a.alt[r]; }
-#pragma unroll
-            for (int k = 0; k < 5; ++k) planes[k * cr + i] = (uint8_t)(ch >> (8 * k));
-#pragma unroll
-            for (int k = 0; k < 4; ++k) {
-                planes[(5 + k) * cr + i] = (uint8_t)(st >> (8 * k));
-                planes[(9 + k) * cr + i] = (uint8_t)(sp >> (8 * k));
-            }
-            planes[13 * cr + i] = rf;
-            planes[23 * cr + i] = al;
-#pragma unroll
-            for (int k = 0; k < 9; ++k) planes[(14 + k) * cr + i] = 0;
-        }
+        site_planes_fill(a, c, planes);
         __syncthreads();
-        {
-            int flit, fhdr, pend;
-            const int len = warp_lz4_segment(planes + sb, se - sb, sb, my_out, table, kSiteHashLog, 4 * (int)cr, a.deep != 0, &flit, &fhdr, &pend);
-            if (lane == 0) { s_len[warp] = len; s_pend[warp] = pend; s_flit[warp] = flit; s_fhdr[warp] = fhdr; }
-        }
-        __syncthreads();
-        if (threadIdx.x == 0) {                   // stitch, as in site_template_kernel
-            int carry = 0, off = 0;
-            for (int w = 0; w < kSiteSegs; ++w) {
-                s_dst[w] = off; s_carry[w] = carry;
-                if (s_len[w] == 0) { carry += s_pend[w]; continue; }
-                const int lit = s_flit[w] + carry;
-                off += 1 + (lit >= 15 ? 1 + (lit - 15) / 255 : 0) + carry + (s_len[w] - s_fhdr[w]);
-                carry = s_pend[w];
-            }
-            s_final[0] = off; s_final[1] = carry;
-        }
-        __syncthreads();
-        uint8_t *g = a.tmpl + c * a.tmpl_cap;
-        uint8_t *lz = g + TMPL_HDR;
-        if (s_len[warp] > 0) {
-            const int carry = s_carry[warp], lit = s_flit[warp] + carry;
-            int o = s_dst[warp];
-            if (lane == 0) lz[o] = (uint8_t)((min(lit, 15) << 4) | (my_out[0] & 15));
-            ++o;
-            if (lit >= 15) {
-                int rem = lit - 15;
-                while (rem >= 255) { if (lane == 0) lz[o] = 255; ++o; rem -= 255; }
-                if (lane == 0) lz[o] = (uint8_t)rem;
-                ++o;
-            }
-            for (int i = lane; i < carry; i += 32) lz[o + i] = planes[sb - carry + i];
-            o += carry;
-            const int rest = s_len[warp] - s_fhdr[warp];
-            for (int i = lane; i < rest; i += 32) lz[o + i] = my_out[s_fhdr[warp] + i];
-        }
-        int o = s_final[0];
-        if (warp == 0) o = warp_emit_seq(lz, o, planes + n1 - s_final[1], s_final[1], 1, (int)n - n1);
-        else o = o + 1 + (s_final[1] >= 15 ? 1 + (s_final[1] - 15) / 255 : 0) + s_final[1] + 2 + ((int)n - n1 >= 19 ? 1 + ((int)n - n1 - 19) / 255 : 0);
-        const uint32_t tl = TMPL_HDR + (uint32_t)o;
-        for (uint32_t i = threadIdx.x; i < TMPL_HDR; i += blockDim.x) g[i] = s_head[i];
-        for (uint32_t i = tl + threadIdx.x; i < ((tl + 15) & ~15u); i += blockDim.x) g[i] = 0;
-        if (threadIdx.x == 0) a.tmpl_len[c] = tl;
+        site_encode_chunk(a, c, planes, outs, table, S);
         __syncthreads();                          // the scratch and the stitch table are re-used by the next chunk
     }
 }
@@ -487,7 +434,6 @@ constexpr int kFramesPerWarp = 8;             // frames (samples of one chunk) a
 
 __device__ __forceinline__ uint32_t low_mask(int n) { return n <= 0 ? 0u : (n >= 32 ? 0xFFFFFFFFu : ((1u << n) - 1u)); }
 __device__ __forceinline__ int ctz32(uint32_t v) { return __clz(__brev(v)); }       // 32 for 0
-__device__ __forceinline__ int lit_ext(int lit) { return lit >= 15 ? 1 + (lit - 15) / 255 : 0; }
 // bits 0..3 of b -> bytes 0..3 (0 / 1)
 __device__ __forceinline__ uint32_t spread4(uint32_t b) { return ((b & 0xFu) * 0x00204081u) & 0x01010101u; }
 
@@ -552,9 +498,321 @@ struct FusedArgs {
                          // literals instead (cr 1075: 64 instead of 68 per lane, 102 of 2150 positions; +0.5 % frame size)
 };
 
+// ---- The allele-tail encoder shared by donor_frames_kernel and donor_frames_large_kernel: steps 1, 2, 3 and 5 and the
+//      closing literals of one frame, run by one warp.
+
+// One frame's allele bytes: block position x (0 .. 2 * cr) is bit alpha + x of the bit strings B and N; a byte with N set
+// is read from the byte planes, row grow + x of gt0 for x < cr and row grow + x - cr of gt1 otherwise.
+struct AlleleBits {
+    const uint32_t *strB, *strN;
+    bool any_n;                          // some allele of the frame is neither 0 nor 1: strN is valid
+    int alpha, cr;
+    const int8_t *gt0, *gt1;
+    uint64_t grow;
+    __device__ __forceinline__ uint32_t byte(int x) const { return (uint8_t)(x < cr ? gt0 : gt1)[grow + (x < cr ? x : x - cr)]; }
+};
+
+// ---- 1. this frame's slices of the bit planes (staged by TMA, words [0, nwst) of each array) -> ONE bit string each for
+//         B and N over both planes, so the parse and the literal emission walk from plane 0 into plane 1 without a seam.
+//         Rows outside [r0, r0 + valid) belong to other chunks (or to nobody) and are masked off in the staging area.
+//         Returns any_n; strN is written only when it is set.
+__device__ __forceinline__ bool build_bit_strings(uint32_t *stage, uint32_t *strB, uint32_t *strN, int nwst, int strw, int alpha,
+                                                  int valid, int cr) {
+    const int lane = threadIdx.x & 31;
+    const int sh = cr & 31, wsh = cr >> 5;       // plane 1 sits cr bits above plane 0 in the strings
+    uint32_t nacc = 0;
+    for (int w = lane; w < nwst; w += 32) {
+        const uint32_t mk = low_mask(alpha + valid - 32 * w) & ~low_mask(alpha - 32 * w);
+        uint32_t *gq = stage + (w >> 2) * kBitGroupWords + (w & 3);
+        if (mk != 0xFFFFFFFFu) { gq[0] &= mk; gq[4] &= mk; gq[8] &= mk; gq[12] &= mk; }
+        nacc |= gq[8] | gq[12];
+    }
+    const bool any_n = __any_sync(0xffffffffu, nacc != 0);
+    __syncwarp();
+    for (int k = lane; k < strw; k += 32) {
+        const int j = k - wsh;
+        uint32_t b = 0, b1lo = 0, b1hi = 0;
+        if (k < nwst) b = stage[(k >> 2) * kBitGroupWords + (k & 3)];
+        if (j >= 1 && j <= nwst) b1lo = stage[((j - 1) >> 2) * kBitGroupWords + 4 + ((j - 1) & 3)];
+        if (j >= 0 && j < nwst) b1hi = stage[(j >> 2) * kBitGroupWords + 4 + (j & 3)];
+        strB[k] = b | __funnelshift_l(b1lo, b1hi, sh);
+        if (any_n) {
+            uint32_t x = 0, x1lo = 0, x1hi = 0;
+            if (k < nwst) x = stage[(k >> 2) * kBitGroupWords + 8 + (k & 3)];
+            if (j >= 1 && j <= nwst) x1lo = stage[((j - 1) >> 2) * kBitGroupWords + 12 + ((j - 1) & 3)];
+            if (j >= 0 && j < nwst) x1hi = stage[(j >> 2) * kBitGroupWords + 12 + (j & 3)];
+            strN[k] = x | __funnelshift_l(x1lo, x1hi, sh);
+        }
+    }
+    fence_proxy_async();                        // the staging area was masked in place: order that before the copy engine's writes
+    __syncwarp();
+    return any_n;
+}
+
+// what the parse of a lane's segment leaves for the scans and the emission
+template <int NW>
+struct LaneParse {
+    uint32_t Rp[NW], K[NW];              // match cover without the last position of each run; C-run cover (match type)
+    int m;                               // matches that start in the segment
+    int matched;                         // positions covered by them
+    int prev_end;                        // end of the last match (0: none)
+    int first_lit;                       // literals in front of the first match
+    int n_ext;                           // extension bytes of literal runs >= 15 and matches >= 19
+    int trail;                           // literals behind the last match (carried into the next sequence)
+};
+
+// ---- 2. per-lane parse of the segment [x0, x0 + seg) of the block, position-parallel
+template <int NW>
+__device__ __forceinline__ void parse_lane(const AlleleBits &ab, int x0, int seg, LaneParse<NW> &P) {
+    const uint32_t *strB = ab.strB, *strN = ab.strN;
+    const bool any_n = ab.any_n;
+    const int cr = ab.cr, n = 2 * cr;
+    const int seglen = max(0, min(seg, n - x0));
+    const int mlim = min(seglen, n - 11 - x0);                    // the last 11 bytes of the block stay literals
+    const int bi = ab.alpha + x0, j0 = bi >> 5, shb = bi & 31;
+    const int ci = bi - cr, jc = ci >> 5, shc = ci & 31;          // the same rows in plane 0 (positions >= cr only)
+    uint32_t Z[NW], C[NW], ZR[NW], S[NW], E[NW];
+#pragma unroll
+    for (int k = 0; k < NW; ++k) {
+        const uint32_t bw = __funnelshift_r(strB[j0 + k], strB[j0 + k + 1], shb);
+        const uint32_t nw = any_n ? __funnelshift_r(strN[j0 + k], strN[j0 + k + 1], shb) : 0u;
+        const uint32_t vm = low_mask(mlim - 32 * k);
+        Z[k] = ~(bw | nw) & vm;
+        C[k] = 0;
+        const uint32_t cm = vm & ~low_mask(cr - x0 - 32 * k);     // the word's positions in plane 1
+        if (cm) {                                                 // (then jc + k >= -1: the zero words in front)
+            const uint32_t b0w = __funnelshift_r(strB[jc + k], strB[jc + k + 1], shc);
+            const uint32_t n0w = any_n ? __funnelshift_r(strN[jc + k], strN[jc + k + 1], shc) : 0u;
+            C[k] = ~((bw ^ b0w) | nw | n0w) & cm;
+        }
+    }
+    runs_cover<NW, kMinZ>(Z, ZR);
+#pragma unroll
+    for (int k = 0; k < NW; ++k) C[k] &= ~ZR[k];
+    runs_cover<NW, kMinC>(C, P.K);        // K = the C-run cover: a match that starts on a K bit copies from plane 0
+    int m = 0, matched = 0;
+#pragma unroll
+    for (int k = 0; k < NW; ++k) {
+        const uint32_t zp = k > 0 ? ZR[k - 1] : 0u, zn = k + 1 < NW ? ZR[k + 1] : 0u;
+        const uint32_t cp = k > 0 ? P.K[k - 1] : 0u, cn = k + 1 < NW ? P.K[k + 1] : 0u;
+        S[k] = (ZR[k] & ~__funnelshift_l(zp, ZR[k], 1)) | (P.K[k] & ~__funnelshift_l(cp, P.K[k], 1));
+        E[k] = (ZR[k] & ~__funnelshift_r(ZR[k], zn, 1)) | (P.K[k] & ~__funnelshift_r(P.K[k], cn, 1));
+        m += __popc(S[k]);
+        matched += __popc(ZR[k] | P.K[k]);
+    }
+    // size of the lane's output from popcounts: 3 bytes per match + its literals + one extension byte per
+    // literal run >= 15 (runs inside a segment are < 270) and per match >= 19 (a match is < 274 long)
+    int prev_end = 0, first_lit = 0, n_ext = 0;
+    if (m > 0) {
+        bool f = false;
+#pragma unroll
+        for (int k = NW - 1; k >= 0; --k)
+            if (!f && E[k]) { prev_end = 32 * k + 32 - __clz(E[k]); f = true; }
+        f = false;
+#pragma unroll
+        for (int k = 0; k < NW; ++k)
+            if (!f && S[k]) { first_lit = 32 * k + ctz32(S[k]); f = true; }
+        // a match [st, en] is >= 19 long iff no end bit lies in [st, st + 17]
+        uint32_t e1[NW], w[NW];
+        or_shr<NW>(E, 1, e1);
+        or_shr<NW>(e1, 2, w);
+        or_shr<NW>(w, 4, w);
+        or_shr<NW>(w, 8, w);
+#pragma unroll
+        for (int k = 0; k < NW; ++k) n_ext += __popc(S[k] & ~(w[k] | shr_word<NW>(e1, k, 16)));
+        // the literal run after end bit e (not the last one: that run is carried) is >= 15 long iff no start
+        // bit lies in [e + 1, e + 15]
+        uint32_t s1[NW], s2[NW], s3[NW];
+        or_shr<NW>(S, 1, s1);
+        or_shr<NW>(s1, 2, s2);
+        or_shr<NW>(s2, 4, s3);
+#pragma unroll
+        for (int k = 0; k < NW; ++k) {
+            uint32_t ek = E[k];
+            if (32 * k <= prev_end - 1 && prev_end - 1 < 32 * k + 32) ek &= ~(1u << ((prev_end - 1) & 31));
+            const uint32_t near = shr_word<NW>(s3, k, 1) | shr_word<NW>(s2, k, 9) | shr_word<NW>(s1, k, 13) | shr_word<NW>(S, k, 15);
+            n_ext += __popc(ek & ~near);
+        }
+    }
+    P.m = m; P.matched = matched; P.prev_end = prev_end; P.first_lit = first_lit; P.n_ext = n_ext;
+    P.trail = seglen - prev_end;
+    // runs of Rp are separated by at least one zero even where a Z run touches a C run, so "lowest run" arithmetic
+    // enumerates the matches in step 5
+#pragma unroll
+    for (int k = 0; k < NW; ++k) P.Rp[k] = (ZR[k] | P.K[k]) & ~E[k];
+}
+
+// ---- 3. carry trailing literals forward (lane 0 takes carry_in, the literals in front of the warp's first segment);
+//         scan: output offsets.  Gives this lane's carried literals, the literals the warp leaves behind its last
+//         match (carry_out), where the lane's output starts and the bytes the whole warp writes.
+template <int NW>
+__device__ __forceinline__ void scan_offsets(const LaneParse<NW> &P, int carry_in, int &carry, int &carry_out, int &out_base,
+                                             int &total) {
+    const int lane = threadIdx.x & 31;
+    int val = P.trail + (lane == 0 && P.m == 0 ? carry_in : 0), flag = P.m > 0;
+#pragma unroll
+    for (int d = 1; d < 32; d <<= 1) {
+        const int v2 = __shfl_up_sync(0xffffffffu, val, d), f2 = __shfl_up_sync(0xffffffffu, flag, d);
+        if (lane >= d && !flag) { val += v2; flag = f2; }
+    }
+    carry = __shfl_up_sync(0xffffffffu, val, 1);
+    if (lane == 0) carry = carry_in;
+    carry_out = __shfl_sync(0xffffffffu, val, 31);
+    const int mysize = P.m > 0 ? 3 * P.m + (P.prev_end - P.matched) + carry + lit_ext(P.first_lit + carry) + P.n_ext : 0;
+    int inc = mysize;
+#pragma unroll
+    for (int d = 1; d < 32; d <<= 1) {
+        const int t1 = __shfl_up_sync(0xffffffffu, inc, d);
+        if (lane >= d) inc += t1;
+    }
+    total = __shfl_sync(0xffffffffu, inc, 31);
+    out_base = inc - mysize;
+}
+
+// ---- 5. emission of the lane's sequences at shared address waddr.  Every lane walks its own byte stream -- per
+//         sequence: token [+ length bytes], literals (rebuilt from the bits), offset [+ length byte] -- in passes of at
+//         most 8 bytes, all lanes in step: a flat state machine, so a lane with a long literal run does not hold up the
+//         others' next sequence.  The bytes of a pass are gathered in a 64-bit value and appended to the lane's region of
+//         the tail buffer through a 64-bit accumulator; a lane's first and last 8-byte word may be shared with its
+//         neighbours: those two are OR-ed into the zeroed buffer at the end, everything between is stored plainly.
+//         `closes`: this lane also writes the token and length bytes of the block's last, literals-only sequence of
+//         final_lit literals (>= 11 of them); the literals themselves are written by closing_literals.
+template <int NW>
+__device__ __forceinline__ void emit_lane(uint32_t waddr, LaneParse<NW> &P, int x0, int carry, bool closes, int final_lit,
+                                          const AlleleBits &ab) {
+    uint32_t (&Rp)[NW] = P.Rp;
+    uint32_t (&K)[NW] = P.K;
+    const int cr = ab.cr;
+    uint32_t fill = waddr & 7u;                      // bytes of the accumulator in use
+    waddr &= ~7u;
+    const uint32_t faddr = waddr;
+    uint64_t acc = 0, fw = 0;
+    uint32_t first = 1;                              // the first word is still being filled: nothing stored yet
+    auto put = [&](uint64_t v, uint32_t nb) {        // append the low nb (<= 8) bytes of v; the bytes above must be zero
+        const uint32_t sh = 8u * fill;
+        acc |= v << sh;
+        const uint64_t spill = (v >> 1) >> (63u - sh);            // = v >> (64 - sh), 0 for sh == 0
+        fill += nb;
+        const bool full = fill >= 8u;
+        if (full && !first) sts64(waddr, acc);
+        fw = (full && first) ? acc : fw;
+        first = full ? 0u : first;
+        waddr += full ? 8u : 0u;
+        acc = full ? spill : acc;
+        fill -= full ? 8u : 0u;
+    };
+    // up to 8 literal bytes of block positions x .. x + nb - 1
+    auto lit8 = [&](int x, int nb) -> uint64_t {
+        const int G = ab.alpha + x;
+        const uint32_t keep = (1u << nb) - 1u;
+        const uint32_t bits = __funnelshift_r(ab.strB[G >> 5], ab.strB[(G >> 5) + 1], G) & keep;
+        uint64_t v = (uint64_t)spread4(bits) | ((uint64_t)spread4(bits >> 4) << 32);
+        if (ab.any_n) {
+            uint32_t nb8 = __funnelshift_r(ab.strN[G >> 5], ab.strN[(G >> 5) + 1], G) & keep;
+#pragma unroll 1
+            while (nb8) {                            // an allele other than 0 / 1: the byte itself
+                const int i = ctz32(nb8);
+                nb8 &= nb8 - 1;
+                const uint64_t byte = ab.byte(x + i);
+                v = (v & ~(0xFFull << (8 * i))) | (byte << (8 * i));
+            }
+        }
+        return v;
+    };
+    int pos = x0 - carry;                            // next block position that has not been emitted
+    int base = x0;                                   // block position of bit 0 of Rp[0]
+    int left = P.m;                                  // matches still to start
+    uint32_t fin = closes ? 1u : 0u;
+    int litrem = 0, cur_ml = 0;
+    uint32_t cur_off = 0, pend = 0;                  // pend: the current sequence's offset has not been emitted yet
+    while ((left | litrem | (int)pend | (int)fin) != 0) {
+        uint64_t v = 0;
+        uint32_t nb = 0;
+        if ((litrem | (int)pend) == 0) {             // the next sequence starts
+            int lit;
+            uint32_t tok;
+            if (left > 0) {
+                // matches are taken in order: whole words that are used up move out (at most NW - 1 times)
+#pragma unroll
+                for (int r = 0; r + 1 < NW; ++r) {
+                    const bool z = Rp[0] == 0u;
+#pragma unroll
+                    for (int k = 0; k + 1 < NW; ++k) { Rp[k] = z ? Rp[k + 1] : Rp[k]; K[k] = z ? K[k + 1] : K[k]; }
+                    Rp[NW - 1] = z ? 0u : Rp[NW - 1];
+                    base += z ? 32 : 0;
+                }
+                // lowest run of Rp: low = its first bit, Rp + low carries through the run (and on into the next words)
+                const uint32_t low = Rp[0] & (0u - Rp[0]);
+                const int ts = __popc(low - 1u);
+                const bool is_k = (K[0] & low) != 0u;
+                uint64_t cy = low;
+                int ml = 1;
+#pragma unroll
+                for (int k = 0; k < NW; ++k) {
+                    cy += Rp[k];
+                    const uint32_t t = (uint32_t)cy;
+                    cy >>= 32;
+                    ml += __popc(Rp[k] & ~t);
+                    Rp[k] &= t;
+                }
+                lit = base + ts - pos;
+                cur_ml = ml;
+                cur_off = is_k ? (uint32_t)cr : 2u * (uint32_t)cr;
+                pend = 1;
+                --left;
+                tok = (uint32_t)((min(lit, 15) << 4) | min(ml - 4, 15));
+            } else {                                 // the last sequence of the block: literals only
+                lit = final_lit;
+                fin = 0;
+                tok = (uint32_t)(min(lit, 15) << 4);
+            }
+            v = tok; nb = 1;
+            if (lit >= 15) {
+                int rem = lit - 15;
+#pragma unroll 1
+                while (rem >= 255) { put(v, nb); v = 255u; nb = 1; rem -= 255; }
+                v |= (uint64_t)(uint32_t)rem << (8u * nb);
+                ++nb;
+            }
+            litrem = pend ? lit : 0;
+        }
+        const int take = min(litrem, 8 - (int)nb);
+        if (take > 0) {
+            v |= lit8(pos, take) << (8u * nb);
+            nb += (uint32_t)take; pos += take; litrem -= take;
+        }
+        if (pend != 0 && litrem == 0) {
+            const uint32_t ob = cur_ml >= 19 ? 3u : 2u;
+            if (nb + ob <= 8u) {
+                v |= (uint64_t)(cur_off | (cur_ml >= 19 ? (uint32_t)(cur_ml - 19) << 16 : 0u)) << (8u * nb);
+                nb += ob; pend = 0; pos += cur_ml;
+            }
+        }
+        put(v, nb);
+    }
+    const uint64_t fv = first ? acc : fw;
+    if ((uint32_t)fv) sts_or32(faddr, (uint32_t)fv);
+    if ((uint32_t)(fv >> 32)) sts_or32(faddr + 4u, (uint32_t)(fv >> 32));
+    if (!first) {
+        if ((uint32_t)acc) sts_or32(waddr, (uint32_t)acc);
+        if ((uint32_t)(acc >> 32)) sts_or32(waddr + 4u, (uint32_t)(acc >> 32));
+    }
+}
+
+// the block's closing literals -- its last final_lit positions (>= 11, and all the positions no lane owns) -- to fdst:
+// one byte per lane and step
+__device__ __forceinline__ void closing_literals(uint8_t *fdst, int final_lit, const AlleleBits &ab) {
+    const int fx = 2 * ab.cr - final_lit;
+    for (int i = threadIdx.x & 31; i < final_lit; i += 32) {
+        const int x = fx + i, G = ab.alpha + x;
+        uint32_t byte = (ab.strB[G >> 5] >> (G & 31)) & 1u;
+        if (ab.any_n && ((ab.strN[G >> 5] >> (G & 31)) & 1u)) byte = ab.byte(x);
+        fdst[i] = (uint8_t)byte;
+    }
+}
+
 template <int NW>
 __global__ void __launch_bounds__(kWpc * 32) donor_frames_kernel(const FusedArgs A) {
-    extern __shared__ __align__(128) uint8_t smem[];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const uint32_t c = blockIdx.x / A.groups, grp = blockIdx.x - c * A.groups;
     const int cr = (int)A.cr, n = 2 * cr;
@@ -599,151 +857,28 @@ __global__ void __launch_bounds__(kWpc * 32) donor_frames_kernel(const FusedArgs
     uint32_t phase = 0;
     bool tmpl_ready = false;
     const unsigned long long row_stride = A.slot_off[A.n_chunks], slot = A.slot_off[c];
-    const int strw = (int)A.strw;
-    const int sh = cr & 31, wsh = cr >> 5;       // plane 1 sits cr bits above plane 0 in the strings
 
     for (; s < s_end; s += kWpc) {
-        int dlen = 0;
-        // state of the parse that the emission needs
-        uint32_t Rp[NW], K[NW];            // match cover without the last position of each run; C-run cover (match type)
-        int m = 0, carry = 0, out_base = 0, total = 0, final_lit = 0;
-        bool any_n = false;
+        // read per frame, not hoisted out of the loop: kept live across it they cost NW >= 5 some 40 registers
         const int seg = (int)A.seg;                  // block positions per lane: lane i owns [i * seg, (i + 1) * seg)
         const int x0 = lane * seg;
-        const uint64_t grow = (uint64_t)(A.s0 + s) * A.gt_stride + r0;         // the frame's first row in the byte planes
-
+        AlleleBits ab{strB, strN, false, alpha, cr, A.gt0, A.gt1, (uint64_t)(A.s0 + s) * A.gt_stride + r0};
+        LaneParse<NW> P;
+        int dlen = n, carry = 0, out_base = 0, final_lit = 0;
         if (!raw) {
-            // ---- 1. this frame's slices of the bit planes (staged by TMA) -> ONE bit string each for B and N over
-            //         both planes: block position x (0 .. 2 * cr) is bit alpha + x, so the parse and the literal
-            //         emission walk from plane 0 into plane 1 without a seam
             mbar_wait(wbar, phase);
             phase ^= 1;
-            uint32_t nacc = 0;
-            for (int w = lane; w < nwst; w += 32) {     // rows outside [r0, r0 + valid) belong to other chunks (or to nobody)
-                const uint32_t mk = low_mask(alpha + valid - 32 * w) & ~low_mask(alpha - 32 * w);
-                uint32_t *gq = stage + (w >> 2) * kBitGroupWords + (w & 3);
-                if (mk != 0xFFFFFFFFu) { gq[0] &= mk; gq[4] &= mk; gq[8] &= mk; gq[12] &= mk; }
-                nacc |= gq[8] | gq[12];
-            }
-            any_n = __any_sync(0xffffffffu, nacc != 0);
-            __syncwarp();
-            for (int k = lane; k < strw; k += 32) {
-                const int j = k - wsh;
-                uint32_t b = 0, b1lo = 0, b1hi = 0;
-                if (k < nwst) b = stage[(k >> 2) * kBitGroupWords + (k & 3)];
-                if (j >= 1 && j <= nwst) b1lo = stage[((j - 1) >> 2) * kBitGroupWords + 4 + ((j - 1) & 3)];
-                if (j >= 0 && j < nwst) b1hi = stage[(j >> 2) * kBitGroupWords + 4 + (j & 3)];
-                strB[k] = b | __funnelshift_l(b1lo, b1hi, sh);
-                if (any_n) {
-                    uint32_t x = 0, x1lo = 0, x1hi = 0;
-                    if (k < nwst) x = stage[(k >> 2) * kBitGroupWords + 8 + (k & 3)];
-                    if (j >= 1 && j <= nwst) x1lo = stage[((j - 1) >> 2) * kBitGroupWords + 12 + ((j - 1) & 3)];
-                    if (j >= 0 && j < nwst) x1hi = stage[(j >> 2) * kBitGroupWords + 12 + (j & 3)];
-                    strN[k] = x | __funnelshift_l(x1lo, x1hi, sh);
-                }
-            }
-            fence_proxy_async();                        // the staging area was masked in place: order that before the copy engine's writes
-            __syncwarp();
+            ab.any_n = build_bit_strings(stage, strB, strN, nwst, (int)A.strw, alpha, valid, cr);
             if (lane == 0 && s + kWpc < s_end) {        // the next frame's slices: one TMA bulk copy, a whole frame ahead
                 mbar_expect_tx(wbar, stg);
                 tma_load_1d(stage, A.bits + (uint64_t)(A.s0 + s + kWpc) * A.bits_stride + (uint64_t)g0 * kBitGroupWords, stg, wbar);
             }
-
-            // ---- 2. per-lane parse of one segment, position-parallel
-            const int seglen = max(0, min(seg, n - x0));
-            const int mlim = min(seglen, n - 11 - x0);                    // the last 11 bytes of the block stay literals
-            const int bi = alpha + x0, j0 = bi >> 5, shb = bi & 31;
-            const int ci = bi - cr, jc = ci >> 5, shc = ci & 31;          // the same rows in plane 0 (positions >= cr only)
-            uint32_t Z[NW], C[NW], ZR[NW], S[NW], E[NW];
-#pragma unroll
-            for (int k = 0; k < NW; ++k) {
-                const uint32_t bw = __funnelshift_r(strB[j0 + k], strB[j0 + k + 1], shb);
-                const uint32_t nw = any_n ? __funnelshift_r(strN[j0 + k], strN[j0 + k + 1], shb) : 0u;
-                const uint32_t vm = low_mask(mlim - 32 * k);
-                Z[k] = ~(bw | nw) & vm;
-                C[k] = 0;
-                const uint32_t cm = vm & ~low_mask(cr - x0 - 32 * k);     // the word's positions in plane 1
-                if (cm) {                                                 // (then jc + k >= -1: the zero words in front)
-                    const uint32_t b0w = __funnelshift_r(strB[jc + k], strB[jc + k + 1], shc);
-                    const uint32_t n0w = any_n ? __funnelshift_r(strN[jc + k], strN[jc + k + 1], shc) : 0u;
-                    C[k] = ~((bw ^ b0w) | nw | n0w) & cm;
-                }
-            }
-            runs_cover<NW, kMinZ>(Z, ZR);
-#pragma unroll
-            for (int k = 0; k < NW; ++k) C[k] &= ~ZR[k];
-            runs_cover<NW, kMinC>(C, K);          // K = the C-run cover: a match that starts on a K bit copies from plane 0
-            int matched = 0;
-#pragma unroll
-            for (int k = 0; k < NW; ++k) {
-                const uint32_t zp = k > 0 ? ZR[k - 1] : 0u, zn = k + 1 < NW ? ZR[k + 1] : 0u;
-                const uint32_t cp = k > 0 ? K[k - 1] : 0u, cn = k + 1 < NW ? K[k + 1] : 0u;
-                S[k] = (ZR[k] & ~__funnelshift_l(zp, ZR[k], 1)) | (K[k] & ~__funnelshift_l(cp, K[k], 1));
-                E[k] = (ZR[k] & ~__funnelshift_r(ZR[k], zn, 1)) | (K[k] & ~__funnelshift_r(K[k], cn, 1));
-                m += __popc(S[k]);
-                matched += __popc(ZR[k] | K[k]);
-            }
-            // size of the lane's output from popcounts: 3 bytes per match + its literals + one extension byte per
-            // literal run >= 15 (runs inside a segment are < 270) and per match >= 19 (a match is < 274 long)
-            int prev_end = 0, first_lit = 0, n_ext = 0;
-            if (m > 0) {
-                bool f = false;
-#pragma unroll
-                for (int k = NW - 1; k >= 0; --k)
-                    if (!f && E[k]) { prev_end = 32 * k + 32 - __clz(E[k]); f = true; }
-                f = false;
-#pragma unroll
-                for (int k = 0; k < NW; ++k)
-                    if (!f && S[k]) { first_lit = 32 * k + ctz32(S[k]); f = true; }
-                // a match [st, en] is >= 19 long iff no end bit lies in [st, st + 17]
-                uint32_t e1[NW], w[NW];
-                or_shr<NW>(E, 1, e1);
-                or_shr<NW>(e1, 2, w);
-                or_shr<NW>(w, 4, w);
-                or_shr<NW>(w, 8, w);
-#pragma unroll
-                for (int k = 0; k < NW; ++k) n_ext += __popc(S[k] & ~(w[k] | shr_word<NW>(e1, k, 16)));
-                // the literal run after end bit e (not the last one: that run is carried) is >= 15 long iff no start
-                // bit lies in [e + 1, e + 15]
-                uint32_t s1[NW], s2[NW], s3[NW];
-                or_shr<NW>(S, 1, s1);
-                or_shr<NW>(s1, 2, s2);
-                or_shr<NW>(s2, 4, s3);
-#pragma unroll
-                for (int k = 0; k < NW; ++k) {
-                    uint32_t ek = E[k];
-                    if (32 * k <= prev_end - 1 && prev_end - 1 < 32 * k + 32) ek &= ~(1u << ((prev_end - 1) & 31));
-                    const uint32_t near = shr_word<NW>(s3, k, 1) | shr_word<NW>(s2, k, 9) | shr_word<NW>(s1, k, 13) | shr_word<NW>(S, k, 15);
-                    n_ext += __popc(ek & ~near);
-                }
-            }
-            const int trail = seglen - prev_end;
-            // runs of Rp are separated by at least one zero even where a Z run touches a C run, so "lowest run" arithmetic
-            // enumerates the matches in step 5
-#pragma unroll
-            for (int k = 0; k < NW; ++k) Rp[k] = (ZR[k] | K[k]) & ~E[k];
-
-            // ---- 3. carry trailing literals forward; scan: output offsets
-            int val = trail, flag = m > 0;
-#pragma unroll
-            for (int d = 1; d < 32; d <<= 1) {
-                const int v2 = __shfl_up_sync(0xffffffffu, val, d), f2 = __shfl_up_sync(0xffffffffu, flag, d);
-                if (lane >= d && !flag) { val += v2; flag = f2; }
-            }
-            carry = __shfl_up_sync(0xffffffffu, val, 1);
-            if (lane == 0) carry = 0;
-            final_lit = __shfl_sync(0xffffffffu, val, 31) + max(0, n - 32 * seg);    // + the positions no lane owns (FusedArgs::seg)
-            const int mysize = m > 0 ? 3 * m + (prev_end - matched) + carry + lit_ext(first_lit + carry) + n_ext : 0;
-            int inc = mysize;
-#pragma unroll
-            for (int d = 1; d < 32; d <<= 1) {
-                const int t1 = __shfl_up_sync(0xffffffffu, inc, d);
-                if (lane >= d) inc += t1;
-            }
-            total = __shfl_sync(0xffffffffu, inc, 31);
-            out_base = inc - mysize;
+            parse_lane<NW>(ab, x0, seg, P);
+            int total;
+            scan_offsets<NW>(P, 0, carry, final_lit, out_base, total);
+            final_lit += max(0, n - 32 * seg);           // + the positions no lane owns (FusedArgs::seg)
             dlen = total + 1 + lit_ext(final_lit) + final_lit;
-        } else dlen = n;
+        }
 
         // ---- 4. the tail buffer: zeroed (neighbouring lanes OR their shared boundary words together), lined up with
         //         the template's end modulo 16 so that the frame leaves as 16-byte aligned bulk copies
@@ -762,147 +897,12 @@ __global__ void __launch_bounds__(kWpc * 32) donor_frames_kernel(const FusedArgs
         if (raw) {
             for (int i = lane; i < n; i += 32) {
                 const int x = i < cr ? i : i - cr;
-                seq[i] = x < valid ? (uint8_t)(i < cr ? A.gt0 : A.gt1)[grow + x] : (uint8_t)0;
+                seq[i] = x < valid ? (uint8_t)ab.byte(i) : (uint8_t)0;
             }
         } else {
-            // ---- 5. emission.  Every lane walks its own byte stream -- per sequence: token [+ length bytes], literals
-            //         (rebuilt from the bits), offset [+ length byte] -- in passes of at most 8 bytes, all lanes in step: a
-            //         flat state machine, so a lane with a long literal run does not hold up the others' next sequence.
-            //         The bytes of a pass are gathered in a 64-bit value and appended to the lane's region of the tail
-            //         buffer through a 64-bit accumulator; a lane's first and last 8-byte word may be shared with its
-            //         neighbours: those two are OR-ed into the zeroed buffer at the end, everything between is stored plainly.
-            uint32_t waddr = smem_u32(seq) + (uint32_t)out_base;
-            uint32_t fill = waddr & 7u;                      // bytes of the accumulator in use
-            waddr &= ~7u;
-            const uint32_t faddr = waddr;
-            uint64_t acc = 0, fw = 0;
-            uint32_t first = 1;                              // the first word is still being filled: nothing stored yet
-            auto put = [&](uint64_t v, uint32_t nb) {        // append the low nb (<= 8) bytes of v; the bytes above must be zero
-                const uint32_t sh = 8u * fill;
-                acc |= v << sh;
-                const uint64_t spill = (v >> 1) >> (63u - sh);            // = v >> (64 - sh), 0 for sh == 0
-                fill += nb;
-                const bool full = fill >= 8u;
-                if (full && !first) sts64(waddr, acc);
-                fw = (full && first) ? acc : fw;
-                first = full ? 0u : first;
-                waddr += full ? 8u : 0u;
-                acc = full ? spill : acc;
-                fill -= full ? 8u : 0u;
-            };
-            // up to 8 literal bytes of block positions x .. x + nb - 1
-            auto lit8 = [&](int x, int nb) -> uint64_t {
-                const int G = alpha + x;
-                const uint32_t keep = (1u << nb) - 1u;
-                const uint32_t bits = __funnelshift_r(strB[G >> 5], strB[(G >> 5) + 1], G) & keep;
-                uint64_t v = (uint64_t)spread4(bits) | ((uint64_t)spread4(bits >> 4) << 32);
-                if (any_n) {
-                    uint32_t nb8 = __funnelshift_r(strN[G >> 5], strN[(G >> 5) + 1], G) & keep;
-#pragma unroll 1
-                    while (nb8) {                            // an allele other than 0 / 1: the byte itself
-                        const int i = ctz32(nb8);
-                        nb8 &= nb8 - 1;
-                        const int xx = x + i;
-                        const uint64_t byte = (uint8_t)(xx < cr ? A.gt0 : A.gt1)[grow + (xx < cr ? xx : xx - cr)];
-                        v = (v & ~(0xFFull << (8 * i))) | (byte << (8 * i));
-                    }
-                }
-                return v;
-            };
-            const int seg_abs = x0;
-            int pos = seg_abs - carry;                       // next block position that has not been emitted
-            int base = seg_abs;                              // block position of bit 0 of Rp[0]
-            int left = m;                                    // matches still to start
-            uint32_t fin = lane == 31 ? 1u : 0u;             // lane 31 closes the block with the token of a literals-only sequence
-            int litrem = 0, cur_ml = 0;
-            uint32_t cur_off = 0, pend = 0;                  // pend: the current sequence's offset has not been emitted yet
-            while ((left | litrem | (int)pend | (int)fin) != 0) {
-                uint64_t v = 0;
-                uint32_t nb = 0;
-                if ((litrem | (int)pend) == 0) {             // the next sequence starts
-                    int lit;
-                    uint32_t tok;
-                    if (left > 0) {
-                        // matches are taken in order: whole words that are used up move out (at most NW - 1 times)
-#pragma unroll
-                        for (int r = 0; r + 1 < NW; ++r) {
-                            const bool z = Rp[0] == 0u;
-#pragma unroll
-                            for (int k = 0; k + 1 < NW; ++k) { Rp[k] = z ? Rp[k + 1] : Rp[k]; K[k] = z ? K[k + 1] : K[k]; }
-                            Rp[NW - 1] = z ? 0u : Rp[NW - 1];
-                            base += z ? 32 : 0;
-                        }
-                        // lowest run of Rp: low = its first bit, Rp + low carries through the run (and on into the next words)
-                        const uint32_t low = Rp[0] & (0u - Rp[0]);
-                        const int ts = __popc(low - 1u);
-                        const bool is_k = (K[0] & low) != 0u;
-                        uint64_t cy = low;
-                        int ml = 1;
-#pragma unroll
-                        for (int k = 0; k < NW; ++k) {
-                            cy += Rp[k];
-                            const uint32_t t = (uint32_t)cy;
-                            cy >>= 32;
-                            ml += __popc(Rp[k] & ~t);
-                            Rp[k] &= t;
-                        }
-                        lit = base + ts - pos;
-                        cur_ml = ml;
-                        cur_off = is_k ? (uint32_t)cr : 2u * (uint32_t)cr;
-                        pend = 1;
-                        --left;
-                        tok = (uint32_t)((min(lit, 15) << 4) | min(ml - 4, 15));
-                    } else {                                 // the last sequence of the block: literals only (>= 11 of them);
-                        lit = final_lit;                     // lane 31 writes its token and length bytes, the literals
-                        fin = 0;                             // themselves are written by the whole warp below
-                        tok = (uint32_t)(min(lit, 15) << 4);
-                    }
-                    v = tok; nb = 1;
-                    if (lit >= 15) {
-                        int rem = lit - 15;
-#pragma unroll 1
-                        while (rem >= 255) { put(v, nb); v = 255u; nb = 1; rem -= 255; }
-                        v |= (uint64_t)(uint32_t)rem << (8u * nb);
-                        ++nb;
-                    }
-                    litrem = pend ? lit : 0;
-                }
-                const int take = min(litrem, 8 - (int)nb);
-                if (take > 0) {
-                    v |= lit8(pos, take) << (8u * nb);
-                    nb += (uint32_t)take; pos += take; litrem -= take;
-                }
-                if (pend != 0 && litrem == 0) {
-                    const uint32_t ob = cur_ml >= 19 ? 3u : 2u;
-                    if (nb + ob <= 8u) {
-                        v |= (uint64_t)(cur_off | (cur_ml >= 19 ? (uint32_t)(cur_ml - 19) << 16 : 0u)) << (8u * nb);
-                        nb += ob; pend = 0; pos += cur_ml;
-                    }
-                }
-                put(v, nb);
-            }
-            {
-                const uint64_t fv = first ? acc : fw;
-                if ((uint32_t)fv) sts_or32(faddr, (uint32_t)fv);
-                if ((uint32_t)(fv >> 32)) sts_or32(faddr + 4u, (uint32_t)(fv >> 32));
-                if (!first) {
-                    if ((uint32_t)acc) sts_or32(waddr, (uint32_t)acc);
-                    if ((uint32_t)(acc >> 32)) sts_or32(waddr + 4u, (uint32_t)(acc >> 32));
-                }
-            }
+            emit_lane<NW>(smem_u32(seq) + (uint32_t)out_base, P, x0, carry, lane == 31, final_lit, ab);
             __syncwarp();
-            // the block's closing literals (>= 11, and all the positions no lane owns): one byte per lane and step
-            {
-                uint8_t *fdst = seq + (dlen - final_lit);
-                const int fx = n - final_lit;
-                for (int i = lane; i < final_lit; i += 32) {
-                    const int x = fx + i, G = alpha + x;
-                    uint32_t byte = (strB[G >> 5] >> (G & 31)) & 1u;
-                    if (any_n && ((strN[G >> 5] >> (G & 31)) & 1u))
-                        byte = (uint8_t)(x < cr ? A.gt0 : A.gt1)[grow + (x < cr ? x : x - cr)];
-                    fdst[i] = (uint8_t)byte;
-                }
-            }
+            closing_literals(seq + (dlen - final_lit), final_lit, ab);
         }
         fence_proxy_async();                 // the tail buffer is read by the bulk-copy engine next
         __syncwarp();
@@ -936,14 +936,17 @@ __global__ void __launch_bounds__(kWpc * 32) donor_frames_kernel(const FusedArgs
 }
 
 // ------------------------------------------------------------------------------------------
-// Kernel 4b-L: the allele tails of chunks of kSmallChunkMax < cr <= kMaxChunkRecords records.  The parse, the scans and
-// the emission are donor_frames_kernel's, run in PASSES: a pass covers 32 lanes x 32 * NW block positions, and the
-// literals a pass leaves at its end are carried into the first sequence of the next pass exactly as a lane carries
-// them into the next lane's.  Z and C match sources (offsets 2 * cr and cr) and the closing literals are unchanged,
-// so the slot bound (template + 2 cr + 2 cr / 255 + 24) still holds.  The template is NOT staged in shared memory
-// (a chunk with high-entropy sites makes a template of up to ~24 * cr bytes): the warp copies its body from global
-// memory (L2-resident: every warp of the chunk reads the same bytes).  Shared memory per warp = bit-plane staging +
-// the two bit strings + the whole tail buffer, zeroed up front because the tail's length is known after the last pass.
+// Kernel 4b-L: the allele tails of chunks of kSmallChunkMax < cr <= kMaxChunkRecords records.  Shared with
+// donor_frames_kernel: the bit strings, the lane parse, the offset scans, the emission and the closing literals, so the
+// frames are built by the same rules (Z and C match sources at offsets 2 * cr and cr, the same closing literals) and
+// the slot bound (template + 2 cr + 2 cr / 255 + 24) still holds.  What differs:
+//   - the parse, scans and emission run in PASSES of 32 lanes x 32 * NW block positions; the literals a pass leaves at
+//     its end are carried into the first sequence of the next pass exactly as a lane carries them into the next lane's,
+//     and lane 31 of the last pass closes the block;
+//   - the template is NOT staged in shared memory (a chunk with high-entropy sites makes a template of up to ~24 * cr
+//     bytes): the warp copies its body from global memory (L2-resident: every warp of the chunk reads the same bytes);
+//   - shared memory per warp = bit-plane staging + the two bit strings + the whole tail buffer, zeroed up front because
+//     the tail's length is known only after the last pass.
 // ------------------------------------------------------------------------------------------
 constexpr int kLargeNW = 4;                   // mask words per lane and pass: 4,096 block positions per pass
 constexpr int kWpcL = 4;                      // warps per CTA: 2-6 CTAs per SM from cr 7,489 down to 2,731
@@ -951,7 +954,6 @@ constexpr int kWpcL = 4;                      // warps per CTA: 2-6 CTAs per SM 
 // __maxnreg__(96) instead of __launch_bounds__: with the bounds alone ptxas settles on 64 registers and spills
 template <int NW>
 __global__ void __maxnreg__(96) donor_frames_large_kernel(const FusedArgs A) {
-    extern __shared__ __align__(128) uint8_t smem[];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const uint32_t c = blockIdx.x / A.groups, grp = blockIdx.x - c * A.groups;
     const int cr = (int)A.cr, n = 2 * cr;
@@ -986,47 +988,19 @@ __global__ void __maxnreg__(96) donor_frames_large_kernel(const FusedArgs A) {
     }
     uint32_t phase = 0;
     const unsigned long long row_stride = A.slot_off[A.n_chunks], slot = A.slot_off[c];
-    const int strw = (int)A.strw;
-    const int sh = cr & 31, wsh = cr >> 5;
     constexpr int seg = 32 * NW;                 // block positions per lane and pass
     const int npass = (n + 32 * seg - 1) / (32 * seg);
 
     for (; s < s_end; s += kWpcL) {
-        const uint64_t grow = (uint64_t)(A.s0 + s) * A.gt_stride + r0;
-        // ---- 1. bit strings, as in donor_frames_kernel
+        AlleleBits ab{strB, strN, false, alpha, cr, A.gt0, A.gt1, (uint64_t)(A.s0 + s) * A.gt_stride + r0};
         mbar_wait(wbar, phase);
         phase ^= 1;
-        uint32_t nacc = 0;
-        for (int w = lane; w < nwst; w += 32) {
-            const uint32_t mk = low_mask(alpha + valid - 32 * w) & ~low_mask(alpha - 32 * w);
-            uint32_t *gq = stage + (w >> 2) * kBitGroupWords + (w & 3);
-            if (mk != 0xFFFFFFFFu) { gq[0] &= mk; gq[4] &= mk; gq[8] &= mk; gq[12] &= mk; }
-            nacc |= gq[8] | gq[12];
-        }
-        const bool any_n = __any_sync(0xffffffffu, nacc != 0);
-        __syncwarp();
-        for (int k = lane; k < strw; k += 32) {
-            const int j = k - wsh;
-            uint32_t b = 0, b1lo = 0, b1hi = 0;
-            if (k < nwst) b = stage[(k >> 2) * kBitGroupWords + (k & 3)];
-            if (j >= 1 && j <= nwst) b1lo = stage[((j - 1) >> 2) * kBitGroupWords + 4 + ((j - 1) & 3)];
-            if (j >= 0 && j < nwst) b1hi = stage[(j >> 2) * kBitGroupWords + 4 + (j & 3)];
-            strB[k] = b | __funnelshift_l(b1lo, b1hi, sh);
-            if (any_n) {
-                uint32_t x = 0, x1lo = 0, x1hi = 0;
-                if (k < nwst) x = stage[(k >> 2) * kBitGroupWords + 8 + (k & 3)];
-                if (j >= 1 && j <= nwst) x1lo = stage[((j - 1) >> 2) * kBitGroupWords + 12 + ((j - 1) & 3)];
-                if (j >= 0 && j < nwst) x1hi = stage[(j >> 2) * kBitGroupWords + 12 + (j & 3)];
-                strN[k] = x | __funnelshift_l(x1lo, x1hi, sh);
-            }
-        }
-        fence_proxy_async();
-        __syncwarp();
+        ab.any_n = build_bit_strings(stage, strB, strN, nwst, (int)A.strw, alpha, valid, cr);
         if (lane == 0 && s + kWpcL < s_end) {
             mbar_expect_tx(wbar, stg);
             tma_load_1d(stage, A.bits + (uint64_t)(A.s0 + s + kWpcL) * A.bits_stride + (uint64_t)g0 * kBitGroupWords, stg, wbar);
         }
-        // ---- 2. the tail buffer: zeroed whole, the template's last partial 16 bytes in front
+        // the tail buffer: zeroed whole, the template's last partial 16 bytes in front
         if (lane == 0) tma_store_wait_read();           // the previous frame's bulk store has read the buffer
         __syncwarp();
         for (uint32_t i = lane; i < A.outcap / 16u; i += 32) reinterpret_cast<uint4 *>(outb)[i] = make_uint4(0, 0, 0, 0);
@@ -1035,231 +1009,20 @@ __global__ void __maxnreg__(96) donor_frames_large_kernel(const FusedArgs A) {
         __syncwarp();
         uint8_t *seq = outb + sh16;
 
-        int carry_in = 0, pass_base = 0, final_lit = 0;
+        int carry_in = 0, pass_base = 0;             // carry_in: literals the passes so far leave behind their last match
         for (int q = 0; q < npass; ++q) {
-            // ---- 3. per-lane parse of one segment of this pass (donor_frames_kernel, step 2)
             const int x0 = q * 32 * seg + lane * seg;
-            uint32_t Rp[NW], K[NW];
-            int m = 0;
-            const int seglen = max(0, min(seg, n - x0));
-            const int mlim = min(seglen, n - 11 - x0);
-            const int bi = alpha + x0, j0 = bi >> 5, shb = bi & 31;
-            const int ci = bi - cr, jc = ci >> 5, shc = ci & 31;
-            uint32_t Z[NW], C[NW], ZR[NW], S[NW], E[NW];
-#pragma unroll
-            for (int k = 0; k < NW; ++k) {
-                const uint32_t bw = __funnelshift_r(strB[j0 + k], strB[j0 + k + 1], shb);
-                const uint32_t nw = any_n ? __funnelshift_r(strN[j0 + k], strN[j0 + k + 1], shb) : 0u;
-                const uint32_t vm = low_mask(mlim - 32 * k);
-                Z[k] = ~(bw | nw) & vm;
-                C[k] = 0;
-                const uint32_t cm = vm & ~low_mask(cr - x0 - 32 * k);
-                if (cm) {
-                    const uint32_t b0w = __funnelshift_r(strB[jc + k], strB[jc + k + 1], shc);
-                    const uint32_t n0w = any_n ? __funnelshift_r(strN[jc + k], strN[jc + k + 1], shc) : 0u;
-                    C[k] = ~((bw ^ b0w) | nw | n0w) & cm;
-                }
-            }
-            runs_cover<NW, kMinZ>(Z, ZR);
-#pragma unroll
-            for (int k = 0; k < NW; ++k) C[k] &= ~ZR[k];
-            runs_cover<NW, kMinC>(C, K);
-            int matched = 0;
-#pragma unroll
-            for (int k = 0; k < NW; ++k) {
-                const uint32_t zp = k > 0 ? ZR[k - 1] : 0u, zn = k + 1 < NW ? ZR[k + 1] : 0u;
-                const uint32_t cp = k > 0 ? K[k - 1] : 0u, cn = k + 1 < NW ? K[k + 1] : 0u;
-                S[k] = (ZR[k] & ~__funnelshift_l(zp, ZR[k], 1)) | (K[k] & ~__funnelshift_l(cp, K[k], 1));
-                E[k] = (ZR[k] & ~__funnelshift_r(ZR[k], zn, 1)) | (K[k] & ~__funnelshift_r(K[k], cn, 1));
-                m += __popc(S[k]);
-                matched += __popc(ZR[k] | K[k]);
-            }
-            int prev_end = 0, first_lit = 0, n_ext = 0;
-            if (m > 0) {
-                bool f = false;
-#pragma unroll
-                for (int k = NW - 1; k >= 0; --k)
-                    if (!f && E[k]) { prev_end = 32 * k + 32 - __clz(E[k]); f = true; }
-                f = false;
-#pragma unroll
-                for (int k = 0; k < NW; ++k)
-                    if (!f && S[k]) { first_lit = 32 * k + ctz32(S[k]); f = true; }
-                uint32_t e1[NW], w[NW];
-                or_shr<NW>(E, 1, e1);
-                or_shr<NW>(e1, 2, w);
-                or_shr<NW>(w, 4, w);
-                or_shr<NW>(w, 8, w);
-#pragma unroll
-                for (int k = 0; k < NW; ++k) n_ext += __popc(S[k] & ~(w[k] | shr_word<NW>(e1, k, 16)));
-                uint32_t s1[NW], s2[NW], s3[NW];
-                or_shr<NW>(S, 1, s1);
-                or_shr<NW>(s1, 2, s2);
-                or_shr<NW>(s2, 4, s3);
-#pragma unroll
-                for (int k = 0; k < NW; ++k) {
-                    uint32_t ek = E[k];
-                    if (32 * k <= prev_end - 1 && prev_end - 1 < 32 * k + 32) ek &= ~(1u << ((prev_end - 1) & 31));
-                    const uint32_t near = shr_word<NW>(s3, k, 1) | shr_word<NW>(s2, k, 9) | shr_word<NW>(s1, k, 13) | shr_word<NW>(S, k, 15);
-                    n_ext += __popc(ek & ~near);
-                }
-            }
-            const int trail = seglen - prev_end;
-#pragma unroll
-            for (int k = 0; k < NW; ++k) Rp[k] = (ZR[k] | K[k]) & ~E[k];
-
-            // ---- 4. carry trailing literals forward (lane 0 takes what the previous pass left); scan: output offsets
-            int val = trail + (lane == 0 && m == 0 ? carry_in : 0), flag = m > 0;
-#pragma unroll
-            for (int d = 1; d < 32; d <<= 1) {
-                const int v2 = __shfl_up_sync(0xffffffffu, val, d), f2 = __shfl_up_sync(0xffffffffu, flag, d);
-                if (lane >= d && !flag) { val += v2; flag = f2; }
-            }
-            int carry = __shfl_up_sync(0xffffffffu, val, 1);
-            if (lane == 0) carry = carry_in;
-            carry_in = __shfl_sync(0xffffffffu, val, 31);
-            const bool last = q == npass - 1;
-            if (last) final_lit = carry_in;
-            const int mysize = m > 0 ? 3 * m + (prev_end - matched) + carry + lit_ext(first_lit + carry) + n_ext : 0;
-            int inc = mysize;
-#pragma unroll
-            for (int d = 1; d < 32; d <<= 1) {
-                const int t1 = __shfl_up_sync(0xffffffffu, inc, d);
-                if (lane >= d) inc += t1;
-            }
-            const int total = __shfl_sync(0xffffffffu, inc, 31);
-            const int out_base = pass_base + inc - mysize;
+            LaneParse<NW> P;
+            parse_lane<NW>(ab, x0, seg, P);
+            int carry, out_base, total;
+            scan_offsets<NW>(P, carry_in, carry, carry_in, out_base, total);
+            emit_lane<NW>(smem_u32(seq) + (uint32_t)(pass_base + out_base), P, x0, carry, lane == 31 && q == npass - 1, carry_in, ab);
             pass_base += total;
-
-            // ---- 5. emission (donor_frames_kernel, step 5); lane 31 of the last pass opens the closing literals
-            uint32_t waddr = smem_u32(seq) + (uint32_t)out_base;
-            uint32_t fill = waddr & 7u;
-            waddr &= ~7u;
-            const uint32_t faddr = waddr;
-            uint64_t acc = 0, fw = 0;
-            uint32_t first = 1;
-            auto put = [&](uint64_t v, uint32_t nb) {
-                const uint32_t sh = 8u * fill;
-                acc |= v << sh;
-                const uint64_t spill = (v >> 1) >> (63u - sh);
-                fill += nb;
-                const bool full = fill >= 8u;
-                if (full && !first) sts64(waddr, acc);
-                fw = (full && first) ? acc : fw;
-                first = full ? 0u : first;
-                waddr += full ? 8u : 0u;
-                acc = full ? spill : acc;
-                fill -= full ? 8u : 0u;
-            };
-            auto lit8 = [&](int x, int nb) -> uint64_t {
-                const int G = alpha + x;
-                const uint32_t keep = (1u << nb) - 1u;
-                const uint32_t bits = __funnelshift_r(strB[G >> 5], strB[(G >> 5) + 1], G) & keep;
-                uint64_t v = (uint64_t)spread4(bits) | ((uint64_t)spread4(bits >> 4) << 32);
-                if (any_n) {
-                    uint32_t nb8 = __funnelshift_r(strN[G >> 5], strN[(G >> 5) + 1], G) & keep;
-#pragma unroll 1
-                    while (nb8) {
-                        const int i = ctz32(nb8);
-                        nb8 &= nb8 - 1;
-                        const int xx = x + i;
-                        const uint64_t byte = (uint8_t)(xx < cr ? A.gt0 : A.gt1)[grow + (xx < cr ? xx : xx - cr)];
-                        v = (v & ~(0xFFull << (8 * i))) | (byte << (8 * i));
-                    }
-                }
-                return v;
-            };
-            int pos = x0 - carry;
-            int base = x0;
-            int left = m;
-            uint32_t fin = lane == 31 && last ? 1u : 0u;
-            int litrem = 0, cur_ml = 0;
-            uint32_t cur_off = 0, pend = 0;
-            while ((left | litrem | (int)pend | (int)fin) != 0) {
-                uint64_t v = 0;
-                uint32_t nb = 0;
-                if ((litrem | (int)pend) == 0) {
-                    int lit;
-                    uint32_t tok;
-                    if (left > 0) {
-#pragma unroll
-                        for (int r = 0; r + 1 < NW; ++r) {
-                            const bool z = Rp[0] == 0u;
-#pragma unroll
-                            for (int k = 0; k + 1 < NW; ++k) { Rp[k] = z ? Rp[k + 1] : Rp[k]; K[k] = z ? K[k + 1] : K[k]; }
-                            Rp[NW - 1] = z ? 0u : Rp[NW - 1];
-                            base += z ? 32 : 0;
-                        }
-                        const uint32_t low = Rp[0] & (0u - Rp[0]);
-                        const int ts = __popc(low - 1u);
-                        const bool is_k = (K[0] & low) != 0u;
-                        uint64_t cy = low;
-                        int ml = 1;
-#pragma unroll
-                        for (int k = 0; k < NW; ++k) {
-                            cy += Rp[k];
-                            const uint32_t t = (uint32_t)cy;
-                            cy >>= 32;
-                            ml += __popc(Rp[k] & ~t);
-                            Rp[k] &= t;
-                        }
-                        lit = base + ts - pos;
-                        cur_ml = ml;
-                        cur_off = is_k ? (uint32_t)cr : 2u * (uint32_t)cr;
-                        pend = 1;
-                        --left;
-                        tok = (uint32_t)((min(lit, 15) << 4) | min(ml - 4, 15));
-                    } else {
-                        lit = final_lit;
-                        fin = 0;
-                        tok = (uint32_t)(min(lit, 15) << 4);
-                    }
-                    v = tok; nb = 1;
-                    if (lit >= 15) {
-                        int rem = lit - 15;
-#pragma unroll 1
-                        while (rem >= 255) { put(v, nb); v = 255u; nb = 1; rem -= 255; }
-                        v |= (uint64_t)(uint32_t)rem << (8u * nb);
-                        ++nb;
-                    }
-                    litrem = pend ? lit : 0;
-                }
-                const int take = min(litrem, 8 - (int)nb);
-                if (take > 0) {
-                    v |= lit8(pos, take) << (8u * nb);
-                    nb += (uint32_t)take; pos += take; litrem -= take;
-                }
-                if (pend != 0 && litrem == 0) {
-                    const uint32_t ob = cur_ml >= 19 ? 3u : 2u;
-                    if (nb + ob <= 8u) {
-                        v |= (uint64_t)(cur_off | (cur_ml >= 19 ? (uint32_t)(cur_ml - 19) << 16 : 0u)) << (8u * nb);
-                        nb += ob; pend = 0; pos += cur_ml;
-                    }
-                }
-                put(v, nb);
-            }
-            {
-                const uint64_t fv = first ? acc : fw;
-                if ((uint32_t)fv) sts_or32(faddr, (uint32_t)fv);
-                if ((uint32_t)(fv >> 32)) sts_or32(faddr + 4u, (uint32_t)(fv >> 32));
-                if (!first) {
-                    if ((uint32_t)acc) sts_or32(waddr, (uint32_t)acc);
-                    if ((uint32_t)(acc >> 32)) sts_or32(waddr + 4u, (uint32_t)(acc >> 32));
-                }
-            }
         }
+        const int final_lit = carry_in;
         const int dlen = pass_base + 1 + lit_ext(final_lit) + final_lit;
         __syncwarp();
-        {   // the block's closing literals: one byte per lane and step
-            uint8_t *fdst = seq + (dlen - final_lit);
-            const int fx = n - final_lit;
-            for (int i = lane; i < final_lit; i += 32) {
-                const int x = fx + i, G = alpha + x;
-                uint32_t byte = (strB[G >> 5] >> (G & 31)) & 1u;
-                if (any_n && ((strN[G >> 5] >> (G & 31)) & 1u))
-                    byte = (uint8_t)(x < cr ? A.gt0 : A.gt1)[grow + (x < cr ? x : x - cr)];
-                fdst[i] = (uint8_t)byte;
-            }
-        }
+        closing_literals(seq + (dlen - final_lit), final_lit, ab);
         // ---- 6. the frame leaves: header + template body from global memory (size fields filled in), own tail by a
         //         TMA bulk store.  A size field that lies behind tl16 sits in the tail buffer's first bytes.
         const uint32_t flen = tl + (uint32_t)dlen;
@@ -1480,7 +1243,6 @@ static int frames_prepare(hb_frames *f, hb_parse *p, bool early) {
     CUF(cudaSetDevice(f->device));
     const uint64_t n = f->n_records;
     const uint32_t cr = (uint32_t)f->cr;
-    const uint64_t n_frames = f->n_chunks * f->n_samples;
     f->layout_valid = false;
     f->totals_valid = false;
     const bool was_early = f->early_site;
@@ -2160,7 +1922,8 @@ int hb_frames_fetch_sample(hb_frames *f, uint32_t s, uint64_t *sizes, uint8_t *b
 // for this path too -- several blocks per chunk, LZ4 / LZ4HC streams, split and unsplit blocks, raw streams,
 // memcpyed chunks -- and the extended (32-byte) header of a c-blosc2 chunk with byte-shuffle as its only filter;
 // anything else, and every field that would make the kernel read or write outside the frame / its output, sets the
-// frame's status to non-zero (a stored file is untrusted input).
+// frame's status to non-zero (a stored file is untrusted input).  The three decoders (decode_frames_kernel, kernels 6
+// and 6-L) read the header with read_blosc_head and walk LZ4 with lz4_walk, so those checks exist once.
 // =============================================================================================
 namespace hb {
 
@@ -2168,10 +1931,12 @@ __device__ __forceinline__ uint32_t ld_le32(const uint8_t *p) {
     return p[0] | (p[1] << 8) | (p[2] << 16) | ((uint32_t)p[3] << 24);
 }
 
-// LZ4 block decode by one warp: sequences are walked in lock-step, bytes are copied 32 per step.
-// dst is global memory written and re-read by different lanes: reads go through L2 (__ldcg).
-__device__ bool warp_lz4_decode(const uint8_t *src, uint32_t n, uint8_t *dst, uint32_t cap) {
-    const int lane = threadIdx.x & 31;
+// LZ4 block walk by one warp: sequences are walked in lock-step, every check on the untrusted stream is made here.  True
+// iff the stream is well-formed and decodes to exactly cap bytes.  `out` says what happens to the bytes:
+// out.lit(op, p, ll) receives the literals of positions [op, op + ll), out.match(op, off, ml) repeats ml bytes from off
+// back (off <= op).
+template <class Out>
+__device__ bool lz4_walk(const uint8_t *__restrict__ src, uint32_t n, uint32_t cap, const Out &out) {
     uint32_t ip = 0, op = 0;
     if (n == 0) return false;
     for (;;) {
@@ -2180,7 +1945,7 @@ __device__ bool warp_lz4_decode(const uint8_t *src, uint32_t n, uint8_t *dst, ui
         uint32_t ll = tok >> 4;
         if (ll == 15) { uint32_t b; do { if (ip >= n) return false; b = src[ip++]; ll += b; } while (b == 255 && ll <= cap); }
         if (ll > n - ip || ll > cap - op) return false;
-        for (uint32_t i = lane; i < ll; i += 32) dst[op + i] = src[ip + i];
+        out.lit(op, src + ip, ll);
         ip += ll; op += ll;
         if (ip == n) break;
         if (ip + 2 > n) return false;
@@ -2191,17 +1956,79 @@ __device__ bool warp_lz4_decode(const uint8_t *src, uint32_t n, uint8_t *dst, ui
         if (ml == 15) { uint32_t b; do { if (ip >= n) return false; b = src[ip++]; ml += b; } while (b == 255 && ml <= cap); }
         ml += 4;
         if (ml > cap - op) return false;
-        __syncwarp();
-        // periodic copy: dst[op+i] = dst[op-off + i % off] only reads bytes written before this match
-        for (uint32_t i = lane; i < ml; i += 32) {
-            const uint32_t k = off >= ml ? i : i % off;
-            dst[op + i] = __ldcg(dst + op - off + k);
-        }
+        out.match(op, off, ml);
         op += ml;
-        __syncwarp();
     }
     __syncwarp();
     return op == cap;
+}
+
+__device__ __forceinline__ void warp_copy(uint8_t *dst, const uint8_t *src, uint32_t n) {
+    for (uint32_t i = threadIdx.x & 31; i < n; i += 32) dst[i] = src[i];
+}
+
+// into global memory, written and re-read by different lanes: matches read through L2 (__ldcg)
+struct Lz4ToGlobal {
+    uint8_t *dst;
+    __device__ void lit(uint32_t op, const uint8_t *p, uint32_t ll) const { warp_copy(dst + op, p, ll); }
+    __device__ void match(uint32_t op, uint32_t off, uint32_t ml) const {
+        __syncwarp();
+        // periodic copy: dst[op+i] = dst[op-off + i % off] only reads bytes written before this match
+        for (uint32_t i = threadIdx.x & 31; i < ml; i += 32) {
+            const uint32_t k = off >= ml ? i : i % off;
+            dst[op + i] = __ldcg(dst + op - off + k);
+        }
+        __syncwarp();
+    }
+};
+
+// into shared memory
+struct Lz4ToShared {
+    uint8_t *dst;
+    __device__ void lit(uint32_t op, const uint8_t *p, uint32_t ll) const { warp_copy(dst + op, p, ll); }
+    __device__ void match(uint32_t op, uint32_t off, uint32_t ml) const {
+        __syncwarp();
+        if (off >= ml) {                                // source and destination do not overlap
+            for (uint32_t i = threadIdx.x & 31; i < ml; i += 32) dst[op + i] = dst[op - off + i];
+        } else {                                        // periodic: dst[op + i] = dst[op - off + i % off]; every source precedes op
+            for (uint32_t i = threadIdx.x & 31; i < ml; i += 32) dst[op + i] = dst[op - off + i % off];
+        }
+        __syncwarp();
+    }
+};
+
+// nowhere: the walk only checks the stream
+struct Lz4Check {
+    __device__ void lit(uint32_t, const uint8_t *, uint32_t) const {}
+    __device__ void match(uint32_t, uint32_t, uint32_t) const {}
+};
+
+// A Blosc chunk's 16-byte header (c-blosc 1.x), or the 32-byte one of c-blosc2 (both shuffle bits set), read and checked.
+struct BloscHead {
+    uint32_t flags, ext, hdr, shuffle, typesize, cn, bs, ccb;   // shuffle: the stored bytes are byte-shuffled
+    int err;
+};
+// Status codes, first failure wins: 1 shorter than a header; 2 format version or reserved bit; then the decoder's own size
+// checks, `sizes(h)`, which returns its code or 0; 3 a c-blosc2 filter other than byte-shuffle; 6 a special chunk
+// (runs of zeros / NaNs / uninit); 5 neither memcpyed nor LZ4 / LZ4HC.
+template <class Sizes>
+__device__ __forceinline__ BloscHead read_blosc_head(const uint8_t *c, uint64_t flen, Sizes sizes) {
+    BloscHead h{0, 0, 16, 0, 1, 0, 0, 0, 0};
+    if (flen < 16) { h.err = 1; return h; }
+    h.flags = c[2]; h.typesize = c[3];
+    h.cn = ld_le32(c + 4); h.bs = ld_le32(c + 8); h.ccb = ld_le32(c + 12);
+    h.ext = (h.flags & 1) && (h.flags & 4);
+    h.hdr = h.ext ? 32 : 16;
+    h.shuffle = !h.ext && (h.flags & 1);
+    if (c[0] < 2 || c[0] > 5 || (!h.ext && (c[0] != 2 || (h.flags & 0x08)))) h.err = 2;
+    else h.err = sizes(h);
+    if (!h.err && h.ext) {
+        for (int i = 0; i < 6; ++i) { if (c[16 + i] == 1) h.shuffle = 1; else if (c[16 + i] != 0) h.err = 3; }
+        if ((c[31] >> 4) & 7) h.err = 6;
+    }
+    if (h.flags & 2) h.shuffle = 0;                  // memcpyed: the bytes as they were given, never shuffled
+    else if (!h.err && ((h.flags >> 5) != 1 || (!h.ext && c[1] != 1))) h.err = 5;
+    return h;
 }
 
 constexpr uint32_t kBloscMaxSplits = 16, kBloscMinBuffer = 128;      // c-blosc: MAX_SPLITS, MIN_BUFFERSIZE
@@ -2219,39 +2046,26 @@ decode_frames_kernel(const uint8_t *__restrict__ frames, const uint64_t *__restr
     const uint64_t flen = len ? (uint64_t)len[wid] : off[wid + 1] - off[wid];
     uint8_t *t = tmp + wid * (uint64_t)chunk_nbytes;
     uint8_t *o = out + wid * (uint64_t)chunk_nbytes;
-    int err = 0;
-    uint32_t typesize = 1, cn = 0, bs = 0, ccb = 0, hdr = 16, flags = 0;
-    bool ext = false, shuffle = false;
-    if (flen < 16) err = 1;
-    if (!err) {
-        flags = c[2]; typesize = c[3];
-        cn = ld_le32(c + 4); bs = ld_le32(c + 8); ccb = ld_le32(c + 12);
-        ext = (flags & 1) && (flags & 4);                    // c-blosc2: both shuffle bits = extended header
-        hdr = ext ? 32 : 16;
-        shuffle = !ext && (flags & 1);
-        if (c[0] < 2 || c[0] > 5 || (!ext && (c[0] != 2 || (flags & 0x08)))) err = 2;      // format version / reserved bit
-        else if (cn != chunk_nbytes || ccb > flen || ccb < hdr || bs == 0 || bs > cn || typesize == 0) err = 4;
-    }
-    if (!err && ext) {
-        for (int i = 0; i < 6; ++i) { if (c[16 + i] == 1) shuffle = true; else if (c[16 + i] != 0) err = 3; }
-        if ((c[31] >> 4) & 7) err = 6;                       // special chunks (runs of zeros / NaNs / uninit)
-    }
-    if (!err && (flags & 2)) {                               // memcpyed: the bytes as they were given, never shuffled
+    const BloscHead h = read_blosc_head(c, flen, [&](const BloscHead &x) {
+        return x.cn != chunk_nbytes || x.ccb > flen || x.ccb < x.hdr || x.bs == 0 || x.bs > x.cn || x.typesize == 0 ? 4 : 0;
+    });
+    const uint32_t typesize = h.typesize, cn = h.cn, bs = h.bs, ccb = h.ccb, hdr = h.hdr;
+    const bool shuffle = h.shuffle;
+    int err = h.err;
+    if (!err && (h.flags & 2)) {                             // memcpyed
         if ((uint64_t)hdr + cn > ccb) err = 7;
-        else for (uint32_t i = lane; i < cn; i += 32) t[i] = c[hdr + i];
-        shuffle = false;
+        else warp_copy(t, c + hdr, cn);
         planar = 1;                                          // nothing to undo
     } else if (!err) {
-        if ((flags >> 5) != 1 || (!ext && c[1] != 1)) err = 5;       // LZ4 / LZ4HC codec format, its format version
-        const bool dont_split = flags & 0x10;
+        const bool dont_split = h.flags & 0x10;
         const uint32_t nblocks = (cn + bs - 1) / bs;
         const uint64_t data0 = (uint64_t)hdr + 4ull * nblocks;        // first byte after bstarts
-        if (!err && data0 > ccb) err = 7;
+        if (data0 > ccb) err = 7;
         for (uint32_t b = 0; b < nblocks && !err; ++b) {
             const bool leftover = (b == nblocks - 1) && (cn % bs);
             const uint32_t bsize = leftover ? cn % bs : bs;
             const bool split = !dont_split && !leftover &&
-                               (ext || (typesize <= kBloscMaxSplits && bs / typesize >= kBloscMinBuffer));
+                               (h.ext || (typesize <= kBloscMaxSplits && bs / typesize >= kBloscMinBuffer));
             const uint32_t nstreams = split ? typesize : 1;
             const uint32_t ne = bsize / nstreams;
             uint64_t ip = ld_le32(c + hdr + 4 * b);
@@ -2261,10 +2075,10 @@ decode_frames_kernel(const uint8_t *__restrict__ frames, const uint64_t *__restr
                 const int32_t cs = (int32_t)ld_le32(c + ip);
                 ip += 4;
                 uint8_t *d = t + (uint64_t)b * bs + (uint64_t)s * ne;
-                if (cs == 0 && ext) { for (uint32_t i = lane; i < ne; i += 32) d[i] = 0; }        // c-blosc2: run of zeros
+                if (cs == 0 && h.ext) { for (uint32_t i = lane; i < ne; i += 32) d[i] = 0; }        // c-blosc2: run of zeros
                 else if (cs <= 0 || ip + (uint32_t)cs > ccb) err = 8;
-                else if ((uint32_t)cs == ne) { for (uint32_t i = lane; i < ne; i += 32) d[i] = c[ip + i]; ip += cs; }
-                else { if (!warp_lz4_decode(c + ip, (uint32_t)cs, d, ne)) err = 9; ip += cs; }
+                else if ((uint32_t)cs == ne) { warp_copy(d, c + ip, ne); ip += cs; }
+                else { if (!lz4_walk(c + ip, (uint32_t)cs, ne, Lz4ToGlobal{d})) err = 9; ip += cs; }
                 __syncwarp();
             }
         }
@@ -2310,216 +2124,112 @@ struct DecodeColsArgs {
     uint32_t warp_smem;
 };
 
-// LZ4 block decode by one warp into shared memory.  Returns true iff exactly cap bytes came out.
-__device__ bool warp_lz4_decode_smem(const uint8_t *__restrict__ src, uint32_t n, uint8_t *dst, uint32_t cap) {
-    const int lane = threadIdx.x & 31;
-    uint32_t ip = 0, op = 0;
-    if (n == 0) return false;
-    for (;;) {
-        if (ip >= n) return false;
-        const uint32_t tok = src[ip++];
-        uint32_t ll = tok >> 4;
-        if (ll == 15) { uint32_t b; do { if (ip >= n) return false; b = src[ip++]; ll += b; } while (b == 255 && ll <= cap); }
-        if (ll > n - ip || ll > cap - op) return false;
-        for (uint32_t i = lane; i < ll; i += 32) dst[op + i] = src[ip + i];
-        ip += ll; op += ll;
-        if (ip == n) break;
-        if (ip + 2 > n) return false;
-        const uint32_t off = src[ip] | ((uint32_t)src[ip + 1] << 8);
-        ip += 2;
-        if (off == 0 || off > op) return false;
-        uint32_t ml = tok & 15;
-        if (ml == 15) { uint32_t b; do { if (ip >= n) return false; b = src[ip++]; ml += b; } while (b == 255 && ml <= cap); }
-        ml += 4;
-        if (ml > cap - op) return false;
-        __syncwarp();
-        if (off >= ml) {                                // source and destination do not overlap
-            for (uint32_t i = lane; i < ml; i += 32) dst[op + i] = dst[op - off + i];
-        } else {                                        // periodic: dst[op + i] = dst[op - off + i % off]; every source precedes op
-            for (uint32_t i = lane; i < ml; i += 32) dst[op + i] = dst[op - off + i % off];
-        }
-        op += ml;
-        __syncwarp();
+// Where the one block of a chunk of `nbytes` bytes is, for kernels 6 and 6-L.  h.err = the status code; without an
+// error: a c-blosc2 run of zeros (zero), or src = the block's bytes in place (memcpyed, or stored raw) or its LZ4 stream
+// of cs bytes (lz).  (src is never compared with null: with absolute offsets the frame base is null.)  Code 11: several blocks per chunk, or a c-blosc2 block split into `typesize` streams (no
+// dont-split flag 0x10); the host-pointer decoder reads those.
+struct SingleBlock {
+    BloscHead h;
+    const uint8_t *src;
+    uint32_t cs;
+    bool zero, lz;
+};
+__device__ __forceinline__ SingleBlock locate_single_block(const uint8_t *c, uint32_t flen, uint32_t nbytes) {
+    SingleBlock b{read_blosc_head(c, flen, [&](const BloscHead &x) {
+                      if (x.typesize != 35 || x.cn != nbytes || x.ccb > flen || x.ccb < x.hdr) return 4;
+                      return !(x.flags & 2) && (x.bs != x.cn || (x.ext && !(x.flags & 0x10))) ? 11 : 0;
+                  }),
+                  nullptr, 0, false, false};
+    BloscHead &h = b.h;
+    if (h.err) return b;
+    if (h.flags & 2) {                                   // memcpyed: record-major
+        if ((uint64_t)h.hdr + nbytes > h.ccb) h.err = 7;
+        else b.src = c + h.hdr;
+        return b;
     }
-    __syncwarp();
-    return op == cap;
+    const uint64_t data0 = (uint64_t)h.hdr + 4;
+    if (data0 + 4 > h.ccb) { h.err = 7; return b; }
+    uint64_t ip = ld_le32(c + h.hdr);
+    if (ip < data0 || ip + 4 > h.ccb) { h.err = 7; return b; }
+    const int32_t cs = (int32_t)ld_le32(c + ip);
+    ip += 4;
+    if (cs == 0 && h.ext) { b.zero = true; return b; }  // c-blosc2: run of zeros
+    if (cs <= 0 || ip + (uint32_t)cs > h.ccb) { h.err = 8; return b; }
+    b.src = c + ip;
+    b.cs = (uint32_t)cs;
+    b.lz = (uint32_t)cs != nbytes;
+    return b;
+}
+
+// the six columns of records [0, cr) at rows row0 + r from B(r, f) = byte f of record r: one record per lane and step
+template <class Byte>
+__device__ __forceinline__ void write_columns(const DecodeColsArgs &a, uint64_t row0, Byte B) {
+    for (uint32_t r = threadIdx.x & 31; r < a.cr; r += 32) {
+        if (a.start) a.start[row0 + r] = B(r, kRecStart) | (B(r, kRecStart + 1) << 8) | (B(r, kRecStart + 2) << 16) | (B(r, kRecStart + 3) << 24);
+        if (a.stop) a.stop[row0 + r] = B(r, kRecStop) | (B(r, kRecStop + 1) << 8) | (B(r, kRecStop + 2) << 16) | (B(r, kRecStop + 3) << 24);
+        if (a.ref) a.ref[row0 + r] = (uint8_t)B(r, kRecRef);
+        if (a.alt) a.alt[row0 + r] = (uint8_t)B(r, kRecAlt);
+        if (a.p1) a.p1[row0 + r] = (int8_t)B(r, kRecP1);
+        if (a.p2) a.p2[row0 + r] = (int8_t)B(r, kRecP2);
+    }
 }
 
 __global__ void __launch_bounds__(128) decode_columns_kernel(const DecodeColsArgs a) {
     extern __shared__ __align__(16) uint8_t dsm[];
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int warp = threadIdx.x >> 5;
     const uint64_t wid = (uint64_t)blockIdx.x * (blockDim.x >> 5) + warp;
     if (wid >= a.n) return;
     uint8_t *t = dsm + (size_t)warp * a.warp_smem;
-    const uint8_t *c = a.frames + a.off[wid];
-    const uint32_t flen = a.len[wid];
-    const uint32_t nbytes = 35u * a.cr;
-    int err = 0;
-    uint32_t flags = 0, bs = 0, ccb = 0, hdr = 16;
-    bool ext = false, shuffle = false;
-    if (flen < 16) err = 1;
+    const uint32_t cr = a.cr, nbytes = 35u * cr;
+    const SingleBlock blk = locate_single_block(a.frames + a.off[wid], a.len[wid], nbytes);
+    int err = blk.h.err;
     if (!err) {
-        flags = c[2];
-        const uint32_t cn = ld_le32(c + 4);
-        bs = ld_le32(c + 8); ccb = ld_le32(c + 12);
-        ext = (flags & 1) && (flags & 4);
-        hdr = ext ? 32 : 16;
-        shuffle = !ext && (flags & 1);
-        if (c[0] < 2 || c[0] > 5 || (!ext && (c[0] != 2 || (flags & 0x08)))) err = 2;
-        else if (c[3] != 35 || cn != nbytes || ccb > flen || ccb < hdr) err = 4;
-        // several blocks per chunk, or a c-blosc2 block split into `typesize` streams (no dont-split flag 0x10): the
-        // host-pointer decoder reads those
-        else if (!(flags & 2) && (bs != cn || (ext && !(flags & 0x10)))) err = 11;
-    }
-    if (!err && ext) {
-        for (int i = 0; i < 6; ++i) { if (c[16 + i] == 1) shuffle = true; else if (c[16 + i] != 0) err = 3; }
-        if ((c[31] >> 4) & 7) err = 6;
-    }
-    if (!err && (flags & 2)) {                                       // memcpyed
-        if ((uint64_t)hdr + nbytes > ccb) err = 7;
-        else for (uint32_t i = lane; i < nbytes; i += 32) t[i] = c[hdr + i];
-        shuffle = false;
-    } else if (!err) {
-        if ((flags >> 5) != 1 || (!ext && c[1] != 1)) err = 5;
-        const uint64_t data0 = (uint64_t)hdr + 4;
-        uint64_t ip = 0;
-        if (!err && data0 + 4 > ccb) err = 7;
-        if (!err) { ip = ld_le32(c + hdr); if (ip < data0 || ip + 4 > ccb) err = 7; }
-        if (!err) {
-            const int32_t cs = (int32_t)ld_le32(c + ip);
-            ip += 4;
-            if (cs == 0 && ext) { for (uint32_t i = lane; i < nbytes; i += 32) t[i] = 0; }
-            else if (cs <= 0 || ip + (uint32_t)cs > ccb) err = 8;
-            else if ((uint32_t)cs == nbytes) { for (uint32_t i = lane; i < nbytes; i += 32) t[i] = c[ip + i]; }
-            else if (!warp_lz4_decode_smem(c + ip, (uint32_t)cs, t, nbytes)) err = 9;
-        }
+        if (blk.lz) { if (!lz4_walk(blk.src, blk.cs, nbytes, Lz4ToShared{t})) err = 9; }
+        else if (blk.zero) for (uint32_t i = threadIdx.x & 31; i < nbytes; i += 32) t[i] = 0;
+        else warp_copy(t, blk.src, nbytes);
     }
     __syncwarp();
-    if (!err) {
-        const uint32_t cr = a.cr;
-        const uint64_t row0 = a.row[wid];
-        // byte f of record r: plane-major when the chunk was byte-shuffled, record-major otherwise
-        for (uint32_t r = lane; r < cr; r += 32) {
-            auto B = [&](uint32_t f) -> uint32_t { return shuffle ? t[f * cr + r] : t[r * 35u + f]; };
-            if (a.start) a.start[row0 + r] = B(5) | (B(6) << 8) | (B(7) << 16) | (B(8) << 24);
-            if (a.stop) a.stop[row0 + r] = B(9) | (B(10) << 8) | (B(11) << 16) | (B(12) << 24);
-            if (a.ref) a.ref[row0 + r] = (uint8_t)B(13);
-            if (a.alt) a.alt[row0 + r] = (uint8_t)B(23);
-            if (a.p1) a.p1[row0 + r] = (int8_t)B(33);
-            if (a.p2) a.p2[row0 + r] = (int8_t)B(34);
-        }
-    }
-    if (lane == 0) a.status[wid] = err;
+    // byte f of record r: plane-major when the chunk was byte-shuffled, record-major otherwise
+    const bool shuffle = blk.h.shuffle;
+    if (!err) write_columns(a, a.row[wid], [&](uint32_t r, uint32_t f) -> uint32_t { return shuffle ? t[f * cr + r] : t[r * 35u + f]; });
+    if ((threadIdx.x & 31) == 0) a.status[wid] = err;
 }
 
 // ---------------------------------------------------------------------------------------------
 // Kernel 6-L: decode_columns_kernel for single-block chunks whose 35 * cr bytes do not fit a warp's shared memory (up to
-// kMaxChunkRecords).  One warp (= one CTA) per chunk.  An LZ4 offset is at most 65,535, so the decoded block streams
-// through a 64 KiB history ring in shared memory and every byte of the planes the columns need (5-13, 23, 33, 34) goes
-// straight to its column.  The stream is first walked once without copying -- the checks of warp_lz4_decode_smem are
-// all structural -- so a chunk that fails writes no row, as in kernel 6.  Stored-raw, memcpyed and zero-run chunks are
-// read in place.  The header checks and status codes are kernel 6's.
+// kMaxChunkRecords).  One warp (= one CTA) per chunk.  Shared with kernel 6: the header and block checks
+// (locate_single_block, so the status codes are the same), the LZ4 checks (lz4_walk) and the column writer.  What
+// differs: an LZ4 offset is at most 65,535, so the decoded block streams through a 64 KiB history ring in shared memory
+// and every byte of the planes the columns need (5-13, 23, 33, 34) goes straight to its column.  The stream is first
+// walked once without copying -- its checks are all structural -- so a chunk that fails writes no row, as in kernel 6.
+// Stored-raw, memcpyed and zero-run chunks are read in place.
 // ---------------------------------------------------------------------------------------------
 constexpr uint32_t kHistRing = 1u << 16;
 
-// The checks of warp_lz4_decode_smem without the copies: true iff the block decodes to exactly cap bytes.
-__device__ bool lz4_block_valid(const uint8_t *__restrict__ src, uint32_t n, uint32_t cap) {
-    uint32_t ip = 0, op = 0;
-    if (n == 0) return false;
-    for (;;) {
-        if (ip >= n) return false;
-        const uint32_t tok = src[ip++];
-        uint32_t ll = tok >> 4;
-        if (ll == 15) { uint32_t b; do { if (ip >= n) return false; b = src[ip++]; ll += b; } while (b == 255 && ll <= cap); }
-        if (ll > n - ip || ll > cap - op) return false;
-        ip += ll; op += ll;
-        if (ip == n) break;
-        if (ip + 2 > n) return false;
-        const uint32_t off = src[ip] | ((uint32_t)src[ip + 1] << 8);
-        ip += 2;
-        if (off == 0 || off > op) return false;
-        uint32_t ml = tok & 15;
-        if (ml == 15) { uint32_t b; do { if (ip >= n) return false; b = src[ip++]; ml += b; } while (b == 255 && ml <= cap); }
-        ml += 4;
-        if (ml > cap - op) return false;
-        op += ml;
-    }
-    return op == cap;
-}
-
 // byte f of record r -> its column (f outside the six columns: nothing)
 __device__ __forceinline__ void put_column_byte(const DecodeColsArgs &a, uint64_t row, uint32_t f, uint8_t v) {
-    if (f >= 5 && f < 9) { if (a.start) reinterpret_cast<uint8_t *>(a.start + row)[f - 5] = v; }
-    else if (f >= 9 && f < 13) { if (a.stop) reinterpret_cast<uint8_t *>(a.stop + row)[f - 9] = v; }
-    else if (f == 13) { if (a.ref) a.ref[row] = v; }
-    else if (f == 23) { if (a.alt) a.alt[row] = v; }
-    else if (f == 33) { if (a.p1) a.p1[row] = (int8_t)v; }
-    else if (f == 34) { if (a.p2) a.p2[row] = (int8_t)v; }
+    if (f >= kRecStart && f < kRecStart + 4) { if (a.start) reinterpret_cast<uint8_t *>(a.start + row)[f - kRecStart] = v; }
+    else if (f >= kRecStop && f < kRecStop + 4) { if (a.stop) reinterpret_cast<uint8_t *>(a.stop + row)[f - kRecStop] = v; }
+    else if (f == kRecRef) { if (a.ref) a.ref[row] = v; }
+    else if (f == kRecAlt) { if (a.alt) a.alt[row] = v; }
+    else if (f == kRecP1) { if (a.p1) a.p1[row] = (int8_t)v; }
+    else if (f == kRecP2) { if (a.p2) a.p2[row] = (int8_t)v; }
 }
 
 __global__ void __launch_bounds__(32) decode_columns_large_kernel(const DecodeColsArgs a) {
     extern __shared__ __align__(16) uint8_t ring[];
     const int lane = threadIdx.x;
     const uint64_t wid = blockIdx.x;
-    const uint8_t *c = a.frames + a.off[wid];
-    const uint32_t flen = a.len[wid];
     const uint32_t cr = a.cr, nbytes = 35u * cr;
-    int err = 0;
-    uint32_t flags = 0, bs = 0, ccb = 0, hdr = 16;
-    bool ext = false, shuffle = false;
-    if (flen < 16) err = 1;
-    if (!err) {
-        flags = c[2];
-        const uint32_t cn = ld_le32(c + 4);
-        bs = ld_le32(c + 8); ccb = ld_le32(c + 12);
-        ext = (flags & 1) && (flags & 4);
-        hdr = ext ? 32 : 16;
-        shuffle = !ext && (flags & 1);
-        if (c[0] < 2 || c[0] > 5 || (!ext && (c[0] != 2 || (flags & 0x08)))) err = 2;
-        else if (c[3] != 35 || cn != nbytes || ccb > flen || ccb < hdr) err = 4;
-        else if (!(flags & 2) && (bs != cn || (ext && !(flags & 0x10)))) err = 11;
-    }
-    if (!err && ext) {
-        for (int i = 0; i < 6; ++i) { if (c[16 + i] == 1) shuffle = true; else if (c[16 + i] != 0) err = 3; }
-        if ((c[31] >> 4) & 7) err = 6;
-    }
-    const uint8_t *src = nullptr;                     // the block's bytes in place (memcpyed / stored raw); null + lz: LZ4
-    bool zero = false, lz = false;
-    uint32_t cs = 0;
-    if (!err && (flags & 2)) {                        // memcpyed: record-major
-        if ((uint64_t)hdr + nbytes > ccb) err = 7;
-        else src = c + hdr;
-        shuffle = false;
-    } else if (!err) {
-        if ((flags >> 5) != 1 || (!ext && c[1] != 1)) err = 5;
-        const uint64_t data0 = (uint64_t)hdr + 4;
-        uint64_t ip = 0;
-        if (!err && data0 + 4 > ccb) err = 7;
-        if (!err) { ip = ld_le32(c + hdr); if (ip < data0 || ip + 4 > ccb) err = 7; }
-        if (!err) {
-            const int32_t s32 = (int32_t)ld_le32(c + ip);
-            ip += 4;
-            cs = (uint32_t)s32;
-            if (s32 == 0 && ext) zero = true;
-            else if (s32 <= 0 || ip + cs > ccb) err = 8;
-            else if (cs == nbytes) src = c + ip;
-            else if (!lz4_block_valid(c + ip, cs, nbytes)) err = 9;
-            else { src = c + ip; lz = true; }
-        }
-    }
-    if (lane == 0) a.status[wid] = err;
-    if (err) return;
+    SingleBlock blk = locate_single_block(a.frames + a.off[wid], a.len[wid], nbytes);
+    if (!blk.h.err && blk.lz && !lz4_walk(blk.src, blk.cs, nbytes, Lz4Check{})) blk.h.err = 9;
+    if (lane == 0) a.status[wid] = blk.h.err;
+    if (blk.h.err) return;
     const uint64_t row0 = a.row[wid];
-    if (!lz) {                                        // in place, one record per lane and step (kernel 6's loop)
-        for (uint32_t r = lane; r < cr; r += 32) {
-            auto B = [&](uint32_t f) -> uint32_t { return zero ? 0u : shuffle ? src[f * cr + r] : src[r * 35u + f]; };
-            if (a.start) a.start[row0 + r] = B(5) | (B(6) << 8) | (B(7) << 16) | (B(8) << 24);
-            if (a.stop) a.stop[row0 + r] = B(9) | (B(10) << 8) | (B(11) << 16) | (B(12) << 24);
-            if (a.ref) a.ref[row0 + r] = (uint8_t)B(13);
-            if (a.alt) a.alt[row0 + r] = (uint8_t)B(23);
-            if (a.p1) a.p1[row0 + r] = (int8_t)B(33);
-            if (a.p2) a.p2[row0 + r] = (int8_t)B(34);
-        }
+    const uint8_t *src = blk.src;
+    const bool shuffle = blk.h.shuffle, zero = blk.zero;
+    if (!blk.lz) {                                      // in place
+        write_columns(a, row0, [&](uint32_t r, uint32_t f) -> uint32_t { return zero ? 0u : shuffle ? src[f * cr + r] : src[r * 35u + f]; });
         return;
     }
     // block position q -> (plane, record) when shuffled, (record, field) otherwise: q / d by a multiply-high, exact for
@@ -2530,6 +2240,7 @@ __global__ void __launch_bounds__(32) decode_columns_large_kernel(const DecodeCo
         if (shuffle) put_column_byte(a, row0 + lo, hi, v);
         else put_column_byte(a, row0 + hi, lo, v);
     };
+    const uint32_t cs = blk.cs;
     uint32_t ip = 0, op = 0;
     for (;;) {                                        // the stream is valid: no bounds checks
         const uint32_t tok = src[ip++];
