@@ -31,8 +31,8 @@ namespace hb {
 
 static thread_local std::string g_err;
 static std::atomic<uint64_t> g_launches{0};
-static std::atomic<uint64_t> g_text_limit{0};
-static std::atomic<uint32_t> g_walker_lines{16};   // hb_set_walker_lines      // hb_parse_set_text_limit: 0 = from free device memory
+static std::atomic<uint64_t> g_text_limit{0};        // hb_parse_set_text_limit: 0 = from free device memory
+static std::atomic<uint32_t> g_walker_lines{16};   // hb_set_walker_lines
 static std::atomic<uint64_t> g_bcf_segment{0};     // hb_set_bcf_segment_bytes: 0 = max(64 KiB, 8 x the first record)
 static const char *const kBcfNoStream =
     "BCF streaming is not supported: read a .bcf with hb_parse_file, hb_parse_vcf_bytes or hb_load_vcf";
@@ -43,12 +43,16 @@ static int fail(int code, const std::string &msg) {
     return code;
 }
 int api_fail(int code, const std::string &msg) { return fail(code, msg); }
-#define CU(expr)                                                                                      \
-    do {                                                                                              \
-        cudaError_t e_ = (expr);                                                                      \
-        if (e_ != cudaSuccess)                                                                        \
-            return fail(HB_ERR_CUDA, std::string("CUDA: ") + cudaGetErrorString(e_) + " at " #expr); \
+static int fail_cuda(cudaError_t e, const char *where = "") {
+    return fail(HB_ERR_CUDA, std::string("CUDA: ") + cudaGetErrorString(e) + where);
+}
+#define CU(expr)                                                   \
+    do {                                                           \
+        cudaError_t e_ = (expr);                                   \
+        if (e_ != cudaSuccess) return fail_cuda(e_, " at " #expr); \
     } while (0)
+
+static double now_ms() { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now().time_since_epoch()).count(); }
 
 static int ensure_device(int device) {
     int n = 0;
@@ -105,7 +109,6 @@ using namespace hb;
 // =============================================================================================
 // hb_parse: one device-resident parse
 // =============================================================================================
-#include "hb_parse_struct.h"
 
 // ---- big device buffers are pooled.  cudaMalloc / cudaFree of GB-sized buffers take anything from 10 to 500 ms on these
 // hosts (measured inside the streaming entry points); a converter that walks 22 chromosome files, or a caller that makes a
@@ -194,6 +197,13 @@ void dev_pool_free(void *p) {
     }
     cudaFree(p);
 }
+void dev_pool_release(void *p) {
+    {
+        std::lock_guard<std::mutex> lk(g_pool.mu);
+        g_pool.live.erase(p);
+    }
+    cudaFree(p);
+}
 }  // namespace hb
 
 static void free_dev(void *p) { hb::dev_pool_free(p); }
@@ -240,14 +250,13 @@ bool host_is_pinned(const void *p) { return is_pinned(p); }
 cudaError_t d2h_copy_2d(void *dst, uint64_t dpitch, const void *src, uint64_t spitch, uint64_t width, uint64_t height, cudaStream_t stream) {
     if (!width || !height) return cudaSuccess;
     cudaError_t e;
-    if (is_pinned(dst)) {
-        e = height == 1 ? cudaMemcpyAsync(dst, src, width, cudaMemcpyDeviceToHost, stream)
-                        : cudaMemcpy2DAsync(dst, dpitch, src, spitch, width, height, cudaMemcpyDeviceToHost, stream);
-        return e == cudaSuccess ? cudaStreamSynchronize(stream) : e;
+    std::unique_lock<std::mutex> lk(g_d2h.mu, std::defer_lock);
+    cudaEvent_t *ev = nullptr;
+    if (!is_pinned(dst)) {
+        lk.lock();
+        ev = d2h_stage_ready() ? d2h_events() : nullptr;
     }
-    std::lock_guard<std::mutex> lk(g_d2h.mu);
-    cudaEvent_t *ev = d2h_stage_ready() ? d2h_events() : nullptr;
-    if (!ev) {                                  // no pinned memory to be had: the plain path
+    if (!ev) {                                  // a pinned destination, or no pinned memory to be had: the plain path
         e = height == 1 ? cudaMemcpyAsync(dst, src, width, cudaMemcpyDeviceToHost, stream)
                         : cudaMemcpy2DAsync(dst, dpitch, src, spitch, width, height, cudaMemcpyDeviceToHost, stream);
         return e == cudaSuccess ? cudaStreamSynchronize(stream) : e;
@@ -295,19 +304,54 @@ cudaError_t d2h_copy(void *dst, const void *src, uint64_t bytes, cudaStream_t st
 
 namespace { void pin_slot_release(hb::DevStatus *s); }
 
+template <typename T>
+static int dev_alloc(T **p, uint64_t n) {
+    if (*p) { free_dev(*p); *p = nullptr; }
+    if (n == 0) n = 1;
+    cudaError_t e = hb::dev_pool_alloc((void **)p, n * sizeof(T));
+    if (e != cudaSuccess) return fail(HB_ERR_MEM, std::string("cudaMalloc: ") + cudaGetErrorString(e));
+    return HB_OK;
+}
+#define TRY(expr) do { int rc_ = (expr); if (rc_ != HB_OK) return rc_; } while (0)
+
+// the capacity a buffer of n elements is made with: exact the first time, with room to grow when it had to grow before
+static uint64_t regrown(uint64_t n, bool had) { return had ? n + n / 8 + 1024 : n; }
+
+// a buffer that only grows: reallocated to exactly `need` elements when it holds fewer or is not there
+template <class T>
+static int grow(T *&p, uint64_t &cap, uint64_t need) {
+    if (cap < need || !p) {
+        TRY(dev_alloc(&p, need));
+        cap = need;
+    }
+    return HB_OK;
+}
+
+static int alloc_rows(SiteRows &r, uint64_t cap) {
+    TRY(dev_alloc(&r.start, cap)); TRY(dev_alloc(&r.stop, cap)); TRY(dev_alloc(&r.ref, cap)); TRY(dev_alloc(&r.alt, cap));
+    TRY(dev_alloc(&r.chrom_abs, cap)); TRY(dev_alloc(&r.chrom_len, cap)); TRY(dev_alloc(&r.chrom5, cap));
+    TRY(dev_alloc(&r.rowinfo, cap));
+    r.cap = cap;
+    return HB_OK;
+}
+
+static void free_rows(SiteRows &r) {
+    free_dev(r.start); free_dev(r.stop); free_dev(r.ref); free_dev(r.alt);
+    free_dev(r.chrom_len); free_dev(r.chrom_abs); free_dev(r.chrom5); free_dev(r.rowinfo);
+    r = SiteRows();
+}
+
 void hb_parse_free(hb_parse *p) {
     if (!p) return;
-    const double t_free0 = getenv("HB_TRACE") ? std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now().time_since_epoch()).count() : 0;
+    const double t_free0 = getenv("HB_TRACE") ? now_ms() : 0;
     cudaSetDevice(p->device);
     if (p->side) cudaStreamSynchronize(p->side);
     free_dev(p->d_text_owned); free_dev(p->d_nl_after); free_dev(p->d_cta); free_dev(p->d_cbase); free_dev(p->d_cp);
-    free_dev(p->d_st); free_dev(p->d_start); free_dev(p->d_stop); free_dev(p->d_ref); free_dev(p->d_alt);
-    free_dev(p->d_chrom_len); free_dev(p->d_chrom_abs); free_dev(p->d_chrom5); free_dev(p->d_rowinfo); free_dev(p->d_nu_rows);
+    free_dev(p->d_st); free_rows(p->rows); free_dev(p->d_nu_rows);
     free_dev(p->d_sites_state); free_dev(p->d_gt[0]); free_dev(p->d_gt[1]); free_dev(p->d_bits); free_dev(p->d_ploidy);
     free_dev(p->d_badgt); free_dev(p->d_run_rows);
     free_dev(p->d_wstart); free_dev(p->d_wrow); free_dev(p->d_verify); free_dev(p->d_wcount);
-    free_dev(p->walk_pad.start); free_dev(p->walk_pad.stop); free_dev(p->walk_pad.ref); free_dev(p->walk_pad.alt);
-    free_dev(p->walk_pad.chrom_abs); free_dev(p->walk_pad.chrom_len); free_dev(p->walk_pad.chrom5); free_dev(p->walk_pad.rowinfo);
+    free_rows(p->walk_pad);
     if (hb_parse::Bcf *b = p->bcf) {
         free_dev(b->d_contigs); free_dev(b->d_names); free_dev(b->d_rec_off); free_dev(b->d_blk_count); free_dev(b->d_blk_base);
         free_dev(b->seg.start); free_dev(b->seg.exit); free_dev(b->seg.bad); free_dev(b->seg.base); free_dev(b->seg.count);
@@ -318,19 +362,9 @@ void hb_parse_free(hb_parse *p) {
     if (p->side) { cudaStreamSynchronize(p->side); cudaStreamDestroy(p->side); }
     if (p->ev_runs) cudaEventDestroy(p->ev_runs);
     pin_slot_release(p->h_st_pin);
-    if (t_free0 > 0) fprintf(stderr, "[hb_parse_free] %.1f ms\n", std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now().time_since_epoch()).count() - t_free0);
+    if (t_free0 > 0) fprintf(stderr, "[hb_parse_free] %.1f ms\n", now_ms() - t_free0);
     delete p;
 }
-
-template <typename T>
-static int dev_alloc(T **p, uint64_t n) {
-    if (*p) { free_dev(*p); *p = nullptr; }
-    if (n == 0) n = 1;
-    cudaError_t e = hb::dev_pool_alloc((void **)p, n * sizeof(T));
-    if (e != cudaSuccess) return fail(HB_ERR_MEM, std::string("cudaMalloc: ") + cudaGetErrorString(e));
-    return HB_OK;
-}
-#define TRY(expr) do { int rc_ = (expr); if (rc_ != HB_OK) return rc_; } while (0)
 
 // device status -> host, through PINNED memory: a D2H copy into pageable memory is staged by the driver and was seen to
 // wait behind the 256 MiB H2D copy of the next slab that streams on another stream (hb_parse_stream_host)
@@ -367,17 +401,12 @@ void pin_slot_release(DevStatus *s) {
 }  // namespace
 
 static int fetch_status(hb_parse *p) {
-    if (!p->h_st_pin && !(p->h_st_pin = pin_slot_acquire())) {
-        // no pinned slot left: the pageable copy still works
-        cudaError_t e = cudaMemcpyAsync(&p->h_st, p->d_st, sizeof(DevStatus), cudaMemcpyDeviceToHost, p->stream);
-        if (e == cudaSuccess) e = cudaStreamSynchronize(p->stream);
-        if (e != cudaSuccess) return fail(HB_ERR_CUDA, std::string("CUDA: ") + cudaGetErrorString(e));
-        return HB_OK;
-    }
-    cudaError_t e = cudaMemcpyAsync(p->h_st_pin, p->d_st, sizeof(DevStatus), cudaMemcpyDeviceToHost, p->stream);
+    if (!p->h_st_pin) p->h_st_pin = pin_slot_acquire();
+    DevStatus *land = p->h_st_pin ? p->h_st_pin : &p->h_st;      // no pinned slot left: the pageable copy still works
+    cudaError_t e = cudaMemcpyAsync(land, p->d_st, sizeof(DevStatus), cudaMemcpyDeviceToHost, p->stream);
     if (e == cudaSuccess) e = cudaStreamSynchronize(p->stream);
-    if (e != cudaSuccess) return fail(HB_ERR_CUDA, std::string("CUDA: ") + cudaGetErrorString(e));
-    p->h_st = *p->h_st_pin;
+    if (e != cudaSuccess) return fail_cuda(e);
+    if (land != &p->h_st) p->h_st = *land;
     return HB_OK;
 }
 
@@ -441,10 +470,10 @@ static int index_by_tokenizer(hb_parse *p, const Launch &L) {
     }
     for (int attempt = 0; attempt < 2; ++attempt) {
         uint64_t need = (uint64_t)p->n_cta * p->stage_cap;
-        if (p->nl_after_cap < need) { TRY(dev_alloc(&p->d_nl_after, need)); p->nl_after_cap = need; }
+        TRY(grow(p->d_nl_after, p->nl_after_cap, need));
         if (p->with_tabs) {
-            if (p->cp_rows < need) { TRY(dev_alloc(&p->d_cp, need * p->ncp)); p->cp_rows = need; }
-            CU(cudaMemsetAsync(p->d_cp, 0xff, p->cp_rows * p->ncp * sizeof(uint64_t), p->stream));
+            TRY(grow(p->d_cp, p->cp_cap, need * p->ncp));
+            CU(cudaMemsetAsync(p->d_cp, 0xff, p->cp_cap * sizeof(uint64_t), p->stream));
         }
         CU(cudaEventRecord(p->ev[0], p->stream));
         launch_tokenize(p->with_tabs, p->d_text, p->nbytes, p->n_cta, p->tiles_per_cta, p->d_nl_after, p->stage_cap,
@@ -468,18 +497,16 @@ static int index_by_tokenizer(hb_parse *p, const Launch &L) {
     p->n_lines = n_lines;
     LineIndex li{p->d_nl_after, p->d_cbase, p->n_cta, p->stage_cap};
 
-    if (p->row_cap < n_lines || !p->d_start || !p->d_sites_state) {
-        uint64_t cap = p->d_start ? std::max(n_lines + n_lines / 8 + 1024, p->row_cap) : n_lines;
-        TRY(dev_alloc(&p->d_start, cap)); TRY(dev_alloc(&p->d_stop, cap));
-        TRY(dev_alloc(&p->d_ref, cap)); TRY(dev_alloc(&p->d_alt, cap));
-        TRY(dev_alloc(&p->d_chrom_abs, cap)); TRY(dev_alloc(&p->d_chrom_len, cap)); TRY(dev_alloc(&p->d_chrom5, cap));
-        TRY(dev_alloc(&p->d_rowinfo, cap)); TRY(dev_alloc(&p->d_nu_rows, cap));
+    SiteRows &r = p->rows;
+    // (a side buffer whose allocation failed is null: the next run allocates the rows again)
+    if (r.cap < n_lines || !r.start || !p->d_nu_rows || !p->d_sites_state) {
+        const uint64_t cap = std::max(regrown(n_lines, r.start), r.cap);
+        TRY(alloc_rows(r, cap));
+        TRY(dev_alloc(&p->d_nu_rows, cap));
         TRY(dev_alloc(&p->d_sites_state, (cap + 255) / 256 + 1));
-        p->row_cap = cap;
     }
-    launch_sites(p->d_text, li, n_lines, p->n_samples, p->rg, p->end_is_int, p->want_gt, p->with_tabs,
-                 p->d_start, p->d_stop, p->d_ref, p->d_alt, p->d_chrom_abs, p->d_chrom_len, p->d_chrom5, p->d_rowinfo,
-                 p->d_nu_rows, p->d_sites_state, p->d_st, L);
+    launch_sites(p->d_text, li, n_lines, p->n_samples, p->rg, p->end_is_int, p->want_gt, p->with_tabs, r, p->d_nu_rows,
+                 p->d_sites_state, p->d_st, L);
     CU(cudaEventRecord(p->ev[2], p->stream));
     TRY(fetch_status(p));
     CU(cudaGetLastError());
@@ -495,22 +522,14 @@ static int index_by_walker(hb_parse *p, const Launch &L) {
         if (!p->d_wstart || p->n_walkers > p->walk_cap) {
             TRY(dev_alloc(&p->d_wstart, (uint64_t)p->n_walkers + 1));
             TRY(dev_alloc(&p->d_wrow, p->n_walkers));
-            uint64_t *wc = (uint64_t *)p->d_wcount;
-            TRY(dev_alloc(&wc, p->n_walkers));
-            p->d_wcount = wc;
+            TRY(dev_alloc(&p->d_wcount, p->n_walkers));
             p->walk_cap = p->n_walkers;
         }
     }
     {   // padded rows of the walk and the list of spans to verify: sized by the walkers, known before anything runs
         const uint64_t cap = (uint64_t)p->n_walkers * kWalkSlots;
-        hb::WalkPad &w = p->walk_pad;
-        if (w.cap < cap) {
-            TRY(dev_alloc(&w.start, cap)); TRY(dev_alloc(&w.stop, cap)); TRY(dev_alloc(&w.ref, cap)); TRY(dev_alloc(&w.alt, cap));
-            TRY(dev_alloc(&w.chrom_abs, cap)); TRY(dev_alloc(&w.chrom_len, cap)); TRY(dev_alloc(&w.chrom5, cap));
-            TRY(dev_alloc(&w.rowinfo, cap));
-            w.cap = cap;
-        }
-        if (p->verify_cap < cap || !p->d_verify) { TRY(dev_alloc(&p->d_verify, cap)); p->verify_cap = cap; }
+        if (p->walk_pad.cap < cap) TRY(alloc_rows(p->walk_pad, cap));
+        TRY(grow(p->d_verify, p->verify_cap, cap));
     }
     CU(cudaEventRecord(p->ev[0], p->stream));
     launch_walk(p->d_text, p->nbytes, p->n_samples, p->walk_range, p->n_walkers, p->rg, p->end_is_int, p->d_wstart, p->d_wcount,
@@ -520,18 +539,17 @@ static int index_by_walker(hb_parse *p, const Launch &L) {
     CU(cudaGetLastError());
     const uint64_t n_lines = p->h_st.n_lines, n_rec = p->h_st.n_records;
     p->n_lines = n_lines;
-    if (p->row_cap < n_rec || !p->d_start) {
-        uint64_t cap = p->d_start ? std::max(n_rec + n_rec / 8 + 1024, p->row_cap) : n_rec;
-        TRY(dev_alloc(&p->d_start, cap)); TRY(dev_alloc(&p->d_stop, cap));
-        TRY(dev_alloc(&p->d_ref, cap)); TRY(dev_alloc(&p->d_alt, cap));
-        TRY(dev_alloc(&p->d_chrom_abs, cap)); TRY(dev_alloc(&p->d_chrom_len, cap)); TRY(dev_alloc(&p->d_chrom5, cap));
-        TRY(dev_alloc(&p->d_rowinfo, cap)); TRY(dev_alloc(&p->d_nu_rows, cap));
-        if (p->d_sites_state) { free_dev(p->d_sites_state); p->d_sites_state = nullptr; }
-        p->row_cap = cap;
+    SiteRows &r = p->rows;
+    if (r.cap < n_rec || !r.start || !p->d_nu_rows) {
+        const uint64_t cap = std::max(regrown(n_rec, r.start), r.cap);
+        TRY(alloc_rows(r, cap));
+        TRY(dev_alloc(&p->d_nu_rows, cap));
+        // the tokenizer sizes its tile state by the rows: a fallback to it on this handle makes it again
+        free_dev(p->d_sites_state);
+        p->d_sites_state = nullptr;
     }
-    launch_walk_compact(p->d_text, p->nbytes, p->n_samples, p->n_walkers, p->d_wcount, p->d_wrow, p->walk_pad, p->d_start, p->d_stop,
-                        p->d_ref, p->d_alt, p->d_chrom_abs, p->d_chrom_len, p->d_chrom5, p->d_rowinfo, p->d_nu_rows, p->d_verify,
-                        p->verify_cap, p->d_st, L);
+    launch_walk_compact(p->d_text, p->nbytes, p->n_samples, p->n_walkers, p->d_wcount, p->d_wrow, p->walk_pad, r, p->d_nu_rows,
+                        p->d_verify, p->verify_cap, p->d_st, L);
     CU(cudaEventRecord(p->ev[2], p->stream));
     p->index_used = 3;
     return HB_OK;
@@ -588,17 +606,11 @@ static int index_bcf(hb_parse *p, const Launch &L) {
     }
     const uint64_t n_all = p->h_st.bcf_records;
     p->n_lines = n_all;
-    if (b.rec_cap < n_all || !b.d_rec_off) { TRY(dev_alloc(&b.d_rec_off, n_all)); b.rec_cap = n_all; }
+    TRY(grow(b.d_rec_off, b.rec_cap, n_all));
     launch_bcf_emit(p->d_text, p->nbytes, sg, b.d_rec_off, L);
     CU(cudaEventRecord(p->ev[1], p->stream));
-    if (p->row_cap < n_all || !p->d_start) {
-        uint64_t cap = p->d_start ? std::max(n_all + n_all / 8 + 1024, p->row_cap) : n_all;
-        TRY(dev_alloc(&p->d_start, cap)); TRY(dev_alloc(&p->d_stop, cap));
-        TRY(dev_alloc(&p->d_ref, cap)); TRY(dev_alloc(&p->d_alt, cap));
-        TRY(dev_alloc(&p->d_chrom_abs, cap)); TRY(dev_alloc(&p->d_chrom_len, cap)); TRY(dev_alloc(&p->d_chrom5, cap));
-        TRY(dev_alloc(&p->d_rowinfo, cap));
-        p->row_cap = cap;
-    }
+    SiteRows &r = p->rows;
+    if (r.cap < n_all || !r.start) TRY(alloc_rows(r, std::max(regrown(n_all, r.start), r.cap)));
     const uint64_t blocks = (n_all + 255) / 256;
     if (b.blk_cap < blocks || !b.d_blk_count) {
         TRY(dev_alloc(&b.d_blk_count, blocks)); TRY(dev_alloc(&b.d_blk_base, blocks));
@@ -614,8 +626,8 @@ static int index_bcf(hb_parse *p, const Launch &L) {
         for (uint32_t i = 0; i < nc; ++i) if (b.contigs[i] == want) { a.rid = (int)i; break; }
     }
     a.beg0 = p->rg.beg0; a.end0 = p->rg.end0; a.want_gt = p->want_gt;
-    a.start = p->d_start; a.stop = p->d_stop; a.ref = p->d_ref; a.alt = p->d_alt; a.chrom_len = p->d_chrom_len;
-    a.chrom_abs = p->d_chrom_abs; a.chrom5 = p->d_chrom5; a.rowinfo = p->d_rowinfo;
+    a.start = r.start; a.stop = r.stop; a.ref = r.ref; a.alt = r.alt; a.chrom_len = r.chrom_len;
+    a.chrom_abs = r.chrom_abs; a.chrom5 = r.chrom5; a.rowinfo = r.rowinfo;
     a.blk_count = b.d_blk_count; a.blk_base = b.d_blk_base; a.st = p->d_st;
     launch_bcf_sites(a, L);
     CU(cudaEventRecord(p->ev[2], p->stream));
@@ -640,19 +652,27 @@ static int ensure_runs(hb_parse *p) {
         std::sort(p->run_rows.begin(), p->run_rows.end());
         for (uint64_t r : p->run_rows) {
             uint64_t abs; uint8_t len; char name[256];
-            CU(cudaMemcpy(&abs, p->d_chrom_abs + r, 8, cudaMemcpyDeviceToHost));
+            CU(cudaMemcpy(&abs, p->rows.chrom_abs + r, 8, cudaMemcpyDeviceToHost));
             if (p->bcf) {                        // BCF rows point into the contig names: the name from the dictionary
                 const auto &off = p->bcf->name_off;
                 const size_t i = (size_t)(std::lower_bound(off.begin(), off.end(), abs) - off.begin());
                 p->run_names.push_back(i < off.size() ? p->bcf->contigs[i] : std::string());
                 continue;
             }
-            CU(cudaMemcpy(&len, p->d_chrom_len + r, 1, cudaMemcpyDeviceToHost));
+            CU(cudaMemcpy(&len, p->rows.chrom_len + r, 1, cudaMemcpyDeviceToHost));
             CU(cudaMemcpy(name, p->d_text + abs, len, cudaMemcpyDeviceToHost));
             p->run_names.emplace_back(name, name + len);
         }
     }
     p->runs_valid = true;
+    return HB_OK;
+}
+
+// kernel 2b: the column checkpoints of the n_nu kept records that need the general decode path
+static int index_nonuniform(hb_parse *p, uint64_t n_nu, const Launch &L) {
+    TRY(grow(p->d_cp, p->cp_cap, n_nu * p->ncp));
+    CU(cudaMemsetAsync(p->d_cp, 0xff, p->cp_cap * sizeof(uint64_t), p->stream));
+    launch_index_columns(p->d_text, p->rows.rowinfo, p->d_nu_rows, n_nu, p->d_cp, p->ncp, L);
     return HB_OK;
 }
 
@@ -701,22 +721,17 @@ static int run_parse(hb_parse *p) {
         CU(cudaStreamWaitEvent(p->side, p->ev_runs, 0));
         Launch Ls = L;
         Ls.stream = p->side;
-        launch_chrom_runs(p->bcf ? p->bcf->d_names : p->d_text, p->d_chrom_abs, p->d_chrom_len, n_rec, p->d_run_rows, hb_parse::kMaxRuns, p->d_st, Ls);
+        launch_chrom_runs(p->bcf ? p->bcf->d_names : p->d_text, p->rows.chrom_abs, p->rows.chrom_len, n_rec, p->d_run_rows, hb_parse::kMaxRuns, p->d_st, Ls);
         CU(cudaEventRecord(p->ev_runs, p->side));
     }
 
     // ---- GT decode
     if (p->want_gt && n_rec && p->n_samples) {
-        if (p->index_used == 1 && p->h_st.n_nonuniform) {
-            uint64_t n_nu = p->h_st.n_nonuniform;
-            if (p->cp_rows < n_nu) { TRY(dev_alloc(&p->d_cp, n_nu * p->ncp)); p->cp_rows = n_nu; }
-            CU(cudaMemsetAsync(p->d_cp, 0xff, p->cp_rows * p->ncp * sizeof(uint64_t), p->stream));
-            launch_index_columns(p->d_text, p->d_rowinfo, p->d_nu_rows, n_nu, p->d_cp, p->ncp, L);
-        }
+        if (p->index_used == 1 && p->h_st.n_nonuniform) TRY(index_nonuniform(p, p->h_st.n_nonuniform, L));
         // the planes are re-used (with their stride) whenever the rows fit: a handle that is re-run on slabs of
         // slightly different length must not re-allocate -- cudaFree synchronises the whole device
         if (!p->d_gt[0] || n_rec > p->gt_stride) {
-            const uint64_t want = p->d_gt[0] ? n_rec + n_rec / 8 + 1024 : n_rec;
+            const uint64_t want = regrown(n_rec, p->d_gt[0]);
             const uint64_t stride = (want + 127) / 128 * 128;         // whole 128-row groups of the bit planes
             const uint64_t bytes = stride * p->n_samples;
             TRY(dev_alloc(&p->d_gt[0], bytes)); TRY(dev_alloc(&p->d_gt[1], bytes));
@@ -726,18 +741,13 @@ static int run_parse(hb_parse *p) {
             // rows between the last decode tile and the end of its group are never written: they read as "no allele"
             CU(cudaMemsetAsync(p->d_bits, 0, p->bits_stride * p->n_samples * 4, p->stream));
         }
-        if (p->index_used == 3 && p->h_st.n_nu_count) {
-            // walker: the count pass told the host how many kept records are not plain "\tX|Y" columns
-            uint64_t n_nu = p->h_st.n_nu_count;
-            if (p->cp_rows < n_nu) { TRY(dev_alloc(&p->d_cp, n_nu * p->ncp)); p->cp_rows = n_nu; }
-            CU(cudaMemsetAsync(p->d_cp, 0xff, p->cp_rows * p->ncp * sizeof(uint64_t), p->stream));
-            launch_index_columns(p->d_text, p->d_rowinfo, p->d_nu_rows, n_nu, p->d_cp, p->ncp, L);
-        }
+        // walker: the count pass told the host how many kept records are not plain "\tX|Y" columns
+        if (p->index_used == 3 && p->h_st.n_nu_count) TRY(index_nonuniform(p, p->h_st.n_nu_count, L));
         if (p->bcf)
-            launch_bcf_decode(p->d_text, p->d_rowinfo, n_rec, p->n_samples, p->d_gt[0], p->d_gt[1], p->gt_stride, p->d_bits,
+            launch_bcf_decode(p->d_text, p->rows.rowinfo, n_rec, p->n_samples, p->d_gt[0], p->d_gt[1], p->gt_stride, p->d_bits,
                               p->bits_stride, p->d_ploidy, p->d_badgt, p->d_st, L);
         else
-            launch_decode_gt(p->d_text, p->d_rowinfo, n_rec, p->n_samples, p->d_cp, p->ncp, p->d_gt[0], p->d_gt[1],
+            launch_decode_gt(p->d_text, p->rows.rowinfo, n_rec, p->n_samples, p->d_cp, p->ncp, p->d_gt[0], p->d_gt[1],
                              p->gt_stride, p->d_bits, p->bits_stride, p->d_ploidy, p->d_badgt, p->d_st, L);
     }
     CU(cudaEventRecord(p->ev[3], p->stream));
@@ -769,10 +779,14 @@ static int run_parse(hb_parse *p) {
     return HB_OK;
 }
 
-static int new_parse(const hb_parse_opts *o, hb_parse **out) {
-    if (!o || !out) return fail(HB_ERR_ARG, "null argument");
-    TRY(ensure_device(o->device));
-    hb_parse *p = new hb_parse();
+// a handle under construction: every early return frees it and what it holds, until the caller releases it
+using ParsePtr = std::unique_ptr<hb_parse, void (*)(hb_parse *)>;
+
+static ParsePtr new_parse(const hb_parse_opts *o, int &rc) {
+    ParsePtr p(nullptr, hb_parse_free);
+    rc = o ? ensure_device(o->device) : fail(HB_ERR_ARG, "null argument");
+    if (rc != HB_OK) return p;
+    p.reset(new hb_parse());
     p->device = o->device;
     p->stream = (cudaStream_t)o->stream;
     cudaDeviceGetAttribute(&p->sm_count, cudaDevAttrMultiProcessorCount, o->device);
@@ -782,38 +796,44 @@ static int new_parse(const hb_parse_opts *o, hb_parse **out) {
     p->want_gt = o->want_gt;
     p->tokenizer = o->tokenizer;
     for (auto &e : p->ev) cudaEventCreate(&e);
-    *out = p;
+    return p;
+}
+
+// zero bytes behind the text of every parse: kernels that read it in whole 16-byte words find zeros past its end
+constexpr uint64_t kTextPad = 256;
+
+// n bytes of host text (+ '\n' when add_newline) become the parse's own device text
+static int upload_text(hb_parse *p, const uint8_t *text, uint64_t n, bool add_newline) {
+    const uint64_t total = n + (add_newline ? 1 : 0);
+    TRY(dev_alloc(&p->d_text_owned, total + kTextPad));
+    cudaError_t e = cudaMemcpyAsync(p->d_text_owned, text, n, cudaMemcpyHostToDevice, p->stream);
+    if (e == cudaSuccess && add_newline) e = cudaMemsetAsync(p->d_text_owned + n, '\n', 1, p->stream);
+    if (e == cudaSuccess) e = cudaMemsetAsync(p->d_text_owned + total, 0, kTextPad, p->stream);
+    if (e != cudaSuccess) return fail_cuda(e);
+    p->d_text = p->d_text_owned;
+    p->nbytes = total;
     return HB_OK;
 }
 
 int hb_parse_device_text(const uint8_t *d_text, uint64_t nbytes, const hb_parse_opts *opts, hb_parse **out) {
-    hb_parse *p = nullptr;
-    TRY(new_parse(opts, &p));
-    if (((uintptr_t)d_text & 15) != 0) { hb_parse_free(p); return fail(HB_ERR_ARG, "d_text must be 16-byte aligned"); }
+    int rc;
+    ParsePtr p = new_parse(opts, rc);
+    if (!p) return rc;
+    if (((uintptr_t)d_text & 15) != 0) return fail(HB_ERR_ARG, "d_text must be 16-byte aligned");
     p->d_text = d_text;
     p->nbytes = nbytes;
-    int rc = run_parse(p);
-    if (rc != HB_OK) { hb_parse_free(p); return rc; }
-    *out = p;
+    TRY(run_parse(p.get()));
+    *out = p.release();
     return HB_OK;
 }
 
 int hb_parse_host_text(const uint8_t *text, uint64_t nbytes, const hb_parse_opts *opts, hb_parse **out) {
-    hb_parse *p = nullptr;
-    TRY(new_parse(opts, &p));
-    bool add_nl = nbytes && text[nbytes - 1] != '\n';
-    uint64_t total = nbytes + (add_nl ? 1 : 0);
-    int rc = dev_alloc(&p->d_text_owned, total + 256);
-    if (rc != HB_OK) { hb_parse_free(p); return rc; }
-    cudaError_t e = cudaMemcpyAsync(p->d_text_owned, text, nbytes, cudaMemcpyHostToDevice, p->stream);
-    if (e == cudaSuccess && add_nl) e = cudaMemsetAsync(p->d_text_owned + nbytes, '\n', 1, p->stream);
-    if (e == cudaSuccess) e = cudaMemsetAsync(p->d_text_owned + total, 0, 256, p->stream);
-    if (e != cudaSuccess) { hb_parse_free(p); return fail(HB_ERR_CUDA, cudaGetErrorString(e)); }
-    p->d_text = p->d_text_owned;
-    p->nbytes = total;
-    rc = run_parse(p);
-    if (rc != HB_OK) { hb_parse_free(p); return rc; }
-    *out = p;
+    int rc;
+    ParsePtr p = new_parse(opts, rc);
+    if (!p) return rc;
+    TRY(upload_text(p.get(), text, nbytes, nbytes && text[nbytes - 1] != '\n'));
+    TRY(run_parse(p.get()));
+    *out = p.release();
     return HB_OK;
 }
 
@@ -916,7 +936,7 @@ int open_slots(SlotCache &c, const hb_parse_opts &opts, size_t n_slots, uint64_t
             cudaEventCreateWithFlags(&s.fetched, cudaEventDisableTiming) != cudaSuccess) { rc = fail(HB_ERR_CUDA, "cannot create streams"); break; }
         hb_parse_opts o = opts;
         o.stream = s.compute;
-        rc = new_parse(&o, &s.p);
+        s.p = new_parse(&o, rc).release();
         if (rc == HB_OK) ss->n_slots = i + 1;
     }
     const bool grow = ss->text_cap < text_cap || ss->carry_cap < carry_cap || ss->comp_cap < comp_cap || ss->n_cap < n_cap;
@@ -947,7 +967,7 @@ int open_slots(SlotCache &c, const hb_parse_opts &opts, size_t n_slots, uint64_t
 // go back to cache c, kept for the next call when all went well
 int close_slots(SlotCache &c, StreamSlots *ss, int rc, cudaError_t e) {
     for (size_t i = 0; i < ss->n_slots && rc == HB_OK && e == cudaSuccess; ++i) e = cudaStreamSynchronize(ss->slot[i].d2h);
-    if (e != cudaSuccess && rc == HB_OK) rc = fail(HB_ERR_CUDA, std::string("CUDA: ") + cudaGetErrorString(e));
+    if (e != cudaSuccess && rc == HB_OK) rc = fail_cuda(e);
     release_slots(c, ss, rc == HB_OK);
     return rc;
 }
@@ -984,16 +1004,18 @@ struct SlabSink {
 // rows into the caller's host arrays: planes [n_samples][out_stride], columns of out_stride records; any of them may be NULL
 struct HostSink : SlabSink {
     int8_t *gt0, *gt1; uint64_t out_stride; uint32_t *start, *stop; char *ref, *alt;
+    HostSink(int8_t *gt0, int8_t *gt1, uint64_t out_stride, uint32_t *start, uint32_t *stop, char *ref, char *alt, uint32_t *pl, uint32_t *bg)
+        : gt0(gt0), gt1(gt1), out_stride(out_stride), start(start), stop(stop), ref(ref), alt(alt) { ploidy_err = pl; badgt_err = bg; }
     int deliver(StreamSlot &s, uint64_t R, uint64_t n, uint64_t, cudaError_t &e) override {
         if (R + n > out_stride && (gt0 || gt1 || start || stop || ref || alt)) return fail(HB_ERR_ARG, "more records than the output arrays hold");
         if (opts.want_gt && opts.n_samples && s.p->d_gt[0]) {
             if (gt0) e = cudaMemcpy2DAsync(gt0 + R, out_stride, s.p->d_gt[0], s.p->gt_stride, n, opts.n_samples, cudaMemcpyDeviceToHost, s.d2h);
             if (gt1 && e == cudaSuccess) e = cudaMemcpy2DAsync(gt1 + R, out_stride, s.p->d_gt[1], s.p->gt_stride, n, opts.n_samples, cudaMemcpyDeviceToHost, s.d2h);
         }
-        if (start && e == cudaSuccess) e = cudaMemcpyAsync(start + R, s.p->d_start, n * 4, cudaMemcpyDeviceToHost, s.d2h);
-        if (stop && e == cudaSuccess) e = cudaMemcpyAsync(stop + R, s.p->d_stop, n * 4, cudaMemcpyDeviceToHost, s.d2h);
-        if (ref && e == cudaSuccess) e = cudaMemcpyAsync(ref + R, s.p->d_ref, n, cudaMemcpyDeviceToHost, s.d2h);
-        if (alt && e == cudaSuccess) e = cudaMemcpyAsync(alt + R, s.p->d_alt, n, cudaMemcpyDeviceToHost, s.d2h);
+        if (start && e == cudaSuccess) e = cudaMemcpyAsync(start + R, s.p->rows.start, n * 4, cudaMemcpyDeviceToHost, s.d2h);
+        if (stop && e == cudaSuccess) e = cudaMemcpyAsync(stop + R, s.p->rows.stop, n * 4, cudaMemcpyDeviceToHost, s.d2h);
+        if (ref && e == cudaSuccess) e = cudaMemcpyAsync(ref + R, s.p->rows.ref, n, cudaMemcpyDeviceToHost, s.d2h);
+        if (alt && e == cudaSuccess) e = cudaMemcpyAsync(alt + R, s.p->rows.alt, n, cudaMemcpyDeviceToHost, s.d2h);
         return HB_OK;
     }
 };
@@ -1018,8 +1040,6 @@ int parse_slab(StreamSlot &s, uint64_t begin, uint64_t nbytes, SlabSink &sink, u
     R += n;
     return HB_OK;
 }
-
-double now_ms() { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now().time_since_epoch()).count(); }
 }  // namespace
 
 int hb_parse_stream_host(const uint8_t *text, uint64_t nbytes, const hb_parse_opts *opts, uint64_t slab_bytes,
@@ -1029,9 +1049,7 @@ int hb_parse_stream_host(const uint8_t *text, uint64_t nbytes, const hb_parse_op
     if (nbytes >= 4 && memcmp(text, "BCF\2", 4) == 0) return fail(HB_ERR_ARG, kBcfNoStream);
     *n_records = 0;
     if (n_slabs) *n_slabs = 0;
-    HostSink sink;
-    sink.gt0 = gt0; sink.gt1 = gt1; sink.out_stride = out_stride; sink.start = start; sink.stop = stop; sink.ref = ref; sink.alt = alt;
-    sink.ploidy_err = ploidy_err; sink.badgt_err = badgt_err;
+    HostSink sink(gt0, gt1, out_stride, start, stop, ref, alt, ploidy_err, badgt_err);
     TRY(sink.begin(*opts, {}, nbytes));
     if (nbytes == 0) return HB_OK;
     if (text[nbytes - 1] != '\n') return fail(HB_ERR_ARG, "the text must end with a newline");
@@ -1091,11 +1109,7 @@ int hb_parse_release_text(hb_parse *p) {
     if (p->d_text_owned) {
         TRY(ensure_runs(p));                     // the CHROM names are read from the text
         CU(cudaSetDevice(p->device));
-        {   // the caller wants the HBM back: not into the idle pool
-            std::lock_guard<std::mutex> lk(g_pool.mu);
-            g_pool.live.erase(p->d_text_owned);
-        }
-        cudaFree(p->d_text_owned);
+        dev_pool_release(p->d_text_owned);       // the caller wants the HBM back: not into the idle pool
         p->d_text_owned = nullptr;
         p->d_text = nullptr;
         p->nbytes = 0;
@@ -1127,7 +1141,7 @@ int hb_parse_get_info(const hb_parse *p, hb_parse_info *info) {
     info->gt_stride = p->gt_stride;
     info->d_gt[0] = p->d_gt[0];
     info->d_gt[1] = p->d_gt[1];
-    info->d_start = p->d_start; info->d_stop = p->d_stop; info->d_ref = p->d_ref; info->d_alt = p->d_alt;
+    info->d_start = p->rows.start; info->d_stop = p->rows.stop; info->d_ref = p->rows.ref; info->d_alt = p->rows.alt;
     info->n_nonuniform = p->h_st.n_nonuniform;
     info->n_bad_gt = p->h_st.n_bad_gt;
     info->n_bad_cols = p->h_st.n_bad_cols;
@@ -1144,10 +1158,10 @@ int hb_parse_fetch_sites(hb_parse *p, uint32_t *start, uint32_t *stop, char *ref
     CU(cudaSetDevice(p->device));
     uint64_t n = p->h_st.n_records;
     if (!n) return HB_OK;
-    if (start) CU(d2h_copy(start, p->d_start, n * 4, p->stream));
-    if (stop) CU(d2h_copy(stop, p->d_stop, n * 4, p->stream));
-    if (ref) CU(d2h_copy(ref, p->d_ref, n, p->stream));
-    if (alt) CU(d2h_copy(alt, p->d_alt, n, p->stream));
+    if (start) CU(d2h_copy(start, p->rows.start, n * 4, p->stream));
+    if (stop) CU(d2h_copy(stop, p->rows.stop, n * 4, p->stream));
+    if (ref) CU(d2h_copy(ref, p->rows.ref, n, p->stream));
+    if (alt) CU(d2h_copy(alt, p->rows.alt, n, p->stream));
     return HB_OK;
 }
 
@@ -1415,33 +1429,43 @@ int parse_file_common(const char *path, const char *region, bool want_gt, int de
     return parse_bytes_common(raw, raw.data(), raw.size(), region, want_gt, device, out, samples);
 }
 
+// a BGZF file: its member table, then its header
+struct BgzfFile {
+    std::vector<uint64_t> coff, ooff;
+    std::vector<uint32_t> clen, olen;
+    uint64_t total = 0;          // bytes of text
+    FileText ft;
+};
+
+// false: the bytes are not BGZF (each caller has its own answer to that)
+bool index_bgzf(const uint8_t *raw, uint64_t n, BgzfFile &f) { return bgzf_index(raw, n, f.coff, f.clen, f.ooff, f.olen, f.total); }
+
 // the VCF header of a BGZF file: leading members are inflated on the host (zlib) until the #CHROM line is complete; with
 // hb_set_bgzf_crc_check on, each is checked against its CRC32 as kernel 0 checks the others
-static int bgzf_header(const uint8_t *raw, const std::vector<uint64_t> &coff, const std::vector<uint32_t> &clen,
-                       const std::vector<uint32_t> &olen, FileText &ft) {
+int bgzf_header(const uint8_t *raw, BgzfFile &f) {
     std::vector<uint8_t> head;
     bool have = false;
     const bool check_crc = bgzf_crc_check();
-    for (size_t i = 0; i < coff.size() && !have; ++i) {
+    for (size_t i = 0; i < f.coff.size() && !have; ++i) {
         const size_t at = head.size();
-        head.resize(at + olen[i]);
+        head.resize(at + f.olen[i]);
         z_stream zs;
         memset(&zs, 0, sizeof zs);
         if (inflateInit2(&zs, -15) != Z_OK) return fail(HB_ERR_IO, "inflateInit2 failed");
-        zs.next_in = const_cast<Bytef *>(raw + coff[i]);
-        zs.avail_in = clen[i];
+        zs.next_in = const_cast<Bytef *>(raw + f.coff[i]);
+        zs.avail_in = f.clen[i];
         zs.next_out = head.data() + at;
-        zs.avail_out = olen[i];
+        zs.avail_out = f.olen[i];
         const int zr = inflate(&zs, Z_FINISH);
         inflateEnd(&zs);
         if (zr != Z_STREAM_END || zs.avail_out != 0) return fail(HB_ERR_IO, "BGZF inflate failed (header)");
         if (check_crc) {
-            const uint8_t *tr = raw + coff[i] + clen[i];
+            const uint8_t *tr = raw + f.coff[i] + f.clen[i];
             const uint32_t want = tr[0] | tr[1] << 8 | tr[2] << 16 | (uint32_t)tr[3] << 24;
-            if ((uint32_t)crc32(crc32(0L, Z_NULL, 0), head.data() + at, olen[i]) != want) return fail(HB_ERR_IO, bgzf_crc_message(raw, coff[i]));
+            if ((uint32_t)crc32(crc32(0L, Z_NULL, 0), head.data() + at, f.olen[i]) != want) return fail(HB_ERR_IO, bgzf_crc_message(raw, f.coff[i]));
         }
-        if (is_bcf(head.data(), head.size())) TRY(bcf_header(head.data(), head.size(), ft, have));
-        else have = parse_header(head.data(), head.size(), i + 1 == coff.size(), ft);
+        if (is_bcf(head.data(), head.size())) TRY(bcf_header(head.data(), head.size(), f.ft, have));
+        else have = parse_header(head.data(), head.size(), i + 1 == f.coff.size(), f.ft);
     }
     if (!have && is_bcf(head.data(), head.size())) return fail(HB_ERR_FORMAT, "BCF header is truncated");
     if (!have) return fail(HB_ERR_HEADER, "no #CHROM header line");
@@ -1494,54 +1518,47 @@ int parse_bcf_host(const FileText &ft, const hb_parse_opts &o, hb_parse **out) {
     uint64_t slab;
     TRY(ensure_device(o.device));
     if (n > text_limit(slab)) return bcf_too_big(n);
-    hb_parse *p = nullptr;
-    TRY(new_parse(&o, &p));
-    int rc = dev_alloc(&p->d_text_owned, n + 256);
-    cudaError_t e = cudaSuccess;
-    if (rc == HB_OK) e = cudaMemcpyAsync(p->d_text_owned, ft.data.data() + ft.body, n, cudaMemcpyHostToDevice, p->stream);
-    if (rc == HB_OK && e == cudaSuccess) e = cudaMemsetAsync(p->d_text_owned + n, 0, 256, p->stream);
-    if (rc == HB_OK && e != cudaSuccess) rc = fail(HB_ERR_CUDA, std::string("CUDA: ") + cudaGetErrorString(e));
-    if (rc == HB_OK) {
-        p->d_text = p->d_text_owned;
-        p->nbytes = n;
-        rc = bcf_attach(p, ft);
-    }
-    if (rc == HB_OK) rc = run_parse(p);
-    if (rc != HB_OK) { hb_parse_free(p); return rc; }
-    *out = p;
+    int rc;
+    ParsePtr p = new_parse(&o, rc);
+    if (!p) return rc;
+    TRY(upload_text(p.get(), ft.data.data() + ft.body, n, false));
+    TRY(bcf_attach(p.get(), ft));
+    TRY(run_parse(p.get()));
+    *out = p.release();
     return HB_OK;
+}
+
+hb_parse_opts opts_for(const FileText &ft, const char *region, bool want_gt, int device) {
+    hb_parse_opts o;
+    memset(&o, 0, sizeof o);
+    o.region = region;
+    o.want_gt = want_gt ? 1 : 0;
+    o.device = device;
+    o.n_samples = (uint32_t)ft.samples.size();
+    o.end_is_int = ft.end_is_int;
+    return o;
 }
 
 // raw_p[0..raw_n): the bytes of a .vcf / .vcf.gz / .bcf; raw_owned: the vector that holds them when the caller read a file
 // (released early on the zlib path), empty when they belong to the caller
 int parse_bytes_common(std::vector<uint8_t> &raw_owned, const uint8_t *raw_p, uint64_t raw_n, const char *region, bool want_gt,
                        int device, hb_parse **out, std::vector<std::string> &samples) {
-    struct View { const uint8_t *p; uint64_t n; const uint8_t *data() const { return p; } uint64_t size() const { return n; }
-                  uint8_t operator[](uint64_t i) const { return p[i]; } } raw{raw_p, raw_n};
-    std::vector<uint64_t> coff, ooff;
-    std::vector<uint32_t> clen, olen;
-    uint64_t total = 0;
-    const bool gpu_inflate = raw.size() >= 28 && raw[0] == 0x1f && raw[1] == 0x8b &&
-                             bgzf_index(raw.data(), raw.size(), coff, clen, ooff, olen, total) && total > 0;
-    hb_parse_opts o;
-    memset(&o, 0, sizeof o);
-    o.region = region;
-    o.want_gt = want_gt ? 1 : 0;
-    o.device = device;
+    BgzfFile bz;
+    const bool gpu_inflate = raw_n >= 28 && raw_p[0] == 0x1f && raw_p[1] == 0x8b && index_bgzf(raw_p, raw_n, bz) && bz.total > 0;
     if (!gpu_inflate) {
         FileText ft;
         if (raw_owned.empty()) raw_owned.assign(raw_p, raw_p + raw_n);
         TRY(read_vcf(raw_owned, ft));
         raw_owned.clear(); raw_owned.shrink_to_fit();
         samples = ft.samples;
-        o.n_samples = (uint32_t)ft.samples.size();
-        o.end_is_int = ft.end_is_int;
+        const hb_parse_opts o = opts_for(ft, region, want_gt, device);
         if (ft.bcf) return parse_bcf_host(ft, o, out);
         return hb_parse_host_text(ft.data.data() + ft.body, ft.data.size() - ft.body, &o, out);
     }
     // ---- header: inflate leading members on the host until the #CHROM line is complete
-    FileText ft;
-    TRY(bgzf_header(raw.data(), coff, clen, olen, ft));
+    TRY(bgzf_header(raw_p, bz));
+    const FileText &ft = bz.ft;
+    const uint64_t total = bz.total;
     samples = ft.samples;
     {   // a file whose text does not fit HBM next to its genotype planes passes through in slabs instead: same rows, same
         // handle minus the text (hb_parse_stream_bgzf_resident)
@@ -1551,35 +1568,31 @@ int parse_bytes_common(std::vector<uint8_t> &raw_owned, const uint8_t *raw_p, ui
         if (total > limit && ft.bcf) return bcf_too_big(total - ft.body);
         if (total > limit) return hb_parse_stream_bgzf_resident(raw_p, raw_n, region, want_gt ? 1 : 0, device, slab, out, nullptr);
     }
-    o.n_samples = (uint32_t)ft.samples.size();
-    o.end_is_int = ft.end_is_int;
-    hb_parse *p = nullptr;
+    const hb_parse_opts o = opts_for(ft, region, want_gt, device);
     const bool trace = getenv("HB_TRACE") != nullptr;
-    auto now = []() { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now().time_since_epoch()).count(); };
-    const double t0 = now();
-    TRY(new_parse(&o, &p));
+    const double t0 = now_ms();
+    int rc;
+    ParsePtr p = new_parse(&o, rc);
+    if (!p) return rc;
     const uint64_t pad = (16 - ft.body % 16) % 16;         // the records must start on a 16-byte boundary
-    int rc = dev_alloc(&p->d_text_owned, pad + total + 1 + 256);
-    const double t1 = now();
-    if (rc == HB_OK) rc = inflate_bgzf_to_device(raw.data(), raw.size(), coff, clen, ooff, olen, p->d_text_owned + pad, p->stream, &p->ms_inflate);
+    TRY(dev_alloc(&p->d_text_owned, pad + total + 1 + kTextPad));
+    const double t1 = now_ms();
+    TRY(inflate_bgzf_to_device(raw_p, raw_n, bz.coff, bz.clen, bz.ooff, bz.olen, p->d_text_owned + pad, p->stream, &p->ms_inflate));
     uint8_t last = 0;
-    cudaError_t e = cudaSuccess;
-    if (rc == HB_OK) e = cudaMemcpy(&last, p->d_text_owned + pad + total - 1, 1, cudaMemcpyDeviceToHost);
+    cudaError_t e = cudaMemcpy(&last, p->d_text_owned + pad + total - 1, 1, cudaMemcpyDeviceToHost);
     uint64_t end = pad + total;
-    if (rc == HB_OK && e == cudaSuccess && last != '\n' && !ft.bcf) { e = cudaMemset(p->d_text_owned + end, '\n', 1); ++end; }
-    if (rc == HB_OK && e == cudaSuccess) e = cudaMemset(p->d_text_owned + end, 0, 256);
-    if (rc == HB_OK && e != cudaSuccess) rc = fail(HB_ERR_CUDA, std::string("CUDA: ") + cudaGetErrorString(e));
-    if (rc == HB_OK) {
-        p->d_text = p->d_text_owned + pad + ft.body;
-        p->nbytes = end - pad - ft.body;
-        p->compressed_bytes = raw.size();
-        const double t2 = now();
-        if (ft.bcf) rc = bcf_attach(p, ft);
-        if (rc == HB_OK) rc = run_parse(p);
-        if (trace) fprintf(stderr, "[parse_bytes_common] text buffer %.1f ms, H2D + inflate %.1f ms, parse %.1f ms\n", t1 - t0, t2 - t1, now() - t2);
-    }
-    if (rc != HB_OK) { hb_parse_free(p); return rc; }
-    *out = p;
+    if (e == cudaSuccess && last != '\n' && !ft.bcf) { e = cudaMemset(p->d_text_owned + end, '\n', 1); ++end; }
+    if (e == cudaSuccess) e = cudaMemset(p->d_text_owned + end, 0, kTextPad);
+    if (e != cudaSuccess) return fail_cuda(e);
+    p->d_text = p->d_text_owned + pad + ft.body;
+    p->nbytes = end - pad - ft.body;
+    p->compressed_bytes = raw_n;
+    const double t2 = now_ms();
+    rc = ft.bcf ? bcf_attach(p.get(), ft) : HB_OK;
+    if (rc == HB_OK) rc = run_parse(p.get());
+    if (trace) fprintf(stderr, "[parse_bytes_common] text buffer %.1f ms, H2D + inflate %.1f ms, parse %.1f ms\n", t1 - t0, t2 - t1, now_ms() - t2);
+    TRY(rc);
+    *out = p.release();
     return HB_OK;
 }
 
@@ -1833,16 +1846,13 @@ int hb_parse_file(const char *in_vcf, const char *region, int want_gt, int devic
 // header of the BGZF bytes of a .vcf.gz: sample count, decompressed size, offset of the first record in it
 int hb_bgzf_vcf_info(const uint8_t *bgzf, uint64_t nbytes, uint32_t *n_samples, uint64_t *text_bytes, uint64_t *body_offset) {
     if (!bgzf) return fail(HB_ERR_ARG, "null argument");
-    std::vector<uint64_t> coff, ooff;
-    std::vector<uint32_t> clen, olen;
-    uint64_t total = 0;
-    if (!bgzf_index(bgzf, nbytes, coff, clen, ooff, olen, total)) return fail(HB_ERR_IO, "not a BGZF file");
-    FileText ft;
-    TRY(bgzf_header(bgzf, coff, clen, olen, ft));
-    if (ft.bcf) return fail(HB_ERR_ARG, kBcfNoStream);
-    if (n_samples) *n_samples = (uint32_t)ft.samples.size();
-    if (text_bytes) *text_bytes = total;
-    if (body_offset) *body_offset = ft.body;
+    BgzfFile bz;
+    if (!index_bgzf(bgzf, nbytes, bz)) return fail(HB_ERR_IO, "not a BGZF file");
+    TRY(bgzf_header(bgzf, bz));
+    if (bz.ft.bcf) return fail(HB_ERR_ARG, kBcfNoStream);
+    if (n_samples) *n_samples = (uint32_t)bz.ft.samples.size();
+    if (text_bytes) *text_bytes = bz.total;
+    if (body_offset) *body_offset = bz.ft.body;
     return HB_OK;
 }
 
@@ -1856,24 +1866,18 @@ static int stream_bgzf(const char *entry, const uint8_t *bgzf, uint64_t nbytes, 
     if (n_slabs) *n_slabs = 0;
     const double t_begin = now_ms();
     double t_wait = 0, t_parse = 0, t_enq = 0;
-    std::vector<uint64_t> coff, ooff;
-    std::vector<uint32_t> clen, olen;
-    uint64_t total = 0;
-    if (!bgzf_index(bgzf, nbytes, coff, clen, ooff, olen, total)) return fail(HB_ERR_IO, "not a BGZF file");
-    FileText ft;
-    TRY(bgzf_header(bgzf, coff, clen, olen, ft));
+    BgzfFile bz;
+    if (!index_bgzf(bgzf, nbytes, bz)) return fail(HB_ERR_IO, "not a BGZF file");
+    TRY(bgzf_header(bgzf, bz));
+    const std::vector<uint64_t> &coff = bz.coff, &ooff = bz.ooff;
+    const std::vector<uint32_t> &clen = bz.clen, &olen = bz.olen;
+    const FileText &ft = bz.ft;
     if (ft.bcf) return fail(HB_ERR_ARG, kBcfNoStream);
     const double t_index = now_ms() - t_begin;
-    hb_parse_opts opts;
-    memset(&opts, 0, sizeof opts);
-    opts.region = region;
-    opts.want_gt = want_gt ? 1 : 0;
-    opts.device = device;
-    opts.n_samples = (uint32_t)ft.samples.size();
-    opts.end_is_int = ft.end_is_int;
+    const hb_parse_opts opts = opts_for(ft, region, want_gt != 0, device);
     TRY(ensure_device(device));
-    TRY(sink.begin(opts, ft.samples, total));
-    if (total <= ft.body) return HB_OK;
+    TRY(sink.begin(opts, ft.samples, bz.total));
+    if (bz.total <= ft.body) return HB_OK;
     if (slab_bytes == 0) slab_bytes = 1ull << 30;
     // slabs of whole members, about slab_bytes of text each
     struct Slab { size_t m0, m1; uint64_t text; uint64_t comp0, comp; };
@@ -1922,7 +1926,7 @@ static int stream_bgzf(const char *entry, const uint8_t *bgzf, uint64_t nbytes, 
         launch_last_newline(s.buf, s.x + skip, s.end, s.sc.d_last_nl, s.compute);
         cudaError_t ee = cudaMemcpyAsync(s.h_pin, s.sc.d_last_nl, 8, cudaMemcpyDeviceToHost, s.compute);
         if (ee == cudaSuccess) ee = cudaMemcpyAsync(s.h_pin + 1, s.sc.d_status, 4ull * n, cudaMemcpyDeviceToHost, s.compute);
-        if (ee != cudaSuccess) return fail(HB_ERR_CUDA, std::string("CUDA: ") + cudaGetErrorString(ee));
+        if (ee != cudaSuccess) return fail_cuda(ee);
         return HB_OK;
     };
     const double t_setup = now_ms() - t_begin - t_index;
@@ -1981,10 +1985,9 @@ namespace {
 // the text never holds more than two slabs.  The result is the handle a whole-file parse would have given (without its
 // text): same rows, so hb_compress_records cuts it into the same HDF5 chunks -- chunk boundaries do not see slab boundaries.
 struct ResidentSink : SlabSink {
-    hb_parse *big = nullptr;
+    ParsePtr big{nullptr, hb_parse_free};
     uint64_t total_text = 0, text_seen = 0, cap = 0;
     std::vector<uint32_t> ploidy, badgt;       // per-sample error counts, summed on the host and put on the device at the end
-    ~ResidentSink() override { if (big) hb_parse_free(big); }
     int begin(const hb_parse_opts &o, const std::vector<std::string> &samples, uint64_t total) override {
         ploidy.assign(std::max<uint32_t>(o.n_samples, 1), 0); badgt.assign(std::max<uint32_t>(o.n_samples, 1), 0);
         ploidy_err = ploidy.data(); badgt_err = badgt.data();
@@ -1992,7 +1995,9 @@ struct ResidentSink : SlabSink {
         total_text = total;
         hb_parse_opts oo = o;
         oo.stream = nullptr;
-        TRY(new_parse(&oo, &big));
+        int rc;
+        big = new_parse(&oo, rc);
+        if (!big) return rc;
         big->samples = samples;
         big->text_released = true;             // there is no text to re-run on
         big->runs_valid = true;                // its CHROM runs are put together from the slabs'
@@ -2001,16 +2006,17 @@ struct ResidentSink : SlabSink {
     int grow(uint64_t need, cudaStream_t st, uint64_t R) {          // capacity for `need` rows, the R rows present are kept
         const uint32_t S = big->n_samples;
         const uint64_t stride = (need + 127) / 128 * 128;
-        struct { uint32_t *start, *stop; uint8_t *ref, *alt; uint64_t *chrom5; int8_t *gt[2]; uint32_t *bits; uint64_t gt_stride; } old =
-            {big->d_start, big->d_stop, big->d_ref, big->d_alt, big->d_chrom5, {big->d_gt[0], big->d_gt[1]}, big->d_bits, big->gt_stride};
+        struct { SiteRows rows; int8_t *gt[2]; uint32_t *bits; uint64_t gt_stride; } old =
+            {big->rows, {big->d_gt[0], big->d_gt[1]}, big->d_bits, big->gt_stride};
         cudaDeviceSynchronize();                   // (rare) copies of the other slot into the old planes are done
-        big->d_start = big->d_stop = nullptr; big->d_ref = big->d_alt = nullptr; big->d_chrom5 = nullptr;
+        big->rows = SiteRows();                    // only the columns of the stored record are kept
         big->d_gt[0] = big->d_gt[1] = nullptr; big->d_bits = nullptr;
-        int rc = dev_alloc(&big->d_start, stride);
-        if (rc == HB_OK) rc = dev_alloc(&big->d_stop, stride);
-        if (rc == HB_OK) rc = dev_alloc(&big->d_ref, stride);
-        if (rc == HB_OK) rc = dev_alloc(&big->d_alt, stride);
-        if (rc == HB_OK) rc = dev_alloc(&big->d_chrom5, stride);
+        SiteRows &r = big->rows;
+        int rc = dev_alloc(&r.start, stride);
+        if (rc == HB_OK) rc = dev_alloc(&r.stop, stride);
+        if (rc == HB_OK) rc = dev_alloc(&r.ref, stride);
+        if (rc == HB_OK) rc = dev_alloc(&r.alt, stride);
+        if (rc == HB_OK) rc = dev_alloc(&r.chrom5, stride);
         if (rc == HB_OK && big->want_gt && S) {
             rc = dev_alloc(&big->d_gt[0], stride * S);
             if (rc == HB_OK) rc = dev_alloc(&big->d_gt[1], stride * S);
@@ -2018,20 +2024,19 @@ struct ResidentSink : SlabSink {
         }
         cudaError_t e = cudaSuccess;
         if (rc == HB_OK && R) {
-            e = cudaMemcpyAsync(big->d_start, old.start, R * 4, cudaMemcpyDeviceToDevice, st);
-            if (e == cudaSuccess) e = cudaMemcpyAsync(big->d_stop, old.stop, R * 4, cudaMemcpyDeviceToDevice, st);
-            if (e == cudaSuccess) e = cudaMemcpyAsync(big->d_ref, old.ref, R, cudaMemcpyDeviceToDevice, st);
-            if (e == cudaSuccess) e = cudaMemcpyAsync(big->d_alt, old.alt, R, cudaMemcpyDeviceToDevice, st);
-            if (e == cudaSuccess) e = cudaMemcpyAsync(big->d_chrom5, old.chrom5, R * 8, cudaMemcpyDeviceToDevice, st);
+            e = cudaMemcpyAsync(r.start, old.rows.start, R * 4, cudaMemcpyDeviceToDevice, st);
+            if (e == cudaSuccess) e = cudaMemcpyAsync(r.stop, old.rows.stop, R * 4, cudaMemcpyDeviceToDevice, st);
+            if (e == cudaSuccess) e = cudaMemcpyAsync(r.ref, old.rows.ref, R, cudaMemcpyDeviceToDevice, st);
+            if (e == cudaSuccess) e = cudaMemcpyAsync(r.alt, old.rows.alt, R, cudaMemcpyDeviceToDevice, st);
+            if (e == cudaSuccess) e = cudaMemcpyAsync(r.chrom5, old.rows.chrom5, R * 8, cudaMemcpyDeviceToDevice, st);
             if (e == cudaSuccess && old.gt[0]) e = cudaMemcpy2DAsync(big->d_gt[0], stride, old.gt[0], old.gt_stride, R, S, cudaMemcpyDeviceToDevice, st);
             if (e == cudaSuccess && old.gt[1]) e = cudaMemcpy2DAsync(big->d_gt[1], stride, old.gt[1], old.gt_stride, R, S, cudaMemcpyDeviceToDevice, st);
             if (e == cudaSuccess) e = cudaStreamSynchronize(st);
         }
-        free_dev(old.start); free_dev(old.stop); free_dev(old.ref); free_dev(old.alt); free_dev(old.chrom5);
-        free_dev(old.gt[0]); free_dev(old.gt[1]); free_dev(old.bits);
+        free_rows(old.rows); free_dev(old.gt[0]); free_dev(old.gt[1]); free_dev(old.bits);
         if (rc != HB_OK) return rc;
-        if (e != cudaSuccess) return fail(HB_ERR_CUDA, std::string("CUDA: ") + cudaGetErrorString(e));
-        big->gt_stride = stride; big->gt_bytes = stride * S; big->bits_stride = stride / 128 * kBitGroupWords; big->row_cap = stride;
+        if (e != cudaSuccess) return fail_cuda(e);
+        big->gt_stride = stride; big->gt_bytes = stride * S; big->bits_stride = stride / 128 * kBitGroupWords; r.cap = stride;
         cap = stride;
         return HB_OK;
     }
@@ -2051,11 +2056,12 @@ struct ResidentSink : SlabSink {
             e = cudaMemcpy2DAsync(big->d_gt[0] + R, big->gt_stride, s.p->d_gt[0], s.p->gt_stride, n, S, cudaMemcpyDeviceToDevice, s.d2h);
             if (e == cudaSuccess) e = cudaMemcpy2DAsync(big->d_gt[1] + R, big->gt_stride, s.p->d_gt[1], s.p->gt_stride, n, S, cudaMemcpyDeviceToDevice, s.d2h);
         }
-        if (e == cudaSuccess) e = cudaMemcpyAsync(big->d_start + R, s.p->d_start, n * 4, cudaMemcpyDeviceToDevice, s.d2h);
-        if (e == cudaSuccess) e = cudaMemcpyAsync(big->d_stop + R, s.p->d_stop, n * 4, cudaMemcpyDeviceToDevice, s.d2h);
-        if (e == cudaSuccess) e = cudaMemcpyAsync(big->d_ref + R, s.p->d_ref, n, cudaMemcpyDeviceToDevice, s.d2h);
-        if (e == cudaSuccess) e = cudaMemcpyAsync(big->d_alt + R, s.p->d_alt, n, cudaMemcpyDeviceToDevice, s.d2h);
-        if (e == cudaSuccess) e = cudaMemcpyAsync(big->d_chrom5 + R, s.p->d_chrom5, n * 8, cudaMemcpyDeviceToDevice, s.d2h);
+        const SiteRows &to = big->rows, &from = s.p->rows;
+        if (e == cudaSuccess) e = cudaMemcpyAsync(to.start + R, from.start, n * 4, cudaMemcpyDeviceToDevice, s.d2h);
+        if (e == cudaSuccess) e = cudaMemcpyAsync(to.stop + R, from.stop, n * 4, cudaMemcpyDeviceToDevice, s.d2h);
+        if (e == cudaSuccess) e = cudaMemcpyAsync(to.ref + R, from.ref, n, cudaMemcpyDeviceToDevice, s.d2h);
+        if (e == cudaSuccess) e = cudaMemcpyAsync(to.alt + R, from.alt, n, cudaMemcpyDeviceToDevice, s.d2h);
+        if (e == cudaSuccess) e = cudaMemcpyAsync(to.chrom5 + R, from.chrom5, n * 8, cudaMemcpyDeviceToDevice, s.d2h);
         // CHROM runs of the slab continue the file's
         TRY(ensure_runs(s.p));
         for (size_t i = 0; i < s.p->run_rows.size(); ++i) {
@@ -2078,9 +2084,7 @@ int hb_parse_stream_bgzf_host(const uint8_t *bgzf, uint64_t nbytes, const char *
                               uint64_t slab_bytes, int8_t *gt0, int8_t *gt1, uint64_t out_stride, uint32_t *start,
                               uint32_t *stop, char *ref, char *alt, uint32_t *ploidy_err, uint32_t *badgt_err,
                               uint64_t *n_records, uint32_t *n_slabs) {
-    HostSink sink;
-    sink.gt0 = gt0; sink.gt1 = gt1; sink.out_stride = out_stride; sink.start = start; sink.stop = stop; sink.ref = ref; sink.alt = alt;
-    sink.ploidy_err = ploidy_err; sink.badgt_err = badgt_err;
+    HostSink sink(gt0, gt1, out_stride, start, stop, ref, alt, ploidy_err, badgt_err);
     return stream_bgzf("hb_parse_stream_bgzf_host", bgzf, nbytes, region, want_gt, device, slab_bytes, sink, n_records, n_slabs);
 }
 
@@ -2091,7 +2095,7 @@ int hb_parse_stream_bgzf_resident(const uint8_t *bgzf, uint64_t nbytes, const ch
     ResidentSink sink;
     uint64_t n = 0;
     TRY(stream_bgzf("hb_parse_stream_bgzf_resident", bgzf, nbytes, region, want_gt, device, slab_bytes, sink, &n, n_slabs));
-    hb_parse *p = sink.big;
+    hb_parse *p = sink.big.get();
     if (!p) return fail(HB_ERR_IO, "empty input");
     const uint32_t S = p->n_samples;
     cudaError_t e = cudaSuccess;
@@ -2107,11 +2111,10 @@ int hb_parse_stream_bgzf_resident(const uint8_t *bgzf, uint64_t nbytes, const ch
             e = cudaStreamSynchronize(p->stream);
         }
     }
-    if (e != cudaSuccess) return fail(HB_ERR_CUDA, std::string("CUDA: ") + cudaGetErrorString(e));
+    if (e != cudaSuccess) return fail_cuda(e);
     p->h_st.n_records = n;
     p->compressed_bytes = nbytes;
-    sink.big = nullptr;
-    *out = p;
+    *out = sink.big.release();
     return HB_OK;
 }
 

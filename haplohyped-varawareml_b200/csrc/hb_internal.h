@@ -82,29 +82,27 @@ void launch_tokenize(bool with_tabs, const uint8_t *d_text, uint64_t nbytes, uin
 uint64_t tokenize_tile_bytes();
 void launch_index_columns(const uint8_t *d_text, const RowInfo *d_rowinfo, const uint32_t *d_nu_rows,
                           uint64_t n_nu, uint64_t *d_cp, uint32_t ncp, const Launch &L);
-void launch_sites(const uint8_t *d_text, const LineIndex &li, uint64_t n_lines, uint32_t n_samples,
-                  const RegionArg &rg, int end_is_int, int want_gt, bool cp_by_line, uint32_t *d_start,
-                  uint32_t *d_stop, uint8_t *d_ref, uint8_t *d_alt, uint64_t *d_chrom_abs, uint8_t *d_chrom_len,
-                  uint64_t *d_chrom5, RowInfo *d_rowinfo, uint32_t *d_nu_rows, uint64_t *d_tile_state, DevStatus *d_st,
-                  const Launch &L);
-// index-free record location for GT-only text (hb_walk.cu)
-uint32_t walk_plan(uint64_t nbytes, uint64_t first_line_len, uint32_t lines_per_walker, uint64_t *range_bytes);
-// walker (hb_walk.cu): padded site rows, kWalkSlots per walker, compacted to dense rows after the prefix sum
-constexpr uint32_t kWalkSlots = 24;
-struct WalkPad {
+// the eight site-row columns of a parse, cap rows each: the site kernels write them, the decoders and kernel 4a read them
+struct SiteRows {
     uint32_t *start = nullptr, *stop = nullptr;
     uint8_t *ref = nullptr, *alt = nullptr, *chrom_len = nullptr;
     uint64_t *chrom_abs = nullptr, *chrom5 = nullptr;
     RowInfo *rowinfo = nullptr;
     uint64_t cap = 0;                        // rows
 };
+void launch_sites(const uint8_t *d_text, const LineIndex &li, uint64_t n_lines, uint32_t n_samples,
+                  const RegionArg &rg, int end_is_int, int want_gt, bool cp_by_line, const SiteRows &rows,
+                  uint32_t *d_nu_rows, uint64_t *d_tile_state, DevStatus *d_st, const Launch &L);
+// index-free record location for GT-only text (hb_walk.cu)
+uint32_t walk_plan(uint64_t nbytes, uint64_t first_line_len, uint32_t lines_per_walker, uint64_t *range_bytes);
+// walker (hb_walk.cu): padded site rows, kWalkSlots per walker, compacted to dense rows after the prefix sum
+constexpr uint32_t kWalkSlots = 24;
 void launch_walk(const uint8_t *d_text, uint64_t nbytes, uint32_t n_samples, uint64_t range_bytes, uint32_t n_walkers,
-                 const RegionArg &rg, int end_is_int, uint64_t *d_wstart, void *d_wcount, uint64_t *d_wrow, const WalkPad &pad,
+                 const RegionArg &rg, int end_is_int, uint64_t *d_wstart, void *d_wcount, uint64_t *d_wrow, const SiteRows &pad,
                  uint64_t *d_verify, uint64_t verify_cap, DevStatus *d_st, const Launch &L);
 void launch_walk_compact(const uint8_t *d_text, uint64_t nbytes, uint32_t n_samples, uint32_t n_walkers, void *d_wcount,
-                         uint64_t *d_wrow, const WalkPad &pad, uint32_t *d_start, uint32_t *d_stop, uint8_t *d_ref, uint8_t *d_alt,
-                         uint64_t *d_chrom_abs, uint8_t *d_chrom_len, uint64_t *d_chrom5, RowInfo *d_rowinfo,
-                         uint32_t *d_nu_rows, uint64_t *d_verify, uint64_t verify_cap, DevStatus *d_st, const Launch &L);
+                         uint64_t *d_wrow, const SiteRows &pad, const SiteRows &rows, uint32_t *d_nu_rows, uint64_t *d_verify,
+                         uint64_t verify_cap, DevStatus *d_st, const Launch &L);
 void launch_chrom_runs(const uint8_t *d_text, const uint64_t *d_chrom_abs, const uint8_t *d_chrom_len,
                        uint64_t n_rows, uint64_t *d_run_rows, uint64_t max_runs, DevStatus *d_st,
                        const Launch &L);
@@ -170,6 +168,7 @@ void count_launch(uint64_t n = 1);
 // pooled big device buffers (hb_api.cu): cudaMalloc / cudaFree of GB-sized buffers are slow and erratic on these hosts
 cudaError_t dev_pool_alloc(void **out, uint64_t bytes);
 void dev_pool_free(void *p);
+void dev_pool_release(void *p);              // back to the driver, not to the idle list
 void dev_pool_flush();
 uint64_t dev_pool_idle_bytes();
 

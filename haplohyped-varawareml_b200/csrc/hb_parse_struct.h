@@ -24,10 +24,9 @@ struct hb_parse {
     bool use_walker = false;            // records located by walking heads (hb_walk.cu) instead of tokenizing
     uint32_t n_walkers = 0, walk_cap = 0;
     uint64_t walk_range = 0;
-    uint64_t *d_wstart = nullptr, *d_wrow = nullptr, *d_verify = nullptr;
-    void *d_wcount = nullptr;
+    uint64_t *d_wstart = nullptr, *d_wrow = nullptr, *d_verify = nullptr, *d_wcount = nullptr;
     uint64_t verify_cap = 0;
-    hb::WalkPad walk_pad;                // padded site rows of the walk (compacted into d_start ... d_rowinfo)
+    hb::SiteRows walk_pad;               // padded site rows of the walk, kWalkSlots per walker (compacted into rows)
     int walker_fallbacks = 0;
     int index_used = 0;                 // 1 newline tokenizer, 2 newline+tab tokenizer, 3 walker, 4 BCF records
     struct Bcf {                        // BCF input: the header's dictionaries and the locator's buffers (hb_bcf.cu)
@@ -53,18 +52,13 @@ struct hb_parse {
     uint64_t first_line_len = 0;
     hb::CtaTok *d_cta = nullptr;
     uint64_t *d_cbase = nullptr;
-    uint64_t *d_cp = nullptr; uint64_t cp_rows = 0;
+    uint64_t *d_cp = nullptr; uint64_t cp_cap = 0;   // column checkpoints, ncp per row
     hb::DevStatus *d_st = nullptr;
     hb::DevStatus h_st;
     hb::DevStatus *h_st_pin = nullptr;       // pinned landing buffer of h_st
-    uint32_t *d_start = nullptr, *d_stop = nullptr;
-    uint8_t *d_ref = nullptr, *d_alt = nullptr, *d_chrom_len = nullptr;
-    uint64_t *d_chrom_abs = nullptr;
-    uint64_t *d_chrom5 = nullptr;       // first 5 CHROM bytes per record (the S5 field of the 35-byte record)
-    hb::RowInfo *d_rowinfo = nullptr;
-    uint32_t *d_nu_rows = nullptr;
-    uint64_t *d_sites_state = nullptr;
-    uint64_t row_cap = 0;
+    hb::SiteRows rows;                  // one per kept record; chrom5 = first 5 CHROM bytes (the S5 field of the 35-byte record)
+    uint32_t *d_nu_rows = nullptr;      // text paths only: the rows that need the general decode path
+    uint64_t *d_sites_state = nullptr;  // tokenizer path only: tile state of the site kernel
     int8_t *d_gt[2] = {nullptr, nullptr};
     uint64_t gt_stride = 0, gt_bytes = 0;
     uint32_t *d_bits = nullptr;         // the same alleles as bit planes (hb_common.cuh, kBitGroupWords): what kernel 4b reads

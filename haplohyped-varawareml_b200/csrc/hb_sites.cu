@@ -134,18 +134,16 @@ __global__ void __launch_bounds__(ST_THREADS) sites_kernel(const SiteArgs a) {
 }
 
 void launch_sites(const uint8_t *d_text, const LineIndex &li, uint64_t n_lines, uint32_t n_samples,
-                  const RegionArg &rg, int end_is_int, int want_gt, bool cp_by_line, uint32_t *d_start,
-                  uint32_t *d_stop, uint8_t *d_ref, uint8_t *d_alt, uint64_t *d_chrom_abs, uint8_t *d_chrom_len,
-                  uint64_t *d_chrom5, RowInfo *d_rowinfo, uint32_t *d_nu_rows, uint64_t *d_tile_state, DevStatus *d_st,
-                  const Launch &L) {
+                  const RegionArg &rg, int end_is_int, int want_gt, bool cp_by_line, const SiteRows &rows,
+                  uint32_t *d_nu_rows, uint64_t *d_tile_state, DevStatus *d_st, const Launch &L) {
     if (!n_lines) return;
     uint64_t tiles = (n_lines + ST_THREADS - 1) / ST_THREADS;
     cudaMemsetAsync(d_tile_state, 0, tiles * sizeof(uint64_t), L.stream);
     SiteArgs a;
     a.text = d_text; a.li = li; a.n_lines = n_lines; a.n_samples = n_samples;
     a.rg = rg; a.end_is_int = end_is_int; a.want_gt = want_gt; a.cp_by_line = cp_by_line ? 1 : 0;
-    a.out.start = d_start; a.out.stop = d_stop; a.out.ref = d_ref; a.out.alt = d_alt;
-    a.out.chrom_abs = d_chrom_abs; a.out.chrom_len = d_chrom_len; a.out.chrom5 = d_chrom5; a.out.rowinfo = d_rowinfo;
+    a.out.start = rows.start; a.out.stop = rows.stop; a.out.ref = rows.ref; a.out.alt = rows.alt;
+    a.out.chrom_abs = rows.chrom_abs; a.out.chrom_len = rows.chrom_len; a.out.chrom5 = rows.chrom5; a.out.rowinfo = rows.rowinfo;
     a.out.nu_rows = d_nu_rows; a.out.st = d_st;
     a.tile_state = d_tile_state; a.st = d_st;
     sites_kernel<<<(unsigned)tiles, ST_THREADS, 0, L.stream>>>(a);

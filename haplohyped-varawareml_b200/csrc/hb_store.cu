@@ -1202,7 +1202,7 @@ static int frames_site_pass(hb_frames *f, hb_parse *p, bool early) {
     cudaError_t e;
 #define CUF(x) do { e = (x); if (e != cudaSuccess) return api_fail(HB_ERR_CUDA, std::string("CUDA: ") + cudaGetErrorString(e) + " at " #x); } while (0)
     SiteArgs4 sa;
-    sa.chrom5 = p->d_chrom5; sa.start = p->d_start; sa.stop = p->d_stop; sa.ref = p->d_ref; sa.alt = p->d_alt;
+    sa.chrom5 = p->rows.chrom5; sa.start = p->rows.start; sa.stop = p->rows.stop; sa.ref = p->rows.ref; sa.alt = p->rows.alt;
     sa.n_records = f->n_records; sa.cr = (uint32_t)f->cr; sa.tmpl = f->d_tmpl; sa.tmpl_cap = f->tmpl_cap; sa.tmpl_len = f->d_tmpl_len;
     sa.deep = g_site_deep.load() ? 1 : 0;
     cudaStream_t st = early ? f->side : f->stream;

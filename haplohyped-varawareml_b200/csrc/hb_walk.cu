@@ -391,7 +391,7 @@ static WalkArgs make_args(const uint8_t *d_text, uint64_t nbytes, uint32_t n_sam
 }
 
 void launch_walk(const uint8_t *d_text, uint64_t nbytes, uint32_t n_samples, uint64_t range_bytes, uint32_t n_walkers,
-                 const RegionArg &rg, int end_is_int, uint64_t *d_wstart, void *d_wcount, uint64_t *d_wrow, const WalkPad &pad,
+                 const RegionArg &rg, int end_is_int, uint64_t *d_wstart, void *d_wcount, uint64_t *d_wrow, const SiteRows &pad,
                  uint64_t *d_verify, uint64_t verify_cap, DevStatus *d_st, const Launch &L) {
     WalkArgs a = make_args(d_text, nbytes, n_samples, range_bytes, n_walkers, rg, end_is_int, d_wstart,
                            (uint2 *)d_wcount, d_wrow, d_st);
@@ -407,16 +407,15 @@ void launch_walk(const uint8_t *d_text, uint64_t nbytes, uint32_t n_samples, uin
 }
 
 void launch_walk_compact(const uint8_t *d_text, uint64_t nbytes, uint32_t n_samples, uint32_t n_walkers, void *d_wcount,
-                         uint64_t *d_wrow, const WalkPad &pad, uint32_t *d_start, uint32_t *d_stop, uint8_t *d_ref, uint8_t *d_alt,
-                         uint64_t *d_chrom_abs, uint8_t *d_chrom_len, uint64_t *d_chrom5, RowInfo *d_rowinfo,
-                         uint32_t *d_nu_rows, uint64_t *d_verify, uint64_t verify_cap, DevStatus *d_st, const Launch &L) {
+                         uint64_t *d_wrow, const SiteRows &pad, const SiteRows &rows, uint32_t *d_nu_rows, uint64_t *d_verify,
+                         uint64_t verify_cap, DevStatus *d_st, const Launch &L) {
     RegionArg rg;
     memset(&rg, 0, sizeof rg);
     WalkArgs a = make_args(d_text, nbytes, n_samples, 0, n_walkers, rg, 0, nullptr, (uint2 *)d_wcount, d_wrow, d_st);
     a.pad.start = pad.start; a.pad.stop = pad.stop; a.pad.ref = pad.ref; a.pad.alt = pad.alt;
     a.pad.chrom_abs = pad.chrom_abs; a.pad.chrom_len = pad.chrom_len; a.pad.chrom5 = pad.chrom5; a.pad.rowinfo = pad.rowinfo;
-    a.out.start = d_start; a.out.stop = d_stop; a.out.ref = d_ref; a.out.alt = d_alt;
-    a.out.chrom_abs = d_chrom_abs; a.out.chrom_len = d_chrom_len; a.out.chrom5 = d_chrom5; a.out.rowinfo = d_rowinfo;
+    a.out.start = rows.start; a.out.stop = rows.stop; a.out.ref = rows.ref; a.out.alt = rows.alt;
+    a.out.chrom_abs = rows.chrom_abs; a.out.chrom_len = rows.chrom_len; a.out.chrom5 = rows.chrom5; a.out.rowinfo = rows.rowinfo;
     a.out.nu_rows = d_nu_rows;
     a.verify = d_verify; a.verify_cap = verify_cap;
     const uint64_t n = (uint64_t)n_walkers * kWalkSlots;
