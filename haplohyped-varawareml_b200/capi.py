@@ -76,7 +76,7 @@ EXPORTS = [
     "hb_parse_fetch_sites", "hb_parse_fetch_sample", "hb_parse_fetch_matrix", "hb_parse_fetch_sample_errors",
     "hb_parse_chrom_runs", "hb_parse_free",
     "hb_bgzf_inflate", "hb_bgzf_compress_host",
-    "hb_compress_records", "hb_compress_sample_range", "hb_frames_set_window", "hb_parse_release_text", "hb_parse_attach_frames", "hb_frames_rerun", "hb_frames_get_info", "hb_frames_layout", "hb_frames_fetch_all", "hb_frames_fetch_packed", "hb_set_fetch_mode", "hb_set_bgzf_crc_check", "hb_get_bgzf_crc_check", "hb_set_host_threads", "hb_frames_last_d2h_bytes",
+    "hb_compress_records", "hb_compress_sample_range", "hb_frames_set_window", "hb_parse_release_text", "hb_parse_attach_frames", "hb_frames_rerun", "hb_frames_get_info", "hb_frames_layout", "hb_frames_fetch_all", "hb_frames_fetch_packed", "hb_set_fetch_mode", "hb_set_bgzf_crc_check", "hb_get_bgzf_crc_check", "hb_set_use_index", "hb_get_use_index", "hb_parse_vcf_bytes_indexed", "hb_parse_index_info", "hb_index_bgzf", "hb_index_file", "hb_set_host_threads", "hb_frames_last_d2h_bytes",
     "hb_frames_fetch_sample", "hb_frames_free",
     "hb_guess_chunk_records", "hb_set_site_matcher", "hb_decode_frames", "hb_decode_columns_device", "hb_decode_columns_device_large",
     "hb_encode_haplotypes",
@@ -109,6 +109,14 @@ def lib():
         L.hb_set_bgzf_crc_check.argtypes = [C.c_int]
         L.hb_set_bgzf_crc_check.restype = None
         L.hb_get_bgzf_crc_check.restype = C.c_int
+        L.hb_set_use_index.argtypes = [C.c_int]
+        L.hb_set_use_index.restype = None
+        L.hb_get_use_index.restype = C.c_int
+        L.hb_parse_vcf_bytes_indexed.argtypes = [C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint64, C.c_char_p, C.c_int, C.c_int,
+                                                 C.POINTER(C.c_void_p)]
+        L.hb_parse_index_info.argtypes = [C.c_void_p, C.POINTER(C.c_int), C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]
+        L.hb_index_bgzf.argtypes = [C.c_void_p, C.c_uint64, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_uint64, C.POINTER(C.c_uint64)]
+        L.hb_index_file.argtypes = [C.c_char_p, C.c_int, C.c_int, C.c_int, C.c_char_p]
         L.hb_set_host_threads.argtypes = [C.c_int]
         L.hb_set_host_threads.restype = None
         L.hb_frames_last_d2h_bytes.argtypes = [C.c_void_p]
@@ -234,8 +242,9 @@ class Parse:
         return cls(h)
 
     @classmethod
-    def from_vcf_bytes(cls, data, region="", want_gt=True, device=0, nbytes=None):
-        """The bytes of a .vcf / .vcf.gz / .bcf in host memory (bytes, uint8 array, or address + nbytes)."""
+    def from_vcf_bytes(cls, data, region="", want_gt=True, device=0, nbytes=None, index=None):
+        """The bytes of a .vcf / .vcf.gz / .bcf in host memory (bytes, uint8 array, or address + nbytes).  index: the bytes
+        of its .tbi / .csi; a region query then inflates only the BGZF members the index lists for the region."""
         if isinstance(data, (bytes, bytearray)):
             keep = np.frombuffer(data, np.uint8); addr, n = keep.ctypes.data, keep.size
         elif isinstance(data, np.ndarray):
@@ -243,7 +252,12 @@ class Parse:
         else:
             keep = None; addr, n = int(data), int(nbytes)
         h = C.c_void_p()
-        check(lib().hb_parse_vcf_bytes(addr, n, (region or "").encode(), int(want_gt), device, C.byref(h)))
+        if index is None:
+            check(lib().hb_parse_vcf_bytes(addr, n, (region or "").encode(), int(want_gt), device, C.byref(h)))
+        else:
+            ix = np.frombuffer(bytes(index), np.uint8)
+            check(lib().hb_parse_vcf_bytes_indexed(addr, n, ix.ctypes.data, ix.size, (region or "").encode(), int(want_gt),
+                                                   device, C.byref(h)))
         del keep
         return cls(h)
 
@@ -277,6 +291,13 @@ class Parse:
         i = ParseInfo()
         check(lib().hb_parse_get_info(self._h, C.byref(i)))
         return i
+
+    @property
+    def index_info(self):
+        """(used, compressed_bytes_read, n_chunks) of a region query through an index (hb_parse_index_info)."""
+        used, nread, nch = C.c_int(), C.c_uint64(), C.c_uint64()
+        check(lib().hb_parse_index_info(self._h, C.byref(used), C.byref(nread), C.byref(nch)))
+        return bool(used.value), int(nread.value), int(nch.value)
 
     def sites(self):
         n = self.info.n_records
@@ -531,6 +552,51 @@ def crc_check(on: bool = True):
         yield
     finally:
         set_bgzf_crc_check(was)
+
+
+def set_use_index(on: bool) -> None:
+    """Answer region queries through <file>.tbi / <file>.csi when one is there (hb_set_use_index; process-wide, on by default)."""
+    lib().hb_set_use_index(1 if on else 0)
+
+
+def get_use_index() -> bool:
+    return bool(lib().hb_get_use_index())
+
+
+@contextlib.contextmanager
+def use_index(on: bool = True):
+    """`with use_index(False): ...` runs the block with region queries through an index set to `on` and restores the setting."""
+    was = get_use_index()
+    set_use_index(on)
+    try:
+        yield
+    finally:
+        set_use_index(was)
+
+
+INDEX_FORMATS = {"tbi": 0, "csi": 1}
+
+
+def build_index(data, fmt: str = "tbi", min_shift: int = 14, device: int = 0) -> bytes:
+    """The .tbi / .csi of BGZF bytes (a .vcf.gz, or a .bcf with fmt="csi"), built on the GPU (hb_index_bgzf): the bytes of
+    the index file, BGZF-compressed."""
+    src = np.frombuffer(bytes(data), np.uint8) if isinstance(data, (bytes, bytearray, memoryview)) else data
+    n = C.c_uint64()
+    cap = max(1 << 20, src.size // 8)
+    out = np.empty(cap, np.uint8)
+    rc = lib().hb_index_bgzf(src.ctypes.data, src.size, INDEX_FORMATS[fmt], min_shift, device, out.ctypes.data, cap, C.byref(n))
+    if rc == 10 and n.value > cap:
+        out = np.empty(n.value, np.uint8)
+        rc = lib().hb_index_bgzf(src.ctypes.data, src.size, INDEX_FORMATS[fmt], min_shift, device, out.ctypes.data, out.size,
+                                 C.byref(n))
+    check(rc)
+    return out[:n.value].tobytes()
+
+
+def index_file(path: str, fmt: str = "tbi", min_shift: int = 14, device: int = 0, out_path: str | None = None) -> str:
+    """Write the index of `path` (hb_index_file) to out_path, by default <path>.tbi / <path>.csi; returns where."""
+    check(lib().hb_index_file(path.encode(), INDEX_FORMATS[fmt], min_shift, device, out_path.encode() if out_path else None))
+    return out_path or path + "." + fmt
 
 
 def bgzf_inflate(data: bytes, device: int = 0, with_ms: bool = False):

@@ -19,13 +19,17 @@
 #include <memory>
 #include <mutex>
 #include <string>
+#include <fcntl.h>
 #include <sys/stat.h>
+#include <unistd.h>
 #include <thread>
 #include <vector>
 
 #include "../../include/haplo_b200.h"
 #include "hb_internal.h"
 #include "hb_parse_struct.h"
+#include "hb_index.h"
+#include "hb_tabix.h"
 
 namespace hb {
 
@@ -1224,7 +1228,7 @@ int hb_parse_chrom_runs(hb_parse *p, uint64_t *n_runs, uint64_t *row_begin, uint
 // =============================================================================================
 namespace hb {
 bool bgzf_index(const uint8_t *raw, uint64_t size, std::vector<uint64_t> &coff, std::vector<uint32_t> &clen,
-                std::vector<uint64_t> &ooff, std::vector<uint32_t> &olen, uint64_t &total);
+                std::vector<uint64_t> &ooff, std::vector<uint32_t> &olen, uint64_t &total, std::vector<uint64_t> *boff = nullptr);
 int inflate_bgzf_to_device(const uint8_t *raw, uint64_t size, const std::vector<uint64_t> &coff,
                            const std::vector<uint32_t> &clen, const std::vector<uint64_t> &ooff,
                            const std::vector<uint32_t> &olen, uint8_t *d_out, cudaStream_t stream, float *ms);
@@ -1239,6 +1243,7 @@ struct FileText {
     int end_is_int = 0;
     bool bcf = false;            // BCF 2.2: body = the records after the header text
     std::vector<std::string> contigs;   // BCF contig dictionary
+    std::vector<uint64_t> contig_len;   // BCF: their ##contig length= (0: not given)
     int gt_key = -1;             // BCF string-dictionary index of GT (-1: not declared)
 };
 
@@ -1386,12 +1391,18 @@ int bcf_header(const uint8_t *d, uint64_t n, FileText &ft, bool &complete) {
             const int c = i >= 0 ? i : cnext;
             cnext = std::max(cnext, c + 1);
             ctg.emplace_back(c, id);
+            std::string len;
+            if (hrec_attr(line, "length", len)) {
+                if ((size_t)c >= ft.contig_len.size()) ft.contig_len.resize((size_t)c + 1, 0);
+                ft.contig_len[(size_t)c] = strtoull(len.c_str(), nullptr, 10);
+            }
         } else if (i >= 0) {
             strs[id] = i;
             next = std::max(next, i + 1);
         } else if (!strs.count(id)) strs[id] = next++;
     }
     ft.contigs.assign((size_t)cnext, std::string());
+    ft.contig_len.resize((size_t)cnext, 0);
     for (auto &c : ctg) ft.contigs[(size_t)c.first] = c.second;
     const auto gt = strs.find("GT");
     ft.gt_key = gt == strs.end() ? -1 : gt->second;
@@ -1422,8 +1433,15 @@ int read_vcf(const std::vector<uint8_t> &raw, FileText &ft) {
 int parse_bytes_common(std::vector<uint8_t> &raw_owned, const uint8_t *raw_p, uint64_t raw_n, const char *region, bool want_gt,
                        int device, hb_parse **out, std::vector<std::string> &samples);
 
+// a region query of a file with a usable .tbi / .csi next to it: HB_OK with used = false when the index is not usable
+int parse_file_indexed(const char *path, const char *region, bool want_gt, int device, hb_parse **out,
+                       std::vector<std::string> &samples, bool &used);
+
 int parse_file_common(const char *path, const char *region, bool want_gt, int device, hb_parse **out,
                       std::vector<std::string> &samples) {
+    bool used = false;
+    TRY(parse_file_indexed(path, region, want_gt, device, out, samples, used));
+    if (used) return HB_OK;
     std::vector<uint8_t> raw;
     TRY(read_all(path, raw));
     return parse_bytes_common(raw, raw.data(), raw.size(), region, want_gt, device, out, samples);
@@ -1441,8 +1459,9 @@ struct BgzfFile {
 bool index_bgzf(const uint8_t *raw, uint64_t n, BgzfFile &f) { return bgzf_index(raw, n, f.coff, f.clen, f.ooff, f.olen, f.total); }
 
 // the VCF header of a BGZF file: leading members are inflated on the host (zlib) until the #CHROM line is complete; with
-// hb_set_bgzf_crc_check on, each is checked against its CRC32 as kernel 0 checks the others
-int bgzf_header(const uint8_t *raw, BgzfFile &f) {
+// hb_set_bgzf_crc_check on, each is checked against its CRC32 as kernel 0 checks the others.  more != NULL: f holds only the
+// leading members of the file, and *more = true asks for more of them when the header does not end inside those
+int bgzf_header(const uint8_t *raw, BgzfFile &f, bool *more = nullptr) {
     std::vector<uint8_t> head;
     bool have = false;
     const bool check_crc = bgzf_crc_check();
@@ -1465,8 +1484,10 @@ int bgzf_header(const uint8_t *raw, BgzfFile &f) {
             if ((uint32_t)crc32(crc32(0L, Z_NULL, 0), head.data() + at, f.olen[i]) != want) return fail(HB_ERR_IO, bgzf_crc_message(raw, f.coff[i]));
         }
         if (is_bcf(head.data(), head.size())) TRY(bcf_header(head.data(), head.size(), f.ft, have));
-        else have = parse_header(head.data(), head.size(), i + 1 == f.coff.size(), f.ft);
+        else have = parse_header(head.data(), head.size(), !more && i + 1 == f.coff.size(), f.ft);
     }
+    if (more) *more = !have;
+    if (!have && more) return HB_OK;
     if (!have && is_bcf(head.data(), head.size())) return fail(HB_ERR_FORMAT, "BCF header is truncated");
     if (!have) return fail(HB_ERR_HEADER, "no #CHROM header line");
     return HB_OK;
@@ -1593,6 +1614,188 @@ int parse_bytes_common(std::vector<uint8_t> &raw_owned, const uint8_t *raw_p, ui
     if (trace) fprintf(stderr, "[parse_bytes_common] text buffer %.1f ms, H2D + inflate %.1f ms, parse %.1f ms\n", t1 - t0, t2 - t1, now_ms() - t2);
     TRY(rc);
     *out = p.release();
+    return HB_OK;
+}
+
+// ---- region queries through a tabix / CSI index: only the BGZF members of the query's span are read and inflated
+std::atomic<int> g_use_index{1};                  // hb_set_use_index
+
+void index_not_used(const std::string &why) {
+    if (getenv("HB_TRACE")) fprintf(stderr, "[index] not used: %s\n", why.c_str());
+}
+
+// the bytes of a file (pread) or of a caller's buffer
+struct ByteSource {
+    const uint8_t *mem = nullptr;
+    int fd = -1;
+    uint64_t size = 0;
+    const uint8_t *get(uint64_t off, uint64_t n, std::vector<uint8_t> &buf) const {
+        if (off > size || n > size - off) return nullptr;
+        if (mem) return mem + off;
+        buf.resize(n);
+        for (uint64_t got = 0; got < n;) {
+            const ssize_t r = pread(fd, buf.data() + got, n - got, (off_t)(off + got));
+            if (r <= 0) return nullptr;
+            got += (uint64_t)r;
+        }
+        return buf.data();
+    }
+};
+
+// bytes of the BGZF member that starts at h (avail bytes readable there), 0 when none starts there
+uint64_t bgzf_member_size(const uint8_t *h, uint64_t avail) {
+    if (avail < 18 || h[0] != 0x1f || h[1] != 0x8b || h[2] != 8 || !(h[3] & 4)) return 0;
+    const uint64_t xe = 12ull + (h[10] | h[11] << 8);
+    if (xe > avail) return 0;
+    for (uint64_t q = 12; q + 4 <= xe; q += 4 + (h[q + 2] | h[q + 3] << 8))
+        if (h[q] == 'B' && h[q + 1] == 'C' && (h[q + 2] | h[q + 3] << 8) == 2 && q + 6 <= xe) return (h[q + 4] | h[q + 5] << 8) + 1ull;
+    return 0;
+}
+
+// The parse of `region` from the members of src that hold the records the index lists for it.  The region filter runs
+// as on a full scan, so the rows are the same.  used = false (with `why`): the index cannot serve this query and the
+// caller takes the full-scan route; nothing has been parsed then.
+int parse_indexed(const ByteSource &src, const uint8_t *ix, uint64_t ix_n, const char *region, bool want_gt, int device,
+                  hb_parse **out, std::vector<std::string> &samples, bool &used, std::string &why) {
+    used = false;
+    std::vector<uint8_t> hbuf, sbuf;
+    {
+        const uint8_t *h = src.get(0, std::min<uint64_t>(src.size, 18), hbuf);
+        if (!h || !bgzf_member_size(h, std::min<uint64_t>(src.size, 18))) { why = "the input is not BGZF"; return HB_OK; }
+    }
+    TabixIndex idx;
+    if (!tabix_load(ix, ix_n, idx, why)) return HB_OK;
+    // the header: leading members, twice as many bytes of them each round until it ends inside them (the rounds
+    // re-inflate what the round before inflated: at most twice the header's members in all)
+    BgzfFile bz;
+    uint64_t head_read = 0;
+    std::vector<uint8_t> head;                              // bytes [0, head_read) of a file source
+    for (bool more = true; more;) {
+        const uint64_t target = std::min(src.size, std::max<uint64_t>(2 * head_read, 1));
+        const uint64_t avail = std::min<uint64_t>(src.size, target + 65536) - head_read;
+        const uint8_t *b = src.get(head_read, avail, hbuf);
+        uint64_t w = 0;
+        for (uint64_t s; b && head_read + w < target && (s = bgzf_member_size(b + w, avail - w)) != 0 && s <= avail - w;) w += s;
+        if (!w) { why = "the input is not BGZF"; return HB_OK; }
+        if (!src.mem) head.insert(head.end(), b, b + w);
+        head_read += w;
+        const uint8_t *all = src.mem ? src.mem : head.data();
+        bz = BgzfFile();
+        if (!index_bgzf(all, head_read, bz)) { why = "the input is not BGZF"; return HB_OK; }
+        const std::string err = g_err;
+        if (bgzf_header(all, bz, head_read < src.size ? &more : nullptr) != HB_OK) { g_err = err; why = "the header does not read"; return HB_OK; }
+        if (head_read == src.size) more = false;
+    }
+    const FileText &ft = bz.ft;
+    if (ft.bcf && !idx.csi) { why = "a BCF is queried through a CSI index only"; return HB_OK; }
+    if (!ft.bcf && idx.names.empty()) { why = "the index names no sequences"; return HB_OK; }
+    RegionArg rg;
+    parse_region(region, rg);
+    const std::vector<std::string> &names = ft.bcf ? ft.contigs : idx.names;
+    const auto at = std::find(names.begin(), names.end(), std::string(rg.chrom, rg.chrom_len));
+    const auto chunks = at == names.end() ? std::vector<std::pair<uint64_t, uint64_t>>()
+                                          : tabix_query(idx, (int)(at - names.begin()), rg.beg0, rg.end0);
+    // the span [first chunk begin, last chunk end): its members, read in one piece
+    BgzfFile sp;
+    const uint8_t *sb = nullptr;
+    uint64_t t0 = 0, t1 = 0, span_comp = 0;
+    if (!chunks.empty()) {
+        const uint64_t c0 = chunks.front().first >> 16, c1 = chunks.back().second >> 16;
+        const uint64_t u0 = chunks.front().first & 0xffff, u1 = chunks.back().second & 0xffff;
+        if (c1 < c0 || c1 > src.size) { why = "the index points past the end of the file"; return HB_OK; }
+        const uint64_t n = std::min<uint64_t>(src.size, c1 + (u1 ? 65536 : 0)) - c0;
+        sb = src.get(c0, n, sbuf);
+        if (!sb) { why = "read error"; return HB_OK; }
+        uint64_t w = 0, last = 0;
+        while (c0 + w < c1 || (u1 && c0 + w == c1)) {
+            const uint64_t s = bgzf_member_size(sb + w, n - w);
+            if (!s || s > n - w) break;
+            last = w;
+            w += s;
+        }
+        if (c0 + w < c1 || (u1 && c0 + last != c1) || !index_bgzf(sb, w, sp) || sp.total == 0) {
+            why = "the index's offsets do not fall on BGZF members of the file";
+            return HB_OK;
+        }
+        t0 = u0;
+        t1 = u1 ? sp.total - sp.olen.back() + u1 : sp.total;
+        if (t0 > t1 || u0 > sp.olen.front() || (u1 && u1 > sp.olen.back())) { why = "the index's offsets do not fall on BGZF members of the file"; return HB_OK; }
+        span_comp = w;
+    }
+    TRY(ensure_device(device));
+    uint64_t slab;
+    if (t1 - t0 > text_limit(slab)) { why = "the region's span is above the text limit"; return HB_OK; }
+    used = true;
+    samples = ft.samples;
+    const hb_parse_opts o = opts_for(ft, region, want_gt, device);
+    const double ta = now_ms();
+    int rc;
+    ParsePtr p = new_parse(&o, rc);
+    if (!p) return rc;
+    const uint64_t pad = (16 - t0 % 16) % 16;           // the records start on a 16-byte boundary
+    TRY(dev_alloc(&p->d_text_owned, pad + sp.total + 1 + kTextPad));
+    if (t1 > t0) TRY(inflate_bgzf_to_device(sb, span_comp, sp.coff, sp.clen, sp.ooff, sp.olen, p->d_text_owned + pad, p->stream, &p->ms_inflate));
+    uint8_t *text = p->d_text_owned + pad + t0;
+    uint64_t nb = t1 - t0;
+    uint8_t last = '\n';
+    cudaError_t e = nb ? cudaMemcpy(&last, text + nb - 1, 1, cudaMemcpyDeviceToHost) : cudaSuccess;
+    if (e == cudaSuccess && last != '\n' && !ft.bcf) { e = cudaMemset(text + nb, '\n', 1); ++nb; }
+    if (e == cudaSuccess) e = cudaMemset(text + nb, 0, kTextPad);
+    if (e != cudaSuccess) return fail_cuda(e);
+    p->d_text = text;
+    p->nbytes = nb;
+    p->compressed_bytes = span_comp;
+    p->idx_used = 1;
+    p->idx_bytes_read = head_read + span_comp;
+    p->idx_chunks = chunks.size();
+    const double tb = now_ms();
+    rc = ft.bcf ? bcf_attach(p.get(), ft) : HB_OK;
+    if (rc == HB_OK) rc = run_parse(p.get());
+    if (getenv("HB_TRACE"))
+        fprintf(stderr, "[index] %zu chunks, %llu of %llu compressed bytes read: H2D + inflate %.1f ms, parse %.1f ms\n", chunks.size(),
+                (unsigned long long)p->idx_bytes_read, (unsigned long long)src.size, tb - ta, now_ms() - tb);
+    TRY(rc);
+    *out = p.release();
+    return HB_OK;
+}
+
+// htslib's order: <path>.tbi then <path>.csi for a .vcf.gz, <path>.csi for a .bcf; an index older than the data is ignored
+bool find_index(const char *path, std::vector<uint8_t> &ix, std::string &why) {
+    const std::string base(path);
+    const bool bcf = base.size() >= 4 && base.compare(base.size() - 4, 4, ".bcf") == 0;
+    struct stat sd, si;
+    if (stat(path, &sd) != 0) { why = "cannot stat the data file"; return false; }
+    for (const char *ext : {".tbi", ".csi"}) {
+        if (bcf && ext[1] == 't') continue;
+        const std::string ip = base + ext;
+        if (stat(ip.c_str(), &si) != 0) continue;
+        if (si.st_mtime < sd.st_mtime) { why = ip + " is older than the data file"; return false; }
+        const std::string err = g_err;
+        if (read_all(ip.c_str(), ix) != HB_OK) { g_err = err; why = "cannot read " + ip; return false; }
+        return true;
+    }
+    why = "no index next to the file";
+    return false;
+}
+
+int parse_file_indexed(const char *path, const char *region, bool want_gt, int device, hb_parse **out,
+                       std::vector<std::string> &samples, bool &used) {
+    used = false;
+    std::string why;
+    std::vector<uint8_t> ix;
+    if (!region || !*region) why = "the region is empty";
+    else if (!g_use_index.load()) why = "hb_set_use_index(0)";
+    else if (find_index(path, ix, why)) {
+        const int fd = open(path, O_RDONLY);
+        struct stat st;
+        int rc = HB_OK;
+        if (fd < 0 || fstat(fd, &st) != 0) why = std::string("cannot open ") + path;
+        else rc = parse_indexed(ByteSource{nullptr, fd, (uint64_t)st.st_size}, ix.data(), ix.size(), region, want_gt, device, out,
+                                samples, used, why);
+        if (fd >= 0) close(fd);
+        if (rc != HB_OK || used) return rc;
+    }
+    index_not_used(why);
     return HB_OK;
 }
 
@@ -2189,5 +2392,121 @@ int hb_parse_samples(hb_parse *p, uint32_t *n, char *names, uint64_t cap, uint64
         used += s.size() + 1;
     }
     if (len) *len = used;
+    return HB_OK;
+}
+
+// ---- region queries through a .tbi / .csi index
+void hb_set_use_index(int on) { g_use_index.store(on ? 1 : 0); }
+int hb_get_use_index(void) { return g_use_index.load(); }
+
+int hb_parse_vcf_bytes_indexed(const uint8_t *data, uint64_t nbytes, const uint8_t *index, uint64_t index_n, const char *region,
+                               int want_gt, int device, hb_parse **out) {
+    if (!data || !out || (index_n && !index)) return fail(HB_ERR_ARG, "null argument");
+    std::vector<std::string> samples;
+    std::string why;
+    bool used = false;
+    if (!region || !*region) why = "the region is empty";
+    else if (!g_use_index.load()) why = "hb_set_use_index(0)";
+    else if (!index_n) why = "no index given";
+    else TRY(parse_indexed(ByteSource{data, -1, nbytes}, index, index_n, region, want_gt != 0, device, out, samples, used, why));
+    if (!used) {
+        index_not_used(why);
+        std::vector<uint8_t> none;
+        TRY(parse_bytes_common(none, data, nbytes, region, want_gt != 0, device, out, samples));
+    }
+    (*out)->samples = samples;
+    return HB_OK;
+}
+
+int hb_parse_index_info(const hb_parse *p, int *used, uint64_t *compressed_bytes_read, uint64_t *n_chunks) {
+    if (!p) return fail(HB_ERR_ARG, "null handle");
+    if (used) *used = p->idx_used;
+    if (compressed_bytes_read) *compressed_bytes_read = p->idx_bytes_read;
+    if (n_chunks) *n_chunks = p->idx_chunks;
+    return HB_OK;
+}
+
+// ---- building an index (kernel 7, hb_index.cu): kernel 0 inflates, the newline tokenizer or the BCF locator finds every
+// record through a parse without a region or genotypes, then kernels 7a / 7b and the host assembly
+int hb_index_bgzf(const uint8_t *data, uint64_t n, int fmt, int min_shift, int device, uint8_t *out, uint64_t cap, uint64_t *len) {
+    if (!data || !len) return fail(HB_ERR_ARG, "null argument");
+    if (fmt != HB_INDEX_TBI && fmt != HB_INDEX_CSI) return fail(HB_ERR_ARG, "fmt is HB_INDEX_TBI or HB_INDEX_CSI");
+    if (fmt == HB_INDEX_CSI && (min_shift < 1 || min_shift > 30)) return fail(HB_ERR_ARG, "min_shift must be 1..30");
+    const bool trace = getenv("HB_TRACE") != nullptr;
+    const double t0 = now_ms();
+    BgzfFile bz;
+    std::vector<uint64_t> boff;
+    if (n < 28 || data[0] != 0x1f || data[1] != 0x8b || !bgzf_index(data, n, bz.coff, bz.clen, bz.ooff, bz.olen, bz.total, &boff) ||
+        bz.total == 0)
+        return fail(HB_ERR_ARG, "an index needs BGZF input (bgzip / bcftools -Ob), not plain gzip or uncompressed bytes");
+    TRY(bgzf_header(data, bz));
+    const FileText &ft = bz.ft;
+    if (ft.bcf && fmt == HB_INDEX_TBI) return fail(HB_ERR_ARG, "a BCF is indexed with CSI only");
+    TRY(ensure_device(device));
+    uint64_t slab;
+    if (bz.total > text_limit(slab)) return fail(HB_ERR_ARG, "the text is above the text limit: slab-wise indexing is not supported");
+    hb_parse *raw = nullptr;
+    std::vector<std::string> samples;
+    std::vector<uint8_t> none;
+    TRY(parse_bytes_common(none, data, n, "", false, device, &raw, samples));
+    ParsePtr p(raw, hb_parse_free);
+    const double t1 = now_ms();
+    IndexJob j;
+    j.d_text = p->d_text;
+    j.text_base = ft.body;
+    j.total = bz.total;
+    j.n_rec = p->n_lines;
+    j.bcf = ft.bcf;
+    if (ft.bcf) {
+        j.d_rec_off = p->bcf->d_rec_off;
+        j.n_contigs = (uint32_t)ft.contigs.size();
+    } else {
+        if (p->index_used != 1) return fail(HB_ERR_ARG, "internal: the index needs the newline tokenizer's line index");
+        j.li = LineIndex{p->d_nl_after, p->d_cbase, p->n_cta, p->stage_cap};
+    }
+    j.ooff = bz.ooff; j.olen = bz.olen; j.boff = boff;
+    for (size_t i = 0; i < bz.coff.size(); ++i) j.bend.push_back(bz.coff[i] + bz.clen[i] + 8);
+    j.csi = fmt == HB_INDEX_CSI;
+    if (!j.csi) { j.min_shift = 14; j.n_lvls = 5; }                            // tabix -p vcf
+    else if (!ft.bcf) { j.min_shift = min_shift; j.n_lvls = (31 - min_shift + 2) / 3; }   // tabix -C: TBX_MAX_SHIFT 31
+    else {                                                                   // bcftools index: the longest contig + 256
+        uint64_t longest = 0;
+        for (uint64_t l : ft.contig_len) longest = std::max(longest, l);
+        longest = (longest ? longest : (1ull << 31) - 1) + 256;
+        j.min_shift = min_shift; j.n_lvls = 0;
+        for (uint64_t s = 1ull << min_shift; longest > s; s <<= 3) ++j.n_lvls;
+    }
+    j.stream = p->stream;
+    std::vector<uint8_t> idx;
+    IndexTimes tm;
+    TRY(build_index(j, idx, &tm));
+    uint64_t need = 0;
+    TRY(hb_bgzf_compress_host(idx.data(), idx.size(), 6, nullptr, 0, &need));
+    std::vector<uint8_t> z(need);
+    TRY(hb_bgzf_compress_host(idx.data(), idx.size(), 6, z.data(), z.size(), &need));
+    *len = need;
+    if (trace)
+        fprintf(stderr, "[hb_index_bgzf] %llu records: parse (H2D + inflate + locate) %.1f ms, kernel 7a %.3f ms, 7b %.3f ms, "
+                        "host assembly %.1f ms, total %.1f ms\n", (unsigned long long)j.n_rec, t1 - t0, tm.ms_keys, tm.ms_chunks,
+                tm.ms_host, now_ms() - t0);
+    if (!out) return HB_OK;
+    if (cap < need) return fail(HB_ERR_ARG, "buffer too small: " + std::to_string(need) + " bytes needed");
+    memcpy(out, z.data(), need);
+    return HB_OK;
+}
+
+int hb_index_file(const char *path, int fmt, int min_shift, int device, const char *out_path) {
+    if (!path) return fail(HB_ERR_ARG, "null argument");
+    std::vector<uint8_t> raw;
+    TRY(read_all(path, raw));
+    uint64_t len = 0;
+    TRY(hb_index_bgzf(raw.data(), raw.size(), fmt, min_shift, device, nullptr, 0, &len));
+    std::vector<uint8_t> z(len);
+    TRY(hb_index_bgzf(raw.data(), raw.size(), fmt, min_shift, device, z.data(), z.size(), &len));
+    const std::string dst = out_path ? std::string(out_path) : std::string(path) + (fmt == HB_INDEX_TBI ? ".tbi" : ".csi");
+    FILE *f = fopen(dst.c_str(), "wb");
+    if (!f) return fail(HB_ERR_IO, "cannot write " + dst);
+    const bool ok = fwrite(z.data(), 1, len, f) == len;
+    if (fclose(f) != 0 || !ok) return fail(HB_ERR_IO, "cannot write " + dst);
     return HB_OK;
 }

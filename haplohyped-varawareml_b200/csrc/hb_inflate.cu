@@ -449,9 +449,9 @@ static void launch_inflate(const InflateArgs &a, cudaStream_t stream) {
     else inflate_bgzf_kernel<false><<<grid, kInfWarps * 32, 0, stream>>>(a);
 }
 
-// BGZF member table of a whole file (host): false when the bytes are not BGZF
+// BGZF member table of a whole file (host): false when the bytes are not BGZF; boff (may be NULL): each member's address
 bool bgzf_index(const uint8_t *raw, uint64_t size, std::vector<uint64_t> &coff, std::vector<uint32_t> &clen,
-                std::vector<uint64_t> &ooff, std::vector<uint32_t> &olen, uint64_t &total) {
+                std::vector<uint64_t> &ooff, std::vector<uint32_t> &olen, uint64_t &total, std::vector<uint64_t> *boff) {
     uint64_t p = 0;
     total = 0;
     while (p < size) {
@@ -479,6 +479,7 @@ bool bgzf_index(const uint8_t *raw, uint64_t size, std::vector<uint64_t> &coff, 
             clen.push_back(bsize - 12 - xlen - 8);
             ooff.push_back(total);
             olen.push_back(isize);
+            if (boff) boff->push_back(p);
         }
         total += isize;
         p += bsize;
@@ -632,7 +633,7 @@ extern "C" int hb_bgzf_inflate(const uint8_t *bgzf, uint64_t nbytes, uint8_t *ou
     std::vector<uint64_t> coff, ooff;
     std::vector<uint32_t> clen, olen;
     uint64_t total = 0;
-    if (!bgzf_index(bgzf, nbytes, coff, clen, ooff, olen, total)) return api_fail(HB_ERR_IO, "not a BGZF file");
+    if (!bgzf_index(bgzf, nbytes, coff, clen, ooff, olen, total, nullptr)) return api_fail(HB_ERR_IO, "not a BGZF file");
     *out_len = total;
     if (!out) return HB_OK;
     if (cap < total) return api_fail(HB_ERR_ARG, "buffer too small");

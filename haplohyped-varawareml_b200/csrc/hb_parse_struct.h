@@ -71,6 +71,9 @@ struct hb_parse {
     cudaEvent_t ev_runs = nullptr;
     float ms_tok = 0, ms_sites = 0, ms_decode = 0, ms_inflate = 0;
     uint64_t compressed_bytes = 0;      // BGZF bytes shipped over PCIe when the file was inflated on the GPU
+    // region query through a .tbi / .csi (hb_parse_index_info): used, compressed bytes read, merged chunks of the query
+    int idx_used = 0;
+    uint64_t idx_bytes_read = 0, idx_chunks = 0;
     // chrom runs (host)
     std::vector<uint64_t> run_rows;
     std::vector<std::string> run_names;

@@ -135,5 +135,7 @@ PYBIND11_MODULE(parse_vcf, m) {
     m.def("cache_clear", &hb_cache_clear, "Drop the device-resident per-(file, region) parse cache");
     m.def("set_bgzf_crc_check", [](bool on) { hb_set_bgzf_crc_check(on ? 1 : 0); }, py::arg("on"),
           "Check the CRC32 of every BGZF member against its trailer, as htslib does (process-wide, off by default)");
+    m.def("set_use_index", [](bool on) { hb_set_use_index(on ? 1 : 0); }, py::arg("on"),
+          "Answer region queries through <file>.tbi / <file>.csi when one is there (process-wide, on by default)");
     m.def("last_error", []() { return std::string(hb_last_error()); });
 }

@@ -267,6 +267,34 @@ void hb_set_host_threads(int n);
  * zlib, which always checks the CRC.  hb_load_vcf keeps parses made with the check on apart from those made with it off. */
 void hb_set_bgzf_crc_check(int on);
 int hb_get_bgzf_crc_check(void);
+/* Region queries through a tabix or CSI index (process-wide, on by default).  When the region is not empty and the input
+ * is BGZF, hb_parse_file, hb_load_vcf and hb_load_vcf_without_sample look for <path>.tbi, then <path>.csi (a .bcf:
+ * <path>.csi only) and read and inflate only the BGZF members between the first and the last chunk the index lists for
+ * the region; the GPU region filter still decides which records are kept, so the rows are those of a full scan.  The
+ * index is ignored (HB_TRACE says why) when it is older than the data file, does not read, names no sequences, or when the
+ * region's span is above the text limit: the file is then scanned whole, as with the setting off.  A contig the index
+ * does not know gives a parse with no records. */
+void hb_set_use_index(int on);
+int hb_get_use_index(void);
+/* hb_parse_vcf_bytes with the bytes of the data file's index (.tbi / .csi, as on disk) next to them; index_n == 0 or
+ * hb_set_use_index(0): what hb_parse_vcf_bytes does */
+int hb_parse_vcf_bytes_indexed(const uint8_t *data, uint64_t nbytes, const uint8_t *index, uint64_t index_n, const char *region,
+                               int want_gt, int device, hb_parse **out);
+/* whether the parse went through an index (used 1) or scanned the whole input (0); the compressed bytes it read from the
+ * data (header members + the span) and the merged chunks of the query.  Any output pointer may be NULL. */
+int hb_parse_index_info(const hb_parse *p, int *used, uint64_t *compressed_bytes_read, uint64_t *n_chunks);
+/* Build the index of BGZF bytes on the GPU (kernel 7): what `tabix -p vcf` (HB_INDEX_TBI), `tabix -C -m min_shift -p vcf`
+ * (HB_INDEX_CSI) or, for a BGZF .bcf, `bcftools index -m min_shift` (CSI only) writes, BGZF-compressed into out[0, *len).
+ * min_shift is used by CSI only (TBI is 14 with 5 levels).  out == NULL: *len is set only; a cap below it fails with
+ * HB_ERR_ARG and sets *len.  Plain gzip or uncompressed input, TBI for a BCF, and text above the text limit
+ * (hb_parse_set_text_limit) fail with HB_ERR_ARG; records out of order ("unsorted positions"), a contig in two blocks
+ * ("chromosome blocks not continuous") and a position TBI cannot hold fail with HB_ERR_FORMAT, as tabix does. */
+#define HB_INDEX_TBI 0
+#define HB_INDEX_CSI 1
+int hb_index_bgzf(const uint8_t *data, uint64_t nbytes, int fmt, int min_shift, int device, uint8_t *out, uint64_t cap,
+                  uint64_t *len);
+/* the index of a file, written to out_path (NULL: <path>.tbi or <path>.csi) */
+int hb_index_file(const char *path, int fmt, int min_shift, int device, const char *out_path);
 /* bytes the last hb_frames_fetch_packed of this handle moved device -> host (frames or tails + headers + templates, + sizes) */
 uint64_t hb_frames_last_d2h_bytes(const hb_frames *f);
 /* sizes[n_chunks] of one sample's frames; then the frames themselves, concatenated without padding */
