@@ -76,7 +76,8 @@ EXPORTS = [
     "hb_parse_fetch_sites", "hb_parse_fetch_sample", "hb_parse_fetch_matrix", "hb_parse_fetch_sample_errors",
     "hb_parse_chrom_runs", "hb_parse_free",
     "hb_bgzf_inflate", "hb_bgzf_compress_host",
-    "hb_compress_records", "hb_compress_sample_range", "hb_frames_set_window", "hb_parse_release_text", "hb_parse_attach_frames", "hb_frames_rerun", "hb_frames_get_info", "hb_frames_layout", "hb_frames_fetch_all", "hb_frames_fetch_packed", "hb_set_fetch_mode", "hb_set_bgzf_crc_check", "hb_get_bgzf_crc_check", "hb_set_use_index", "hb_get_use_index", "hb_parse_vcf_bytes_indexed", "hb_parse_index_info", "hb_index_bgzf", "hb_index_file", "hb_set_host_threads", "hb_frames_last_d2h_bytes",
+    "hb_compress_records", "hb_compress_sample_range", "hb_frames_set_window", "hb_parse_release_text", "hb_parse_attach_frames", "hb_frames_rerun", "hb_frames_get_info", "hb_frames_layout", "hb_frames_fetch_all", "hb_frames_fetch_packed", "hb_set_fetch_mode", "hb_set_bgzf_crc_check", "hb_get_bgzf_crc_check", "hb_set_use_index", "hb_get_use_index", "hb_parse_vcf_bytes_indexed", "hb_parse_index_info",
+    "hb_parse_host_text_subset", "hb_parse_device_text_subset", "hb_parse_file_subset", "hb_parse_vcf_bytes_subset", "hb_file_samples", "hb_index_bgzf", "hb_index_file", "hb_set_host_threads", "hb_frames_last_d2h_bytes",
     "hb_frames_fetch_sample", "hb_frames_free",
     "hb_guess_chunk_records", "hb_set_site_matcher", "hb_decode_frames", "hb_decode_columns_device", "hb_decode_columns_device_large",
     "hb_encode_haplotypes",
@@ -114,6 +115,14 @@ def lib():
         L.hb_get_use_index.restype = C.c_int
         L.hb_parse_vcf_bytes_indexed.argtypes = [C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint64, C.c_char_p, C.c_int, C.c_int,
                                                  C.POINTER(C.c_void_p)]
+        L.hb_parse_host_text_subset.argtypes = [C.c_void_p, C.c_uint64, C.POINTER(ParseOpts), C.c_void_p, C.c_uint32,
+                                                C.POINTER(C.c_void_p)]
+        L.hb_parse_device_text_subset.argtypes = [C.c_void_p, C.c_uint64, C.POINTER(ParseOpts), C.c_void_p, C.c_uint32,
+                                                  C.POINTER(C.c_void_p)]
+        L.hb_parse_file_subset.argtypes = [C.c_char_p, C.c_char_p, C.c_void_p, C.c_uint32, C.c_int, C.POINTER(C.c_void_p)]
+        L.hb_parse_vcf_bytes_subset.argtypes = [C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint64, C.c_char_p, C.c_void_p, C.c_uint32,
+                                                C.c_int, C.POINTER(C.c_void_p)]
+        L.hb_file_samples.argtypes = [C.c_char_p, C.POINTER(C.c_uint32), C.c_void_p, C.c_uint64, C.POINTER(C.c_uint64)]
         L.hb_parse_index_info.argtypes = [C.c_void_p, C.POINTER(C.c_int), C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]
         L.hb_index_bgzf.argtypes = [C.c_void_p, C.c_uint64, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_uint64, C.POINTER(C.c_uint64)]
         L.hb_index_file.argtypes = [C.c_char_p, C.c_int, C.c_int, C.c_int, C.c_char_p]
@@ -191,6 +200,26 @@ def kernel_launches() -> int:
     return int(lib().hb_kernel_launches())
 
 
+def _columns(samples) -> np.ndarray:
+    """Column indices of a text-level sample subset as the C ABI takes them (the library checks them)."""
+    return np.ascontiguousarray(np.asarray(list(samples), dtype=np.int64).astype(np.uint32))
+
+
+def _names(samples):
+    """(encoded names, const char *[] over them) of a file-level sample subset."""
+    names = [s.encode() if isinstance(s, str) else bytes(s) for s in samples]
+    return names, (C.c_char_p * max(1, len(names)))(*names)
+
+
+def file_sample_names(path: str):
+    """The header's sample names of a .vcf / .vcf.gz / .bcf, read from its leading bytes only (hb_file_samples; host only)."""
+    n, ln = C.c_uint32(), C.c_uint64()
+    check(lib().hb_file_samples(path.encode(), C.byref(n), None, 0, C.byref(ln)))
+    buf = C.create_string_buffer(max(1, ln.value))
+    check(lib().hb_file_samples(path.encode(), C.byref(n), buf, ln.value, C.byref(ln)))
+    return [x.decode() for x in buf.raw[:ln.value].split(b"\0")[:n.value]]
+
+
 # ------------------------------------------------------------------------------------------------
 class Parse:
     """Device-resident parse of decompressed VCF body text (section B of the C ABI)."""
@@ -212,8 +241,9 @@ class Parse:
 
     @classmethod
     def from_host(cls, text, n_samples, region="", end_is_int=False, want_gt=True, device=0, tokenizer=0,
-                  stream=None, nbytes=None):
-        """text: bytes / numpy uint8 array / raw host address (with nbytes)."""
+                  stream=None, nbytes=None, samples=None):
+        """text: bytes / numpy uint8 array / raw host address (with nbytes).  samples: column indices of a sample subset
+        (ascending, distinct; hb_parse_host_text_subset), None = every sample."""
         if isinstance(text, (bytes, bytearray)):
             keep = np.frombuffer(text, np.uint8)
             addr, n = keep.ctypes.data, keep.size
@@ -223,28 +253,44 @@ class Parse:
             addr, n, keep = int(text), int(nbytes), None
         h = C.c_void_p()
         o = cls._opts(n_samples, region, end_is_int, want_gt, device, tokenizer, stream)
-        check(lib().hb_parse_host_text(addr, n, C.byref(o), C.byref(h)))
+        if samples is None:
+            check(lib().hb_parse_host_text(addr, n, C.byref(o), C.byref(h)))
+        else:
+            cols = _columns(samples)
+            check(lib().hb_parse_host_text_subset(addr, n, C.byref(o), cols.ctypes.data, cols.size, C.byref(h)))
         del keep
         return cls(h)
 
     @classmethod
     def from_device(cls, d_ptr: int, nbytes: int, n_samples, region="", end_is_int=False, want_gt=True, device=0,
-                    tokenizer=0, stream=None):
+                    tokenizer=0, stream=None, samples=None):
+        """samples: column indices of a sample subset (hb_parse_device_text_subset), None = every sample."""
         h = C.c_void_p()
         o = cls._opts(n_samples, region, end_is_int, want_gt, device, tokenizer, stream)
-        check(lib().hb_parse_device_text(d_ptr, nbytes, C.byref(o), C.byref(h)))
+        if samples is None:
+            check(lib().hb_parse_device_text(d_ptr, nbytes, C.byref(o), C.byref(h)))
+        else:
+            cols = _columns(samples)
+            check(lib().hb_parse_device_text_subset(d_ptr, nbytes, C.byref(o), cols.ctypes.data, cols.size, C.byref(h)))
         return cls(h)
 
     @classmethod
-    def from_file(cls, path: str, region="", want_gt=True, device=0):
+    def from_file(cls, path: str, region="", want_gt=True, device=0, samples=None):
+        """samples: names of a sample subset, in any order (hb_parse_file_subset; the planes come in header order), None =
+        every sample."""
         h = C.c_void_p()
-        check(lib().hb_parse_file(path.encode(), (region or "").encode(), int(want_gt), device, C.byref(h)))
+        if samples is None:
+            check(lib().hb_parse_file(path.encode(), (region or "").encode(), int(want_gt), device, C.byref(h)))
+        else:
+            names, arr = _names(samples)
+            check(lib().hb_parse_file_subset(path.encode(), (region or "").encode(), arr, len(names), device, C.byref(h)))
         return cls(h)
 
     @classmethod
-    def from_vcf_bytes(cls, data, region="", want_gt=True, device=0, nbytes=None, index=None):
+    def from_vcf_bytes(cls, data, region="", want_gt=True, device=0, nbytes=None, index=None, samples=None):
         """The bytes of a .vcf / .vcf.gz / .bcf in host memory (bytes, uint8 array, or address + nbytes).  index: the bytes
-        of its .tbi / .csi; a region query then inflates only the BGZF members the index lists for the region."""
+        of its .tbi / .csi; a region query then inflates only the BGZF members the index lists for the region.  samples:
+        names of a sample subset, as for from_file."""
         if isinstance(data, (bytes, bytearray)):
             keep = np.frombuffer(data, np.uint8); addr, n = keep.ctypes.data, keep.size
         elif isinstance(data, np.ndarray):
@@ -252,10 +298,14 @@ class Parse:
         else:
             keep = None; addr, n = int(data), int(nbytes)
         h = C.c_void_p()
-        if index is None:
+        ix = None if index is None else np.frombuffer(bytes(index), np.uint8)
+        if samples is not None:
+            names, arr = _names(samples)
+            check(lib().hb_parse_vcf_bytes_subset(addr, n, None if ix is None else ix.ctypes.data, 0 if ix is None else ix.size,
+                                                  (region or "").encode(), arr, len(names), device, C.byref(h)))
+        elif ix is None:
             check(lib().hb_parse_vcf_bytes(addr, n, (region or "").encode(), int(want_gt), device, C.byref(h)))
         else:
-            ix = np.frombuffer(bytes(index), np.uint8)
             check(lib().hb_parse_vcf_bytes_indexed(addr, n, ix.ctypes.data, ix.size, (region or "").encode(), int(want_gt),
                                                    device, C.byref(h)))
         del keep

@@ -356,6 +356,7 @@ void hb_parse_free(hb_parse *p) {
     free_dev(p->d_badgt); free_dev(p->d_run_rows);
     free_dev(p->d_wstart); free_dev(p->d_wrow); free_dev(p->d_verify); free_dev(p->d_wcount);
     free_rows(p->walk_pad);
+    free_dev(p->d_sel_mask); free_dev(p->d_sel_base);
     if (hb_parse::Bcf *b = p->bcf) {
         free_dev(b->d_contigs); free_dev(b->d_names); free_dev(b->d_rec_off); free_dev(b->d_blk_count); free_dev(b->d_blk_base);
         free_dev(b->seg.start); free_dev(b->seg.exit); free_dev(b->seg.bad); free_dev(b->seg.base); free_dev(b->seg.count);
@@ -509,7 +510,7 @@ static int index_by_tokenizer(hb_parse *p, const Launch &L) {
         TRY(dev_alloc(&p->d_nu_rows, cap));
         TRY(dev_alloc(&p->d_sites_state, (cap + 255) / 256 + 1));
     }
-    launch_sites(p->d_text, li, n_lines, p->n_samples, p->rg, p->end_is_int, p->want_gt, p->with_tabs, r, p->d_nu_rows,
+    launch_sites(p->d_text, li, n_lines, p->n_cols, p->rg, p->end_is_int, p->want_gt, p->with_tabs, r, p->d_nu_rows,
                  p->d_sites_state, p->d_st, L);
     CU(cudaEventRecord(p->ev[2], p->stream));
     TRY(fetch_status(p));
@@ -536,7 +537,7 @@ static int index_by_walker(hb_parse *p, const Launch &L) {
         TRY(grow(p->d_verify, p->verify_cap, cap));
     }
     CU(cudaEventRecord(p->ev[0], p->stream));
-    launch_walk(p->d_text, p->nbytes, p->n_samples, p->walk_range, p->n_walkers, p->rg, p->end_is_int, p->d_wstart, p->d_wcount,
+    launch_walk(p->d_text, p->nbytes, p->n_cols, p->walk_range, p->n_walkers, p->rg, p->end_is_int, p->d_wstart, p->d_wcount,
                 p->d_wrow, p->walk_pad, p->d_verify, p->verify_cap, p->d_st, L);
     CU(cudaEventRecord(p->ev[1], p->stream));
     TRY(fetch_status(p));
@@ -552,7 +553,7 @@ static int index_by_walker(hb_parse *p, const Launch &L) {
         free_dev(p->d_sites_state);
         p->d_sites_state = nullptr;
     }
-    launch_walk_compact(p->d_text, p->nbytes, p->n_samples, p->n_walkers, p->d_wcount, p->d_wrow, p->walk_pad, r, p->d_nu_rows,
+    launch_walk_compact(p->d_text, p->nbytes, p->n_cols, p->n_walkers, p->d_wcount, p->d_wrow, p->walk_pad, r, p->d_nu_rows,
                         p->d_verify, p->verify_cap, p->d_st, L);
     CU(cudaEventRecord(p->ev[2], p->stream));
     p->index_used = 3;
@@ -592,7 +593,7 @@ static int index_bcf(hb_parse *p, const Launch &L) {
         sg.cap = sg.n;
     }
     CU(cudaEventRecord(p->ev[0], p->stream));
-    launch_bcf_chain(p->d_text, p->nbytes, p->n_samples, nc, sg, true, L);
+    launch_bcf_chain(p->d_text, p->nbytes, p->n_cols, nc, sg, true, L);
     for (;;) {                                   // until every segment's start is the exit of the segment before it
         CU(cudaMemsetAsync(&p->d_st->bcf_fail, 0xff, 8, p->stream));
         CU(cudaMemsetAsync(&p->d_st->bcf_records, 0, 8, p->stream));
@@ -604,9 +605,9 @@ static int index_bcf(hb_parse *p, const Launch &L) {
         if (f & 1) {                             // a proven chain met a record that fails the header test
             uint64_t bad = 0;
             CU(cudaMemcpy(&bad, sg.bad + (f >> 1), 8, cudaMemcpyDeviceToHost));
-            return bcf_malformed(bad, p->n_samples, nc);
+            return bcf_malformed(bad, p->n_cols, nc);
         }
-        launch_bcf_chain(p->d_text, p->nbytes, p->n_samples, nc, sg, false, L);
+        launch_bcf_chain(p->d_text, p->nbytes, p->n_cols, nc, sg, false, L);
     }
     const uint64_t n_all = p->h_st.bcf_records;
     p->n_lines = n_all;
@@ -621,7 +622,7 @@ static int index_bcf(hb_parse *p, const Launch &L) {
         b.blk_cap = blocks;
     }
     BcfSiteArgs a;
-    a.text = p->d_text; a.rec_off = b.d_rec_off; a.n_rec = n_all; a.n_samples = p->n_samples; a.n_contigs = nc;
+    a.text = p->d_text; a.rec_off = b.d_rec_off; a.n_rec = n_all; a.n_samples = p->n_cols; a.n_contigs = nc;
     a.contigs = b.d_contigs; a.gt_key = b.gt_key;
     a.rid = -1;
     if (p->rg.has_region) {
@@ -687,23 +688,23 @@ static int run_parse(hb_parse *p) {
     if (!p->d_st) TRY(dev_alloc(&p->d_st, 1));
     CU(cudaMemsetAsync(p->d_st, 0, sizeof(DevStatus), p->stream));
     memset(&p->h_st, 0, sizeof p->h_st);
-    p->ncp = (p->n_samples + kCP - 1) / kCP;
+    p->ncp = (p->n_cols + kCP - 1) / kCP;
     if (p->nbytes == 0) return HB_OK;
 
     // ---- how to locate the records, from the first one
     if (!p->probed && !p->bcf) {
         // the whole first record: 4 bytes per sample when it is GT-only (800 KB at 200,000 samples) + its head
-        std::vector<uint8_t> head((size_t)std::min<uint64_t>(4ull * p->n_samples + 65536, p->nbytes));
+        std::vector<uint8_t> head((size_t)std::min<uint64_t>(4ull * p->n_cols + 65536, p->nbytes));
         const size_t hn = head.size();
         CU(cudaMemcpyAsync(head.data(), p->d_text, hn, cudaMemcpyDeviceToHost, p->stream));
         CU(cudaStreamSynchronize(p->stream));
         bool gt_only, uniform; uint64_t l0;
-        probe_head(head.data(), hn, p->n_samples, gt_only, uniform, l0);
+        probe_head(head.data(), hn, p->n_cols, gt_only, uniform, l0);
         p->with_tabs = p->tokenizer == 2 || ((p->tokenizer == 0 || p->tokenizer == 3) && !gt_only);
         if (!p->want_gt) p->with_tabs = false;
         // walking pays when a record is much longer than its head (and needs the decoder to validate the jumps)
-        p->use_walker = p->want_gt && p->n_samples > 0 &&
-                        (p->tokenizer == 3 || (p->tokenizer == 0 && uniform && p->n_samples >= 256));
+        p->use_walker = p->want_gt && p->n_cols > 0 &&
+                        (p->tokenizer == 3 || (p->tokenizer == 0 && uniform && p->n_cols >= 256));
         p->first_line_len = l0 ? l0 : hn;
         p->probed = true;
     }
@@ -747,12 +748,14 @@ static int run_parse(hb_parse *p) {
         }
         // walker: the count pass told the host how many kept records are not plain "\tX|Y" columns
         if (p->index_used == 3 && p->h_st.n_nu_count) TRY(index_nonuniform(p, p->h_st.n_nu_count, L));
+        // the decoders run over the file's columns; a subset picks which of them are decoded and into which planes
+        const SampleSel sel{p->d_sel_mask, p->d_sel_base};
         if (p->bcf)
-            launch_bcf_decode(p->d_text, p->rows.rowinfo, n_rec, p->n_samples, p->d_gt[0], p->d_gt[1], p->gt_stride, p->d_bits,
-                              p->bits_stride, p->d_ploidy, p->d_badgt, p->d_st, L);
+            launch_bcf_decode(p->d_text, p->rows.rowinfo, n_rec, p->n_cols, p->d_gt[0], p->d_gt[1], p->gt_stride, p->d_bits,
+                              p->bits_stride, p->d_ploidy, p->d_badgt, p->d_st, sel, L);
         else
-            launch_decode_gt(p->d_text, p->rows.rowinfo, n_rec, p->n_samples, p->d_cp, p->ncp, p->d_gt[0], p->d_gt[1],
-                             p->gt_stride, p->d_bits, p->bits_stride, p->d_ploidy, p->d_badgt, p->d_st, L);
+            launch_decode_gt(p->d_text, p->rows.rowinfo, n_rec, p->n_cols, p->d_cp, p->ncp, p->d_gt[0], p->d_gt[1],
+                             p->gt_stride, p->d_bits, p->bits_stride, p->d_ploidy, p->d_badgt, p->d_st, sel, L);
     }
     CU(cudaEventRecord(p->ev[3], p->stream));
     // frames attached to this parse: their kernel is queued right behind the decoder now (the host waits for the templates
@@ -794,13 +797,46 @@ static ParsePtr new_parse(const hb_parse_opts *o, int &rc) {
     p->device = o->device;
     p->stream = (cudaStream_t)o->stream;
     cudaDeviceGetAttribute(&p->sm_count, cudaDevAttrMultiProcessorCount, o->device);
-    p->n_samples = o->n_samples;
+    p->n_cols = p->n_samples = o->n_samples;
     parse_region(o->region, p->rg);
     p->end_is_int = o->end_is_int;
     p->want_gt = o->want_gt;
     p->tokenizer = o->tokenizer;
     for (auto &e : p->ev) cudaEventCreate(&e);
     return p;
+}
+
+// ---- sample subsets (hb_parse_*_subset)
+// cols[0..n) of records with n_cols sample columns: at least one, ascending, each once, all in range
+static int check_cols(const uint32_t *cols, uint32_t n, uint32_t n_cols) {
+    if (!cols || n == 0) return fail(HB_ERR_ARG, "a sample subset names at least one column");
+    for (uint32_t i = 0; i < n; ++i) {
+        if (cols[i] >= n_cols)
+            return fail(HB_ERR_ARG, "sample column " + std::to_string(cols[i]) + " is out of range (" + std::to_string(n_cols) + " samples)");
+        if (i && cols[i] <= cols[i - 1]) return fail(HB_ERR_ARG, "sample columns must be ascending and distinct");
+    }
+    return HB_OK;
+}
+
+// The subset cols (checked; empty = every sample) on a handle that has not run yet: its planes are cols.size() wide, plane j
+// is column cols[j].  A subset of every column is the ordinary parse and changes nothing.
+static int set_subset(hb_parse *p, const std::vector<uint32_t> &cols) {
+    if (cols.empty() || cols.size() == p->n_cols) return HB_OK;
+    const uint32_t nb = (p->n_cols + kTS - 1) / kTS;
+    std::vector<uint32_t> mask(4ull * nb, 0), base(nb, 0);          // mask: 4 words per block, word c / 32 holds column c
+    for (uint32_t c : cols) mask[c / 32] |= 1u << (c % 32);
+    for (uint32_t b = 1; b < nb; ++b) {
+        uint32_t in_block = 0;
+        for (int q = 0; q < 4; ++q) in_block += (uint32_t)__builtin_popcount(mask[4 * (b - 1) + q]);
+        base[b] = base[b - 1] + in_block;
+    }
+    TRY(dev_alloc(&p->d_sel_mask, nb));
+    TRY(dev_alloc(&p->d_sel_base, nb));
+    CU(cudaMemcpy(p->d_sel_mask, mask.data(), 16ull * nb, cudaMemcpyHostToDevice));
+    CU(cudaMemcpy(p->d_sel_base, base.data(), 4ull * nb, cudaMemcpyHostToDevice));
+    p->sel_cols = cols;
+    p->n_samples = (uint32_t)cols.size();
+    return HB_OK;
 }
 
 // zero bytes behind the text of every parse: kernels that read it in whole 16-byte words find zeros past its end
@@ -819,11 +855,14 @@ static int upload_text(hb_parse *p, const uint8_t *text, uint64_t n, bool add_ne
     return HB_OK;
 }
 
-int hb_parse_device_text(const uint8_t *d_text, uint64_t nbytes, const hb_parse_opts *opts, hb_parse **out) {
+// cols: the sample subset (empty = every sample)
+static int device_text(const uint8_t *d_text, uint64_t nbytes, const hb_parse_opts *opts, const std::vector<uint32_t> &cols,
+                       hb_parse **out) {
     int rc;
     ParsePtr p = new_parse(opts, rc);
     if (!p) return rc;
     if (((uintptr_t)d_text & 15) != 0) return fail(HB_ERR_ARG, "d_text must be 16-byte aligned");
+    TRY(set_subset(p.get(), cols));
     p->d_text = d_text;
     p->nbytes = nbytes;
     TRY(run_parse(p.get()));
@@ -831,14 +870,40 @@ int hb_parse_device_text(const uint8_t *d_text, uint64_t nbytes, const hb_parse_
     return HB_OK;
 }
 
-int hb_parse_host_text(const uint8_t *text, uint64_t nbytes, const hb_parse_opts *opts, hb_parse **out) {
+static int host_text(const uint8_t *text, uint64_t nbytes, const hb_parse_opts *opts, const std::vector<uint32_t> &cols,
+                     hb_parse **out) {
     int rc;
     ParsePtr p = new_parse(opts, rc);
     if (!p) return rc;
+    TRY(set_subset(p.get(), cols));
     TRY(upload_text(p.get(), text, nbytes, nbytes && text[nbytes - 1] != '\n'));
     TRY(run_parse(p.get()));
     *out = p.release();
     return HB_OK;
+}
+
+int hb_parse_device_text(const uint8_t *d_text, uint64_t nbytes, const hb_parse_opts *opts, hb_parse **out) {
+    return device_text(d_text, nbytes, opts, {}, out);
+}
+
+int hb_parse_host_text(const uint8_t *text, uint64_t nbytes, const hb_parse_opts *opts, hb_parse **out) {
+    return host_text(text, nbytes, opts, {}, out);
+}
+
+int hb_parse_device_text_subset(const uint8_t *d_text, uint64_t nbytes, const hb_parse_opts *opts, const uint32_t *cols,
+                                uint32_t n_cols, hb_parse **out) {
+    TRY(ensure_device(opts ? opts->device : 0));
+    if (!opts) return fail(HB_ERR_ARG, "null argument");
+    TRY(check_cols(cols, n_cols, opts->n_samples));
+    return device_text(d_text, nbytes, opts, std::vector<uint32_t>(cols, cols + n_cols), out);
+}
+
+int hb_parse_host_text_subset(const uint8_t *text, uint64_t nbytes, const hb_parse_opts *opts, const uint32_t *cols,
+                              uint32_t n_cols, hb_parse **out) {
+    TRY(ensure_device(opts ? opts->device : 0));
+    if (!opts) return fail(HB_ERR_ARG, "null argument");
+    TRY(check_cols(cols, n_cols, opts->n_samples));
+    return host_text(text, nbytes, opts, std::vector<uint32_t>(cols, cols + n_cols), out);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -868,6 +933,7 @@ struct StreamSlots {
     size_t n_slots = 0;
     int device = -1, want_gt = 0, end_is_int = 0, tokenizer = 0;
     uint32_t n_samples = 0;
+    std::vector<uint32_t> cols;                   // the slot parses' sample subset (empty = every sample)
     std::string region;
     uint64_t text_cap = 0, comp_cap = 0, carry_cap = 0;
     uint32_t n_cap = 0;
@@ -887,19 +953,19 @@ struct StreamSlots {
         }
         n_slots = 0;
     }
-    bool same_options(const hb_parse_opts &o) const {
+    bool same_options(const hb_parse_opts &o, const std::vector<uint32_t> &c) const {
         return device == o.device && n_samples == o.n_samples && want_gt == (o.want_gt ? 1 : 0) && end_is_int == (o.end_is_int ? 1 : 0) &&
-               tokenizer == o.tokenizer && region == (o.region ? o.region : "");
+               tokenizer == o.tokenizer && region == (o.region ? o.region : "") && cols == c;
     }
 };
 struct SlotCache { std::mutex mu; StreamSlots *kept = nullptr; bool in_use = false; };
 SlotCache g_text_slots, g_bgzf_slots;
 
-// the cached slots when they were made with these options and are free, else fresh (empty) ones
-StreamSlots *acquire_slots(SlotCache &c, const hb_parse_opts &o, size_t n_slots) {
+// the cached slots when they were made with these options and sample subset and are free, else fresh (empty) ones
+StreamSlots *acquire_slots(SlotCache &c, const hb_parse_opts &o, const std::vector<uint32_t> &cols, size_t n_slots) {
     std::lock_guard<std::mutex> lk(c.mu);
     if (c.kept && !c.in_use) {
-        if (c.kept->same_options(o) && c.kept->n_slots >= n_slots) { c.in_use = true; return c.kept; }
+        if (c.kept->same_options(o, cols) && c.kept->n_slots >= n_slots) { c.in_use = true; return c.kept; }
         c.kept->destroy();
         delete c.kept;
         c.kept = nullptr;
@@ -907,6 +973,7 @@ StreamSlots *acquire_slots(SlotCache &c, const hb_parse_opts &o, size_t n_slots)
     StreamSlots *ss = new StreamSlots();
     ss->device = o.device; ss->n_samples = o.n_samples; ss->want_gt = o.want_gt ? 1 : 0; ss->end_is_int = o.end_is_int ? 1 : 0;
     ss->tokenizer = o.tokenizer; ss->region = o.region ? o.region : "";
+    ss->cols = cols;
     return ss;
 }
 void release_slots(SlotCache &c, StreamSlots *ss, bool keep) {
@@ -928,10 +995,11 @@ void clear_slot_cache(SlotCache &c) {
 
 // the slots of one streaming call from cache c: streams, event and parse are made for a slot that has none, and the buffers of
 // every slot grow together when a capacity is short (the carry offset is part of the layout).  text_cap: text of one slab;
-// carry_cap, comp_cap, n_cap: BGZF only -- host text (all 0) has no inflate scratch and no pinned tables.
-int open_slots(SlotCache &c, const hb_parse_opts &opts, size_t n_slots, uint64_t text_cap, uint64_t carry_cap, uint64_t comp_cap,
-               uint32_t n_cap, StreamSlots **out) {
-    StreamSlots *ss = acquire_slots(c, opts, n_slots);
+// carry_cap, comp_cap, n_cap: BGZF only -- host text (all 0) has no inflate scratch and no pinned tables.  cols: the sample
+// subset of the slot parses (empty = every sample).
+int open_slots(SlotCache &c, const hb_parse_opts &opts, const std::vector<uint32_t> &cols, size_t n_slots, uint64_t text_cap,
+               uint64_t carry_cap, uint64_t comp_cap, uint32_t n_cap, StreamSlots **out) {
+    StreamSlots *ss = acquire_slots(c, opts, cols, n_slots);
     int rc = HB_OK;
     for (size_t i = ss->n_slots; i < n_slots && rc == HB_OK; ++i) {
         StreamSlot &s = ss->slot[i];
@@ -941,6 +1009,7 @@ int open_slots(SlotCache &c, const hb_parse_opts &opts, size_t n_slots, uint64_t
         hb_parse_opts o = opts;
         o.stream = s.compute;
         s.p = new_parse(&o, rc).release();
+        if (rc == HB_OK) rc = set_subset(s.p, cols);
         if (rc == HB_OK) ss->n_slots = i + 1;
     }
     const bool grow = ss->text_cap < text_cap || ss->carry_cap < carry_cap || ss->comp_cap < comp_cap || ss->n_cap < n_cap;
@@ -1077,7 +1146,7 @@ int hb_parse_stream_host(const uint8_t *text, uint64_t nbytes, const hb_parse_op
     TRY(ensure_device(opts->device));
     const double t_begin = now_ms();
     StreamSlots *ss = nullptr;
-    TRY(open_slots(g_text_slots, *opts, std::min<size_t>(2, slabs.size()), cap, 0, 0, 0, &ss));
+    TRY(open_slots(g_text_slots, *opts, {}, std::min<size_t>(2, slabs.size()), cap, 0, 0, 0, &ss));
     StreamSlot *slot = ss->slot;
     auto h2d = [&](size_t k) -> cudaError_t {
         StreamSlot &s = slot[k & 1];
@@ -1414,6 +1483,37 @@ int bcf_header(const uint8_t *d, uint64_t n, FileText &ft, bool &complete) {
 
 bool is_bcf(const uint8_t *d, uint64_t n) { return n >= 3 && memcmp(d, "BCF", 3) == 0; }
 
+// the sample names of hb_parse_file_subset / hb_parse_vcf_bytes_subset
+struct Subset {
+    const char *const *names;
+    uint32_t n;
+};
+
+// The columns of subset ss among the header's samples, ascending: the planes come out in header order whatever the order of
+// the names, as htslib's bcf_hdr_set_samples gives them.  samples becomes the names of the planes.  ss == nullptr: every
+// sample, cols stays empty.
+int resolve_subset(const Subset *ss, std::vector<std::string> &samples, std::vector<uint32_t> &cols) {
+    cols.clear();
+    if (!ss) return HB_OK;
+    if (!ss->names || ss->n == 0) return fail(HB_ERR_ARG, "a sample subset names at least one sample");
+    std::map<std::string, uint32_t> at;
+    for (uint32_t i = 0; i < samples.size(); ++i) at.emplace(samples[i], i);
+    std::vector<uint8_t> taken(samples.size(), 0);
+    for (uint32_t k = 0; k < ss->n; ++k) {
+        if (!ss->names[k]) return fail(HB_ERR_ARG, "null sample name");
+        const auto it = at.find(ss->names[k]);
+        if (it == at.end()) return fail(HB_ERR_SAMPLE, std::string("sample ") + ss->names[k] + " is not in the VCF header");
+        if (taken[it->second]) return fail(HB_ERR_ARG, std::string("sample ") + ss->names[k] + " is named twice");
+        taken[it->second] = 1;
+        cols.push_back(it->second);
+    }
+    std::sort(cols.begin(), cols.end());
+    std::vector<std::string> picked;
+    for (uint32_t c : cols) picked.push_back(samples[c]);
+    samples.swap(picked);
+    return HB_OK;
+}
+
 int read_vcf(const std::vector<uint8_t> &raw, FileText &ft) {
     TRY(inflate_all(raw, ft.data));
     if (is_bcf(ft.data.data(), ft.data.size())) {
@@ -1430,21 +1530,26 @@ int read_vcf(const std::vector<uint8_t> &raw, FileText &ft) {
 // reads) travel over PCIe COMPRESSED and are inflated on the GPU (hb_inflate.cu) straight into the text buffer;
 // only the header members are also inflated on the host, to learn the sample names.  Any other gzip input (plain
 // gzip, or BGZF that bgzip would not have written) and plain text go through zlib / as they are.
+// hb_parse_stream_bgzf_resident with the sample subset cols (empty = every sample)
+int stream_resident(const uint8_t *bgzf, uint64_t nbytes, const char *region, int want_gt, int device, uint64_t slab_bytes,
+                    hb_parse **out, uint32_t *n_slabs, const std::vector<uint32_t> &cols);
+
+// ss: a sample subset (nullptr = every sample); samples: the names of the parse's planes
 int parse_bytes_common(std::vector<uint8_t> &raw_owned, const uint8_t *raw_p, uint64_t raw_n, const char *region, bool want_gt,
-                       int device, hb_parse **out, std::vector<std::string> &samples);
+                       int device, hb_parse **out, std::vector<std::string> &samples, const Subset *ss);
 
 // a region query of a file with a usable .tbi / .csi next to it: HB_OK with used = false when the index is not usable
 int parse_file_indexed(const char *path, const char *region, bool want_gt, int device, hb_parse **out,
-                       std::vector<std::string> &samples, bool &used);
+                       std::vector<std::string> &samples, bool &used, const Subset *ss);
 
 int parse_file_common(const char *path, const char *region, bool want_gt, int device, hb_parse **out,
-                      std::vector<std::string> &samples) {
+                      std::vector<std::string> &samples, const Subset *ss = nullptr) {
     bool used = false;
-    TRY(parse_file_indexed(path, region, want_gt, device, out, samples, used));
+    TRY(parse_file_indexed(path, region, want_gt, device, out, samples, used, ss));
     if (used) return HB_OK;
     std::vector<uint8_t> raw;
     TRY(read_all(path, raw));
-    return parse_bytes_common(raw, raw.data(), raw.size(), region, want_gt, device, out, samples);
+    return parse_bytes_common(raw, raw.data(), raw.size(), region, want_gt, device, out, samples, ss);
 }
 
 // a BGZF file: its member table, then its header
@@ -1534,7 +1639,7 @@ int bcf_too_big(uint64_t body) {
 }
 
 // the body of an uncompressed or plain-gzip BCF, inflated on the host
-int parse_bcf_host(const FileText &ft, const hb_parse_opts &o, hb_parse **out) {
+int parse_bcf_host(const FileText &ft, const hb_parse_opts &o, const std::vector<uint32_t> &cols, hb_parse **out) {
     const uint64_t n = ft.data.size() - ft.body;
     uint64_t slab;
     TRY(ensure_device(o.device));
@@ -1542,6 +1647,7 @@ int parse_bcf_host(const FileText &ft, const hb_parse_opts &o, hb_parse **out) {
     int rc;
     ParsePtr p = new_parse(&o, rc);
     if (!p) return rc;
+    TRY(set_subset(p.get(), cols));
     TRY(upload_text(p.get(), ft.data.data() + ft.body, n, false));
     TRY(bcf_attach(p.get(), ft));
     TRY(run_parse(p.get()));
@@ -1563,8 +1669,9 @@ hb_parse_opts opts_for(const FileText &ft, const char *region, bool want_gt, int
 // raw_p[0..raw_n): the bytes of a .vcf / .vcf.gz / .bcf; raw_owned: the vector that holds them when the caller read a file
 // (released early on the zlib path), empty when they belong to the caller
 int parse_bytes_common(std::vector<uint8_t> &raw_owned, const uint8_t *raw_p, uint64_t raw_n, const char *region, bool want_gt,
-                       int device, hb_parse **out, std::vector<std::string> &samples) {
+                       int device, hb_parse **out, std::vector<std::string> &samples, const Subset *ss) {
     BgzfFile bz;
+    std::vector<uint32_t> cols;
     const bool gpu_inflate = raw_n >= 28 && raw_p[0] == 0x1f && raw_p[1] == 0x8b && index_bgzf(raw_p, raw_n, bz) && bz.total > 0;
     if (!gpu_inflate) {
         FileText ft;
@@ -1572,22 +1679,24 @@ int parse_bytes_common(std::vector<uint8_t> &raw_owned, const uint8_t *raw_p, ui
         TRY(read_vcf(raw_owned, ft));
         raw_owned.clear(); raw_owned.shrink_to_fit();
         samples = ft.samples;
+        TRY(resolve_subset(ss, samples, cols));
         const hb_parse_opts o = opts_for(ft, region, want_gt, device);
-        if (ft.bcf) return parse_bcf_host(ft, o, out);
-        return hb_parse_host_text(ft.data.data() + ft.body, ft.data.size() - ft.body, &o, out);
+        if (ft.bcf) return parse_bcf_host(ft, o, cols, out);
+        return host_text(ft.data.data() + ft.body, ft.data.size() - ft.body, &o, cols, out);
     }
     // ---- header: inflate leading members on the host until the #CHROM line is complete
     TRY(bgzf_header(raw_p, bz));
     const FileText &ft = bz.ft;
     const uint64_t total = bz.total;
     samples = ft.samples;
+    TRY(resolve_subset(ss, samples, cols));
     {   // a file whose text does not fit HBM next to its genotype planes passes through in slabs instead: same rows, same
         // handle minus the text (hb_parse_stream_bgzf_resident)
         TRY(ensure_device(device));
         uint64_t slab;
         const uint64_t limit = text_limit(slab);
         if (total > limit && ft.bcf) return bcf_too_big(total - ft.body);
-        if (total > limit) return hb_parse_stream_bgzf_resident(raw_p, raw_n, region, want_gt ? 1 : 0, device, slab, out, nullptr);
+        if (total > limit) return stream_resident(raw_p, raw_n, region, want_gt ? 1 : 0, device, slab, out, nullptr, cols);
     }
     const hb_parse_opts o = opts_for(ft, region, want_gt, device);
     const bool trace = getenv("HB_TRACE") != nullptr;
@@ -1595,6 +1704,7 @@ int parse_bytes_common(std::vector<uint8_t> &raw_owned, const uint8_t *raw_p, ui
     int rc;
     ParsePtr p = new_parse(&o, rc);
     if (!p) return rc;
+    TRY(set_subset(p.get(), cols));
     const uint64_t pad = (16 - ft.body % 16) % 16;         // the records must start on a 16-byte boundary
     TRY(dev_alloc(&p->d_text_owned, pad + total + 1 + kTextPad));
     const double t1 = now_ms();
@@ -1655,20 +1765,17 @@ uint64_t bgzf_member_size(const uint8_t *h, uint64_t avail) {
 // The parse of `region` from the members of src that hold the records the index lists for it.  The region filter runs
 // as on a full scan, so the rows are the same.  used = false (with `why`): the index cannot serve this query and the
 // caller takes the full-scan route; nothing has been parsed then.
-int parse_indexed(const ByteSource &src, const uint8_t *ix, uint64_t ix_n, const char *region, bool want_gt, int device,
-                  hb_parse **out, std::vector<std::string> &samples, bool &used, std::string &why) {
-    used = false;
-    std::vector<uint8_t> hbuf, sbuf;
+// The header of BGZF input, from its leading members only: twice as many bytes of them each round until the header ends
+// inside them (the rounds re-inflate what the round before inflated: at most twice the header's members in all).  false
+// (with `why`): the input is not BGZF or its header does not read.  head_read: the compressed bytes read.
+bool leading_bgzf_header(const ByteSource &src, FileText &ft, uint64_t &head_read, std::string &why) {
+    std::vector<uint8_t> hbuf;
     {
         const uint8_t *h = src.get(0, std::min<uint64_t>(src.size, 18), hbuf);
-        if (!h || !bgzf_member_size(h, std::min<uint64_t>(src.size, 18))) { why = "the input is not BGZF"; return HB_OK; }
+        if (!h || !bgzf_member_size(h, std::min<uint64_t>(src.size, 18))) { why = "the input is not BGZF"; return false; }
     }
-    TabixIndex idx;
-    if (!tabix_load(ix, ix_n, idx, why)) return HB_OK;
-    // the header: leading members, twice as many bytes of them each round until it ends inside them (the rounds
-    // re-inflate what the round before inflated: at most twice the header's members in all)
     BgzfFile bz;
-    uint64_t head_read = 0;
+    head_read = 0;
     std::vector<uint8_t> head;                              // bytes [0, head_read) of a file source
     for (bool more = true; more;) {
         const uint64_t target = std::min(src.size, std::max<uint64_t>(2 * head_read, 1));
@@ -1676,17 +1783,34 @@ int parse_indexed(const ByteSource &src, const uint8_t *ix, uint64_t ix_n, const
         const uint8_t *b = src.get(head_read, avail, hbuf);
         uint64_t w = 0;
         for (uint64_t s; b && head_read + w < target && (s = bgzf_member_size(b + w, avail - w)) != 0 && s <= avail - w;) w += s;
-        if (!w) { why = "the input is not BGZF"; return HB_OK; }
+        if (!w) { why = "the input is not BGZF"; return false; }
         if (!src.mem) head.insert(head.end(), b, b + w);
         head_read += w;
         const uint8_t *all = src.mem ? src.mem : head.data();
         bz = BgzfFile();
-        if (!index_bgzf(all, head_read, bz)) { why = "the input is not BGZF"; return HB_OK; }
+        if (!index_bgzf(all, head_read, bz)) { why = "the input is not BGZF"; return false; }
         const std::string err = g_err;
-        if (bgzf_header(all, bz, head_read < src.size ? &more : nullptr) != HB_OK) { g_err = err; why = "the header does not read"; return HB_OK; }
+        if (bgzf_header(all, bz, head_read < src.size ? &more : nullptr) != HB_OK) { g_err = err; why = "the header does not read"; return false; }
         if (head_read == src.size) more = false;
     }
-    const FileText &ft = bz.ft;
+    ft = bz.ft;
+    return true;
+}
+
+int parse_indexed(const ByteSource &src, const uint8_t *ix, uint64_t ix_n, const char *region, bool want_gt, int device,
+                  hb_parse **out, std::vector<std::string> &samples, bool &used, std::string &why, const Subset *ss) {
+    used = false;
+    std::vector<uint8_t> sbuf;
+    {
+        std::vector<uint8_t> hbuf;
+        const uint8_t *h = src.get(0, std::min<uint64_t>(src.size, 18), hbuf);
+        if (!h || !bgzf_member_size(h, std::min<uint64_t>(src.size, 18))) { why = "the input is not BGZF"; return HB_OK; }
+    }
+    TabixIndex idx;
+    if (!tabix_load(ix, ix_n, idx, why)) return HB_OK;
+    FileText ft;
+    uint64_t head_read = 0;
+    if (!leading_bgzf_header(src, ft, head_read, why)) return HB_OK;
     if (ft.bcf && !idx.csi) { why = "a BCF is queried through a CSI index only"; return HB_OK; }
     if (!ft.bcf && idx.names.empty()) { why = "the index names no sequences"; return HB_OK; }
     RegionArg rg;
@@ -1727,11 +1851,14 @@ int parse_indexed(const ByteSource &src, const uint8_t *ix, uint64_t ix_n, const
     if (t1 - t0 > text_limit(slab)) { why = "the region's span is above the text limit"; return HB_OK; }
     used = true;
     samples = ft.samples;
+    std::vector<uint32_t> cols;
+    TRY(resolve_subset(ss, samples, cols));
     const hb_parse_opts o = opts_for(ft, region, want_gt, device);
     const double ta = now_ms();
     int rc;
     ParsePtr p = new_parse(&o, rc);
     if (!p) return rc;
+    TRY(set_subset(p.get(), cols));
     const uint64_t pad = (16 - t0 % 16) % 16;           // the records start on a 16-byte boundary
     TRY(dev_alloc(&p->d_text_owned, pad + sp.total + 1 + kTextPad));
     if (t1 > t0) TRY(inflate_bgzf_to_device(sb, span_comp, sp.coff, sp.clen, sp.ooff, sp.olen, p->d_text_owned + pad, p->stream, &p->ms_inflate));
@@ -1779,7 +1906,7 @@ bool find_index(const char *path, std::vector<uint8_t> &ix, std::string &why) {
 }
 
 int parse_file_indexed(const char *path, const char *region, bool want_gt, int device, hb_parse **out,
-                       std::vector<std::string> &samples, bool &used) {
+                       std::vector<std::string> &samples, bool &used, const Subset *ss) {
     used = false;
     std::string why;
     std::vector<uint8_t> ix;
@@ -1791,7 +1918,7 @@ int parse_file_indexed(const char *path, const char *region, bool want_gt, int d
         int rc = HB_OK;
         if (fd < 0 || fstat(fd, &st) != 0) why = std::string("cannot open ") + path;
         else rc = parse_indexed(ByteSource{nullptr, fd, (uint64_t)st.st_size}, ix.data(), ix.size(), region, want_gt, device, out,
-                                samples, used, why);
+                                samples, used, why, ss);
         if (fd >= 0) close(fd);
         if (rc != HB_OK || used) return rc;
     }
@@ -2046,6 +2173,15 @@ int hb_parse_file(const char *in_vcf, const char *region, int want_gt, int devic
     return HB_OK;
 }
 
+int hb_parse_file_subset(const char *in_vcf, const char *region, const char *const *names, uint32_t n, int device, hb_parse **out) {
+    if (!in_vcf || !out) return fail(HB_ERR_ARG, "null argument");
+    std::vector<std::string> samples;
+    const Subset ss{names, n};
+    TRY(parse_file_common(in_vcf, region, true, device, out, samples, &ss));
+    (*out)->samples = samples;
+    return HB_OK;
+}
+
 // header of the BGZF bytes of a .vcf.gz: sample count, decompressed size, offset of the first record in it
 int hb_bgzf_vcf_info(const uint8_t *bgzf, uint64_t nbytes, uint32_t *n_samples, uint64_t *text_bytes, uint64_t *body_offset) {
     if (!bgzf) return fail(HB_ERR_ARG, "null argument");
@@ -2062,8 +2198,10 @@ int hb_bgzf_vcf_info(const uint8_t *bgzf, uint64_t nbytes, uint32_t *n_samples, 
 // BGZF bytes in host memory -> results in host memory, streamed: slabs of whole BGZF members cross PCIe compressed,
 // are inflated on the GPU behind the unfinished last line of the slab before, parsed up to their own last newline and
 // fetched -- H2D + inflate of slab k + 1 and the D2H of slab k - 1 run while slab k is parsed.
+// cols: the sample subset of the slab parses (empty = every sample); the sink gets planes of the subset's width
 static int stream_bgzf(const char *entry, const uint8_t *bgzf, uint64_t nbytes, const char *region, int want_gt, int device,
-                       uint64_t slab_bytes, SlabSink &sink, uint64_t *n_records, uint32_t *n_slabs) {
+                       uint64_t slab_bytes, SlabSink &sink, uint64_t *n_records, uint32_t *n_slabs,
+                       const std::vector<uint32_t> &cols = {}) {
     if (!bgzf || !n_records) return fail(HB_ERR_ARG, "null argument");
     *n_records = 0;
     if (n_slabs) *n_slabs = 0;
@@ -2079,7 +2217,13 @@ static int stream_bgzf(const char *entry, const uint8_t *bgzf, uint64_t nbytes, 
     const double t_index = now_ms() - t_begin;
     const hb_parse_opts opts = opts_for(ft, region, want_gt != 0, device);
     TRY(ensure_device(device));
-    TRY(sink.begin(opts, ft.samples, bz.total));
+    {
+        hb_parse_opts planes = opts;
+        std::vector<std::string> names;
+        for (uint32_t c : cols) names.push_back(ft.samples[c]);
+        if (!cols.empty()) planes.n_samples = (uint32_t)cols.size();
+        TRY(sink.begin(planes, cols.empty() ? ft.samples : names, bz.total));
+    }
     if (bz.total <= ft.body) return HB_OK;
     if (slab_bytes == 0) slab_bytes = 1ull << 30;
     // slabs of whole members, about slab_bytes of text each
@@ -2099,7 +2243,7 @@ static int stream_bgzf(const char *entry, const uint8_t *bgzf, uint64_t nbytes, 
     if (ft.body >= slabs[0].text) return fail(HB_ERR_ARG, "the VCF header is longer than a slab: raise slab_bytes");
     const uint64_t carry_cap = std::min<uint64_t>((text_cap + 15) & ~15ull, 256ull << 20);   // longest unfinished line carried over
     StreamSlots *ss = nullptr;
-    TRY(open_slots(g_bgzf_slots, opts, std::min<size_t>(2, slabs.size()), text_cap, carry_cap, comp_cap, (uint32_t)n_cap, &ss));
+    TRY(open_slots(g_bgzf_slots, opts, cols, std::min<size_t>(2, slabs.size()), text_cap, carry_cap, comp_cap, (uint32_t)n_cap, &ss));
     StreamSlot *slot = ss->slot;
     const uint64_t carry_base = ss->carry_cap;                 // offset of a slab's text when nothing is carried
     int rc = HB_OK;
@@ -2293,11 +2437,17 @@ int hb_parse_stream_bgzf_host(const uint8_t *bgzf, uint64_t nbytes, const char *
 
 int hb_parse_stream_bgzf_resident(const uint8_t *bgzf, uint64_t nbytes, const char *region, int want_gt, int device,
                                   uint64_t slab_bytes, hb_parse **out, uint32_t *n_slabs) {
+    return stream_resident(bgzf, nbytes, region, want_gt, device, slab_bytes, out, n_slabs, {});
+}
+
+namespace {
+int stream_resident(const uint8_t *bgzf, uint64_t nbytes, const char *region, int want_gt, int device, uint64_t slab_bytes,
+                    hb_parse **out, uint32_t *n_slabs, const std::vector<uint32_t> &cols) {
     if (!out) return fail(HB_ERR_ARG, "null argument");
     *out = nullptr;
     ResidentSink sink;
     uint64_t n = 0;
-    TRY(stream_bgzf("hb_parse_stream_bgzf_resident", bgzf, nbytes, region, want_gt, device, slab_bytes, sink, &n, n_slabs));
+    TRY(stream_bgzf("hb_parse_stream_bgzf_resident", bgzf, nbytes, region, want_gt, device, slab_bytes, sink, &n, n_slabs, cols));
     hb_parse *p = sink.big.get();
     if (!p) return fail(HB_ERR_IO, "empty input");
     const uint32_t S = p->n_samples;
@@ -2320,6 +2470,7 @@ int hb_parse_stream_bgzf_resident(const uint8_t *bgzf, uint64_t nbytes, const ch
     *out = sink.big.release();
     return HB_OK;
 }
+}  // namespace
 
 // Host utility (tests, bench): text -> BGZF with stock zlib on all host threads -- what `bgzip -@` does.
 // Not part of the product path (the path READS BGZF); it exists so that BGZF inputs of bench size can be made
@@ -2378,7 +2529,7 @@ int hb_parse_vcf_bytes(const uint8_t *data, uint64_t nbytes, const char *region,
     if (!data || !out) return fail(HB_ERR_ARG, "null argument");
     std::vector<std::string> samples;
     std::vector<uint8_t> none;
-    TRY(parse_bytes_common(none, data, nbytes, region, want_gt != 0, device, out, samples));
+    TRY(parse_bytes_common(none, data, nbytes, region, want_gt != 0, device, out, samples, nullptr));
     (*out)->samples = samples;
     return HB_OK;
 }
@@ -2395,12 +2546,92 @@ int hb_parse_samples(hb_parse *p, uint32_t *n, char *names, uint64_t cap, uint64
     return HB_OK;
 }
 
+namespace {
+// The header of a .vcf, .vcf.gz (BGZF or plain gzip) or .bcf from its leading bytes only.  BGZF: the leading members, as a
+// region query reads them.  Anything else: read in rounds that double the bytes read, inflated as a stream when it is gzip,
+// until the #CHROM line (or the BCF header text) is complete.
+int leading_header(const ByteSource &src, FileText &ft) {
+    {
+        uint64_t head_read = 0;
+        std::string why;
+        if (leading_bgzf_header(src, ft, head_read, why)) return HB_OK;   // (else the stream below gives the reason)
+    }
+    std::vector<uint8_t> buf, text;
+    const uint8_t *h = src.get(0, std::min<uint64_t>(src.size, 2), buf);
+    const bool gz = h && src.size >= 2 && h[0] == 0x1f && h[1] == 0x8b;
+    struct Z {
+        z_stream zs;
+        bool on = false;
+        ~Z() { if (on) inflateEnd(&zs); }
+    } z;
+    if (gz) {
+        memset(&z.zs, 0, sizeof z.zs);
+        if (inflateInit2(&z.zs, 15 + 32) != Z_OK) return fail(HB_ERR_IO, "inflateInit2 failed");
+        z.on = true;
+    }
+    for (uint64_t off = 0, chunk = 1 << 16;; chunk *= 2) {
+        const uint64_t n = std::min<uint64_t>(chunk, src.size - off);
+        const uint8_t *b = src.get(off, n, buf);
+        if (!b) return fail(HB_ERR_IO, "read error");
+        off += n;
+        const bool eof = off == src.size;
+        if (!gz) text.insert(text.end(), b, b + n);
+        else {
+            z.zs.next_in = const_cast<Bytef *>(b);
+            z.zs.avail_in = (uInt)n;
+            while (z.zs.avail_in) {
+                const size_t at = text.size();
+                text.resize(at + (1 << 16));
+                z.zs.next_out = text.data() + at;
+                z.zs.avail_out = 1 << 16;
+                const int zr = inflate(&z.zs, Z_NO_FLUSH);
+                text.resize(at + (1 << 16) - z.zs.avail_out);
+                if (zr == Z_STREAM_END) { if (inflateReset(&z.zs) != Z_OK) return fail(HB_ERR_IO, "gzip member reset failed"); }
+                else if (zr != Z_OK) return fail(HB_ERR_IO, "gzip inflate failed");
+            }
+        }
+        if (is_bcf(text.data(), text.size())) {
+            bool complete = false;
+            TRY(bcf_header(text.data(), text.size(), ft, complete));
+            if (complete) return HB_OK;
+            if (eof) return fail(HB_ERR_FORMAT, "BCF header is truncated");
+        } else if (parse_header(text.data(), text.size(), eof, ft)) {
+            return HB_OK;
+        } else if (eof) {
+            return fail(HB_ERR_HEADER, "no #CHROM header line");
+        }
+    }
+}
+}  // namespace
+
+int hb_file_samples(const char *path, uint32_t *n, char *names, uint64_t cap, uint64_t *len) {
+    if (!path) return fail(HB_ERR_ARG, "null argument");
+    const int fd = open(path, O_RDONLY);
+    struct stat st;
+    if (fd < 0 || fstat(fd, &st) != 0) {
+        if (fd >= 0) close(fd);
+        return fail(HB_ERR_IO, std::string("cannot open ") + path);
+    }
+    FileText ft;
+    const int rc = leading_header(ByteSource{nullptr, fd, (uint64_t)st.st_size}, ft);
+    close(fd);
+    TRY(rc);
+    if (n) *n = (uint32_t)ft.samples.size();
+    uint64_t used = 0;
+    for (const std::string &s : ft.samples) {
+        if (names && used + s.size() + 1 <= cap) memcpy(names + used, s.c_str(), s.size() + 1);
+        used += s.size() + 1;
+    }
+    if (len) *len = used;
+    return HB_OK;
+}
+
 // ---- region queries through a .tbi / .csi index
 void hb_set_use_index(int on) { g_use_index.store(on ? 1 : 0); }
 int hb_get_use_index(void) { return g_use_index.load(); }
 
-int hb_parse_vcf_bytes_indexed(const uint8_t *data, uint64_t nbytes, const uint8_t *index, uint64_t index_n, const char *region,
-                               int want_gt, int device, hb_parse **out) {
+static int vcf_bytes_indexed(const uint8_t *data, uint64_t nbytes, const uint8_t *index, uint64_t index_n, const char *region,
+                             int want_gt, int device, hb_parse **out, const Subset *ss) {
     if (!data || !out || (index_n && !index)) return fail(HB_ERR_ARG, "null argument");
     std::vector<std::string> samples;
     std::string why;
@@ -2408,14 +2639,25 @@ int hb_parse_vcf_bytes_indexed(const uint8_t *data, uint64_t nbytes, const uint8
     if (!region || !*region) why = "the region is empty";
     else if (!g_use_index.load()) why = "hb_set_use_index(0)";
     else if (!index_n) why = "no index given";
-    else TRY(parse_indexed(ByteSource{data, -1, nbytes}, index, index_n, region, want_gt != 0, device, out, samples, used, why));
+    else TRY(parse_indexed(ByteSource{data, -1, nbytes}, index, index_n, region, want_gt != 0, device, out, samples, used, why, ss));
     if (!used) {
         index_not_used(why);
         std::vector<uint8_t> none;
-        TRY(parse_bytes_common(none, data, nbytes, region, want_gt != 0, device, out, samples));
+        TRY(parse_bytes_common(none, data, nbytes, region, want_gt != 0, device, out, samples, ss));
     }
     (*out)->samples = samples;
     return HB_OK;
+}
+
+int hb_parse_vcf_bytes_indexed(const uint8_t *data, uint64_t nbytes, const uint8_t *index, uint64_t index_n, const char *region,
+                               int want_gt, int device, hb_parse **out) {
+    return vcf_bytes_indexed(data, nbytes, index, index_n, region, want_gt, device, out, nullptr);
+}
+
+int hb_parse_vcf_bytes_subset(const uint8_t *data, uint64_t nbytes, const uint8_t *index, uint64_t index_n, const char *region,
+                              const char *const *names, uint32_t n, int device, hb_parse **out) {
+    const Subset ss{names, n};
+    return vcf_bytes_indexed(data, nbytes, index, index ? index_n : 0, region, 1, device, out, &ss);
 }
 
 int hb_parse_index_info(const hb_parse *p, int *used, uint64_t *compressed_bytes_read, uint64_t *n_chunks) {
@@ -2448,7 +2690,7 @@ int hb_index_bgzf(const uint8_t *data, uint64_t n, int fmt, int min_shift, int d
     hb_parse *raw = nullptr;
     std::vector<std::string> samples;
     std::vector<uint8_t> none;
-    TRY(parse_bytes_common(none, data, n, "", false, device, &raw, samples));
+    TRY(parse_bytes_common(none, data, n, "", false, device, &raw, samples, nullptr));
     ParsePtr p(raw, hb_parse_free);
     const double t1 = now_ms();
     IndexJob j;

@@ -360,11 +360,14 @@ __device__ __noinline__ int bcf_gt_sample(const uint8_t *p, uint32_t ty, uint32_
     return pl != 2 || tail ? 1 : 0;
 }
 
+// kSubset: as kernel 3's, only the columns of `sel` are decoded, counted and written, to their planes.  Every sample's values
+// sit at a fixed stride, so the records' column counts are known without reading the others.
+template <bool kSubset>
 __global__ void __launch_bounds__(BD_THREADS, 4)
 bcf_decode_kernel(const uint8_t *__restrict__ text, const RowInfo *__restrict__ rowinfo, uint64_t n_rows, uint32_t n_samples,
                   uint32_t n_stiles, int8_t *__restrict__ gt0, int8_t *__restrict__ gt1, uint64_t gt_stride,
                   uint32_t *__restrict__ bits, uint64_t bits_stride, uint32_t *__restrict__ ploidy_err,
-                  uint32_t *__restrict__ badgt_err, DevStatus *__restrict__ st) {
+                  uint32_t *__restrict__ badgt_err, DevStatus *__restrict__ st, SampleSel sel) {
     __shared__ BcfGtSmem sm;
     const int tid = threadIdx.x;
     const uint32_t tile = blockIdx.x;
@@ -374,6 +377,9 @@ bcf_decode_kernel(const uint8_t *__restrict__ text, const RowInfo *__restrict__ 
     const uint32_t ns = min((uint32_t)kTS, n_samples - s0);
     const uint64_t r0 = (uint64_t)tile_r * kTV;
     const uint32_t nr = (uint32_t)min((uint64_t)kTV, n_rows - r0);
+    uint4 msk = make_uint4(0, 0, 0, 0);                    // kSubset: the tile's selected columns and the plane of the first
+    uint32_t sbase = 0;
+    if constexpr (kSubset) { msk = sel.mask[tile_s]; sbase = sel.base[tile_s]; }
     if (tid == 0) {
         mbar_init(&sm.bar, kTV);                           // every record's thread arrives, with the bytes it requested
         mbar_fence_init();
@@ -414,7 +420,7 @@ bcf_decode_kernel(const uint8_t *__restrict__ text, const RowInfo *__restrict__ 
     for (int item = tid; item < kTS * (kTV / 16); item += BD_THREADS) {
         const int s = item % kTS, rg = item / kTS;
         uint32_t acc0[4] = {0, 0, 0, 0}, acc1[4] = {0, 0, 0, 0};
-        if ((uint32_t)s < ns) {
+        if ((uint32_t)s < ns && (!kSubset || sel_has(msk, s))) {
 #pragma unroll
             for (int i = 0; i < 16; ++i) {
                 const int r = 16 * rg + i;
@@ -430,8 +436,8 @@ bcf_decode_kernel(const uint8_t *__restrict__ text, const RowInfo *__restrict__ 
                     const uint32_t ty = sm.type[r], c = sm.count[r];
                     rc = bcf_gt_sample(text + sm.off[r] + (uint64_t)s * c * (ty == 1 ? 1u : ty == 2 ? 2u : 4u), ty, c, a0, a1);
                 }
-                if (rc == 2) { atomicAdd(&st->n_bad_gt, 1ull); atomicAdd(&badgt_err[s0 + s], 1u); }
-                else if (rc == 1) atomicAdd(&ploidy_err[s0 + s], 1u);
+                if (rc == 2) { atomicAdd(&st->n_bad_gt, 1ull); atomicAdd(&badgt_err[sel_plane<kSubset>(msk, sbase, s0, s)], 1u); }
+                else if (rc == 1) atomicAdd(&ploidy_err[sel_plane<kSubset>(msk, sbase, s0, s)], 1u);
                 acc0[i >> 2] |= (uint32_t)(uint8_t)a0 << (8 * (i & 3));
                 acc1[i >> 2] |= (uint32_t)(uint8_t)a1 << (8 * (i & 3));
             }
@@ -449,11 +455,11 @@ bcf_decode_kernel(const uint8_t *__restrict__ text, const RowInfo *__restrict__ 
             const int piece = item % PIECES;
             const int ps = item / PIECES;
             const int s = ps % kTS, p = ps / kTS;
-            const bool live = (uint32_t)s < ns;
+            const bool live = (uint32_t)s < ns && (!kSubset || sel_has(msk, s));
             uint4 v = make_uint4(0, 0, 0, 0);
             if (live) {
                 v = *reinterpret_cast<const uint4 *>(&sm.out[p][s][16 * piece]);
-                int8_t *dst = (p ? gt1 : gt0) + (uint64_t)(s0 + s) * gt_stride + r0 + 16ull * piece;
+                int8_t *dst = (p ? gt1 : gt0) + (uint64_t)sel_plane<kSubset>(msk, sbase, s0, s) * gt_stride + r0 + 16ull * piece;
                 stg_stream(reinterpret_cast<uint4 *>(dst), v);
             }
             uint32_t t = pack_lsb4(v.x) | (pack_lsb4(v.y) << 4) | (pack_lsb4(v.z) << 8) | (pack_lsb4(v.w) << 12);
@@ -463,7 +469,7 @@ bcf_decode_kernel(const uint8_t *__restrict__ text, const RowInfo *__restrict__ 
             const uint32_t bw = (t & 0xffffu) | (u << 16), nw = (t >> 16) | (u & 0xffff0000u);
             const uint32_t bw1 = __shfl_down_sync(0xffffffffu, bw, 2), nw1 = __shfl_down_sync(0xffffffffu, nw, 2);
             if (live && piece == 0) {
-                uint32_t *row = bits + (uint64_t)(s0 + s) * bits_stride + (r0 >> 7) * kBitGroupWords + ((r0 >> 5) & 3u);
+                uint32_t *row = bits + (uint64_t)sel_plane<kSubset>(msk, sbase, s0, s) * bits_stride + (r0 >> 7) * kBitGroupWords + ((r0 >> 5) & 3u);
                 *reinterpret_cast<uint2 *>(row + 4 * p) = make_uint2(bw, bw1);
                 *reinterpret_cast<uint2 *>(row + 4 * (2 + p)) = make_uint2(nw, nw1);
             }
@@ -473,12 +479,13 @@ bcf_decode_kernel(const uint8_t *__restrict__ text, const RowInfo *__restrict__ 
 
 void launch_bcf_decode(const uint8_t *d_text, const RowInfo *d_rowinfo, uint64_t n_rows, uint32_t n_samples, int8_t *d_gt0,
                        int8_t *d_gt1, uint64_t gt_stride, uint32_t *d_bits, uint64_t bits_stride, uint32_t *d_ploidy_err,
-                       uint32_t *d_badgt_err, DevStatus *d_st, const Launch &L) {
+                       uint32_t *d_badgt_err, DevStatus *d_st, const SampleSel &sel, const Launch &L) {
     if (!n_rows || !n_samples) return;
     const uint32_t n_stiles = (n_samples + kTS - 1) / kTS;
     const uint64_t tiles = (n_rows + kTV - 1) / kTV * n_stiles;
-    bcf_decode_kernel<<<(unsigned)tiles, BD_THREADS, 0, L.stream>>>(d_text, d_rowinfo, n_rows, n_samples, n_stiles, d_gt0, d_gt1,
-                                                                    gt_stride, d_bits, bits_stride, d_ploidy_err, d_badgt_err, d_st);
+    auto kernel = sel.mask ? bcf_decode_kernel<true> : bcf_decode_kernel<false>;
+    kernel<<<(unsigned)tiles, BD_THREADS, 0, L.stream>>>(d_text, d_rowinfo, n_rows, n_samples, n_stiles, d_gt0, d_gt1, gt_stride,
+                                                         d_bits, bits_stride, d_ploidy_err, d_badgt_err, d_st, sel);
     count_launch();
 }
 

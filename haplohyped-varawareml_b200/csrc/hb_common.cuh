@@ -112,4 +112,23 @@ __device__ __forceinline__ uint32_t pack_nz4(uint32_t w) {
     return (nz * 0x01020408u) >> 24;
 }
 
+// ---------------------------------------------------------------- sample subset (SampleSel, hb_internal.h)
+// word s / 32 of a 128-bit block mask; s is a column of the block, 0..127
+__device__ __forceinline__ uint32_t sel_word(const uint4 &m, uint32_t s) {
+    const uint32_t q = s >> 5;
+    return q == 0 ? m.x : q == 1 ? m.y : q == 2 ? m.z : m.w;
+}
+__device__ __forceinline__ bool sel_has(const uint4 &m, uint32_t s) { return (sel_word(m, s) >> (s & 31)) & 1u; }
+// selected columns of the block below s
+__device__ __forceinline__ uint32_t sel_rank(const uint4 &m, uint32_t s) {
+    const uint32_t q = s >> 5;
+    const uint32_t below = (q > 0 ? __popc(m.x) : 0) + (q > 1 ? __popc(m.y) : 0) + (q > 2 ? __popc(m.z) : 0);
+    return below + __popc(sel_word(m, s) & ((1u << (s & 31)) - 1u));
+}
+// the plane of column s of the tile whose first column is s0 (without a subset: s0 + s)
+template <bool kSubset>
+__device__ __forceinline__ uint32_t sel_plane(const uint4 &m, uint32_t base, uint32_t s0, uint32_t s) {
+    return kSubset ? base + sel_rank(m, s) : s0 + s;
+}
+
 }  // namespace hb

@@ -99,13 +99,19 @@ __device__ __noinline__ uint32_t decode_group_slow(uint32_t w, int *mode, uint32
     return (a0 << 8) | (a1 << 24);
 }
 
+// kSubset: only the columns of `sel` are decoded and written, to their planes.  Every column of every kept record is still
+// staged and read as in the full decode: the shape check of phase 1, decode_group_slow's newline check and phase 2's TAB
+// count see them all, so a record with too many or too few columns is still found, and so is a newline inside a span the
+// head walker jumped over (DevStatus::index_invalid).  Per-sample decoding, per-sample error counts and output are for
+// selected columns only.
+template <bool kSubset>
 __global__ void __launch_bounds__(GT_THREADS, 4)
 decode_gt_kernel(const uint8_t *__restrict__ text, const RowInfo *__restrict__ rowinfo, uint64_t n_rows,
                  uint32_t n_samples, uint32_t n_stiles, const uint64_t *__restrict__ cp, uint32_t ncp,
                  int8_t *__restrict__ gt0, int8_t *__restrict__ gt1, uint64_t gt_stride,
                  uint32_t *__restrict__ bits, uint64_t bits_stride,
                  uint32_t *__restrict__ ploidy_err, uint32_t *__restrict__ badgt_err,
-                 DevStatus *__restrict__ st, uint32_t pf_dist) {
+                 DevStatus *__restrict__ st, uint32_t pf_dist, SampleSel sel) {
     extern __shared__ __align__(128) uint8_t smem_raw[];
     GtSmem &sm = *reinterpret_cast<GtSmem *>(smem_raw);
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -116,6 +122,9 @@ decode_gt_kernel(const uint8_t *__restrict__ text, const RowInfo *__restrict__ r
     const uint32_t ns = min((uint32_t)kTS, n_samples - s0);
     const uint64_t r0 = (uint64_t)tile_r * kTV;
     const uint32_t nr = (uint32_t)min((uint64_t)kTV, n_rows - r0);
+    uint4 msk = make_uint4(0, 0, 0, 0);                    // kSubset: the tile's selected columns and the plane of the first
+    uint32_t sbase = 0;
+    if constexpr (kSubset) { msk = sel.mask[tile_s]; sbase = sel.base[tile_s]; }
 
     if (tid == 0) {
         mbar_init(&sm.bar, kTV);                           // every record's thread arrives, with the bytes it requested
@@ -290,7 +299,7 @@ decode_gt_kernel(const uint8_t *__restrict__ text, const RowInfo *__restrict__ r
             while (mm) {
                 const int bit = __ffs(mm) - 1;                                   // byte of the TAB inside the lane's 16
                 mm &= mm - 1;
-                if (k < ns) {
+                if (k < ns && (!kSubset || sel_has(msk, k))) {
                     int a0, a1, pl;
                     const int rel = 16 * lane + bit + 1;                         // first byte of the field, in `row`
                     const uint32_t *fw = reinterpret_cast<const uint32_t *>(row + (rel & ~3));
@@ -303,8 +312,8 @@ decode_gt_kernel(const uint8_t *__restrict__ text, const RowInfo *__restrict__ r
                         a1 = Y == '.' ? -9 : (int)dy;
                         pl = 2;
                     } else pl = decode_field(text, o + (uint64_t)bit + 1, g, a0, a1);
-                    if (pl < 0) { atomicAdd(&st->n_bad_gt, 1ull); atomicAdd(&badgt_err[s0 + k], 1u); a0 = 0; a1 = 0; }
-                    else if (pl != 2) atomicAdd(&ploidy_err[s0 + k], 1u);
+                    if (pl < 0) { atomicAdd(&st->n_bad_gt, 1ull); atomicAdd(&badgt_err[sel_plane<kSubset>(msk, sbase, s0, k)], 1u); a0 = 0; a1 = 0; }
+                    else if (pl != 2) atomicAdd(&ploidy_err[sel_plane<kSubset>(msk, sbase, s0, k)], 1u);
                     sm.out[0][k][r] = (uint8_t)a0;
                     sm.out[1][k][r] = (uint8_t)a1;
                 }
@@ -327,15 +336,27 @@ decode_gt_kernel(const uint8_t *__restrict__ text, const RowInfo *__restrict__ r
     {
         constexpr int PIECES = kTV / 16;
         static_assert(PIECES == 4 && (2 * kTS * PIECES) % GT_THREADS == 0, "the 4 pieces of a row sit in 4 neighbouring lanes");
+        // kSubset: a thread's items are columns tid / 4 and tid / 4 + 64 only (of both planes): their selection and their
+        // planes are worked out once here, not per item
+        static_assert(GT_THREADS * 2 == kTS * PIECES, "item >> 8 & 1 picks the column");
+        bool take[2] = {true, true};
+        uint32_t plane[2] = {0, 0};
+        if constexpr (kSubset) {
+            for (int h = 0; h < 2; ++h) {
+                const uint32_t c = (uint32_t)(tid / PIECES) + 64u * h;
+                take[h] = sel_has(msk, c);
+                plane[h] = sbase + sel_rank(msk, c);
+            }
+        }
         for (int item = tid; item < 2 * kTS * PIECES; item += GT_THREADS) {
             const int piece = item % PIECES;
             const int ps = item / PIECES;       // plane * kTS + s
             const int s = ps % kTS, p = ps / kTS;
-            const bool live = (uint32_t)s < ns;
+            const bool live = (uint32_t)s < ns && (!kSubset || take[(item >> 8) & 1]);
             uint4 v = make_uint4(0, 0, 0, 0);
             if (live) {
                 v = *reinterpret_cast<const uint4 *>(&sm.out[p][s][16 * piece]);
-                int8_t *dst = (p ? gt1 : gt0) + (uint64_t)(s0 + s) * gt_stride + r0 + 16ull * piece;
+                int8_t *dst = (p ? gt1 : gt0) + (uint64_t)(kSubset ? plane[(item >> 8) & 1] : s0 + s) * gt_stride + r0 + 16ull * piece;
                 stg_stream(reinterpret_cast<uint4 *>(dst), v);
             }
             if (bits) {
@@ -346,7 +367,7 @@ decode_gt_kernel(const uint8_t *__restrict__ text, const RowInfo *__restrict__ r
                 const uint32_t bw = (t & 0xffffu) | (u << 16), nw = (t >> 16) | (u & 0xffff0000u);   // valid in even lanes
                 const uint32_t bw1 = __shfl_down_sync(0xffffffffu, bw, 2), nw1 = __shfl_down_sync(0xffffffffu, nw, 2);
                 if (live && piece == 0) {
-                    uint32_t *row = bits + (uint64_t)(s0 + s) * bits_stride + (r0 >> 7) * kBitGroupWords + ((r0 >> 5) & 3u);
+                    uint32_t *row = bits + (uint64_t)(kSubset ? plane[(item >> 8) & 1] : s0 + s) * bits_stride + (r0 >> 7) * kBitGroupWords + ((r0 >> 5) & 3u);
                     *reinterpret_cast<uint2 *>(row + 4 * p) = make_uint2(bw, bw1);
                     *reinterpret_cast<uint2 *>(row + 4 * (2 + p)) = make_uint2(nw, nw1);
                 }
@@ -358,19 +379,21 @@ decode_gt_kernel(const uint8_t *__restrict__ text, const RowInfo *__restrict__ r
 void launch_decode_gt(const uint8_t *d_text, const RowInfo *d_rowinfo, uint64_t n_rows, uint32_t n_samples,
                       const uint64_t *d_cp, uint32_t ncp, int8_t *d_gt0, int8_t *d_gt1, uint64_t gt_stride,
                       uint32_t *d_bits, uint64_t bits_stride, uint32_t *d_ploidy_err, uint32_t *d_badgt_err, DevStatus *d_st,
-                      const Launch &L) {
+                      const SampleSel &sel, const Launch &L) {
     if (!n_rows || !n_samples) return;
     size_t smem = sizeof(GtSmem);
+    const bool subset = sel.mask != nullptr;
+    auto kernel = subset ? decode_gt_kernel<true> : decode_gt_kernel<false>;
     // > 48 KB of dynamic shared memory is opt-in per function AND per device: set on every launch (a microsecond), so a
     // process that moves to another device is served too
-    cudaFuncSetAttribute(decode_gt_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     uint32_t n_stiles = (n_samples + kTS - 1) / kTS;
     uint64_t n_rtiles = (n_rows + kTV - 1) / kTV;
     uint64_t tiles = n_rtiles * n_stiles;
     const uint32_t pf_dist = 4u * (uint32_t)L.sm_count;      // 4 CTAs per SM are resident (__launch_bounds__)
-    decode_gt_kernel<<<(unsigned)tiles, GT_THREADS, smem, L.stream>>>(d_text, d_rowinfo, n_rows, n_samples, n_stiles,
-                                                                      d_cp, ncp, d_gt0, d_gt1, gt_stride, d_bits, bits_stride,
-                                                                      d_ploidy_err, d_badgt_err, d_st, pf_dist);
+    kernel<<<(unsigned)tiles, GT_THREADS, smem, L.stream>>>(d_text, d_rowinfo, n_rows, n_samples, n_stiles, d_cp, ncp, d_gt0,
+                                                            d_gt1, gt_stride, d_bits, bits_stride, d_ploidy_err, d_badgt_err,
+                                                            d_st, pf_dist, sel);
     count_launch();
 }
 

@@ -70,6 +70,14 @@ struct RegionArg {
     long long beg0, end0;
 };
 
+// A sample subset on the device (hb_parse_*_subset), for the decoders (kernels 3 and 3b): per 128-column block b of the
+// file's samples, bit s of mask[b] selects column 128 b + s, and base[b] is the plane of the block's first selected column.
+// The plane of a selected column is base[b] + the popc of the mask below it.  mask == nullptr: every column, plane = column.
+struct SampleSel {
+    const uint4 *mask = nullptr;
+    const uint32_t *base = nullptr;
+};
+
 struct Launch {   // filled by the host, one per parse
     cudaStream_t stream;
     int sm_count;
@@ -109,7 +117,7 @@ void launch_chrom_runs(const uint8_t *d_text, const uint64_t *d_chrom_abs, const
 void launch_decode_gt(const uint8_t *d_text, const RowInfo *d_rowinfo, uint64_t n_rows, uint32_t n_samples,
                       const uint64_t *d_cp, uint32_t ncp, int8_t *d_gt0, int8_t *d_gt1, uint64_t gt_stride,
                       uint32_t *d_bits, uint64_t bits_stride, uint32_t *d_ploidy_err, uint32_t *d_badgt_err, DevStatus *d_st,
-                      const Launch &L);
+                      const SampleSel &sel, const Launch &L);
 
 void launch_bits_from_planes(const int8_t *d_gt0, const int8_t *d_gt1, uint64_t gt_stride, uint64_t n_rows, uint32_t n_samples,
                              uint32_t *d_bits, uint64_t bits_stride, const Launch &L);
@@ -161,7 +169,7 @@ void launch_bcf_emit(const uint8_t *d_text, uint64_t nbytes, const BcfSegs &sg, 
 void launch_bcf_sites(const BcfSiteArgs &a, const Launch &L);
 void launch_bcf_decode(const uint8_t *d_text, const RowInfo *d_rowinfo, uint64_t n_rows, uint32_t n_samples, int8_t *d_gt0,
                        int8_t *d_gt1, uint64_t gt_stride, uint32_t *d_bits, uint64_t bits_stride, uint32_t *d_ploidy_err,
-                       uint32_t *d_badgt_err, DevStatus *d_st, const Launch &L);
+                       uint32_t *d_badgt_err, DevStatus *d_st, const SampleSel &sel, const Launch &L);
 
 void count_launch(uint64_t n = 1);
 

@@ -17,7 +17,12 @@ struct hb_parse {
     uint8_t *d_text_owned = nullptr;
     bool text_released = false;         // hb_parse_release_text: the results stay, a re-run is no longer possible
     uint64_t nbytes = 0;
-    uint32_t n_samples = 0;
+    // n_cols: sample columns of every record of the file (what locates records and checks their column counts);
+    // n_samples: genotype planes -- the subset's size under a sample subset, else n_cols
+    uint32_t n_cols = 0, n_samples = 0;
+    std::vector<uint32_t> sel_cols;     // sample subset (hb_parse_*_subset): the selected columns, ascending; empty = every one
+    uint4 *d_sel_mask = nullptr;        // its device tables (hb::SampleSel), one entry per 128-column block
+    uint32_t *d_sel_base = nullptr;
     hb::RegionArg rg;
     int end_is_int = 0, want_gt = 1, tokenizer = 0;
     bool with_tabs = false;

@@ -50,12 +50,24 @@ def _configure_logging():
 class _ChromParse:
     """One chromosome file: device-resident parse + Blosc2 frames of the donors' chunks.
 
+    When the donors of the sample list that the file has are fewer than its samples, only theirs are decoded (a sample
+    subset, in header order): 1,000 donors of a 200,000-sample cohort keep 1/200 of the genotype planes.  The datasets are
+    those an all-sample parse gives.
+
     The frames of ALL donors of a big chromosome may not fit in HBM next to the genotype planes (1000G chr1: 64 GB of
     text, 32 GB of planes, ~100 GB of frames), so the text is given back right after the parse and the frames are made
     for a WINDOW of samples at a time; the window is as large as free HBM allows -- all samples for anything chr22-sized."""
 
-    def __init__(self, data_path: str, chromosome: int, device: int, window: Optional[int] = None):
-        self.parse = capi.Parse.from_file(data_path, region=f"chr{chromosome}", want_gt=True, device=device)
+    def __init__(self, data_path: str, chromosome: int, device: int, window: Optional[int] = None,
+                 donors: Optional[List[str]] = None):
+        subset = None
+        if donors is not None:
+            wanted = set(donors)
+            header = capi.file_sample_names(data_path)
+            subset = list(dict.fromkeys(s for s in header if s in wanted))
+            if not subset or len(subset) == len(header):
+                subset = None                           # nothing to leave out (or no donor here: the file is still checked)
+        self.parse = capi.Parse.from_file(data_path, region=f"chr{chromosome}", want_gt=True, device=device, samples=subset)
         self.samples = self.parse.sample_names()
         self.index = {s: i for i, s in enumerate(self.samples)}
         info = self.parse.info
@@ -169,7 +181,8 @@ class VCFtoHDF5Converter:
             cp = self._chrom.get(chromosome)
         if cp is None:
             with self._crc_scope():
-                cp = _ChromParse(data_path, chromosome, self.device if device is None else device, self.sample_window)
+                cp = _ChromParse(data_path, chromosome, self.device if device is None else device, self.sample_window,
+                                 self.donor_ids)
             with self._wlock:
                 self._chrom[chromosome] = cp
         return cp
@@ -326,7 +339,8 @@ class VCFtoHDF5Converter:
     def _safe_parse(self, chromosome: int, device: Optional[int] = None):
         vcf_file = os.path.join(self.vcf_dir, f"chr{chromosome}.filtered.vcf.gz")
         try:
-            return _ChromParse(vcf_file, chromosome, self.device if device is None else device, self.sample_window)
+            return _ChromParse(vcf_file, chromosome, self.device if device is None else device, self.sample_window,
+                               self.donor_ids)
         except capi.HaploError as e:
             logger.error(f"An error occurred while processing VCF file: Error parsing VCF file: {e}")
             if e.code in (capi.HB_ERR_MEM, capi.HB_ERR_CUDA):

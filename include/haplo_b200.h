@@ -160,8 +160,34 @@ void hb_set_walker_lines(uint32_t lines);
  * other values are raised to at least 64.  Tests use small segments to put segment boundaries at every offset of a
  * record and to make records longer than a segment. */
 void hb_set_bcf_segment_bytes(uint64_t bytes);
-/* sample names of a file-level parse, NUL-separated */
+/* sample names of a file-level parse, NUL-separated (under a sample subset: the subset's, in header order) */
 int hb_parse_samples(hb_parse *p, uint32_t *n, char *names, uint64_t cap, uint64_t *len);
+/* Sample subsets: only the listed samples' genotypes are decoded and kept, as htslib's bcf_hdr_set_samples does before it
+ * parses.  Planes come out in header order whatever the order of the list: plane j is the j-th selected column of the
+ * header, and n_samples (hb_parse_get_info, hb_parse_samples, the frame calls) is the subset's size.  For every selected
+ * sample the result is what the full parse of the same bytes gives: the same rows, site columns, CHROM runs and planes,
+ * the same per-sample error counts.  The columns of unselected samples are still counted, so a record with too many or
+ * too few columns fails with HB_ERR_FORMAT as in the full parse, but their GT text is not parsed: a bad allele or a
+ * haploid call there neither fails nor counts (n_bad_gt counts selected samples only).  A list of every sample is the
+ * ordinary parse.  hb_parse_rerun repeats the subset.
+ * Text level: cols[0..n_cols) are column indices into the opts->n_samples sample columns, ascending and distinct;
+ * an empty list, an index out of range, unsorted or repeated fails with HB_ERR_ARG. */
+int hb_parse_host_text_subset(const uint8_t *text, uint64_t nbytes, const hb_parse_opts *opts, const uint32_t *cols,
+                              uint32_t n_cols, hb_parse **out);
+int hb_parse_device_text_subset(const uint8_t *d_text, uint64_t nbytes, const hb_parse_opts *opts, const uint32_t *cols,
+                                uint32_t n_cols, hb_parse **out);
+/* File level (hb_parse_file / hb_parse_vcf_bytes_indexed with genotypes and a subset; every route they take -- BCF, an
+ * index, the slab-streamed route -- takes the subset): names[0..n) in any order.  A name the header does not have fails
+ * with HB_ERR_SAMPLE and names it; an empty list or a name given twice fails with HB_ERR_ARG.  index == NULL: what
+ * hb_parse_vcf_bytes does. */
+int hb_parse_file_subset(const char *in_vcf, const char *region, const char *const *names, uint32_t n, int device,
+                         hb_parse **out);
+int hb_parse_vcf_bytes_subset(const uint8_t *data, uint64_t nbytes, const uint8_t *index, uint64_t index_n, const char *region,
+                              const char *const *names, uint32_t n, int device, hb_parse **out);
+/* The header's sample names of a .vcf, .vcf.gz (BGZF or plain gzip) or .bcf, NUL-separated, read from the leading bytes
+ * (BGZF members) of the file only; host only, no device needed.  As hb_parse_samples: the names that fit cap are written,
+ * *len is what all of them need. */
+int hb_file_samples(const char *path, uint32_t *n, char *names, uint64_t cap, uint64_t *len);
 /* re-run the kernels of an existing handle on (new contents of) the same device buffer: no allocation */
 int hb_parse_rerun(hb_parse *p);
 /* the same for a handle made by hb_parse_device_text whose buffer now holds nbytes of (other) text: slab streaming */
